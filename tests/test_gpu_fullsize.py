@@ -166,6 +166,45 @@ def test_c5_batched_replay_matches_single_shot(big):
     pipe.close()
 
 
+def test_bench_dump_outputs_are_the_last_steps_results(big, tmp_path):
+    """bench.py --dump-outputs: the counters of every frame and the rows / plane of each lane's last frame,
+    as the timed steps left them, equal one-scan-at-a-time runs of the same frames; --steps sets the
+    number of timed steps."""
+    import json
+    import os
+    import subprocess
+    import sys
+    import bench
+    ctx, engine, capi = big["ctx"], big["engine"], big["capi"]
+    FT, lanes, steps = 10, 3, 2
+    r = subprocess.run([sys.executable, os.path.abspath(bench.__file__), "--steps", str(steps), "--frames-total", str(FT),
+                        "--lanes", str(lanes), "--no-configs", "--no-cpu-baseline", "--no-e2e",
+                        "--dump-outputs", str(tmp_path)], capture_output=True, text=True, timeout=600)
+    assert r.returncode == 0, r.stderr[-3000:]
+    line = json.loads(r.stdout)
+    assert line["steps"] == steps
+    counts = np.load(tmp_path / "counts.npy")
+    assert counts.dtype == np.float64 and counts.shape == (FT, 8)
+    assert sorted(os.listdir(tmp_path)) == ["counts.npy"] + [f"{k}_{f:05d}.npy" for k in ("plane", "xyzi")
+                                                             for f in range(FT - lanes, FT)]
+    block = bench.make_c5_block(0, FT, workers=1)
+    fcfg = engine.make_filter_cfg(skip_nans=True, dedup_mode=capi.DEDUP_OPEN3D, remove_nan=True, remove_inf=True,
+                                  transforms=[bench.TF], crop=bench.CROP)
+    pcfg = engine.make_pipeline_cfg(fcfg, **bench.STAGES)
+    fields = bench.frame_msg(b"").fields
+    for f in range(FT):
+        data = torch.from_numpy(block[f].copy()).cuda()
+        out, c, plane = ctx.pipeline_run([engine.make_cloud_desc(fields, bench.POINT_STEP, bench.N_POINTS, data)], pcfg)
+        ctx.check()
+        c = c.cpu().numpy()
+        assert np.array_equal(counts[f], c.astype(np.float64)), f
+        if f >= FT - lanes:
+            rows = np.load(tmp_path / f"xyzi_{f:05d}.npy")
+            assert rows.dtype == np.float32
+            assert np.array_equal(rows.view(np.uint32), out[:int(c[capi.CNT_OUTPUT])].cpu().numpy().view(np.uint32)), f
+            assert np.array_equal(np.load(tmp_path / f"plane_{f:05d}.npy"), plane.cpu().numpy()), f
+
+
 def test_c1_full_size_131072_crop_voxel_ground(big):
     """configs[0] at its own size: 64 x 2048 = 131 072 points, crop_box + 0.1 m voxels + RANSAC ground
     removal, every intermediate count and the published rows bit-exact against the oracle."""
