@@ -14,6 +14,7 @@ LIB_PATH = os.path.join(PKG, "libapc.so")
 
 APC_MAX_FIELDS = 16
 APC_MAX_CLOUDS = 8
+APC_MAX_NEIGHBORS = 1024   # statistical nb_neighbors and normals max_nn
 APC_MAX_TRANSFORMS = 3
 APC_MAX_MIRRORS = 8
 

@@ -22,7 +22,9 @@
 APC_TRACE_EXPORT(neighbors)
 
 #define KNN_LEVELS 12
-#define KNN_KMAX 64
+#define KNN_KMAX 64           // k_knn_query / k_knn_stragglers; above it the *_wide kernels, up to APC_MAX_NEIGHBORS
+#define APC_STRINGIFY2(x) #x
+#define APC_STRINGIFY(x) APC_STRINGIFY2(x)
 
 // counters[] slots used by this file (zeroed by k_begin)
 #define CTR_CURSOR 0        // [0..KNN_LEVELS) per-level scatter cursors of the KNN grid
@@ -949,6 +951,221 @@ k_knn_stragglers(const float4* __restrict__ pts, uint32_t n_max, const uint32_t*
   }
 }
 
+// ---- k > 64 (up to APC_MAX_NEIGHBORS): per-warp shared candidate buffers ---------------------------
+// Keys are compared as unsigned integers and have their top bit clear: float32 d2 bit patterns
+// (non-negative floats order like integers), or (d2 bits << 32 | index) for the normals.
+//
+// WarpKeep: a warp streams candidate keys into its buffer (warp-collective add(), one key per lane);
+// when the next batch might not fit, the k smallest are found by a binary search on the bit pattern
+// (each step a strided count + REDUX) and compacted to the front in place (ties at the k-th value are
+// interchangeable: equal keys are equal distances).  From then on the k-th value bounds the batch:
+// a key not below it cannot enter the k smallest, so it never takes a buffer slot.  After finish()
+// the k smallest (or all, if fewer arrived) sit unordered in buf[0, m).
+template <typename K>
+struct WarpKeep {
+  K* buf;
+  uint32_t cap, k, m;   // cap > k + 32: every selection frees room for at least one more batch
+  K bound;              // keys >= bound are rejected (all ones before the first selection)
+  __device__ __forceinline__ void init(K* b, uint32_t capacity, uint32_t kk) { buf = b; cap = capacity; k = kk; m = 0; bound = ~(K)0; }
+  __device__ __forceinline__ void select(uint32_t lane) {
+    __syncwarp();
+    K V = 0;                                                   // the k-th smallest key
+    for (int bit = (int)sizeof(K) * 8 - 2; bit >= 0; --bit) {
+      const K trial = V | ((K)1 << bit);
+      uint32_t below = 0;
+      for (uint32_t i = lane; i < m; i += 32) below += buf[i] < trial ? 1u : 0u;
+      if (__reduce_add_sync(0xffffffffu, below) < k) V = trial;
+    }
+    uint32_t below = 0;
+    for (uint32_t i = lane; i < m; i += 32) below += buf[i] < V ? 1u : 0u;
+    const uint32_t need_eq = k - __reduce_add_sync(0xffffffffu, below);
+    const uint32_t lt_mask = (1u << lane) - 1u;
+    uint32_t kept = 0, eq_seen = 0;
+    for (uint32_t base = 0; base < m; base += 32) {           // in place: writes never pass the batch being read
+      const uint32_t i = base + lane;
+      const K x = i < m ? buf[i] : ~(K)0;
+      const bool is_eq = i < m && x == V;
+      const uint32_t beq = __ballot_sync(0xffffffffu, is_eq);
+      const bool keep = (i < m && x < V) || (is_eq && eq_seen + __popc(beq & lt_mask) < need_eq);
+      const uint32_t bk = __ballot_sync(0xffffffffu, keep);
+      __syncwarp();
+      if (keep) buf[kept + __popc(bk & lt_mask)] = x;
+      kept += __popc(bk);
+      eq_seen += __popc(beq);
+      __syncwarp();
+    }
+    m = k;
+    bound = V;
+  }
+  __device__ __forceinline__ void add(K key, bool valid, uint32_t lane) {
+    const bool take = valid && key < bound;
+    const uint32_t b = __ballot_sync(0xffffffffu, take);
+    if (take) buf[m + __popc(b & ((1u << lane) - 1u))] = key;
+    m += __popc(b);
+    if (m + 32u > cap) select(lane);
+  }
+  __device__ __forceinline__ void finish(uint32_t lane) {
+    if (m > k) select(lane);
+    __syncwarp();
+  }
+};
+
+// Buffer entries per warp for k > 64: more than k + 32 (a selection always makes room for a batch)
+// and at least the power of two warp_sort pads k to.  k = 1024: 1280 entries, 5 KB (KNN) /
+// 10 KB (normals) per warp, 20 / 40 KB per block of 4 warps - under the 48 KB of a default launch.
+static inline uint32_t wide_cap(uint32_t k) {
+  uint32_t pow2 = 1;
+  while (pow2 < k) pow2 <<= 1;
+  return max(pow2, (k + 31u) / 32u * 32u + 256u);
+}
+
+// Ascending bitonic sort of buf[0, n) over the padded power of two (buf must hold it).  Warp-collective.
+template <typename K>
+__device__ void warp_sort(K* buf, uint32_t n, uint32_t lane) {
+  uint32_t len = 1;
+  while (len < n) len <<= 1;
+  for (uint32_t i = n + lane; i < len; i += 32) buf[i] = ~(K)0;
+  __syncwarp();
+  for (uint32_t kk = 2; kk <= len; kk <<= 1)
+    for (uint32_t jj = kk >> 1; jj > 0; jj >>= 1) {
+      for (uint32_t i = lane; i < len; i += 32) {
+        const uint32_t p = i ^ jj;
+        if (p > i) {
+          const K a = buf[i], b = buf[p];
+          if ((a > b) == ((i & kk) == 0)) { buf[i] = b; buf[p] = a; }
+        }
+      }
+      __syncwarp();
+    }
+}
+
+// Mean of sqrtf over the k_eff keys in buf[0, k_eff) (float32 d2 bit patterns, unordered): sorted, then
+// the sequential ascending float32 sum of oracle/outliers.py.  Warp-collective; every lane returns the mean.
+__device__ float wide_average(uint32_t* buf, uint32_t k_eff, uint32_t lane) {
+  warp_sort(buf, k_eff, lane);
+  float sum = 0.0f;
+  for (uint32_t base = 0; base < k_eff; base += 32) {
+    const float r = base + lane < k_eff ? sqrtf(__uint_as_float(buf[base + lane])) : 0.0f;
+    const uint32_t cnt = min(32u, k_eff - base);
+    for (uint32_t i = 0; i < cnt; ++i) {                          // sequential float32 sum, ascending
+      const float v = __shfl_sync(0xffffffffu, r, i);
+      sum = base + i == 0 ? v : __fadd_rn(sum, v);
+    }
+  }
+  __syncwarp();
+  return __fdiv_rn(sum, (float)k_eff);
+}
+
+extern __shared__ __align__(16) unsigned char wide_smem[];
+
+// k_knn_query for 64 < k <= APC_MAX_NEIGHBORS: the same level climb, 27-cell flat candidate list and
+// coverage test (`safe`, exact_margin), the candidates through a WarpKeep of wide_cap(k) entries per
+// warp (dynamic shared memory), the accepted level's k distances sorted and summed by wide_average.
+__global__ void __launch_bounds__(KNN_WARPS * 32)
+k_knn_query_wide(uint32_t n_max, const uint32_t* n_dev, GridDev g, uint32_t k, uint32_t cap, float* __restrict__ avg,
+                 uint32_t* __restrict__ stragglers, ApcCtrl* ctrl, int exact_margin) {
+  const uint32_t n = apc_count(n_dev, n_max);
+  const uint32_t n_sorted = grid_sorted_count(g, ctrl, n);
+  const uint32_t k_eff = min(k, n);
+  const uint32_t lane = threadIdx.x & 31u, w = threadIdx.x >> 5;
+  uint32_t* buf = reinterpret_cast<uint32_t*>(wide_smem) + (size_t)w * cap;
+  for (uint32_t j = blockIdx.x * KNN_WARPS + w; j < n_sorted; j += gridDim.x * KNN_WARPS) {
+    const float4 q = g.sorted[j];
+    const uint32_t orig = __float_as_uint(q.w);
+    bool done = false;
+    for (uint32_t level = 0; level < g.levels && !done; ++level) {
+      const float c = g.cell[level];
+      int32_t ix, iy, iz;
+      if (!grid_coord_g(g, c, q.x, q.y, q.z, ix, iy, iz)) continue;
+      uint32_t cs = 0, cf = 0;
+      if (lane < 27) {
+        const int dx = (int)(lane % 3u) - 1, dy = (int)((lane / 3u) % 3u) - 1, dz = (int)(lane / 9u) - 1;
+        uint32_t b, f;
+        if (grid_lookup(g, grid_key(level, ix + dx, iy + dy, iz + dz), b, f)) { cs = b; cf = f; }
+      }
+      uint32_t incl = cf;
+#pragma unroll
+      for (int o = 1; o < 32; o <<= 1) {
+        const uint32_t v = __shfl_up_sync(0xffffffffu, incl, o);
+        if (lane >= (uint32_t)o) incl += v;
+      }
+      const uint32_t ps = incl - cf;
+      const uint32_t total = __shfl_sync(0xffffffffu, incl, 31);
+      if (total < k_eff) continue;
+      const float4* sp = g.sorted + (size_t)level * n_max;
+      float safe = c;
+      if (exact_margin) {
+        const float mx = fminf(__fsub_rn(q.x, __fmul_rn((float)ix, c)), __fsub_rn(__fmul_rn((float)(ix + 1), c), q.x));
+        const float my = fminf(__fsub_rn(q.y, __fmul_rn((float)iy, c)), __fsub_rn(__fmul_rn((float)(iy + 1), c), q.y));
+        const float mz = fminf(__fsub_rn(q.z, __fmul_rn((float)iz, c)), __fsub_rn(__fmul_rn((float)(iz + 1), c), q.z));
+        safe = __fadd_rn(c, fmaxf(0.0f, fminf(mx, fminf(my, mz))));
+      }
+      safe = __fmul_rn(safe, 0.999f);
+      WarpKeep<uint32_t> wk;
+      wk.init(buf, cap, k_eff);
+      for (uint32_t base = 0; base < total; base += 32) {
+        const uint32_t ci = base + lane;
+        const uint32_t flat = min(ci, total - 1u);
+        uint32_t run = 0;                                          // largest t with ps[t] <= flat
+#pragma unroll
+        for (int step = 16; step > 0; step >>= 1) {
+          const uint32_t mid = run + step;
+          const uint32_t v = __shfl_sync(0xffffffffu, ps, mid & 31u);
+          if (mid < 27u && v <= flat) run = mid;
+        }
+        const uint32_t rs = __shfl_sync(0xffffffffu, cs, run), rp = __shfl_sync(0xffffffffu, ps, run);
+        uint32_t key = 0;
+        if (ci < total) {
+          const float4 p = sp[rs + (flat - rp)];
+          key = __float_as_uint(d2_f32(q.x, q.y, q.z, p.x, p.y, p.z));
+        }
+        wk.add(key, ci < total, lane);
+      }
+      wk.finish(lane);
+      uint32_t mx = 0;                                             // covered by the block?
+      for (uint32_t i = lane; i < k_eff; i += 32) mx = max(mx, buf[i]);
+      if (__uint_as_float(__reduce_max_sync(0xffffffffu, mx)) <= __fmul_rn(safe, safe)) done = true;
+    }
+    if (done) {
+      const float a = wide_average(buf, k_eff, lane);
+      if (lane == 0) avg[orig] = a;
+    } else if (lane == 0) {
+      stragglers[atomicAdd(&ctrl->counters[CTR_STRAGGLERS], 1u)] = orig;
+    }
+    __syncwarp();
+  }
+}
+
+// Exact brute force for the points no level of k_knn_query_wide covers: one warp per straggler streams
+// every point through its WarpKeep (after the first selection nearly all are rejected by the bound).
+__global__ void __launch_bounds__(KNN_WARPS * 32)
+k_knn_stragglers_wide(const float4* __restrict__ pts, uint32_t n_max, const uint32_t* n_dev, uint32_t k, uint32_t cap,
+                      const uint32_t* __restrict__ stragglers, const ApcCtrl* ctrl, float* __restrict__ avg) {
+  const uint32_t n = apc_count(n_dev, n_max);
+  const uint32_t k_eff = min(k, n);
+  const uint32_t n_str = ctrl->counters[CTR_STRAGGLERS];
+  const uint32_t lane = threadIdx.x & 31u, w = threadIdx.x >> 5;
+  uint32_t* buf = reinterpret_cast<uint32_t*>(wide_smem) + (size_t)w * cap;
+  for (uint32_t sidx = blockIdx.x * KNN_WARPS + w; sidx < n_str; sidx += gridDim.x * KNN_WARPS) {
+    const uint32_t orig = stragglers[sidx];
+    const float4 q = pts[orig];
+    WarpKeep<uint32_t> wk;
+    wk.init(buf, cap, k_eff);
+    for (uint32_t base = 0; base < n; base += 32) {
+      const uint32_t i = base + lane;
+      uint32_t key = 0;
+      if (i < n) {
+        const float4 p = pts[i];
+        key = __float_as_uint(d2_f32(q.x, q.y, q.z, p.x, p.y, p.z));
+      }
+      wk.add(key, i < n, lane);
+    }
+    wk.finish(lane);
+    const float a = wide_average(buf, k_eff, lane);
+    if (lane == 0) avg[orig] = a;
+  }
+}
+
 // ---- float64 adjacent-pairwise tree reductions (mirrors oracle/outliers.py tree_sum) ------------
 // in[i] (i < n) -> out[b] = tree sum of the 256 consecutive elements of block b (zero padded).
 // mode 0: v = (double)avgf[i]; mode 1: v = ((double)avgf[i] - mu)^2 with mu = stats[0];
@@ -1289,7 +1506,8 @@ int apc_statistical_nobegin(apc_ctx* ctx, const float* xyzi, uint32_t n_max, con
   if (n_max == 0) return APC_OK;
   APC_REQUIRE(ctx, xyzi && out_mask, "NULL pointer");
   APC_REQUIRE(ctx, n_max <= ctx->max_points, "more points than the context was created for");
-  APC_REQUIRE(ctx, nb_neighbors >= 1 && nb_neighbors <= KNN_KMAX, "nb_neighbors must be in 1..64");
+  APC_REQUIRE(ctx, nb_neighbors >= 1 && nb_neighbors <= APC_MAX_NEIGHBORS,
+              "nb_neighbors must be in 1..APC_MAX_NEIGHBORS (" APC_STRINGIFY(APC_MAX_NEIGHBORS) ")");
   APC_REQUIRE(ctx, std_ratio > 0.0, "std_ratio must be > 0");
   int rc = apc_neighbors_prepare(ctx, 1);
   if (rc) return rc;
@@ -1301,23 +1519,38 @@ int apc_statistical_nobegin(apc_ctx* ctx, const float* xyzi, uint32_t n_max, con
   rc = grid_build(ctx, g, pts, n_max, n_dev, cell_hint, !(cell_hint > 0.0f), s);
   if (rc) return rc;
   const uint32_t bq = min(apc_div_up(n_max, KNN_WARPS), (uint32_t)APC_SM_COUNT * 16);   // one warp per query, grid-stride
-  {
-    APC_PROF(ctx, "k_knn_query", s);
-    // APC_KNN_START_FILL: own-cell population that selects the starting level (default 0 = always level 0: skipping
-    // fine levels by this estimate examines more candidates than the failed passes cost - 2.49 / 2.94 / 3.34 ms
-    // against 1.86 ms for a population of 5 / 10 / 16 on the C4 scan);
-    // APC_KNN_MARGIN=0: guaranteed radius = the cell edge only (profiles/r2x_knn_ab.json)
-    static const int fill_env = []() { const char* e = getenv("APC_KNN_START_FILL"); return e ? atoi(e) : -1; }();
-    static const int margin_env = []() { const char* e = getenv("APC_KNN_MARGIN"); return e ? atoi(e) : 1; }();
-    const uint32_t start_fill = fill_env > 0 ? (uint32_t)fill_env : 0u;
-    // newcomers in a batch of 32 above which the batch is sorted and merged instead of inserted one by one
-    static const uint32_t merge_min = []() { const char* e = getenv("APC_KNN_MERGE_MIN"); return e ? (uint32_t)atoi(e) : 6u; }();
-    k_knn_query<<<bq, KNN_WARPS * 32, 0, s>>>(n_max, n_dev, g.d, (uint32_t)nb_neighbors, avg, sc->stragglers, ctx->ctrl,
-                                              start_fill, margin_env, merge_min);
-  }
-  {
-    APC_PROF(ctx, "k_knn_stragglers", s);
-    k_knn_stragglers<<<APC_SM_COUNT * 2, 256, 0, s>>>(pts, n_max, n_dev, (uint32_t)nb_neighbors, sc->stragglers, ctx->ctrl, avg);
+  static const int margin_env = []() { const char* e = getenv("APC_KNN_MARGIN"); return e ? atoi(e) : 1; }();
+  if (nb_neighbors > KNN_KMAX) {
+    const uint32_t cap = wide_cap((uint32_t)nb_neighbors);
+    const size_t smem = (size_t)KNN_WARPS * cap * sizeof(uint32_t);
+    {
+      APC_PROF(ctx, "k_knn_query_wide", s);
+      k_knn_query_wide<<<bq, KNN_WARPS * 32, smem, s>>>(n_max, n_dev, g.d, (uint32_t)nb_neighbors, cap, avg, sc->stragglers,
+                                                        ctx->ctrl, margin_env);
+    }
+    {
+      APC_PROF(ctx, "k_knn_stragglers_wide", s);
+      k_knn_stragglers_wide<<<APC_SM_COUNT * 2, KNN_WARPS * 32, smem, s>>>(pts, n_max, n_dev, (uint32_t)nb_neighbors, cap,
+                                                                           sc->stragglers, ctx->ctrl, avg);
+    }
+  } else {
+    {
+      APC_PROF(ctx, "k_knn_query", s);
+      // APC_KNN_START_FILL: own-cell population that selects the starting level (default 0 = always level 0: skipping
+      // fine levels by this estimate examines more candidates than the failed passes cost - 2.49 / 2.94 / 3.34 ms
+      // against 1.86 ms for a population of 5 / 10 / 16 on the C4 scan);
+      // APC_KNN_MARGIN=0: guaranteed radius = the cell edge only (profiles/r2x_knn_ab.json)
+      static const int fill_env = []() { const char* e = getenv("APC_KNN_START_FILL"); return e ? atoi(e) : -1; }();
+      const uint32_t start_fill = fill_env > 0 ? (uint32_t)fill_env : 0u;
+      // newcomers in a batch of 32 above which the batch is sorted and merged instead of inserted one by one
+      static const uint32_t merge_min = []() { const char* e = getenv("APC_KNN_MERGE_MIN"); return e ? (uint32_t)atoi(e) : 6u; }();
+      k_knn_query<<<bq, KNN_WARPS * 32, 0, s>>>(n_max, n_dev, g.d, (uint32_t)nb_neighbors, avg, sc->stragglers, ctx->ctrl,
+                                                start_fill, margin_env, merge_min);
+    }
+    {
+      APC_PROF(ctx, "k_knn_stragglers", s);
+      k_knn_stragglers<<<APC_SM_COUNT * 2, 256, 0, s>>>(pts, n_max, n_dev, (uint32_t)nb_neighbors, sc->stragglers, ctx->ctrl, avg);
+    }
   }
   const dim3 gridc(min(apc_div_up(n_max, 256), (uint32_t)APC_SM_COUNT * 4), g.d.levels);
   {
@@ -1671,6 +1904,98 @@ k_normals_cov(uint32_t n_max, const uint32_t* n_dev, GridDev g, float r2, uint32
   }
 }
 
+// 64 < max_nn <= APC_MAX_NEIGHBORS: one warp per query over the same 27-cell flat candidate list as
+// k_normals_cov; the in-radius candidates stream through a WarpKeep of 64-bit keys (d2 bits << 32 |
+// original index: the oracle's total order, so the neighbourhood is exact) of wide_cap(max_nn) entries per
+// warp; the kept keys are sorted, and the lanes read the neighbours by original index from the input and add up
+// their float64 moments about the query point.  k_normals_eigen turns cov9 into normals.
+__global__ void __launch_bounds__(128)
+k_normals_wide(uint32_t n_max, const uint32_t* n_dev, GridDev g, const float4* __restrict__ pts, float r2, uint32_t max_nn,
+               uint32_t cap, uint32_t* __restrict__ counts, double* __restrict__ cov9, const ApcCtrl* __restrict__ ctrl) {
+  const uint32_t n = grid_sorted_count(g, ctrl, apc_count(n_dev, n_max));
+  const float c = grid_cell_size(g, 0);
+  const uint32_t lane = threadIdx.x & 31u;
+  unsigned long long* buf = reinterpret_cast<unsigned long long*>(wide_smem) + (size_t)(threadIdx.x >> 5) * cap;
+  for (uint32_t j = (blockIdx.x * blockDim.x + threadIdx.x) >> 5; j < n; j += (gridDim.x * blockDim.x) >> 5) {
+    const float4 q = g.sorted[j];
+    const uint32_t orig = __float_as_uint(q.w);
+    int32_t ix, iy, iz;
+    grid_coord_g(g, c, q.x, q.y, q.z, ix, iy, iz);  // succeeded at insert time
+    uint32_t cs = 0, cf = 0;
+    if (lane < 27) {
+      const int dx = (int)(lane % 3u) - 1, dy = (int)((lane / 3u) % 3u) - 1, dz = (int)(lane / 9u) - 1;
+      uint32_t b, f;
+      if (grid_lookup(g, grid_key(0, ix + dx, iy + dy, iz + dz), b, f)) { cs = b; cf = f; }
+    }
+    uint32_t incl = cf;
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+      const uint32_t v = __shfl_up_sync(0xffffffffu, incl, o);
+      if (lane >= (uint32_t)o) incl += v;
+    }
+    const uint32_t ps = incl - cf;
+    const uint32_t total = __shfl_sync(0xffffffffu, incl, 31);
+    WarpKeep<unsigned long long> wk;
+    wk.init(buf, cap, max_nn);
+    uint32_t in_radius = 0;
+    for (uint32_t base = 0; base < total; base += 32) {
+      const uint32_t ci = base + lane;
+      const uint32_t flat = min(ci, total - 1u);
+      uint32_t run = 0;
+#pragma unroll
+      for (int step = 16; step > 0; step >>= 1) {
+        const uint32_t mid = run + step;
+        const uint32_t v = __shfl_sync(0xffffffffu, ps, mid & 31u);
+        if (mid < 27u && v <= flat) run = mid;
+      }
+      const uint32_t rs = __shfl_sync(0xffffffffu, cs, run), rp = __shfl_sync(0xffffffffu, ps, run);
+      unsigned long long key = 0;
+      bool inside = false;
+      if (ci < total) {
+        const float4 p = g.sorted[rs + (flat - rp)];
+        const float d2 = d2_f32(q.x, q.y, q.z, p.x, p.y, p.z);
+        inside = d2 <= r2;
+        key = ((unsigned long long)__float_as_uint(d2) << 32) | __float_as_uint(p.w);
+      }
+      in_radius += __popc(__ballot_sync(0xffffffffu, inside));
+      wk.add(key, inside, lane);
+    }
+    wk.finish(lane);
+    const uint32_t n_sel = min(in_radius, max_nn);                 // == wk.m
+    double C[9] = {1.0, 0.0, 0.0, 0.0, 1.0, 0.0, 0.0, 0.0, 1.0};   // fewer than 3 neighbours: identity
+    if (n_sel >= 3) {
+      // the kept keys arrive in the grid's in-cell order, which the build's atomics decide: sorted, the sums
+      // below take the same order on every run
+      warp_sort(buf, n_sel, lane);
+      double v[9] = {0.0, 0.0, 0.0, 0.0, 0.0, 0.0, 0.0, 0.0, 0.0};
+      for (uint32_t i = lane; i < n_sel; i += 32) {
+        const float4 p = pts[(uint32_t)buf[i]];
+        const double x = (double)p.x - (double)q.x, y = (double)p.y - (double)q.y, z = (double)p.z - (double)q.z;
+        v[0] += x; v[1] += y; v[2] += z;
+        v[3] += x * x; v[4] += x * y; v[5] += x * z; v[6] += y * y; v[7] += y * z; v[8] += z * z;
+      }
+#pragma unroll
+      for (int k = 0; k < 9; ++k)
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) v[k] += __shfl_xor_sync(0xffffffffu, v[k], o);
+      const double inv = 1.0 / (double)n_sel;
+      const double s0 = v[0] * inv, s1 = v[1] * inv, s2 = v[2] * inv;
+      C[0] = v[3] * inv - s0 * s0;
+      C[1] = C[3] = v[4] * inv - s0 * s1;
+      C[2] = C[6] = v[5] * inv - s0 * s2;
+      C[4] = v[6] * inv - s1 * s1;
+      C[5] = C[7] = v[7] * inv - s1 * s2;
+      C[8] = v[8] * inv - s2 * s2;
+    }
+    double mine = C[0];                                            // C[lane] without a local-memory array
+#pragma unroll
+    for (int k = 1; k < 9; ++k) mine = lane == (uint32_t)k ? C[k] : mine;
+    if (lane < 9) cov9[9 * (size_t)orig + lane] = mine;
+    if (lane == 0 && counts) counts[orig] = n_sel;
+    __syncwarp();                                                  // buf is reused by the next query
+  }
+}
+
 __global__ void __launch_bounds__(256)
 k_normals_eigen(uint32_t n_max, const uint32_t* n_dev, const double* __restrict__ cov9, float* __restrict__ normals) {
   const uint32_t n = apc_count(n_dev, n_max);
@@ -1690,7 +2015,9 @@ int apc_normals_prepare(apc_ctx* ctx, int max_nn) {
   int rc = apc_neighbors_prepare(ctx, 0);
   if (rc) return rc;
   NeighborScratch* sc = scratch_of(ctx);
-  if (max_nn <= 32 && !sc->cov) APC_CUDA(ctx, cudaMalloc((void**)&sc->cov, (size_t)ctx->max_points * 9 * sizeof(double)));
+  // k_normals_cov (max_nn <= 32) and k_normals_wide (max_nn > 64) hand their covariances to k_normals_eigen
+  const bool via_cov = max_nn <= 32 || max_nn > NRM_KMAX;
+  if (via_cov && !sc->cov) APC_CUDA(ctx, cudaMalloc((void**)&sc->cov, (size_t)ctx->max_points * 9 * sizeof(double)));
   return APC_OK;
 }
 
@@ -1699,7 +2026,8 @@ int apc_normals_nobegin(apc_ctx* ctx, const float* xyzi, uint32_t n_max, const u
   if (n_max == 0) return APC_OK;
   APC_REQUIRE(ctx, xyzi && out_normals, "NULL pointer");
   APC_REQUIRE(ctx, n_max <= ctx->max_points, "more points than the context was created for");
-  APC_REQUIRE(ctx, max_nn >= 1 && max_nn <= NRM_KMAX && radius > 0.0, "max_nn must be in 1..64 and radius > 0");
+  APC_REQUIRE(ctx, max_nn >= 1 && max_nn <= APC_MAX_NEIGHBORS && radius > 0.0,
+              "max_nn must be in 1..APC_MAX_NEIGHBORS (" APC_STRINGIFY(APC_MAX_NEIGHBORS) ") and radius > 0");
   int rc = apc_neighbors_prepare(ctx, 0);
   if (rc) return rc;
   GridHost& g = scratch_of(ctx)->grid[0];
@@ -1711,7 +2039,7 @@ int apc_normals_nobegin(apc_ctx* ctx, const float* xyzi, uint32_t n_max, const u
   // the range the division with its 2^-10 margin guaranteed.
   rc = grid_build(ctx, g, pts, n_max, n_dev, r32 * 1.00390625f, false, s, false, CTR_CURSOR_NORMALS, true);
   if (rc) return rc;
-  if (max_nn <= 32) {
+  if (max_nn <= 32 || max_nn > NRM_KMAX) {
     // warp per query -> covariances (caller's buffer or context scratch), then thread per point -> eigenvector
     NeighborScratch* sc = scratch_of(ctx);
     double* cov = out_cov;
@@ -1720,9 +2048,14 @@ int apc_normals_nobegin(apc_ctx* ctx, const float* xyzi, uint32_t n_max, const u
       cov = sc->cov;
     }
     const uint32_t bq = min(apc_div_up(n_max, 4), (uint32_t)APC_SM_COUNT * 16);
-    {
+    if (max_nn <= 32) {
       APC_PROF(ctx, "k_normals_cov", s);
       k_normals_cov<<<bq, 128, 0, s>>>(n_max, n_dev, g.d, r32 * r32, (uint32_t)max_nn, out_counts, cov, ctx->ctrl);
+    } else {
+      const uint32_t cap = wide_cap((uint32_t)max_nn);
+      APC_PROF(ctx, "k_normals_wide", s);
+      k_normals_wide<<<bq, 128, (size_t)4 * cap * sizeof(unsigned long long), s>>>(n_max, n_dev, g.d, pts, r32 * r32, (uint32_t)max_nn,
+                                                                                   cap, out_counts, cov, ctx->ctrl);
     }
     APC_PROF(ctx, "k_normals_eigen", s);
     k_normals_eigen<<<min(apc_div_up(n_max, 256), (uint32_t)APC_SM_COUNT * 8), 256, 0, s>>>(n_max, n_dev, cov, out_normals);

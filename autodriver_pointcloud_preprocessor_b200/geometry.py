@@ -249,8 +249,9 @@ class PointCloud:
     def estimate_normals(self, max_nn=30, radius=None):   # pp.py:523
         """Open3D ``estimate_normals``: hybrid search (``max_nn`` nearest within ``radius``) ->
         covariance -> eigenvector of the smallest eigenvalue; sets ``point['normals']`` (float32
-        N x 3), not oriented.  Both arguments are required here (the reference passes both,
-        pp.py:523-526); pure-KNN / pure-radius searches are not implemented."""
+        N x 3), not oriented.  ``max_nn`` in 1..``APC_MAX_NEIGHBORS`` (1024; beyond it the call raises
+        ``ApcError``).  Both arguments are required here (the reference passes both, pp.py:523-526);
+        pure-KNN / pure-radius searches are not implemented."""
         if radius is None or max_nn is None:
             raise NotImplementedError("estimate_normals needs both radius and max_nn (hybrid search, pp.py:523-526)")
         if self._n() == 0:
@@ -397,6 +398,9 @@ class PointCloud:
 
     # -- outliers (pp.py:516; TODO pp.py:37)
     def remove_statistical_outliers(self, nb_neighbors, std_ratio):
+        """Open3D ``remove_statistical_outliers``: keep the points whose mean distance to their
+        ``nb_neighbors`` nearest (self included) is at most mu + std_ratio * sigma.  ``nb_neighbors`` in
+        1..``APC_MAX_NEIGHBORS`` (1024; beyond it the call raises ``ApcError``)."""
         if nb_neighbors < 1 or std_ratio <= 0:
             raise ValueError("Illegal input parameters, the number of neighbors and standard deviation ratio must be positive")
         ctx = self._ctx()

@@ -297,8 +297,8 @@ class PointcloudPreprocessorNode(Node):
             return False
         # 'auto': the fused pipeline carries x, y, z, intensity itself, estimates the normals between the
         # outlier and the ground stage, and ring / time / return_type / rgb travel through its index maps.
-        # Only parameter values beyond the kernels' caps (INTEGRATION.md) take the staged carrier path.
-        return not (self.estimate_normals and self.estimate_normals_max_neighbors > 64)
+        # Both paths accept the same parameter ranges (INTEGRATION.md, "Parameter caps").
+        return True
 
     # ------------------------------------------------------------------------------------------------
     def _upload_message(self, ros_cloud):

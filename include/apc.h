@@ -56,6 +56,7 @@ enum { APC_INT8 = 1, APC_UINT8 = 2, APC_INT16 = 3, APC_UINT16 = 4, APC_INT32 = 5
 #define APC_MAX_FIELDS 16     /* fields read_points may test for NaN */
 #define APC_MAX_CLOUDS 8      /* sensors merged in one launch */
 #define APC_MAX_TRANSFORMS 3  /* offset(lidar) -> TF -> offset(robot), pp.py:480-491 */
+#define APC_MAX_NEIGHBORS 1024 /* statistical nb_neighbors and normals max_nn */
 
 typedef struct apc_field {
   int32_t offset;   /* byte offset inside a point record */
@@ -241,7 +242,8 @@ int apc_radius_outliers(apc_ctx* ctx, const float* xyzi, uint32_t n_max, const u
                         int nb_points, double radius, uint8_t* out_mask,
                         uint32_t* out_neighbor_counts, void* stream);
 
-/* remove_statistical_outliers(nb_neighbors, std_ratio) (pp.py:514-519).  out_avg
+/* remove_statistical_outliers(nb_neighbors, std_ratio) (pp.py:514-519), nb_neighbors in
+ * 1..APC_MAX_NEIGHBORS (APC_ERR_BAD_ARG beyond).  out_avg
  * float32[n_max] (mean distance to the k nearest, self included) may be NULL;
  * out_stats_dev double[3] = (mu, sigma, threshold) may be NULL. */
 int apc_statistical_outliers(apc_ctx* ctx, const float* xyzi, uint32_t n_max,
@@ -250,7 +252,7 @@ int apc_statistical_outliers(apc_ctx* ctx, const float* xyzi, uint32_t n_max,
                              void* stream);
 
 /* estimate_normals(radius, max_nn) (pp.py:521-530, on by default pp.py:176; Open3D hybrid search):
- * neighbourhood = the max_nn (<= 64) nearest of the points with d2 <= float32(radius)^2, query
+ * neighbourhood = the max_nn (1..APC_MAX_NEIGHBORS) nearest of the points with d2 <= float32(radius)^2, query
  * included, ties by lower index; normal = eigenvector of the smallest eigenvalue of the
  * neighbourhood covariance (analytic symmetric 3x3 solver), not oriented; fewer than 3 neighbours
  * -> (0, 0, 1).  out_normals float32[3*n_max]; out_neighbor_counts uint32[n_max] and
@@ -302,7 +304,7 @@ typedef struct apc_pipeline_cfg {
   apc_filter_cfg filter;
   float voxel_size;            /* <= 0 disables (pp.py:509) */
   int32_t stat_enable;         /* pp.py:514 */
-  int32_t stat_nb_neighbors;
+  int32_t stat_nb_neighbors;   /* 1..APC_MAX_NEIGHBORS */
   double stat_std_ratio;
   int32_t radius_enable;       /* additive stage, TODO pp.py:37 */
   int32_t radius_nb_points;
@@ -315,7 +317,7 @@ typedef struct apc_pipeline_cfg {
   uint64_t ground_seed;
   int32_t normals_enable;      /* estimate_normals (pp.py:521-530, on by default pp.py:176): runs on the cloud that
                                   enters the ground stage; the normals travel through its selection (pp.py:542) */
-  int32_t normals_max_nn;      /* 1..64 */
+  int32_t normals_max_nn;      /* 1..APC_MAX_NEIGHBORS */
   double normals_radius;
 } apc_pipeline_cfg;
 
