@@ -15,6 +15,7 @@
 // until the k-th distance is covered by the 27-cell block, and the rare points that never
 // are (fewer than k points in range of the coarsest level) fall to an exact brute-force
 // kernel.  The table is cleaned by the points that own rank 0 of their cell, not by memset.
+#include <cmath>
 #include <cstdlib>
 #include <cstring>
 #include "apc_scan.cuh"
@@ -1058,6 +1059,99 @@ __device__ float wide_average(uint32_t* buf, uint32_t k_eff, uint32_t lane) {
 
 extern __shared__ __align__(16) unsigned char wide_smem[];
 
+// Selection key of a candidate at float32 distance d2 whose original index is idx: the d2 bit pattern for
+// the statistical stage (equal distances are interchangeable there), (d2 bits << 32 | index) for the
+// normals (the oracle's total order (d2, index): the neighbourhood itself is exact).
+template <typename K> __device__ __forceinline__ K knn_key(float d2, uint32_t idx);
+template <> __device__ __forceinline__ uint32_t knn_key<uint32_t>(float d2, uint32_t) { return __float_as_uint(d2); }
+template <> __device__ __forceinline__ unsigned long long knn_key<unsigned long long>(float d2, uint32_t idx) {
+  return ((unsigned long long)__float_as_uint(d2) << 32) | idx;
+}
+
+// The KNN grid's level climb for query q (warp-collective), shared by k_knn_query_wide and k_normals_knn:
+// per level, lanes 0..26 resolve the 27 cells, the flat candidate list streams through a WarpKeep of `cap`
+// keys at buf, and the level stands if the k_eff-th distance is covered by the block (`safe`, exact_margin).
+// Returns true with the k_eff smallest keys in buf[0, k_eff) (unordered); false when no level covers q
+// (a straggler).
+template <typename K>
+__device__ __forceinline__ bool knn_levels(const GridDev& g, uint32_t n_max, float4 q, uint32_t k_eff, K* buf, uint32_t cap,
+                                           int exact_margin, uint32_t lane) {
+  for (uint32_t level = 0; level < g.levels; ++level) {
+    const float c = g.cell[level];
+    int32_t ix, iy, iz;
+    if (!grid_coord_g(g, c, q.x, q.y, q.z, ix, iy, iz)) continue;
+    uint32_t cs = 0, cf = 0;
+    if (lane < 27) {
+      const int dx = (int)(lane % 3u) - 1, dy = (int)((lane / 3u) % 3u) - 1, dz = (int)(lane / 9u) - 1;
+      uint32_t b, f;
+      if (grid_lookup(g, grid_key(level, ix + dx, iy + dy, iz + dz), b, f)) { cs = b; cf = f; }
+    }
+    uint32_t incl = cf;
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+      const uint32_t v = __shfl_up_sync(0xffffffffu, incl, o);
+      if (lane >= (uint32_t)o) incl += v;
+    }
+    const uint32_t ps = incl - cf;
+    const uint32_t total = __shfl_sync(0xffffffffu, incl, 31);
+    if (total < k_eff) continue;
+    const float4* sp = g.sorted + (size_t)level * n_max;
+    float safe = c;
+    if (exact_margin) {
+      const float mx = fminf(__fsub_rn(q.x, __fmul_rn((float)ix, c)), __fsub_rn(__fmul_rn((float)(ix + 1), c), q.x));
+      const float my = fminf(__fsub_rn(q.y, __fmul_rn((float)iy, c)), __fsub_rn(__fmul_rn((float)(iy + 1), c), q.y));
+      const float mz = fminf(__fsub_rn(q.z, __fmul_rn((float)iz, c)), __fsub_rn(__fmul_rn((float)(iz + 1), c), q.z));
+      safe = __fadd_rn(c, fmaxf(0.0f, fminf(mx, fminf(my, mz))));
+    }
+    safe = __fmul_rn(safe, 0.999f);
+    WarpKeep<K> wk;
+    wk.init(buf, cap, k_eff);
+    for (uint32_t base = 0; base < total; base += 32) {
+      const uint32_t ci = base + lane;
+      const uint32_t flat = min(ci, total - 1u);
+      uint32_t run = 0;                                          // largest t with ps[t] <= flat
+#pragma unroll
+      for (int step = 16; step > 0; step >>= 1) {
+        const uint32_t mid = run + step;
+        const uint32_t v = __shfl_sync(0xffffffffu, ps, mid & 31u);
+        if (mid < 27u && v <= flat) run = mid;
+      }
+      const uint32_t rs = __shfl_sync(0xffffffffu, cs, run), rp = __shfl_sync(0xffffffffu, ps, run);
+      K key = 0;
+      if (ci < total) {
+        const float4 p = sp[rs + (flat - rp)];
+        key = knn_key<K>(d2_f32(q.x, q.y, q.z, p.x, p.y, p.z), __float_as_uint(p.w));
+      }
+      wk.add(key, ci < total, lane);
+    }
+    wk.finish(lane);
+    uint32_t mx = 0;                                             // covered by the block? (the d2 bits of the keys)
+    for (uint32_t i = lane; i < k_eff; i += 32) mx = max(mx, (uint32_t)(buf[i] >> (8 * sizeof(K) - 32)));
+    if (__uint_as_float(__reduce_max_sync(0xffffffffu, mx)) <= __fmul_rn(safe, safe)) return true;
+  }
+  return false;
+}
+
+// Exact brute force for a query no level covers (warp-collective): every point streams through the
+// WarpKeep (after the first selection nearly all are rejected by the bound).  The k_eff smallest keys
+// end in buf[0, k_eff), unordered.
+template <typename K>
+__device__ __forceinline__ void knn_brute(const float4* __restrict__ pts, uint32_t n, float4 q, uint32_t k_eff, K* buf,
+                                          uint32_t cap, uint32_t lane) {
+  WarpKeep<K> wk;
+  wk.init(buf, cap, k_eff);
+  for (uint32_t base = 0; base < n; base += 32) {
+    const uint32_t i = base + lane;
+    K key = 0;
+    if (i < n) {
+      const float4 p = pts[i];
+      key = knn_key<K>(d2_f32(q.x, q.y, q.z, p.x, p.y, p.z), i);
+    }
+    wk.add(key, i < n, lane);
+  }
+  wk.finish(lane);
+}
+
 // k_knn_query for 64 < k <= APC_MAX_NEIGHBORS: the same level climb, 27-cell flat candidate list and
 // coverage test (`safe`, exact_margin), the candidates through a WarpKeep of wide_cap(k) entries per
 // warp (dynamic shared memory), the accepted level's k distances sorted and summed by wide_average.
@@ -1072,61 +1166,7 @@ k_knn_query_wide(uint32_t n_max, const uint32_t* n_dev, GridDev g, uint32_t k, u
   for (uint32_t j = blockIdx.x * KNN_WARPS + w; j < n_sorted; j += gridDim.x * KNN_WARPS) {
     const float4 q = g.sorted[j];
     const uint32_t orig = __float_as_uint(q.w);
-    bool done = false;
-    for (uint32_t level = 0; level < g.levels && !done; ++level) {
-      const float c = g.cell[level];
-      int32_t ix, iy, iz;
-      if (!grid_coord_g(g, c, q.x, q.y, q.z, ix, iy, iz)) continue;
-      uint32_t cs = 0, cf = 0;
-      if (lane < 27) {
-        const int dx = (int)(lane % 3u) - 1, dy = (int)((lane / 3u) % 3u) - 1, dz = (int)(lane / 9u) - 1;
-        uint32_t b, f;
-        if (grid_lookup(g, grid_key(level, ix + dx, iy + dy, iz + dz), b, f)) { cs = b; cf = f; }
-      }
-      uint32_t incl = cf;
-#pragma unroll
-      for (int o = 1; o < 32; o <<= 1) {
-        const uint32_t v = __shfl_up_sync(0xffffffffu, incl, o);
-        if (lane >= (uint32_t)o) incl += v;
-      }
-      const uint32_t ps = incl - cf;
-      const uint32_t total = __shfl_sync(0xffffffffu, incl, 31);
-      if (total < k_eff) continue;
-      const float4* sp = g.sorted + (size_t)level * n_max;
-      float safe = c;
-      if (exact_margin) {
-        const float mx = fminf(__fsub_rn(q.x, __fmul_rn((float)ix, c)), __fsub_rn(__fmul_rn((float)(ix + 1), c), q.x));
-        const float my = fminf(__fsub_rn(q.y, __fmul_rn((float)iy, c)), __fsub_rn(__fmul_rn((float)(iy + 1), c), q.y));
-        const float mz = fminf(__fsub_rn(q.z, __fmul_rn((float)iz, c)), __fsub_rn(__fmul_rn((float)(iz + 1), c), q.z));
-        safe = __fadd_rn(c, fmaxf(0.0f, fminf(mx, fminf(my, mz))));
-      }
-      safe = __fmul_rn(safe, 0.999f);
-      WarpKeep<uint32_t> wk;
-      wk.init(buf, cap, k_eff);
-      for (uint32_t base = 0; base < total; base += 32) {
-        const uint32_t ci = base + lane;
-        const uint32_t flat = min(ci, total - 1u);
-        uint32_t run = 0;                                          // largest t with ps[t] <= flat
-#pragma unroll
-        for (int step = 16; step > 0; step >>= 1) {
-          const uint32_t mid = run + step;
-          const uint32_t v = __shfl_sync(0xffffffffu, ps, mid & 31u);
-          if (mid < 27u && v <= flat) run = mid;
-        }
-        const uint32_t rs = __shfl_sync(0xffffffffu, cs, run), rp = __shfl_sync(0xffffffffu, ps, run);
-        uint32_t key = 0;
-        if (ci < total) {
-          const float4 p = sp[rs + (flat - rp)];
-          key = __float_as_uint(d2_f32(q.x, q.y, q.z, p.x, p.y, p.z));
-        }
-        wk.add(key, ci < total, lane);
-      }
-      wk.finish(lane);
-      uint32_t mx = 0;                                             // covered by the block?
-      for (uint32_t i = lane; i < k_eff; i += 32) mx = max(mx, buf[i]);
-      if (__uint_as_float(__reduce_max_sync(0xffffffffu, mx)) <= __fmul_rn(safe, safe)) done = true;
-    }
-    if (done) {
+    if (knn_levels(g, n_max, q, k_eff, buf, cap, exact_margin, lane)) {
       const float a = wide_average(buf, k_eff, lane);
       if (lane == 0) avg[orig] = a;
     } else if (lane == 0) {
@@ -1136,8 +1176,7 @@ k_knn_query_wide(uint32_t n_max, const uint32_t* n_dev, GridDev g, uint32_t k, u
   }
 }
 
-// Exact brute force for the points no level of k_knn_query_wide covers: one warp per straggler streams
-// every point through its WarpKeep (after the first selection nearly all are rejected by the bound).
+// Exact brute force for the points no level of k_knn_query_wide covers: one warp per straggler.
 __global__ void __launch_bounds__(KNN_WARPS * 32)
 k_knn_stragglers_wide(const float4* __restrict__ pts, uint32_t n_max, const uint32_t* n_dev, uint32_t k, uint32_t cap,
                       const uint32_t* __restrict__ stragglers, const ApcCtrl* ctrl, float* __restrict__ avg) {
@@ -1148,19 +1187,7 @@ k_knn_stragglers_wide(const float4* __restrict__ pts, uint32_t n_max, const uint
   uint32_t* buf = reinterpret_cast<uint32_t*>(wide_smem) + (size_t)w * cap;
   for (uint32_t sidx = blockIdx.x * KNN_WARPS + w; sidx < n_str; sidx += gridDim.x * KNN_WARPS) {
     const uint32_t orig = stragglers[sidx];
-    const float4 q = pts[orig];
-    WarpKeep<uint32_t> wk;
-    wk.init(buf, cap, k_eff);
-    for (uint32_t base = 0; base < n; base += 32) {
-      const uint32_t i = base + lane;
-      uint32_t key = 0;
-      if (i < n) {
-        const float4 p = pts[i];
-        key = __float_as_uint(d2_f32(q.x, q.y, q.z, p.x, p.y, p.z));
-      }
-      wk.add(key, i < n, lane);
-    }
-    wk.finish(lane);
+    knn_brute(pts, n, pts[orig], k_eff, buf, cap, lane);
     const float a = wide_average(buf, k_eff, lane);
     if (lane == 0) avg[orig] = a;
   }
@@ -1244,16 +1271,22 @@ __global__ void __launch_bounds__(256) k_bbox(const float4* __restrict__ pts, ui
     }
   }
 }
-// level sizes: c0 = hint if > 0 else max extent / 4096 (>= 1e-4), c_l = c0 * 2^l
+// level sizes: c0 = hint if > 0 else max extent / 4096 (>= 1e-4), c_l = c0 * 2^l.  Without a hint c0 is also
+// kept large enough for the farthest coordinate to have a level-0 cell index (|index| < 262 143): a small cloud
+// far from the origin (a single point at 30 m: extent 0, cells of 1e-4 m) would otherwise fail with
+// APC_ERR_KEY_RANGE.  Clouds whose indices stay below 262 000 keep their cell size.
 __global__ void k_grid_cells(const ApcCtrl* ctrl, float hint, uint32_t levels, float* cell) {
   float c0 = hint;
   if (!(c0 > 0.0f)) {
-    float ext = 0.0f;
+    float ext = 0.0f, big = 0.0f;
     for (int a = 0; a < 3; ++a) {
       const float lo = ord2f((int32_t)ctrl->counters[CTR_BBOX + a]), hi = ord2f((int32_t)ctrl->counters[CTR_BBOX + 3 + a]);
-      if (hi >= lo) ext = fmaxf(ext, hi - lo);
+      if (hi >= lo) {
+        ext = fmaxf(ext, hi - lo);
+        big = fmaxf(big, fmaxf(fabsf(lo), fabsf(hi)));
+      }
     }
-    c0 = fmaxf(ext * (1.0f / 4096.0f), 1.0e-4f);
+    c0 = fmaxf(fmaxf(ext * (1.0f / 4096.0f), 1.0e-4f), big * (1.0f / 262000.0f));
   }
   for (uint32_t l = 0; l < levels; ++l) { cell[l] = c0; c0 = c0 * 2.0f; }
 }
@@ -1904,6 +1937,43 @@ k_normals_cov(uint32_t n_max, const uint32_t* n_dev, GridDev g, float r2, uint32
   }
 }
 
+// Covariance of a kept neighbourhood (warp-collective): buf[0, n_sel) holds the neighbours' 64-bit keys (d2 bits
+// << 32 | original index), unordered.  The float64 moments about q are summed in key order, the same on every run
+// (the keys arrive in the grid's in-cell order, which the build's atomics decide); lanes 0..8 write cov9 of point
+// orig, lane 0 the count.  Fewer than 3 neighbours: identity.
+__device__ __forceinline__ void normals_cov_of_keys(unsigned long long* buf, uint32_t n_sel, const float4* __restrict__ pts,
+                                                    float4 q, uint32_t orig, uint32_t lane, uint32_t* __restrict__ counts,
+                                                    double* __restrict__ cov9) {
+  double C[9] = {1.0, 0.0, 0.0, 0.0, 1.0, 0.0, 0.0, 0.0, 1.0};
+  if (n_sel >= 3) {
+    warp_sort(buf, n_sel, lane);
+    double v[9] = {0.0, 0.0, 0.0, 0.0, 0.0, 0.0, 0.0, 0.0, 0.0};
+    for (uint32_t i = lane; i < n_sel; i += 32) {
+      const float4 p = pts[(uint32_t)buf[i]];
+      const double x = (double)p.x - (double)q.x, y = (double)p.y - (double)q.y, z = (double)p.z - (double)q.z;
+      v[0] += x; v[1] += y; v[2] += z;
+      v[3] += x * x; v[4] += x * y; v[5] += x * z; v[6] += y * y; v[7] += y * z; v[8] += z * z;
+    }
+#pragma unroll
+    for (int k = 0; k < 9; ++k)
+#pragma unroll
+      for (int o = 16; o > 0; o >>= 1) v[k] += __shfl_xor_sync(0xffffffffu, v[k], o);
+    const double inv = 1.0 / (double)n_sel;
+    const double s0 = v[0] * inv, s1 = v[1] * inv, s2 = v[2] * inv;
+    C[0] = v[3] * inv - s0 * s0;
+    C[1] = C[3] = v[4] * inv - s0 * s1;
+    C[2] = C[6] = v[5] * inv - s0 * s2;
+    C[4] = v[6] * inv - s1 * s1;
+    C[5] = C[7] = v[7] * inv - s1 * s2;
+    C[8] = v[8] * inv - s2 * s2;
+  }
+  double mine = C[0];                                            // C[lane] without a local-memory array
+#pragma unroll
+  for (int k = 1; k < 9; ++k) mine = lane == (uint32_t)k ? C[k] : mine;
+  if (lane < 9) cov9[9 * (size_t)orig + lane] = mine;
+  if (lane == 0 && counts) counts[orig] = n_sel;
+}
+
 // 64 < max_nn <= APC_MAX_NEIGHBORS: one warp per query over the same 27-cell flat candidate list as
 // k_normals_cov; the in-radius candidates stream through a WarpKeep of 64-bit keys (d2 bits << 32 |
 // original index: the oracle's total order, so the neighbourhood is exact) of wide_cap(max_nn) entries per
@@ -1961,38 +2031,129 @@ k_normals_wide(uint32_t n_max, const uint32_t* n_dev, GridDev g, const float4* _
       wk.add(key, inside, lane);
     }
     wk.finish(lane);
-    const uint32_t n_sel = min(in_radius, max_nn);                 // == wk.m
-    double C[9] = {1.0, 0.0, 0.0, 0.0, 1.0, 0.0, 0.0, 0.0, 1.0};   // fewer than 3 neighbours: identity
-    if (n_sel >= 3) {
-      // the kept keys arrive in the grid's in-cell order, which the build's atomics decide: sorted, the sums
-      // below take the same order on every run
-      warp_sort(buf, n_sel, lane);
-      double v[9] = {0.0, 0.0, 0.0, 0.0, 0.0, 0.0, 0.0, 0.0, 0.0};
-      for (uint32_t i = lane; i < n_sel; i += 32) {
-        const float4 p = pts[(uint32_t)buf[i]];
-        const double x = (double)p.x - (double)q.x, y = (double)p.y - (double)q.y, z = (double)p.z - (double)q.z;
-        v[0] += x; v[1] += y; v[2] += z;
-        v[3] += x * x; v[4] += x * y; v[5] += x * z; v[6] += y * y; v[7] += y * z; v[8] += z * z;
+    normals_cov_of_keys(buf, min(in_radius, max_nn), pts, q, orig, lane, counts, cov9);   // n_sel == wk.m
+    __syncwarp();                                                  // buf is reused by the next query
+  }
+}
+
+// KNN search (Open3D estimate_normals with max_nn only): the max_nn nearest points by (d2, original index),
+// no distance bound.  One warp per query climbs the levels of the KNN grid like k_knn_query_wide, with the
+// 64-bit keys of k_normals_wide; the queries no level covers go to k_normals_knn_stragglers.
+__global__ void __launch_bounds__(KNN_WARPS * 32)
+k_normals_knn(uint32_t n_max, const uint32_t* n_dev, GridDev g, const float4* __restrict__ pts, uint32_t k, uint32_t cap,
+              uint32_t* __restrict__ counts, double* __restrict__ cov9, uint32_t* __restrict__ stragglers, ApcCtrl* ctrl) {
+  const uint32_t n = apc_count(n_dev, n_max);
+  const uint32_t n_sorted = grid_sorted_count(g, ctrl, n);
+  const uint32_t k_eff = min(k, n);
+  const uint32_t lane = threadIdx.x & 31u, w = threadIdx.x >> 5;
+  unsigned long long* buf = reinterpret_cast<unsigned long long*>(wide_smem) + (size_t)w * cap;
+  for (uint32_t j = blockIdx.x * KNN_WARPS + w; j < n_sorted; j += gridDim.x * KNN_WARPS) {
+    const float4 q = g.sorted[j];
+    const uint32_t orig = __float_as_uint(q.w);
+    if (knn_levels(g, n_max, q, k_eff, buf, cap, 1, lane)) normals_cov_of_keys(buf, k_eff, pts, q, orig, lane, counts, cov9);
+    else if (lane == 0) stragglers[atomicAdd(&ctrl->counters[CTR_STRAGGLERS], 1u)] = orig;
+    __syncwarp();
+  }
+}
+
+__global__ void __launch_bounds__(KNN_WARPS * 32)
+k_normals_knn_stragglers(const float4* __restrict__ pts, uint32_t n_max, const uint32_t* n_dev, uint32_t k, uint32_t cap,
+                         const uint32_t* __restrict__ stragglers, const ApcCtrl* ctrl, uint32_t* __restrict__ counts,
+                         double* __restrict__ cov9) {
+  const uint32_t n = apc_count(n_dev, n_max);
+  const uint32_t k_eff = min(k, n);
+  const uint32_t n_str = ctrl->counters[CTR_STRAGGLERS];
+  const uint32_t lane = threadIdx.x & 31u, w = threadIdx.x >> 5;
+  unsigned long long* buf = reinterpret_cast<unsigned long long*>(wide_smem) + (size_t)w * cap;
+  for (uint32_t sidx = blockIdx.x * KNN_WARPS + w; sidx < n_str; sidx += gridDim.x * KNN_WARPS) {
+    const uint32_t orig = stragglers[sidx];
+    const float4 q = pts[orig];
+    knn_brute(pts, n, q, k_eff, buf, cap, lane);
+    normals_cov_of_keys(buf, k_eff, pts, q, orig, lane, counts, cov9);
+    __syncwarp();
+  }
+}
+
+// Radius search (Open3D estimate_normals with radius only): every point with d2 <= float32(r)^2, no cap on the
+// count.  One warp per query over the 27-cell flat candidate list of k_normals_wide, nothing kept: each
+// in-radius neighbour adds its moments about the query in fixed point, rint(d * 2^40 / r) for the 3 first and
+// rint(d d' * 2^40 / r^2) for the 6 second moments, in int64.  Integer sums do not depend on the order the
+// grid's atomics leave inside a cell, so the covariance is bit-identical across runs and input permutations.
+// Every term is at most ~2^40 and a context holds at most 2^22 points: the sums stay below 2^62.
+#define NRM_FIX_ONE 1099511627776.0   // 2^40
+__global__ void __launch_bounds__(128)
+k_normals_radius(uint32_t n_max, const uint32_t* n_dev, GridDev g, float r, float r2, uint32_t* __restrict__ counts,
+                 double* __restrict__ cov9, const ApcCtrl* __restrict__ ctrl) {
+  const uint32_t n = grid_sorted_count(g, ctrl, apc_count(n_dev, n_max));
+  const float c = grid_cell_size(g, 0);
+  const uint32_t lane = threadIdx.x & 31u;
+  const double s1 = NRM_FIX_ONE / (double)r, s2 = NRM_FIX_ONE / ((double)r * (double)r);
+  for (uint32_t j = (blockIdx.x * blockDim.x + threadIdx.x) >> 5; j < n; j += (gridDim.x * blockDim.x) >> 5) {
+    const float4 q = g.sorted[j];
+    const uint32_t orig = __float_as_uint(q.w);
+    int32_t ix, iy, iz;
+    grid_coord_g(g, c, q.x, q.y, q.z, ix, iy, iz);  // succeeded at insert time
+    uint32_t cs = 0, cf = 0;
+    if (lane < 27) {
+      const int dx = (int)(lane % 3u) - 1, dy = (int)((lane / 3u) % 3u) - 1, dz = (int)(lane / 9u) - 1;
+      uint32_t b, f;
+      if (grid_lookup(g, grid_key(0, ix + dx, iy + dy, iz + dz), b, f)) { cs = b; cf = f; }
+    }
+    uint32_t incl = cf;
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+      const uint32_t v = __shfl_up_sync(0xffffffffu, incl, o);
+      if (lane >= (uint32_t)o) incl += v;
+    }
+    const uint32_t ps = incl - cf;
+    const uint32_t total = __shfl_sync(0xffffffffu, incl, 31);
+    long long m[9] = {0, 0, 0, 0, 0, 0, 0, 0, 0};
+    uint32_t cnt = 0;
+    for (uint32_t base = 0; base < total; base += 32) {
+      const uint32_t ci = base + lane;
+      const uint32_t flat = min(ci, total - 1u);
+      uint32_t run = 0;
+#pragma unroll
+      for (int step = 16; step > 0; step >>= 1) {
+        const uint32_t mid = run + step;
+        const uint32_t v = __shfl_sync(0xffffffffu, ps, mid & 31u);
+        if (mid < 27u && v <= flat) run = mid;
       }
+      const uint32_t rs = __shfl_sync(0xffffffffu, cs, run), rp = __shfl_sync(0xffffffffu, ps, run);
+      bool inside = false;
+      if (ci < total) {
+        const float4 p = g.sorted[rs + (flat - rp)];
+        inside = d2_f32(q.x, q.y, q.z, p.x, p.y, p.z) <= r2;
+        if (inside) {
+          const double x = (double)p.x - (double)q.x, y = (double)p.y - (double)q.y, z = (double)p.z - (double)q.z;
+          m[0] += __double2ll_rn(x * s1); m[1] += __double2ll_rn(y * s1); m[2] += __double2ll_rn(z * s1);
+          m[3] += __double2ll_rn(x * x * s2); m[4] += __double2ll_rn(x * y * s2); m[5] += __double2ll_rn(x * z * s2);
+          m[6] += __double2ll_rn(y * y * s2); m[7] += __double2ll_rn(y * z * s2); m[8] += __double2ll_rn(z * z * s2);
+        }
+      }
+      cnt += __popc(__ballot_sync(0xffffffffu, inside));
+    }
+    double C[9] = {1.0, 0.0, 0.0, 0.0, 1.0, 0.0, 0.0, 0.0, 1.0};   // fewer than 3 neighbours: identity
+    if (cnt >= 3) {
 #pragma unroll
       for (int k = 0; k < 9; ++k)
 #pragma unroll
-        for (int o = 16; o > 0; o >>= 1) v[k] += __shfl_xor_sync(0xffffffffu, v[k], o);
-      const double inv = 1.0 / (double)n_sel;
-      const double s0 = v[0] * inv, s1 = v[1] * inv, s2 = v[2] * inv;
-      C[0] = v[3] * inv - s0 * s0;
-      C[1] = C[3] = v[4] * inv - s0 * s1;
-      C[2] = C[6] = v[5] * inv - s0 * s2;
-      C[4] = v[6] * inv - s1 * s1;
-      C[5] = C[7] = v[7] * inv - s1 * s2;
-      C[8] = v[8] * inv - s2 * s2;
+        for (int o = 16; o > 0; o >>= 1) m[k] += __shfl_xor_sync(0xffffffffu, m[k], o);
+      const double inv = 1.0 / (double)cnt;
+      const double u1 = (double)r / NRM_FIX_ONE, u2 = (double)r * (double)r / NRM_FIX_ONE;
+      const double a0 = (double)m[0] * u1 * inv, a1 = (double)m[1] * u1 * inv, a2 = (double)m[2] * u1 * inv;
+      C[0] = (double)m[3] * u2 * inv - a0 * a0;
+      C[1] = C[3] = (double)m[4] * u2 * inv - a0 * a1;
+      C[2] = C[6] = (double)m[5] * u2 * inv - a0 * a2;
+      C[4] = (double)m[6] * u2 * inv - a1 * a1;
+      C[5] = C[7] = (double)m[7] * u2 * inv - a1 * a2;
+      C[8] = (double)m[8] * u2 * inv - a2 * a2;
     }
     double mine = C[0];                                            // C[lane] without a local-memory array
 #pragma unroll
     for (int k = 1; k < 9; ++k) mine = lane == (uint32_t)k ? C[k] : mine;
     if (lane < 9) cov9[9 * (size_t)orig + lane] = mine;
-    if (lane == 0 && counts) counts[orig] = n_sel;
-    __syncwarp();                                                  // buf is reused by the next query
+    if (lane == 0 && counts) counts[orig] = cnt;
   }
 }
 
@@ -2082,4 +2243,95 @@ extern "C" int apc_estimate_normals(apc_ctx* ctx, const float* xyzi, uint32_t n_
   if (out_normals && n_max) APC_CUDA(ctx, cudaMemsetAsync(out_normals, 0, (size_t)n_max * 3 * sizeof(float), s));
   if (out_neighbor_counts && n_max) APC_CUDA(ctx, cudaMemsetAsync(out_neighbor_counts, 0, (size_t)n_max * sizeof(uint32_t), s));
   return apc_normals_nobegin(ctx, xyzi, n_max, n_dev, max_nn, radius, out_normals, out_neighbor_counts, out_covariances, s);
+}
+
+// ---- estimate_normals with one search bound: max_nn only (KNN) or radius only ---------------------------------
+// Common start of apc_estimate_normals_knn / _radius once the mode's argument is checked: allocates grid `which`
+// and the covariance scratch before anything is launched (nothing is allocated between the call's kernels),
+// begins the call and zeroes the outputs.  Points the grid cannot key are never queried: their covariance stays
+// zero, so k_normals_eigen gives them the normal (0, 0, 0), and their count is 0.
+static int normals_search_begin(apc_ctx* ctx, const float* xyzi, uint32_t n_max, int which, float* out_normals,
+                                uint32_t* out_counts, double* out_cov, double** cov, cudaStream_t s) {
+  APC_REQUIRE(ctx, xyzi && out_normals, "NULL pointer");
+  APC_REQUIRE(ctx, n_max <= ctx->max_points, "more points than the context was created for");
+  int rc = apc_neighbors_prepare(ctx, which);
+  if (rc) return rc;
+  NeighborScratch* sc = scratch_of(ctx);
+  if (!out_cov && !sc->cov) APC_CUDA(ctx, cudaMalloc((void**)&sc->cov, (size_t)ctx->max_points * 9 * sizeof(double)));
+  *cov = out_cov ? out_cov : sc->cov;
+  rc = apc_begin(ctx, s);
+  if (rc) return rc;
+  APC_CUDA(ctx, cudaMemsetAsync(*cov, 0, (size_t)n_max * 9 * sizeof(double), s));
+  APC_CUDA(ctx, cudaMemsetAsync(out_normals, 0, (size_t)n_max * 3 * sizeof(float), s));
+  if (out_counts) APC_CUDA(ctx, cudaMemsetAsync(out_counts, 0, (size_t)n_max * sizeof(uint32_t), s));
+  return APC_OK;
+}
+
+// covariances -> normals, then the grid cleans itself for the next call of any mode
+static int normals_search_finish(apc_ctx* ctx, const GridHost& g, uint32_t n_max, const uint32_t* n_dev, const double* cov,
+                                 float* out_normals, cudaStream_t s) {
+  {
+    APC_PROF(ctx, "k_normals_eigen", s);
+    k_normals_eigen<<<min(apc_div_up(n_max, 256), (uint32_t)APC_SM_COUNT * 8), 256, 0, s>>>(n_max, n_dev, cov, out_normals);
+  }
+  APC_PROF(ctx, "k_grid_clean", s);
+  k_grid_clean<<<dim3(min(apc_div_up(n_max, 256), (uint32_t)APC_SM_COUNT * 4), g.d.levels), 256, 0, s>>>(n_max, n_dev, g.d);
+  APC_LAUNCH_CHECK(ctx, "estimate_normals");
+  return APC_OK;
+}
+
+extern "C" int apc_estimate_normals_knn(apc_ctx* ctx, const float* xyzi, uint32_t n_max, const uint32_t* n_dev, int max_nn,
+                                        float* out_normals, uint32_t* out_neighbor_counts, double* out_covariances,
+                                        void* stream) {
+  if (!ctx) return APC_ERR_BAD_ARG;
+  APC_REQUIRE(ctx, max_nn >= 1 && max_nn <= APC_MAX_NEIGHBORS,
+              "max_nn must be in 1..APC_MAX_NEIGHBORS (" APC_STRINGIFY(APC_MAX_NEIGHBORS) ")");
+  if (n_max == 0) return APC_OK;
+  cudaStream_t s = (cudaStream_t)stream;
+  double* cov = nullptr;
+  int rc = normals_search_begin(ctx, xyzi, n_max, 1, out_normals, out_neighbor_counts, out_covariances, &cov, s);
+  if (rc) return rc;
+  NeighborScratch* sc = scratch_of(ctx);
+  GridHost& g = sc->grid[1];
+  const float4* pts = reinterpret_cast<const float4*>(xyzi);
+  rc = grid_build(ctx, g, pts, n_max, n_dev, 0.0f, true, s);
+  if (rc) return rc;
+  const uint32_t cap = wide_cap((uint32_t)max_nn);
+  const size_t smem = (size_t)KNN_WARPS * cap * sizeof(unsigned long long);
+  const uint32_t bq = min(apc_div_up(n_max, KNN_WARPS), (uint32_t)APC_SM_COUNT * 16);   // one warp per query, grid-stride
+  {
+    APC_PROF(ctx, "k_normals_knn", s);
+    k_normals_knn<<<bq, KNN_WARPS * 32, smem, s>>>(n_max, n_dev, g.d, pts, (uint32_t)max_nn, cap, out_neighbor_counts, cov,
+                                                   sc->stragglers, ctx->ctrl);
+  }
+  {
+    APC_PROF(ctx, "k_normals_knn_stragglers", s);
+    k_normals_knn_stragglers<<<APC_SM_COUNT * 2, KNN_WARPS * 32, smem, s>>>(pts, n_max, n_dev, (uint32_t)max_nn, cap,
+                                                                            sc->stragglers, ctx->ctrl, out_neighbor_counts, cov);
+  }
+  return normals_search_finish(ctx, g, n_max, n_dev, cov, out_normals, s);
+}
+
+extern "C" int apc_estimate_normals_radius(apc_ctx* ctx, const float* xyzi, uint32_t n_max, const uint32_t* n_dev,
+                                           double radius, float* out_normals, uint32_t* out_neighbor_counts,
+                                           double* out_covariances, void* stream) {
+  if (!ctx) return APC_ERR_BAD_ARG;
+  const float r32 = (float)radius;
+  APC_REQUIRE(ctx, radius > 0.0 && r32 > 0.0f && std::isfinite(r32 * r32), "radius must be finite and > 0");
+  if (n_max == 0) return APC_OK;
+  cudaStream_t s = (cudaStream_t)stream;
+  double* cov = nullptr;
+  int rc = normals_search_begin(ctx, xyzi, n_max, 0, out_normals, out_neighbor_counts, out_covariances, &cov, s);
+  if (rc) return rc;
+  GridHost& g = scratch_of(ctx)->grid[0];
+  const float4* pts = reinterpret_cast<const float4*>(xyzi);
+  // the grid of the hybrid search (apc_normals_nobegin): cells of r * (1 + 2^-8), reciprocal indexing
+  rc = grid_build(ctx, g, pts, n_max, n_dev, r32 * 1.00390625f, false, s, false, CTR_CURSOR_NORMALS, true);
+  if (rc) return rc;
+  {
+    APC_PROF(ctx, "k_normals_radius", s);
+    k_normals_radius<<<min(apc_div_up(n_max, 4), (uint32_t)APC_SM_COUNT * 16), 128, 0, s>>>(n_max, n_dev, g.d, r32, r32 * r32,
+                                                                                        out_neighbor_counts, cov, ctx->ctrl);
+  }
+  return normals_search_finish(ctx, g, n_max, n_dev, cov, out_normals, s);
 }

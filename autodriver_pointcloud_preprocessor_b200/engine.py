@@ -306,6 +306,24 @@ class Context:
                                           _ptr(normals), _ptr(counts), _ptr(cov), _stream()))
         return normals[:n], (counts[:n] if counts is not None else None), (cov[:n] if cov is not None else None)
 
+    def estimate_normals_knn(self, xyzi, max_nn, want_counts=False, want_cov=False, n_dev=None):
+        """KNN search (``apc_estimate_normals_knn``): the ``max_nn`` nearest points, no distance bound.
+        Returns the same tuple as :meth:`estimate_normals`."""
+        return self._normals_search(lib.apc_estimate_normals_knn, xyzi, int(max_nn), want_counts, want_cov, n_dev)
+
+    def estimate_normals_radius(self, xyzi, radius, want_counts=False, want_cov=False, n_dev=None):
+        """Radius search (``apc_estimate_normals_radius``): every point within ``radius``, no cap on the count.
+        Returns the same tuple as :meth:`estimate_normals`."""
+        return self._normals_search(lib.apc_estimate_normals_radius, xyzi, float(radius), want_counts, want_cov, n_dev)
+
+    def _normals_search(self, fn, xyzi, bound, want_counts, want_cov, n_dev):
+        n = xyzi.shape[0]
+        normals = self._empty((max(n, 1), 3), torch.float32)
+        counts = self._empty((max(n, 1),), torch.int32) if want_counts else None
+        cov = self._empty((max(n, 1), 3, 3), torch.float64) if want_cov else None
+        self._ok(fn(self.h, _ptr(xyzi), n, _ptr(n_dev), bound, _ptr(normals), _ptr(counts), _ptr(cov), _stream()))
+        return normals[:n], (counts[:n] if counts is not None else None), (cov[:n] if cov is not None else None)
+
     # ---- ransac ------------------------------------------------------------------------------------
     def segment_plane(self, xyzi, distance_threshold, ransac_n, num_iterations, probability, seed=0,
                       sample_table=None, n_dev=None):

@@ -247,17 +247,28 @@ class PointCloud:
         raise NotImplementedError("legacy Open3D geometry (visualisation) is outside the CUDA hot path")
 
     def estimate_normals(self, max_nn=30, radius=None):   # pp.py:523
-        """Open3D ``estimate_normals``: hybrid search (``max_nn`` nearest within ``radius``) ->
-        covariance -> eigenvector of the smallest eigenvalue; sets ``point['normals']`` (float32
-        N x 3), not oriented.  ``max_nn`` in 1..``APC_MAX_NEIGHBORS`` (1024; beyond it the call raises
-        ``ApcError``).  Both arguments are required here (the reference passes both, pp.py:523-526);
-        pure-KNN / pure-radius searches are not implemented."""
-        if radius is None or max_nn is None:
-            raise NotImplementedError("estimate_normals needs both radius and max_nn (hybrid search, pp.py:523-526)")
+        """Open3D ``estimate_normals``: neighbourhood search -> covariance -> eigenvector of the
+        smallest eigenvalue; sets ``point['normals']`` (float32 N x 3), not oriented.  The search
+        follows the arguments, as in Open3D:
+
+        * both given (the reference's call, pp.py:523-526): hybrid, the ``max_nn`` nearest within ``radius``;
+        * ``max_nn`` only (the default call ``estimate_normals()``): KNN, the ``max_nn`` nearest;
+        * ``radius`` only (``max_nn=None``): every point within ``radius``, no cap on the count;
+        * neither: ``ValueError``.
+
+        ``max_nn`` in 1..``APC_MAX_NEIGHBORS`` (1024) and ``radius`` finite and > 0; otherwise the call
+        raises ``ApcError``."""
+        if radius is None and max_nn is None:
+            raise ValueError("estimate_normals needs max_nn, radius or both")
         if self._n() == 0:
             self.point["normals"] = self._home(torch.zeros((0, 3), dtype=torch.float32, device="cuda"))
             return self
-        normals, _, _ = self._ctx().estimate_normals(self._xyzi(), int(max_nn), float(radius))
+        if radius is None:
+            normals, _, _ = self._ctx().estimate_normals_knn(self._xyzi(), int(max_nn))
+        elif max_nn is None:
+            normals, _, _ = self._ctx().estimate_normals_radius(self._xyzi(), float(radius))
+        else:
+            normals, _, _ = self._ctx().estimate_normals(self._xyzi(), int(max_nn), float(radius))
         self.point["normals"] = self._home(normals.contiguous())
         return self
 

@@ -261,6 +261,21 @@ int apc_estimate_normals(apc_ctx* ctx, const float* xyzi, uint32_t n_max, const 
                          int max_nn, double radius, float* out_normals,
                          uint32_t* out_neighbor_counts, double* out_covariances, void* stream);
 
+/* estimate_normals(max_nn) (Open3D KNN search): the same, with the neighbourhood = the min(max_nn, n) points
+ * first in the order (d2, index), query included, no distance bound; max_nn in 1..APC_MAX_NEIGHBORS
+ * (APC_ERR_BAD_ARG beyond).  Points the grid cannot key get the normal (0, 0, 0) and the count 0. */
+int apc_estimate_normals_knn(apc_ctx* ctx, const float* xyzi, uint32_t n_max, const uint32_t* n_dev,
+                             int max_nn, float* out_normals, uint32_t* out_neighbor_counts,
+                             double* out_covariances, void* stream);
+
+/* estimate_normals(radius) (Open3D radius search): the same, with the neighbourhood = every point with
+ * d2 <= float32(radius)^2, query included, no cap on the count; radius finite and > 0 (APC_ERR_BAD_ARG
+ * otherwise).  Moments are accumulated in 64-bit fixed point (2^-40 r): the covariances and normals are
+ * bit-identical across runs and input orders, within 1e-11 r^2 of the float64 covariance. */
+int apc_estimate_normals_radius(apc_ctx* ctx, const float* xyzi, uint32_t n_max, const uint32_t* n_dev,
+                                double radius, float* out_normals, uint32_t* out_neighbor_counts,
+                                double* out_covariances, void* stream);
+
 /* ---- (4) RANSAC ground plane --------------------------------------------------------- */
 
 /* segment_plane(distance_threshold, ransac_n, num_iterations, probability) (pp.py:533-543).
