@@ -103,6 +103,7 @@ def _load():
         "apc_estimate_normals": [vp, vp, u32, vp, i32, f64, vp, vp, vp, vp],
         "apc_estimate_normals_knn": [vp, vp, u32, vp, i32, vp, vp, vp, vp],
         "apc_estimate_normals_radius": [vp, vp, u32, vp, f64, vp, vp, vp, vp],
+        "apc_cluster_dbscan": [vp, vp, u32, vp, f64, i32, vp, vp, vp, vp],
         "apc_segment_plane": [vp, vp, u32, vp, f64, i32, i32, f64, C.c_uint64, vp, vp, vp, vp, vp],
         "apc_segment_plane_scores": [vp, vp, u32, vp],
         "apc_repack": [vp, vp, u32, vp, C.POINTER(OutField), u32, u32, vp, vp],
@@ -144,7 +145,7 @@ SYMBOLS = ["apc_ctx_create", "apc_ctx_destroy", "apc_ctx_set_low_latency", "apc_
            "apc_non_finite_mask", "apc_duplicate_mask", "apc_unique_rows", "apc_select_by_mask", "apc_gather",
            "apc_voxel_downsample", "apc_voxel_downsample_sorted", "apc_voxel_mean_attr", "apc_radius_outliers",
            "apc_statistical_outliers", "apc_estimate_normals", "apc_estimate_normals_knn",
-           "apc_estimate_normals_radius", "apc_segment_plane", "apc_segment_plane_scores", "apc_repack", "apc_pipeline_run", "apc_pipeline_run_maps",
+           "apc_estimate_normals_radius", "apc_cluster_dbscan", "apc_segment_plane", "apc_segment_plane_scores", "apc_repack", "apc_pipeline_run", "apc_pipeline_run_maps",
            "apc_pipeline_run_mirrored", "apc_pipeline_run_ex", "apc_graph_capture_pipeline_ex",
            "apc_graph_capture_pipeline", "apc_graph_capture_pipeline_mirrored",
            "apc_graph_launch", "apc_graph_destroy",

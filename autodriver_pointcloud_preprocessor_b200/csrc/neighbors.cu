@@ -1303,6 +1303,9 @@ struct NeighborScratch {
   uint32_t* stragglers = nullptr;
   double* stats = nullptr;
   double* cov = nullptr;            // [max_points][9] covariances between k_normals_cov and k_normals_eigen
+  uint32_t* dbscan_parent = nullptr;   // [max_points] union-find forest of apc_cluster_dbscan's core points
+  uint32_t* dbscan_id = nullptr;       // [max_points] cluster id of every root
+  uint8_t* dbscan_core = nullptr;      // [max_points] core flags
 };
 // one scratch set per context, owned by the context (created on first use, freed by apc_ctx_destroy)
 static NeighborScratch* scratch_of(apc_ctx* ctx) {
@@ -1321,6 +1324,9 @@ void apc_neighbors_release(apc_ctx* ctx) {
   if (s->stragglers) cudaFree(s->stragglers);
   if (s->stats) cudaFree(s->stats);
   if (s->cov) cudaFree(s->cov);
+  void* dbscan[] = {s->dbscan_parent, s->dbscan_id, s->dbscan_core};
+  for (void* p : dbscan)
+    if (p) cudaFree(p);
   delete s;
   ctx->neighbors = nullptr;
 }
@@ -2334,4 +2340,260 @@ extern "C" int apc_estimate_normals_radius(apc_ctx* ctx, const float* xyzi, uint
                                                                                         out_neighbor_counts, cov, ctx->ctrl);
   }
   return normals_search_finish(ctx, g, n_max, n_dev, cov, out_normals, s);
+}
+
+// ---- cluster_dbscan(eps, min_points) (Open3D PointCloud::ClusterDBSCAN) ----------------------------------------
+// Contract (oracle/dbscan.py): N(i) = {j : d2 <= float32(eps)^2}, i included; core iff |N(i)| >= min_points;
+// clusters = connected components of the core points linked by N; ids 0, 1, ... in the order of each component's
+// lowest core index; a core point gets its component's id, a non-core point the smallest id among the components
+// of the core points in N(i), else -1.
+//   k_dbscan_core    |N(i)| (stops at min_points when the counts are not wanted) -> core flag, parent[i] = i
+//   k_dbscan_union   every core point unions itself with its lower-indexed core neighbours
+//   k_dbscan_roots   points every core point at its root, ranks the roots in index order -> ids, n_clusters
+//   k_dbscan_label   core: id[root]; non-core: id of the lowest root among its core neighbours, or -1
+// The union-find is lock-free over original indices: a union always hooks the larger root under the smaller one
+// (atomicCAS on the root's own entry), so every tree's root is its minimum index whatever the thread schedule,
+// and the output does not depend on the order the grid's atomics leave inside a cell.  Finds halve paths with
+// relaxed stores: every value stored is an ancestor, so the trees stay the same whichever store lands last.
+// Points the grid cannot key (APC_ERR_KEY_RANGE) are never in the cell-sorted array: they are in no one's N,
+// stay non-core and keep the label -1.
+
+// The 27 cells around q as one flat candidate list, for a warp that walks it 32 records at a time: lane l < 27
+// resolves cell l and keeps its run's start in the cell-sorted array (cs) and the flat index of the run's first
+// record (ps); returns the list's length (all lanes).  This is k_normals_radius's walk; that kernel keeps its inline
+// copy because calling these helpers changes its instruction schedule.
+__device__ __forceinline__ uint32_t flat27_runs(const GridDev& g, float c, float4 q, uint32_t lane, uint32_t& cs, uint32_t& ps) {
+  int32_t ix, iy, iz;
+  grid_coord_g(g, c, q.x, q.y, q.z, ix, iy, iz);  // succeeded at insert time
+  uint32_t s0 = 0, cf = 0;
+  if (lane < 27) {
+    const int dx = (int)(lane % 3u) - 1, dy = (int)((lane / 3u) % 3u) - 1, dz = (int)(lane / 9u) - 1;
+    uint32_t b, f;
+    if (grid_lookup(g, grid_key(0, ix + dx, iy + dy, iz + dz), b, f)) { s0 = b; cf = f; }
+  }
+  uint32_t incl = cf;
+#pragma unroll
+  for (int o = 1; o < 32; o <<= 1) {
+    const uint32_t v = __shfl_up_sync(0xffffffffu, incl, o);
+    if (lane >= (uint32_t)o) incl += v;
+  }
+  cs = s0;
+  ps = incl - cf;
+  return __shfl_sync(0xffffffffu, incl, 31);
+}
+// Position in g.sorted of record `flat` of that list (called by all lanes of the warp).
+__device__ __forceinline__ uint32_t flat27_at(uint32_t cs, uint32_t ps, uint32_t flat) {
+  uint32_t run = 0;                                  // largest cell with ps <= flat
+#pragma unroll
+  for (int step = 16; step > 0; step >>= 1) {
+    const uint32_t mid = run + step;
+    const uint32_t v = __shfl_sync(0xffffffffu, ps, mid & 31u);
+    if (mid < 27u && v <= flat) run = mid;
+  }
+  const uint32_t rs = __shfl_sync(0xffffffffu, cs, run), rp = __shfl_sync(0xffffffffu, ps, run);
+  return rs + (flat - rp);
+}
+
+__device__ __forceinline__ uint32_t ld_relaxed_u32(const uint32_t* p) {
+  uint32_t v;
+  asm volatile("ld.relaxed.gpu.global.u32 %0, [%1];" : "=r"(v) : "l"(p) : "memory");
+  return v;
+}
+__device__ __forceinline__ void st_relaxed_u32(uint32_t* p, uint32_t v) {
+  asm volatile("st.relaxed.gpu.global.u32 [%0], %1;" ::"l"(p), "r"(v) : "memory");
+}
+__device__ __forceinline__ uint32_t uf_find(uint32_t* parent, uint32_t x) {
+  uint32_t p = ld_relaxed_u32(&parent[x]);
+  while (p != x) {
+    const uint32_t gp = ld_relaxed_u32(&parent[p]);
+    if (gp == p) return p;
+    st_relaxed_u32(&parent[x], gp);                  // path halving
+    x = gp;
+    p = ld_relaxed_u32(&parent[x]);
+  }
+  return x;
+}
+__device__ __forceinline__ void uf_union(uint32_t* parent, uint32_t a, uint32_t b) {
+  a = uf_find(parent, a);
+  b = uf_find(parent, b);
+  while (a != b) {
+    if (a > b) { const uint32_t t = a; a = b; b = t; }
+    const uint32_t old = atomicCAS(&parent[b], b, a);   // hook the larger root under the smaller
+    if (old == b) return;
+    b = uf_find(parent, old);                            // b was hooked meanwhile: go on from its new root
+    a = uf_find(parent, a);
+  }
+}
+
+__global__ void __launch_bounds__(128)
+k_dbscan_core(uint32_t n_max, const uint32_t* n_dev, GridDev g, float r2, uint32_t min_points, uint32_t* __restrict__ counts,
+              uint8_t* __restrict__ core, uint32_t* __restrict__ parent, const ApcCtrl* __restrict__ ctrl) {
+  const uint32_t n = grid_sorted_count(g, ctrl, apc_count(n_dev, n_max));
+  const float c = grid_cell_size(g, 0);
+  const uint32_t lane = threadIdx.x & 31u;
+  for (uint32_t j = (blockIdx.x * blockDim.x + threadIdx.x) >> 5; j < n; j += (gridDim.x * blockDim.x) >> 5) {
+    const float4 q = g.sorted[j];
+    const uint32_t orig = __float_as_uint(q.w);
+    uint32_t cs, ps;
+    const uint32_t total = flat27_runs(g, c, q, lane, cs, ps);
+    uint32_t cnt = 0;
+    for (uint32_t base = 0; base < total && (counts || cnt < min_points); base += 32) {
+      const uint32_t ci = base + lane;
+      const uint32_t at = flat27_at(cs, ps, min(ci, total - 1u));
+      bool inside = false;
+      if (ci < total) {
+        const float4 p = g.sorted[at];
+        inside = d2_f32(q.x, q.y, q.z, p.x, p.y, p.z) <= r2;
+      }
+      cnt += __popc(__ballot_sync(0xffffffffu, inside));
+    }
+    if (lane == 0) {
+      core[orig] = cnt >= min_points ? 1 : 0;
+      parent[orig] = orig;
+      if (counts) counts[orig] = cnt;
+    }
+  }
+}
+
+__global__ void __launch_bounds__(128)
+k_dbscan_union(uint32_t n_max, const uint32_t* n_dev, GridDev g, float r2, const uint8_t* __restrict__ core,
+               uint32_t* parent, const ApcCtrl* __restrict__ ctrl) {
+  const uint32_t n = grid_sorted_count(g, ctrl, apc_count(n_dev, n_max));
+  const float c = grid_cell_size(g, 0);
+  const uint32_t lane = threadIdx.x & 31u;
+  for (uint32_t j = (blockIdx.x * blockDim.x + threadIdx.x) >> 5; j < n; j += (gridDim.x * blockDim.x) >> 5) {
+    const float4 q = g.sorted[j];
+    const uint32_t orig = __float_as_uint(q.w);
+    if (!core[orig]) continue;                               // warp-uniform
+    uint32_t cs, ps;
+    const uint32_t total = flat27_runs(g, c, q, lane, cs, ps);
+    for (uint32_t base = 0; base < total; base += 32) {
+      const uint32_t ci = base + lane;
+      const uint32_t at = flat27_at(cs, ps, min(ci, total - 1u));
+      if (ci < total) {
+        const float4 p = g.sorted[at];
+        const uint32_t o = __float_as_uint(p.w);
+        // each edge once, from its higher end (the predicate is symmetric)
+        if (o < orig && d2_f32(q.x, q.y, q.z, p.x, p.y, p.z) <= r2 && core[o]) uf_union(parent, orig, o);
+      }
+    }
+  }
+}
+
+// One tile of 1024 points in index order: roots flagged, ranked by the look-back scan of apc_scan.cuh.
+__global__ void __launch_bounds__(APC_TILE_THREADS)
+k_dbscan_roots(uint32_t n_max, const uint32_t* n_dev, const uint8_t* __restrict__ core, uint32_t* parent,
+               uint32_t* __restrict__ id, uint32_t* out_count, uint64_t* scan_state, const ApcCtrl* ctrl, uint32_t n_tiles) {
+  __shared__ uint32_t sm_scan[34];
+  const uint32_t n = apc_count(n_dev, n_max);
+  const uint32_t tile = blockIdx.x;
+  bool root[APC_TILE_ITEMS];
+#pragma unroll
+  for (int k = 0; k < APC_TILE_ITEMS; ++k) {
+    const uint32_t i = tile * APC_TILE_POINTS + k * APC_TILE_THREADS + threadIdx.x;
+    root[k] = false;
+    if (i < n && core[i]) {
+      uint32_t r = i, p = ld_relaxed_u32(&parent[i]);
+      while (p != r) {                                      // no halving here: the only store is parent[i] = root
+        r = p;
+        p = ld_relaxed_u32(&parent[r]);
+      }
+      st_relaxed_u32(&parent[i], r);
+      root[k] = r == i;
+    }
+  }
+  uint32_t rank[APC_TILE_ITEMS];
+  const uint32_t base = tile_compact_offsets(root, rank, sm_scan, scan_state, tile, ctrl->epoch, out_count, n_tiles);
+#pragma unroll
+  for (int k = 0; k < APC_TILE_ITEMS; ++k)
+    if (root[k]) id[tile * APC_TILE_POINTS + k * APC_TILE_THREADS + threadIdx.x] = base + rank[k];
+}
+
+__global__ void __launch_bounds__(128)
+k_dbscan_label(uint32_t n_max, const uint32_t* n_dev, GridDev g, float r2, const uint8_t* __restrict__ core,
+               const uint32_t* __restrict__ parent, const uint32_t* __restrict__ id, int32_t* __restrict__ labels,
+               const ApcCtrl* __restrict__ ctrl) {
+  const uint32_t n = grid_sorted_count(g, ctrl, apc_count(n_dev, n_max));
+  const float c = grid_cell_size(g, 0);
+  const uint32_t lane = threadIdx.x & 31u;
+  for (uint32_t j = (blockIdx.x * blockDim.x + threadIdx.x) >> 5; j < n; j += (gridDim.x * blockDim.x) >> 5) {
+    const float4 q = g.sorted[j];
+    const uint32_t orig = __float_as_uint(q.w);
+    if (core[orig]) {                                       // warp-uniform
+      if (lane == 0) labels[orig] = (int32_t)id[parent[orig]];
+      continue;
+    }
+    uint32_t cs, ps;
+    const uint32_t total = flat27_runs(g, c, q, lane, cs, ps);
+    uint32_t low = 0xffffffffu;                             // lowest root among the core neighbours
+    for (uint32_t base = 0; base < total; base += 32) {
+      const uint32_t ci = base + lane;
+      const uint32_t at = flat27_at(cs, ps, min(ci, total - 1u));
+      if (ci < total) {
+        const float4 p = g.sorted[at];
+        const uint32_t o = __float_as_uint(p.w);
+        if (d2_f32(q.x, q.y, q.z, p.x, p.y, p.z) <= r2 && core[o]) low = min(low, parent[o]);
+      }
+    }
+    low = __reduce_min_sync(0xffffffffu, low);
+    if (lane == 0) labels[orig] = low == 0xffffffffu ? -1 : (int32_t)id[low];
+  }
+}
+
+extern "C" int apc_cluster_dbscan(apc_ctx* ctx, const float* xyzi, uint32_t n_max, const uint32_t* n_dev, double eps,
+                                  int min_points, int32_t* out_labels, uint32_t* out_cluster_count_dev,
+                                  uint32_t* out_neighbor_counts, void* stream) {
+  if (!ctx) return APC_ERR_BAD_ARG;
+  const float r32 = (float)eps;
+  APC_REQUIRE(ctx, eps > 0.0 && r32 > 0.0f && std::isfinite(r32 * r32), "eps must be finite and > 0");
+  APC_REQUIRE(ctx, min_points >= 0, "min_points must be >= 0");
+  if (n_max == 0) return APC_OK;
+  APC_REQUIRE(ctx, xyzi && out_labels, "NULL pointer");
+  APC_REQUIRE(ctx, n_max <= ctx->max_points, "more points than the context was created for");
+  const uint32_t n_tiles = apc_div_up(n_max, APC_TILE_POINTS);
+  APC_REQUIRE(ctx, n_tiles <= ctx->max_tiles, "more points than the context was created for");
+  // everything is allocated before the first launch
+  int rc = apc_neighbors_prepare(ctx, 0);
+  if (rc) return rc;
+  NeighborScratch* sc = scratch_of(ctx);
+  const size_t M = ctx->max_points;
+  if (!sc->dbscan_parent) APC_CUDA(ctx, cudaMalloc((void**)&sc->dbscan_parent, M * sizeof(uint32_t)));
+  if (!sc->dbscan_id) APC_CUDA(ctx, cudaMalloc((void**)&sc->dbscan_id, M * sizeof(uint32_t)));
+  if (!sc->dbscan_core) APC_CUDA(ctx, cudaMalloc((void**)&sc->dbscan_core, M));
+  cudaStream_t s = (cudaStream_t)stream;
+  rc = apc_begin(ctx, s);
+  if (rc) return rc;
+  APC_CUDA(ctx, cudaMemsetAsync(out_labels, 0xff, (size_t)n_max * sizeof(int32_t), s));
+  APC_CUDA(ctx, cudaMemsetAsync(sc->dbscan_core, 0, n_max, s));
+  if (out_neighbor_counts) APC_CUDA(ctx, cudaMemsetAsync(out_neighbor_counts, 0, (size_t)n_max * sizeof(uint32_t), s));
+  GridHost& g = sc->grid[0];
+  const float4* pts = reinterpret_cast<const float4*>(xyzi);
+  const float r2 = r32 * r32;
+  // the grid of the normals radius search (apc_estimate_normals_radius): cells of eps * (1 + 2^-8), reciprocal indexing
+  rc = grid_build(ctx, g, pts, n_max, n_dev, r32 * 1.00390625f, false, s, false, CTR_CURSOR_NORMALS, true);
+  if (rc) return rc;
+  const uint32_t bq = min(apc_div_up(n_max, 4), (uint32_t)APC_SM_COUNT * 16);   // one warp per query, grid-stride
+  {
+    APC_PROF(ctx, "k_dbscan_core", s);
+    k_dbscan_core<<<bq, 128, 0, s>>>(n_max, n_dev, g.d, r2, (uint32_t)min_points, out_neighbor_counts, sc->dbscan_core,
+                                     sc->dbscan_parent, ctx->ctrl);
+  }
+  {
+    APC_PROF(ctx, "k_dbscan_union", s);
+    k_dbscan_union<<<bq, 128, 0, s>>>(n_max, n_dev, g.d, r2, sc->dbscan_core, sc->dbscan_parent, ctx->ctrl);
+  }
+  {
+    APC_PROF(ctx, "k_dbscan_roots", s);
+    k_dbscan_roots<<<n_tiles, APC_TILE_THREADS, 0, s>>>(n_max, n_dev, sc->dbscan_core, sc->dbscan_parent, sc->dbscan_id,
+                                                        out_cluster_count_dev, ctx->scan_state[0], ctx->ctrl, n_tiles);
+  }
+  {
+    APC_PROF(ctx, "k_dbscan_label", s);
+    k_dbscan_label<<<bq, 128, 0, s>>>(n_max, n_dev, g.d, r2, sc->dbscan_core, sc->dbscan_parent, sc->dbscan_id,
+                                      out_labels, ctx->ctrl);
+  }
+  APC_PROF(ctx, "k_grid_clean", s);
+  k_grid_clean<<<dim3(min(apc_div_up(n_max, 256), (uint32_t)APC_SM_COUNT * 4), 1), 256, 0, s>>>(n_max, n_dev, g.d);
+  APC_LAUNCH_CHECK(ctx, "cluster_dbscan");
+  return APC_OK;
 }

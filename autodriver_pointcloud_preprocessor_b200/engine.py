@@ -324,6 +324,18 @@ class Context:
         self._ok(fn(self.h, _ptr(xyzi), n, _ptr(n_dev), bound, _ptr(normals), _ptr(counts), _ptr(cov), _stream()))
         return normals[:n], (counts[:n] if counts is not None else None), (cov[:n] if cov is not None else None)
 
+    # ---- clustering ----------------------------------------------------------------------------------
+    def cluster_dbscan(self, xyzi, eps, min_points, want_counts=False, n_dev=None):
+        """DBSCAN (``apc_cluster_dbscan``).  Returns ``(labels int32[n], n_clusters int32[1] (device),
+        counts int32[n] | None)``; label -1 = noise."""
+        n = xyzi.shape[0]
+        labels = self._empty((max(n, 1),), torch.int32)
+        n_clusters = torch.zeros((1,), dtype=torch.int32, device=self.device)
+        counts = self._empty((max(n, 1),), torch.int32) if want_counts else None
+        self._ok(lib.apc_cluster_dbscan(self.h, _ptr(xyzi), n, _ptr(n_dev), float(eps), int(min_points), _ptr(labels),
+                                        _ptr(n_clusters), _ptr(counts), _stream()))
+        return labels[:n], n_clusters, (counts[:n] if counts is not None else None)
+
     # ---- ransac ------------------------------------------------------------------------------------
     def segment_plane(self, xyzi, distance_threshold, ransac_n, num_iterations, probability, seed=0,
                       sample_table=None, n_dev=None):

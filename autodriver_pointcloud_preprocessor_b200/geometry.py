@@ -13,6 +13,8 @@ stages them through the GPU for each operation; there is no CPU implementation.
 """
 from __future__ import annotations
 
+import math
+
 import numpy as np
 import torch
 
@@ -426,6 +428,24 @@ class PointCloud:
         mask, _ = ctx.radius_outliers(self._xyzi(), nb_points, search_radius)
         ctx.check()
         return self.select_by_mask(Tensor(mask)), self._home(mask.to(torch.bool))
+
+    # -- clustering
+    def cluster_dbscan(self, eps, min_points, print_progress=False):
+        """Open3D ``cluster_dbscan``: int32 label of every point (``Tensor`` [N] on the cloud's device), -1 for
+        noise.  Neighbours are the points within ``eps`` (self included, the float32 distance of
+        ``remove_radius_outliers``); a point with at least ``min_points`` neighbours is a core point; clusters are
+        the connected components of the core points, numbered in the order of their lowest point index; a
+        non-core point joins the lowest-numbered cluster among its core neighbours.  ``print_progress`` is
+        accepted and ignored."""
+        if not (math.isfinite(eps) and eps > 0) or min_points < 0:
+            raise ValueError("Illegal input parameters, eps must be positive and finite and min_points >= 0")
+        n = self._n()
+        if n == 0:
+            return self._home(torch.zeros((0,), dtype=torch.int32, device="cuda"))
+        ctx = self._ctx()
+        labels, _, _ = ctx.cluster_dbscan(self._xyzi(), float(eps), min(int(min_points), n + 1))
+        ctx.check()
+        return self._home(labels.contiguous())
 
     # -- RANSAC plane (pp.py:535)
     def segment_plane(self, distance_threshold=0.01, ransac_n=3, num_iterations=100, probability=0.99999999,

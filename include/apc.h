@@ -276,6 +276,18 @@ int apc_estimate_normals_radius(apc_ctx* ctx, const float* xyzi, uint32_t n_max,
                                 double radius, float* out_normals, uint32_t* out_neighbor_counts,
                                 double* out_covariances, void* stream);
 
+/* cluster_dbscan(eps, min_points) (Open3D PointCloud::ClusterDBSCAN): N(i) = every point with
+ * d2 <= float32(eps)^2, i included; i is core iff |N(i)| >= min_points; clusters are the connected components of
+ * the core points linked by N, numbered 0, 1, ... in the order of each component's lowest core index.
+ * out_labels int32[n_max]: a core point's cluster; a non-core point's smallest cluster among the core points in
+ * N(i); else -1 (noise).  out_cluster_count_dev uint32[1] (device, may be NULL): the number of clusters.
+ * out_neighbor_counts uint32[n_max] (may be NULL): |N(i)|.  eps finite and > 0 with float32(eps)^2 finite,
+ * min_points >= 0 (APC_ERR_BAD_ARG otherwise); no cap on |N(i)|.  The labels do not depend on the thread
+ * schedule.  Points the grid cannot key get -1 and are in no N(i).  No host synchronisation. */
+int apc_cluster_dbscan(apc_ctx* ctx, const float* xyzi, uint32_t n_max, const uint32_t* n_dev,
+                       double eps, int min_points, int32_t* out_labels,
+                       uint32_t* out_cluster_count_dev, uint32_t* out_neighbor_counts, void* stream);
+
 /* ---- (4) RANSAC ground plane --------------------------------------------------------- */
 
 /* segment_plane(distance_threshold, ransac_n, num_iterations, probability) (pp.py:533-543).
