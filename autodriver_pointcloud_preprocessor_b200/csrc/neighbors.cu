@@ -1306,6 +1306,8 @@ struct NeighborScratch {
   uint32_t* dbscan_parent = nullptr;   // [max_points] union-find forest of apc_cluster_dbscan's core points
   uint32_t* dbscan_id = nullptr;       // [max_points] cluster id of every root
   uint8_t* dbscan_core = nullptr;      // [max_points] core flags
+  double* icp_part = nullptr;          // [ICP_MAX_BLOCKS][32] block partials of k_icp_match's moments
+  struct IcpState* icp_state = nullptr;   // apc_icp's T, previous metrics and done flag
 };
 // one scratch set per context, owned by the context (created on first use, freed by apc_ctx_destroy)
 static NeighborScratch* scratch_of(apc_ctx* ctx) {
@@ -1326,6 +1328,9 @@ void apc_neighbors_release(apc_ctx* ctx) {
   if (s->cov) cudaFree(s->cov);
   void* dbscan[] = {s->dbscan_parent, s->dbscan_id, s->dbscan_core};
   for (void* p : dbscan)
+    if (p) cudaFree(p);
+  void* icp[] = {s->icp_part, s->icp_state};
+  for (void* p : icp)
     if (p) cudaFree(p);
   delete s;
   ctx->neighbors = nullptr;
@@ -2596,4 +2601,423 @@ extern "C" int apc_cluster_dbscan(apc_ctx* ctx, const float* xyzi, uint32_t n_ma
   k_grid_clean<<<dim3(min(apc_div_up(n_max, 256), (uint32_t)APC_SM_COUNT * 4), 1), 256, 0, s>>>(n_max, n_dev, g.d);
   APC_LAUNCH_CHECK(ctx, "cluster_dbscan");
   return APC_OK;
+}
+
+// ---- ICP registration (Open3D t::pipelines::registration::ICP / EvaluateRegistration) -------------------------
+// Contract (oracle/registration.py): s' = float32(T s) with every coordinate ((T[r,0]*x + T[r,1]*y) + T[r,2]*z)
+// + T[r,3] in float64, unfused, from the ORIGINAL source; the correspondence of s' is the target point with the
+// smallest (d2, index) among those with d2_f32 <= float32(r)^2, else -1.
+//   k_icp_init    T = init (a kernel argument), zero metrics, clears the done flag
+//   k_icp_match   one warp per source point in index order, grid-stride: transform, 27-cell walk over the target's
+//                 grid (the grid of apc_cluster_dbscan, cells of r * (1 + 2^-8)), 64-bit (d2 bits, index) warp
+//                 minimum -> correspondence; lane k accumulates moment k of the estimation in float64 over the
+//                 warp's queries, and the block writes one row of 32 partials
+//   k_icp_solve   one block: the partials reduced in a fixed order -> fitness, rmse, the convergence test, the
+//                 update (Horn's quaternion for point-to-point, Cholesky for point-to-plane) and T = update T
+// apc_icp launches max_iteration (match, solve) pairs up front; both kernels return at once when the loop has
+// stopped (done flag), so the call needs no host synchronisation.  The launch configuration depends on n_max
+// only, and every sum has a fixed order: results are bit-identical from run to run.
+#define ICP_MAX_BLOCKS (APC_SM_COUNT * 16)
+#define ICP_PIVOT_REL 1e-12     // Cholesky pivot floor relative to its diagonal entry (oracle PIVOT_REL)
+
+struct IcpState {
+  double T[16];
+  double prev_f, prev_r;
+  uint32_t done;
+  uint32_t iterations;
+};
+struct IcpT16 {
+  double v[16];
+};
+
+// Lane k accumulates v[a] * v[b] with (a, b) = c_icp_pairs[method][k] (a | b << 4).  v[0..6] depend on the method,
+// v[7] = 1, v[8] = d2, v[9] = 0.  Lanes 0 and 1 are n_corr and sum d2 for both methods.
+//   point-to-point: v = (s', t); sum s' (2-4), sum t (5-7), sum s'_i t_j (8-16)
+//   point-to-plane: v = (J = [s' x n, n], r = (s' - t) . n); J^T J upper triangle (2-22), J^T r (23-28)
+__constant__ uint8_t c_icp_pairs[2][32] = {
+    {0x77, 0x78, 0x70, 0x71, 0x72, 0x73, 0x74, 0x75, 0x30, 0x40, 0x50, 0x31, 0x41, 0x51, 0x32, 0x42,
+     0x52, 0x99, 0x99, 0x99, 0x99, 0x99, 0x99, 0x99, 0x99, 0x99, 0x99, 0x99, 0x99, 0x99, 0x99, 0x99},
+    {0x77, 0x78, 0x00, 0x10, 0x20, 0x30, 0x40, 0x50, 0x11, 0x21, 0x31, 0x41, 0x51, 0x22, 0x32, 0x42,
+     0x52, 0x33, 0x43, 0x53, 0x44, 0x54, 0x55, 0x60, 0x61, 0x62, 0x63, 0x64, 0x65, 0x99, 0x99, 0x99}};
+
+__device__ __forceinline__ double icp_pick(const double (&v)[10], uint32_t a) {
+  double x = v[0];
+#pragma unroll
+  for (uint32_t k = 1; k < 10; ++k) x = a == k ? v[k] : x;
+  return x;
+}
+__device__ __forceinline__ float icp_row(const double (&T)[12], int r, double x, double y, double z) {
+  return __double2float_rn(__dadd_rn(__dadd_rn(__dadd_rn(__dmul_rn(T[4 * r], x), __dmul_rn(T[4 * r + 1], y)),
+                                               __dmul_rn(T[4 * r + 2], z)), T[4 * r + 3]));
+}
+// flat27_runs for a query that was not inserted into the grid: a point whose cell cannot be keyed (beyond the
+// key range or not finite) has an empty list.  Warp-uniform.
+__device__ __forceinline__ uint32_t flat27_runs_outside(const GridDev& g, float c, float4 q, uint32_t lane, uint32_t& cs,
+                                                        uint32_t& ps) {
+  int32_t ix, iy, iz;
+  cs = ps = 0;
+  if (!grid_coord_g(g, c, q.x, q.y, q.z, ix, iy, iz)) return 0;
+  return flat27_runs(g, c, q, lane, cs, ps);
+}
+// warp minimum of a 64-bit key: high words, then the low words of the lanes that hold the high minimum
+__device__ __forceinline__ uint64_t warp_min_u64(uint64_t k) {
+  const uint32_t hi = __reduce_min_sync(0xffffffffu, (uint32_t)(k >> 32));
+  const uint32_t lo = __reduce_min_sync(0xffffffffu, (uint32_t)(k >> 32) == hi ? (uint32_t)k : 0xffffffffu);
+  return ((uint64_t)hi << 32) | lo;
+}
+
+__global__ void k_icp_init(IcpT16 init, IcpState* __restrict__ st, double* __restrict__ out_T, double* __restrict__ out_stats,
+                           int32_t* __restrict__ out_info, int32_t status) {
+#pragma unroll
+  for (int k = 0; k < 16; ++k) {
+    st->T[k] = init.v[k];
+    if (out_T) out_T[k] = init.v[k];
+  }
+  st->prev_f = st->prev_r = 0.0;
+  st->done = status != APC_ICP_OK;
+  st->iterations = 0;
+  out_stats[0] = out_stats[1] = 0.0;
+  if (out_info) {
+    out_info[0] = out_info[1] = out_info[3] = 0;
+    out_info[2] = status;
+  }
+}
+
+__global__ void __launch_bounds__(128)
+k_icp_match(const float4* __restrict__ src, uint32_t n_max, const uint32_t* n_dev, const float4* __restrict__ tgt,
+            const float* __restrict__ tgt_normals, GridDev g, float r2, int method, const IcpState* __restrict__ st,
+            int32_t* __restrict__ corr_out, float* __restrict__ d2_out, double* __restrict__ partials) {
+  if (st->done) return;                                     // the loop has stopped: block-uniform
+  __shared__ double sm[4][32];
+  const uint32_t n = apc_count(n_dev, n_max);
+  const float c = grid_cell_size(g, 0);
+  const uint32_t lane = threadIdx.x & 31u, warp = threadIdx.x >> 5;
+  const uint32_t pair = c_icp_pairs[method][lane], pa = pair & 15u, pb = pair >> 4;
+  double T[12];
+#pragma unroll
+  for (int k = 0; k < 12; ++k) T[k] = st->T[k];
+  double acc = 0.0;
+  for (uint32_t i = (blockIdx.x * blockDim.x + threadIdx.x) >> 5; i < n; i += (gridDim.x * blockDim.x) >> 5) {
+    const float4 p = src[i];
+    const double x = p.x, y = p.y, z = p.z;
+    const float4 q = make_float4(icp_row(T, 0, x, y, z), icp_row(T, 1, x, y, z), icp_row(T, 2, x, y, z), 0.0f);
+    uint32_t cs, ps;
+    const uint32_t total = flat27_runs_outside(g, c, q, lane, cs, ps);
+    uint64_t best = ~0ull;
+    for (uint32_t base = 0; base < total; base += 32) {
+      const uint32_t ci = base + lane;
+      const uint32_t at = flat27_at(cs, ps, min(ci, total - 1u));
+      if (ci < total) {
+        const float4 t = g.sorted[at];
+        const float d2 = d2_f32(q.x, q.y, q.z, t.x, t.y, t.z);
+        if (d2 <= r2) best = min(best, ((uint64_t)__float_as_uint(d2) << 32) | __float_as_uint(t.w));
+      }
+    }
+    best = warp_min_u64(best);
+    const bool found = best != ~0ull;                       // warp-uniform
+    const uint32_t j = (uint32_t)best;
+    const float d2 = __uint_as_float((uint32_t)(best >> 32));
+    if (found) {
+      const float4 t = tgt[j];
+      double v[10];
+      const double sx = q.x, sy = q.y, sz = q.z, tx = t.x, ty = t.y, tz = t.z;
+      if (method == APC_ICP_POINT_TO_PLANE) {
+        const double nx = tgt_normals[3 * (size_t)j], ny = tgt_normals[3 * (size_t)j + 1], nz = tgt_normals[3 * (size_t)j + 2];
+        v[0] = sy * nz - sz * ny; v[1] = sz * nx - sx * nz; v[2] = sx * ny - sy * nx;
+        v[3] = nx; v[4] = ny; v[5] = nz;
+        v[6] = ((sx - tx) * nx + (sy - ty) * ny) + (sz - tz) * nz;
+      } else {
+        v[0] = sx; v[1] = sy; v[2] = sz; v[3] = tx; v[4] = ty; v[5] = tz; v[6] = 0.0;
+      }
+      v[7] = 1.0; v[8] = d2; v[9] = 0.0;
+      acc += icp_pick(v, pa) * icp_pick(v, pb);
+    }
+    if (lane == 0) {
+      if (corr_out) corr_out[i] = found ? (int32_t)j : -1;
+      if (d2_out) d2_out[i] = found ? d2 : 0.0f;
+    }
+  }
+  sm[warp][lane] = acc;
+  __syncthreads();
+  if (threadIdx.x < 32) partials[32 * (size_t)blockIdx.x + lane] = ((sm[0][lane] + sm[1][lane]) + sm[2][lane]) + sm[3][lane];
+}
+
+// The serial solve of k_icp_solve (one thread) keeps its matrices in shared memory: as local arrays they spilled.
+struct IcpWork {
+  double N[4][4], V[4][4];    // point-to-point: Horn's matrix and its Jacobi rotations
+  double L[6][6];             // point-to-plane: the normal equations, overwritten by their Cholesky factor
+};
+
+// Largest-eigenvalue eigenvector of the symmetric 4x4 N (cyclic Jacobi)
+__device__ __forceinline__ void icp_top_eigvec4(double (&N)[4][4], double (&V)[4][4], double (&q)[4]) {
+  for (int a = 0; a < 4; ++a)
+    for (int b = 0; b < 4; ++b) V[a][b] = a == b ? 1.0 : 0.0;
+  for (int sweep = 0; sweep < 30; ++sweep) {
+    double off = 0.0, diag = 0.0;
+    for (int a = 0; a < 4; ++a) {
+      diag += N[a][a] * N[a][a];
+      for (int b = a + 1; b < 4; ++b) off += N[a][b] * N[a][b];
+    }
+    if (!(off > 1e-36 * diag)) break;
+    for (int a = 0; a < 3; ++a)
+      for (int b = a + 1; b < 4; ++b) {
+        if (N[a][b] == 0.0) continue;
+        const double theta = (N[b][b] - N[a][a]) / (2.0 * N[a][b]);
+        const double t = (theta >= 0.0 ? 1.0 : -1.0) / (fabs(theta) + sqrt(theta * theta + 1.0));
+        const double cs = 1.0 / sqrt(t * t + 1.0), sn = t * cs;
+        for (int k = 0; k < 4; ++k) {                        // N = J^T N J, columns then rows
+          const double x = N[k][a], y = N[k][b];
+          N[k][a] = cs * x - sn * y;
+          N[k][b] = sn * x + cs * y;
+        }
+        for (int k = 0; k < 4; ++k) {
+          const double x = N[a][k], y = N[b][k];
+          N[a][k] = cs * x - sn * y;
+          N[b][k] = sn * x + cs * y;
+        }
+        for (int k = 0; k < 4; ++k) {
+          const double x = V[k][a], y = V[k][b];
+          V[k][a] = cs * x - sn * y;
+          V[k][b] = sn * x + cs * y;
+        }
+      }
+  }
+  int m = 0;
+  for (int a = 1; a < 4; ++a)
+    if (N[a][a] > N[m][m]) m = a;
+  for (int k = 0; k < 4; ++k) q[k] = V[k][m];
+}
+
+// Kabsch from the raw moments: H = sum s' t^T - sum s' sum t^T / n; the proper rotation maximising tr(R^T H) is
+// the quaternion of the largest eigenvalue of Horn's matrix (the SVD solution with its reflection fix).
+__device__ __forceinline__ void icp_point_to_point(const double* M, IcpWork& wk, double (&U)[16]) {
+  const double n = M[0];
+  const double ms[3] = {M[2] / n, M[3] / n, M[4] / n}, mt[3] = {M[5] / n, M[6] / n, M[7] / n};
+  double H[3][3];
+  for (int a = 0; a < 3; ++a)
+    for (int b = 0; b < 3; ++b) H[a][b] = M[8 + 3 * a + b] - n * ms[a] * mt[b];   // lane 8 + 3a + b: sum s'_a t_b
+  const double Sxx = H[0][0], Sxy = H[0][1], Sxz = H[0][2], Syx = H[1][0], Syy = H[1][1], Syz = H[1][2], Szx = H[2][0],
+               Szy = H[2][1], Szz = H[2][2];
+  const double N[4][4] = {{Sxx + Syy + Szz, Syz - Szy, Szx - Sxz, Sxy - Syx},
+                          {Syz - Szy, Sxx - Syy - Szz, Sxy + Syx, Szx + Sxz},
+                          {Szx - Sxz, Sxy + Syx, -Sxx + Syy - Szz, Syz + Szy},
+                          {Sxy - Syx, Szx + Sxz, Syz + Szy, -Sxx - Syy + Szz}};
+  for (int a = 0; a < 4; ++a)
+    for (int b = 0; b < 4; ++b) wk.N[a][b] = N[a][b];
+  double q[4];
+  icp_top_eigvec4(wk.N, wk.V, q);
+  const double nq = sqrt(((q[0] * q[0] + q[1] * q[1]) + q[2] * q[2]) + q[3] * q[3]);
+  const double w = q[0] / nq, x = q[1] / nq, y = q[2] / nq, z = q[3] / nq;
+  const double R[3][3] = {{w * w + x * x - y * y - z * z, 2.0 * (x * y - w * z), 2.0 * (x * z + w * y)},
+                          {2.0 * (x * y + w * z), w * w - x * x + y * y - z * z, 2.0 * (y * z - w * x)},
+                          {2.0 * (x * z - w * y), 2.0 * (y * z + w * x), w * w - x * x - y * y + z * z}};
+  for (int a = 0; a < 3; ++a) {
+    for (int b = 0; b < 3; ++b) U[4 * a + b] = R[a][b];
+    U[4 * a + 3] = mt[a] - ((R[a][0] * ms[0] + R[a][1] * ms[1]) + R[a][2] * ms[2]);
+  }
+  U[12] = U[13] = U[14] = 0.0;
+  U[15] = 1.0;
+}
+
+// One Gauss-Newton step: (sum J^T J) x = -(sum J^T r) by Cholesky; false when a pivot is not above ICP_PIVOT_REL
+// times its diagonal entry.  x = (alpha, beta, gamma, tx, ty, tz) -> Rz(gamma) Ry(beta) Rx(alpha) (Open3D's
+// PoseToTransformation).
+__device__ __forceinline__ bool icp_point_to_plane(const double* M, IcpWork& wk, double (&U)[16]) {
+  double (&L)[6][6] = wk.L;
+  int k = 2;
+  for (int c = 0; c < 6; ++c)
+    for (int r = c; r < 6; ++r) L[r][c] = M[k++];          // lower triangle of sum J^T J
+  for (int j = 0; j < 6; ++j) {
+    const double ajj = L[j][j];
+    double d = ajj;
+    for (int m = 0; m < j; ++m) d -= L[j][m] * L[j][m];
+    if (!(isfinite(d) && d > ICP_PIVOT_REL * ajj)) return false;
+    L[j][j] = sqrt(d);
+    for (int i = j + 1; i < 6; ++i) {
+      double e = L[i][j];
+      for (int m = 0; m < j; ++m) e -= L[i][m] * L[j][m];
+      L[i][j] = e / L[j][j];
+    }
+  }
+  double y[6], x[6];
+  for (int i = 0; i < 6; ++i) {
+    double e = -M[23 + i];
+    for (int m = 0; m < i; ++m) e -= L[i][m] * y[m];
+    y[i] = e / L[i][i];
+  }
+  for (int i = 5; i >= 0; --i) {
+    double e = y[i];
+    for (int m = i + 1; m < 6; ++m) e -= L[m][i] * x[m];
+    x[i] = e / L[i][i];
+  }
+  double sa, ca, sb, cb, sg, cg;
+  sincos(x[0], &sa, &ca);
+  sincos(x[1], &sb, &cb);
+  sincos(x[2], &sg, &cg);
+  U[0] = cg * cb;  U[1] = -sg * ca + cg * sb * sa;  U[2] = sg * sa + cg * sb * ca;   U[3] = x[3];
+  U[4] = sg * cb;  U[5] = cg * ca + sg * sb * sa;   U[6] = -cg * sa + sg * sb * ca;  U[7] = x[4];
+  U[8] = -sb;      U[9] = cb * sa;                  U[10] = cb * ca;                 U[11] = x[5];
+  U[12] = 0.0;     U[13] = 0.0;                     U[14] = 0.0;                     U[15] = 1.0;
+  return true;
+}
+
+// method < 0: evaluate_registration, metrics only.
+// 8 warps reduce the partials; one thread solves.  __maxnreg__: with the default budget of a 256-thread block the
+// serial solve spilled (64 registers); it needs 90.
+#define ICP_SOLVE_WARPS 8
+__global__ void __maxnreg__(128)
+k_icp_solve(const double* __restrict__ partials, uint32_t n_parts, uint32_t n_max, const uint32_t* n_dev, int method,
+            int iteration, double relative_fitness, double relative_rmse, IcpState* __restrict__ st,
+            double* __restrict__ out_T, double* __restrict__ out_stats, int32_t* __restrict__ out_info) {
+  if (st->done) return;                                     // block-uniform
+  __shared__ double sm[ICP_SOLVE_WARPS][32];
+  __shared__ IcpWork wk;
+  const uint32_t m = threadIdx.x & 31u, w = threadIdx.x >> 5;
+  // thread (w, m): moment m of blocks w, w + 8, ..., in four independent chains (the loads overlap)
+  double part[4] = {0.0, 0.0, 0.0, 0.0};
+  uint32_t b = w;
+  for (; b + 3 * ICP_SOLVE_WARPS < n_parts; b += 4 * ICP_SOLVE_WARPS)
+#pragma unroll
+    for (int u = 0; u < 4; ++u) part[u] += partials[32 * (size_t)(b + u * ICP_SOLVE_WARPS) + m];
+  for (; b < n_parts; b += ICP_SOLVE_WARPS) part[0] += partials[32 * (size_t)b + m];
+  sm[w][m] = (part[0] + part[1]) + (part[2] + part[3]);
+  __syncthreads();
+  if (w != 0) return;
+  double tot = 0.0;
+#pragma unroll
+  for (int k = 0; k < ICP_SOLVE_WARPS; ++k) tot += sm[k][m];
+  __syncwarp();
+  sm[0][m] = tot;
+  __syncwarp();
+  if (m != 0) return;
+  const double* M = sm[0];
+  const double n_corr = M[0];
+  const uint32_t n = apc_count(n_dev, n_max);
+  const double fitness = n_corr > 0.0 ? n_corr / (double)n : 0.0, rmse = n_corr > 0.0 ? sqrt(M[1] / n_corr) : 0.0;
+  out_stats[0] = fitness;
+  out_stats[1] = rmse;
+  if (method < 0) return;
+  int32_t status = APC_ICP_OK;
+  double U[16];
+  if (n_corr == 0.0) status = APC_ICP_NO_CORRESPONDENCE;
+  else if (method == APC_ICP_POINT_TO_POINT) icp_point_to_point(M, wk, U);
+  else if (!icp_point_to_plane(M, wk, U)) status = APC_ICP_DEGENERATE;
+  int32_t converged = 0;
+  if (status == APC_ICP_OK) {
+    double T[16];
+    for (int r = 0; r < 4; ++r)
+      for (int c = 0; c < 4; ++c)
+        T[4 * r + c] = ((U[4 * r] * st->T[c] + U[4 * r + 1] * st->T[4 + c]) + U[4 * r + 2] * st->T[8 + c]) +
+                       U[4 * r + 3] * st->T[12 + c];
+    for (int k = 0; k < 16; ++k) st->T[k] = out_T[k] = T[k];
+    st->iterations = iteration + 1;
+    converged = iteration > 0 && fabs(st->prev_f - fitness) < relative_fitness && fabs(st->prev_r - rmse) < relative_rmse;
+    st->prev_f = fitness;
+    st->prev_r = rmse;
+  }
+  st->done = status != APC_ICP_OK || converged;
+  out_info[0] = (int32_t)st->iterations;
+  out_info[1] = converged;
+  out_info[2] = status;
+  out_info[3] = 0;
+}
+
+// Checks, scratch (allocated before the first launch), the call's begin, output initialisation and the target's
+// grid.  *empty: one cloud has no points, nothing more to launch.
+static int icp_begin(apc_ctx* ctx, const float* src_xyzi, uint32_t n_src, const float* tgt_xyzi, uint32_t n_tgt,
+                     const uint32_t* n_tgt_dev, double r, const double* T16_host, double* out_stats, int32_t* out_corr, float* out_d2,
+                     double* out_T, int32_t* out_info, int32_t empty_status, bool* empty, cudaStream_t s) {
+  APC_REQUIRE(ctx, src_xyzi && tgt_xyzi && T16_host && out_stats, "NULL pointer");
+  APC_REQUIRE(ctx, n_src <= ctx->max_points && n_tgt <= ctx->max_points, "more points than the context was created for");
+  const float r32 = (float)r;
+  APC_REQUIRE(ctx, r > 0.0 && r32 > 0.0f && std::isfinite(r32 * r32), "max_correspondence_distance must be finite and > 0");
+  int rc = apc_neighbors_prepare(ctx, 0);
+  if (rc) return rc;
+  NeighborScratch* sc = scratch_of(ctx);
+  if (!sc->icp_part) APC_CUDA(ctx, cudaMalloc((void**)&sc->icp_part, (size_t)ICP_MAX_BLOCKS * 32 * sizeof(double)));
+  if (!sc->icp_state) APC_CUDA(ctx, cudaMalloc((void**)&sc->icp_state, sizeof(IcpState)));
+  rc = apc_begin(ctx, s);
+  if (rc) return rc;
+  if (out_corr && n_src) APC_CUDA(ctx, cudaMemsetAsync(out_corr, 0xff, (size_t)n_src * sizeof(int32_t), s));
+  if (out_d2 && n_src) APC_CUDA(ctx, cudaMemsetAsync(out_d2, 0, (size_t)n_src * sizeof(float), s));
+  *empty = n_src == 0 || n_tgt == 0;
+  IcpT16 init;
+  memcpy(init.v, T16_host, sizeof(init.v));
+  k_icp_init<<<1, 1, 0, s>>>(init, sc->icp_state, out_T, out_stats, out_info, *empty ? empty_status : APC_ICP_OK);
+  APC_LAUNCH_CHECK(ctx, "k_icp_init");
+  if (*empty) return APC_OK;
+  // the grid of apc_cluster_dbscan / apc_estimate_normals_radius: cells of r * (1 + 2^-8), reciprocal indexing
+  return grid_build(ctx, sc->grid[0], reinterpret_cast<const float4*>(tgt_xyzi), n_tgt, n_tgt_dev, r32 * 1.00390625f,
+                    false, s, false, CTR_CURSOR_NORMALS, true);
+}
+
+static int icp_finish(apc_ctx* ctx, uint32_t n_tgt, const uint32_t* n_tgt_dev, cudaStream_t s) {
+  const GridHost& g = scratch_of(ctx)->grid[0];
+  APC_PROF(ctx, "k_grid_clean", s);
+  k_grid_clean<<<dim3(min(apc_div_up(n_tgt, 256), (uint32_t)APC_SM_COUNT * 4), 1), 256, 0, s>>>(n_tgt, n_tgt_dev, g.d);
+  APC_LAUNCH_CHECK(ctx, "icp");
+  return APC_OK;
+}
+
+static uint32_t icp_blocks(uint32_t n_src) { return min(apc_div_up(n_src, 4), (uint32_t)ICP_MAX_BLOCKS); }
+
+extern "C" int apc_evaluate_registration(apc_ctx* ctx, const float* src_xyzi, uint32_t n_src, const uint32_t* n_src_dev,
+                                         const float* tgt_xyzi, uint32_t n_tgt, const uint32_t* n_tgt_dev,
+                                         double max_correspondence_distance, const double* T16_host,
+                                         int32_t* out_correspondences, float* out_d2, double* out_stats_dev, void* stream) {
+  if (!ctx) return APC_ERR_BAD_ARG;
+  cudaStream_t s = (cudaStream_t)stream;
+  bool empty = false;
+  int rc = icp_begin(ctx, src_xyzi, n_src, tgt_xyzi, n_tgt, n_tgt_dev, max_correspondence_distance, T16_host, out_stats_dev,
+                     out_correspondences, out_d2, nullptr, nullptr, APC_ICP_OK, &empty, s);
+  if (rc || empty) return rc;
+  NeighborScratch* sc = scratch_of(ctx);
+  const float r32 = (float)max_correspondence_distance;
+  const uint32_t bq = icp_blocks(n_src);
+  {
+    APC_PROF(ctx, "k_icp_match", s);
+    k_icp_match<<<bq, 128, 0, s>>>(reinterpret_cast<const float4*>(src_xyzi), n_src, n_src_dev,
+                                   reinterpret_cast<const float4*>(tgt_xyzi), nullptr, sc->grid[0].d, r32 * r32,
+                                   APC_ICP_POINT_TO_POINT, sc->icp_state, out_correspondences, out_d2, sc->icp_part);
+  }
+  {
+    APC_PROF(ctx, "k_icp_solve", s);
+    k_icp_solve<<<1, ICP_SOLVE_WARPS * 32, 0, s>>>(sc->icp_part, bq, n_src, n_src_dev, -1, 0, 0.0, 0.0, sc->icp_state, nullptr,
+                                   out_stats_dev, nullptr);
+  }
+  return icp_finish(ctx, n_tgt, n_tgt_dev, s);
+}
+
+extern "C" int apc_icp(apc_ctx* ctx, const float* src_xyzi, uint32_t n_src, const uint32_t* n_src_dev,
+                       const float* tgt_xyzi, const float* tgt_normals, uint32_t n_tgt, const uint32_t* n_tgt_dev,
+                       double max_correspondence_distance, const double* init_T16_host, int method, int max_iteration,
+                       double relative_fitness, double relative_rmse, double* out_T16_dev, double* out_stats_dev,
+                       int32_t* out_info_dev, int32_t* out_correspondences, void* stream) {
+  if (!ctx) return APC_ERR_BAD_ARG;
+  APC_REQUIRE(ctx, out_T16_dev && out_info_dev, "NULL pointer");
+  APC_REQUIRE(ctx, max_iteration >= 0, "max_iteration must be >= 0");
+  APC_REQUIRE(ctx, method == APC_ICP_POINT_TO_POINT || method == APC_ICP_POINT_TO_PLANE, "unknown ICP method");
+  APC_REQUIRE(ctx, method != APC_ICP_POINT_TO_PLANE || tgt_normals, "point-to-plane ICP needs the target's normals");
+  cudaStream_t s = (cudaStream_t)stream;
+  bool empty = false;
+  int rc = icp_begin(ctx, src_xyzi, n_src, tgt_xyzi, n_tgt, n_tgt_dev, max_correspondence_distance, init_T16_host, out_stats_dev,
+                     out_correspondences, nullptr, out_T16_dev, out_info_dev,
+                     max_iteration > 0 ? APC_ICP_NO_CORRESPONDENCE : APC_ICP_OK, &empty, s);
+  if (rc || empty) return rc;
+  NeighborScratch* sc = scratch_of(ctx);
+  const float r32 = (float)max_correspondence_distance;
+  const uint32_t bq = icp_blocks(n_src);
+  for (int j = 0; j < max_iteration; ++j) {
+    {
+      APC_PROF(ctx, "k_icp_match", s);
+      k_icp_match<<<bq, 128, 0, s>>>(reinterpret_cast<const float4*>(src_xyzi), n_src, n_src_dev,
+                                     reinterpret_cast<const float4*>(tgt_xyzi), tgt_normals, sc->grid[0].d, r32 * r32,
+                                     method, sc->icp_state, out_correspondences, nullptr, sc->icp_part);
+    }
+    APC_PROF(ctx, "k_icp_solve", s);
+    k_icp_solve<<<1, ICP_SOLVE_WARPS * 32, 0, s>>>(sc->icp_part, bq, n_src, n_src_dev, method, j, relative_fitness, relative_rmse,
+                                   sc->icp_state, out_T16_dev, out_stats_dev, out_info_dev);
+  }
+  APC_LAUNCH_CHECK(ctx, "icp");
+  return icp_finish(ctx, n_tgt, n_tgt_dev, s);
 }

@@ -23,6 +23,14 @@ def _ptr(t):
     return C.c_void_p(t.data_ptr()) if t is not None else None
 
 
+def _t16(T):
+    """A 4x4 transform as the ``double[16]`` (row-major) of the C ABI; identity when None."""
+    v = np.eye(4) if T is None else np.asarray(T.cpu() if isinstance(T, torch.Tensor) else T, np.float64)
+    if v.shape != (4, 4):
+        raise ValueError("the transformation must be 4x4")
+    return (C.c_double * 16)(*v.reshape(16).tolist())
+
+
 def _stream():
     return C.c_void_p(torch.cuda.current_stream().cuda_stream)
 
@@ -335,6 +343,37 @@ class Context:
         self._ok(lib.apc_cluster_dbscan(self.h, _ptr(xyzi), n, _ptr(n_dev), float(eps), int(min_points), _ptr(labels),
                                         _ptr(n_clusters), _ptr(counts), _stream()))
         return labels[:n], n_clusters, (counts[:n] if counts is not None else None)
+
+    # ---- registration ---------------------------------------------------------------------------------
+    def evaluate_registration(self, src_xyzi, tgt_xyzi, max_correspondence_distance, T=None, n_src_dev=None,
+                              n_tgt_dev=None):
+        """``apc_evaluate_registration`` at ``T`` (float64 4x4, identity by default).  Returns ``(stats float64[2]
+        {fitness, inlier_rmse}, correspondences int32[n_src] (-1: none), d2 float32[n_src])`` on the device."""
+        n_src, n_tgt = src_xyzi.shape[0], tgt_xyzi.shape[0]
+        corr = self._empty((max(n_src, 1),), torch.int32)
+        d2 = self._empty((max(n_src, 1),), torch.float32)
+        stats = self._empty((2,), torch.float64)
+        self._ok(lib.apc_evaluate_registration(self.h, _ptr(src_xyzi), n_src, _ptr(n_src_dev), _ptr(tgt_xyzi), n_tgt,
+                                               _ptr(n_tgt_dev), float(max_correspondence_distance), _t16(T),
+                                               _ptr(corr), _ptr(d2), _ptr(stats), _stream()))
+        return stats, corr[:n_src], d2[:n_src]
+
+    def icp(self, src_xyzi, tgt_xyzi, max_correspondence_distance, init=None, method=_capi.APC_ICP_POINT_TO_POINT,
+            tgt_normals=None, max_iteration=30, relative_fitness=1e-6, relative_rmse=1e-6, n_src_dev=None,
+            n_tgt_dev=None):
+        """``apc_icp``.  Returns ``(T float64[4,4], stats float64[2] {fitness, inlier_rmse}, info int32[4]
+        {iterations, converged, APC_ICP_* status, 0}, correspondences int32[n_src])`` on the device, with no host
+        synchronisation."""
+        n_src, n_tgt = src_xyzi.shape[0], tgt_xyzi.shape[0]
+        T = self._empty((4, 4), torch.float64)
+        stats = self._empty((2,), torch.float64)
+        info = self._empty((4,), torch.int32)
+        corr = self._empty((max(n_src, 1),), torch.int32)
+        self._ok(lib.apc_icp(self.h, _ptr(src_xyzi), n_src, _ptr(n_src_dev), _ptr(tgt_xyzi), _ptr(tgt_normals), n_tgt,
+                             _ptr(n_tgt_dev), float(max_correspondence_distance), _t16(init), int(method),
+                             int(max_iteration), float(relative_fitness), float(relative_rmse), _ptr(T), _ptr(stats),
+                             _ptr(info), _ptr(corr), _stream()))
+        return T, stats, info, corr[:n_src]
 
     # ---- ransac ------------------------------------------------------------------------------------
     def segment_plane(self, xyzi, distance_threshold, ransac_n, num_iterations, probability, seed=0,

@@ -288,6 +288,48 @@ int apc_cluster_dbscan(apc_ctx* ctx, const float* xyzi, uint32_t n_max, const ui
                        double eps, int min_points, int32_t* out_labels,
                        uint32_t* out_cluster_count_dev, uint32_t* out_neighbor_counts, void* stream);
 
+/* ---- (3b) ICP registration (Open3D t.pipelines.registration) -------------------------- */
+
+enum { APC_ICP_POINT_TO_POINT = 0, APC_ICP_POINT_TO_PLANE = 1 };
+enum { APC_ICP_OK = 0, APC_ICP_NO_CORRESPONDENCE = 1, APC_ICP_DEGENERATE = 2 };
+
+/* evaluate_registration(source, target, max_correspondence_distance, transformation) (Open3D
+ * t::pipelines::registration::EvaluateRegistration).  Contract (oracle/registration.py): s' = float32(T s) with
+ * T = T16_host (float64, row-major, passed to the kernels by value); the correspondence of source point i is the
+ * target point with the smallest (d2, index) among those with d2 = (dx*dx + dy*dy) + dz*dz (float32, unfused)
+ * <= float32(r)^2, else -1.  out_correspondences int32[n_src] and out_d2 float32[n_src] (d2, 0 for none) may be
+ * NULL; out_stats_dev double[2] (device) = {fitness = n_corr / n_src, inlier_rmse = sqrt(sum d2 / n_corr)}, both
+ * 0 when n_corr = 0.  xyzi clouds (float4 per point); r finite and > 0 with float32(r)^2 finite (APC_ERR_BAD_ARG
+ * otherwise).  Target points the grid cannot key raise APC_ERR_KEY_RANGE at apc_check; a transformed source
+ * point the grid cannot key has no correspondence.  Every target point within r is found for coordinates below
+ * 16384 r.  No host synchronisation. */
+int apc_evaluate_registration(apc_ctx* ctx, const float* src_xyzi, uint32_t n_src, const uint32_t* n_src_dev,
+                              const float* tgt_xyzi, uint32_t n_tgt, const uint32_t* n_tgt_dev,
+                              double max_correspondence_distance, const double* T16_host,
+                              int32_t* out_correspondences, float* out_d2, double* out_stats_dev, void* stream);
+
+/* icp(source, target, max_correspondence_distance, init, estimation, criteria) (Open3D
+ * t::pipelines::registration::ICP, one scale; DoSingleScaleICPIterations).  Every iteration matches the ORIGINAL
+ * source transformed by the T accumulated so far (as apc_evaluate_registration), computes fitness and rmse, and
+ * estimates an update: APC_ICP_POINT_TO_POINT Kabsch (no scaling), APC_ICP_POINT_TO_PLANE one Gauss-Newton step
+ * of sum ((s' - t) . n)^2 over the pose (alpha, beta, gamma, tx, ty, tz) -> Rz Ry Rx (PoseToTransformation), with
+ * the 6x6 system solved by Cholesky; T = update T.  The loop stops after max_iteration iterations, when
+ * |delta fitness| < relative_fitness and |delta rmse| < relative_rmse (never at the first iteration), at an
+ * iteration without correspondences (APC_ICP_NO_CORRESPONDENCE; Open3D raises) or when the 6x6 system is not
+ * positive definite (APC_ICP_DEGENERATE, no update).  Outputs (device): out_T16_dev double[16] (row-major),
+ * out_stats_dev double[2] {fitness, inlier_rmse} and out_correspondences int32[n_src] (may be NULL) of the last
+ * matching, out_info_dev int32[4] {iterations, converged, APC_ICP_* status, 0}.  max_iteration = 0 gives init,
+ * 0, 0, all -1, 0 iterations.  tgt_normals float32[3 * n_tgt] (point-to-plane only).  init_T16_host is passed to
+ * the kernels by value, and all max_iteration (match, solve) pairs are launched up front and return at once
+ * after the loop has stopped: the call makes no host synchronisation and can be captured in a CUDA graph.
+ * APC_ERR_BAD_ARG: NULL pointers, n_src or n_tgt above the context's max_points, r as in
+ * apc_evaluate_registration, max_iteration < 0, an unknown method, point-to-plane without normals. */
+int apc_icp(apc_ctx* ctx, const float* src_xyzi, uint32_t n_src, const uint32_t* n_src_dev,
+            const float* tgt_xyzi, const float* tgt_normals, uint32_t n_tgt, const uint32_t* n_tgt_dev,
+            double max_correspondence_distance, const double* init_T16_host, int method, int max_iteration,
+            double relative_fitness, double relative_rmse, double* out_T16_dev, double* out_stats_dev,
+            int32_t* out_info_dev, int32_t* out_correspondences, void* stream);
+
 /* ---- (4) RANSAC ground plane --------------------------------------------------------- */
 
 /* segment_plane(distance_threshold, ransac_n, num_iterations, probability) (pp.py:533-543).
