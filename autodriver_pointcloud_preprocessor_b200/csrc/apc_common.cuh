@@ -73,8 +73,9 @@ struct apc_ctx {
   uint32_t* nb_count = nullptr;     // [max_points]
   // ransac
   double* rs_planes = nullptr;      // [max_iters*4]
-  unsigned long long* rs_scores = nullptr;  // per-CTA tally rows of k_rs_score {inliers, err}
-  unsigned long long* rs_scores_copy = nullptr;  // [max_iters*2] readable copy of the last call's tallies
+  unsigned long long* rs_scores = nullptr;  // per-CTA tally rows of k_rs_score {inliers, err}, column by column
+  unsigned long long* rs_scores_copy = nullptr;  // [max_iters*2] the last call's tallies, summed over the CTAs
+  uint32_t* rs_col_tickets = nullptr;  // [max_iters] retired CTAs of each chunk column of k_rs_score
   double* rs_partials = nullptr;    // refit partial sums
   uint32_t rs_max_iters = 0;
   // pipeline ping-pong buffers

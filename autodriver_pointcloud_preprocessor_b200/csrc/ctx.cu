@@ -79,7 +79,7 @@ extern "C" int apc_ctx_destroy(apc_ctx* ctx) {
   for (cudaEvent_t e : ctx->prof.ev) cudaEventDestroy(e);
   void* ptrs[] = {ctx->ctrl, ctx->vox_slots, ctx->vox_acc, ctx->vox_rank, ctx->p2slot,
                   ctx->dedup_slots, ctx->sorted_pts, ctx->knn_avg, ctx->red_a,
-                  ctx->red_b, ctx->nb_count, ctx->rs_planes, ctx->rs_scores, ctx->rs_scores_copy, ctx->rs_partials, ctx->buf_a, ctx->buf_b,
+                  ctx->red_b, ctx->nb_count, ctx->rs_planes, ctx->rs_scores, ctx->rs_scores_copy, ctx->rs_col_tickets, ctx->rs_partials, ctx->buf_a, ctx->buf_b,
                   ctx->mask_a, ctx->idx_a, ctx->idx_b, ctx->dev_counts, ctx->nrm_scratch};
   for (void* p : ptrs)
     if (p) cudaFree(p);
@@ -140,6 +140,7 @@ extern "C" int apc_ctx_create(int device, uint32_t max_points, apc_ctx** out) {
   A(dalloc(&ctx->rs_scores, (size_t)(APC_SM_COUNT * 2 * 20 + ctx->rs_max_iters + 64) * 2));
   A(dalloc(&ctx->rs_scores_copy, (size_t)ctx->rs_max_iters * 2));
   A(cudaMemset(ctx->rs_scores_copy, 0, (size_t)ctx->rs_max_iters * 2 * sizeof(unsigned long long)));
+  A(dalloc(&ctx->rs_col_tickets, ctx->rs_max_iters));
   A(dalloc(&ctx->rs_partials, (size_t)(M / 256 + 64) * 10));
   A(dalloc(&ctx->buf_a, M));
   A(dalloc(&ctx->buf_b, M));

@@ -78,6 +78,13 @@ __device__ __forceinline__ unsigned long long fma2(unsigned long long a, unsigne
   return r;
 }
 
+// acc += bits(v) if c, as ONE predicated integer add (the compiler's own choice for the C form
+// is a SEL of the value or zero followed by an add)
+__device__ __forceinline__ void add_if(uint32_t& acc, bool c, float v) {
+  asm("{\n\t.reg .pred p;\n\tsetp.ne.u32 p, %1, 0;\n\t@p add.u32 %0, %0, %2;\n\t}"
+      : "+r"(acc) : "r"((uint32_t)c), "r"(__float_as_uint(v)));
+}
+
 // One hypothesis from its sample points (s[0..n), staged in shared memory): plane through three
 // points, or the least-squares "fast plane fit" - same operation order as oracle/ransac.py.
 __device__ void rs_fit(const float4* s, uint32_t n, double* out) {
@@ -116,16 +123,14 @@ __device__ __forceinline__ double plane_dist(const double* pl, double x, double 
   return fabs(__dadd_rn(__dadd_rn(__dadd_rn(__dmul_rn(pl[0], x), __dmul_rn(pl[1], y)), __dmul_rn(pl[2], z)), pl[3]));
 }
 
-#define RS_SELECT_CHUNK 512
 #define RS_EPS 5.0e-7f          // relative slack of the float32 pre-test (see k_rs_score)
 #define RS_MAGIC 8388608.0f     // 2^23: (u + 2^23) has rint(u) in its low mantissa bits for 0 <= u < 2^23
 #define RS_MAGIC_BITS 0x4B000000u
 #define RS_FLUSH_TILES 32       // the packed per-thread accumulators hold at most 128 points (see k_rs_score)
-#define CTR_RS_SCORE_TICKET 21  // ctrl->counters slot: retired CTAs of k_rs_score
-__device__ __noinline__ void rs_select_cta(const double* __restrict__ planes, const unsigned long long* scores_in,
-                                           uint32_t n_rows, uint32_t row_stride, uint32_t P, uint32_t ransac_n,
-                                           uint32_t iters, double log1mp, double* __restrict__ plane8,
-                                           uint32_t* __restrict__ info, unsigned long long* __restrict__ scores_copy);
+#define CTR_RS_SCORE_TICKET 21  // ctrl->counters slot: chunk columns of k_rs_score whose tallies are summed
+__device__ __noinline__ void rs_select_cta(const double* __restrict__ planes, const unsigned long long* scores,
+                                           uint32_t P, uint32_t ransac_n, uint32_t iters, double log1mp,
+                                           double* __restrict__ plane8, uint32_t* __restrict__ info);
 
 // Scoring + selection in one launch (the hypotheses come from k_rs_hypotheses).
 // grid = (persistent CTAs striding over point tiles, chunks of CH hypotheses).
@@ -139,8 +144,9 @@ __device__ __noinline__ void rs_select_cta(const double* __restrict__ planes, co
 //             rint(d32^2 * 2^16/thr^2) comes out of the same packed pipeline: one FFMA2 adds the
 //             2^23 magic number, leaving the integer in the mantissa (no F2I); summed as integers.
 //   epilogue  warp REDUX -> per-warp rows in shared memory -> one row of per-CTA tallies in
-//             global memory (no atomics); the last CTA to retire (ticket) adds the rows up and
-//             applies Open3D's sequential selection rule.
+//             global memory (no atomics); the last CTA of each chunk column (a ticket per column)
+//             adds that column's rows up into scores_copy, and the last column to finish applies
+//             Open3D's sequential selection rule.
 #define RS_QCAP 128
 // Exact re-decision of one queued point against hypotheses h_first, h_first + h_step, ...: the
 // evaluations whose float32 distance lies inside the rounding band [lo, hi) are decided by the
@@ -192,7 +198,8 @@ __device__ __forceinline__ unsigned long long gtime() {
 #define RS_HYP_THREADS 64
 __global__ void __launch_bounds__(RS_HYP_THREADS)
 k_rs_hypotheses(const float4* __restrict__ pts, uint32_t n_max, const uint32_t* n_dev, uint32_t ransac_n, uint32_t iters,
-                uint64_t seed, const int32_t* __restrict__ table, double* __restrict__ planes) {
+                uint64_t seed, const int32_t* __restrict__ table, double* __restrict__ planes,
+                uint32_t* __restrict__ col_tickets) {
   __shared__ uint32_t s_idx[RS_HYP_THREADS][RS_MAX_N + 1];   // +1: rows on different banks
   __shared__ float4 s_sp[RS_HYP_THREADS][RS_MAX_N];
   pdl_enter();
@@ -216,6 +223,7 @@ k_rs_hypotheses(const float4* __restrict__ pts, uint32_t n_max, const uint32_t* 
     for (uint32_t j = 0; j < ransac_n; ++j) s_sp[tid][j] = pts[s_idx[tid][j]];   // independent loads, all in flight
   }
   if (it < iters) {
+    col_tickets[it] = 0;   // k_rs_score's chunk columns (fewer than iters), counted from zero on every call
     double pl[4] = {0.0, 0.0, 0.0, 0.0};
     if (live) rs_fit(s_sp[tid], ransac_n, pl);
 #pragma unroll
@@ -228,7 +236,7 @@ __global__ void __launch_bounds__(APC_TILE_THREADS, CH <= 10 ? 3 : 1)
 k_rs_score(const float4* __restrict__ pts, uint32_t n_max, const uint32_t* n_dev, uint32_t ransac_n, uint32_t iters,
            const double* __restrict__ planes, double thr,
            unsigned long long* scores, double log1mp, double* __restrict__ plane8, uint32_t* __restrict__ info,
-           unsigned long long* __restrict__ scores_copy, ApcCtrl* ctrl) {
+           unsigned long long* __restrict__ scores_copy, uint32_t* __restrict__ col_tickets, ApcCtrl* ctrl) {
   static_assert(CH % 2 == 0, "hypotheses are scored in pairs");
   __shared__ double s_pl[CH][4];
   __shared__ __align__(16) float s_pk[CH / 2][8];   // {a0,a1, b0,b1, c0,c1, d0,d1} of a pair, float32
@@ -246,7 +254,13 @@ k_rs_score(const float4* __restrict__ pts, uint32_t n_max, const uint32_t* n_dev
   RS_STAMP(0);
   APC_STAMP(0, 0);
 #ifdef RS_TRACE
-  if (threadIdx.x == 0) { uint32_t sm; asm volatile("mov.u32 %0, %%smid;" : "=r"(sm)); g_rs_trace[(blockIdx.y * gridDim.x + blockIdx.x) * 8 + 7] = sm; }
+  if (threadIdx.x == 0) {
+    uint32_t sm;
+    asm volatile("mov.u32 %0, %%smid;" : "=r"(sm));
+    unsigned long long* t = &g_rs_trace[(blockIdx.y * gridDim.x + blockIdx.x) * 8];
+    t[7] = sm;
+    t[5] = t[6] = 0;   // written by the column's last CTA / the selecting CTA only
+  }
 #endif
   // ---- prologue: the first tile's points are requested before anything else; the chunk's planes
   // (k_rs_hypotheses) are staged in shared memory while those loads are in flight ---------------
@@ -351,8 +365,8 @@ k_rs_score(const float4* __restrict__ pts, uint32_t n_max, const uint32_t* n_dev
         upk2(v2, v0, v1);
         const bool in0 = fabsf(d0) < lo[j], in1 = fabsf(d1) < lo[j];
         amb = amb | (in0 != (fabsf(d0) < hi[j])) | (in1 != (fabsf(d1) < hi[j]));
-        acc[2 * hp] += in0 ? __float_as_uint(v0) : 0u;
-        acc[2 * hp + 1] += in1 ? __float_as_uint(v1) : 0u;
+        add_if(acc[2 * hp], in0, v0);
+        add_if(acc[2 * hp + 1], in1, v1);
       }
     }
     // an evaluation inside the rounding band (a few per million): the thread queues its points of
@@ -381,28 +395,56 @@ k_rs_score(const float4* __restrict__ pts, uint32_t n_max, const uint32_t* n_dev
     if (nq) __syncthreads();   // nq is CTA-uniform
   }
   RS_STAMP(3);
+  // per-CTA partial tallies {count, error}, plain stores: row blockIdx.x of the column's [gridDim.x][CH]
+  // block, the blocks of the columns one after the other (thousands of same-line global atomics from 260
+  // CTAs cost ~17 us of serialisation in L2)
+  ulonglong2* col = reinterpret_cast<ulonglong2*>(scores) + (size_t)blockIdx.y * gridDim.x * CH;
   if (tid < nh) {
     unsigned long long c = s_cnt[tid], e = s_err[tid];
 #pragma unroll
     for (int w = 0; w < APC_TILE_THREADS / 32; ++w) { c += s_wcnt[w][tid]; e += s_werr[w][tid]; }
-    // per-CTA partial tallies, plain stores: row blockIdx.x of a [gridDim.x][gridDim.y * CH] table
-    // (thousands of same-line global atomics from 260 CTAs cost ~17 us of serialisation in L2)
-    const size_t slot = (size_t)blockIdx.x * (gridDim.y * CH) + h0 + tid;
-    scores[2 * slot] = c;
-    scores[2 * slot + 1] = e;
+    col[blockIdx.x * CH + tid] = make_ulonglong2(c, e);
   }
-  // the last CTA to retire (ticket) runs the selection: one launch and one inter-kernel
-  // dependency less on the per-scan critical path.  Barrier, then ONE thread takes the ticket with
-  // an acq_rel atomic (see ticket_acq_rel).
+  // the last CTA of the column (ticket) sums the column's rows; the last column to be summed runs the
+  // selection: one launch and one inter-kernel dependency less on the per-scan critical path.  Barrier,
+  // then ONE thread takes each ticket with an acq_rel atomic (see ticket_acq_rel).
   __shared__ bool s_last;
   __syncthreads();
-  if (tid == 0) s_last = (ticket_acq_rel(&ctrl->counters[CTR_RS_SCORE_TICKET]) == gridDim.x * gridDim.y - 1);
+  if (tid == 0) s_last = (ticket_acq_rel(&col_tickets[blockIdx.y]) == gridDim.x - 1);
   __syncthreads();
   RS_STAMP(4);
   APC_STAMP(0, 1);
   if (!s_last) return;
-  rs_select_cta(planes, scores, gridDim.x, gridDim.y * CH, P, ransac_n, iters, log1mp, plane8, info, scores_copy);
+  {
+    // G groups of CH threads add every G-th row (integer sums: the order is immaterial)
+    constexpr uint32_t G = APC_TILE_THREADS / CH;
+    __shared__ ulonglong2 s_col[G][CH];
+    const uint32_t h = tid % CH, g = tid / CH;
+    if (g < G) {
+      unsigned long long c = 0, e = 0;
+      if (h < nh)
+        for (uint32_t r = g; r < gridDim.x; r += G) {
+          const ulonglong2 v = __ldcg(col + r * CH + h);
+          c += v.x;
+          e += v.y;
+        }
+      s_col[g][h] = make_ulonglong2(c, e);
+    }
+    __syncthreads();
+    if (tid < nh) {
+      unsigned long long c = 0, e = 0;
+#pragma unroll
+      for (uint32_t k = 0; k < G; ++k) { c += s_col[k][tid].x; e += s_col[k][tid].y; }
+      reinterpret_cast<ulonglong2*>(scores_copy)[h0 + tid] = make_ulonglong2(c, e);
+    }
+  }
+  __syncthreads();
+  if (tid == 0) s_last = (ticket_acq_rel(&ctrl->counters[CTR_RS_SCORE_TICKET]) == gridDim.y - 1);
+  __syncthreads();
   RS_STAMP(5);
+  if (!s_last) return;
+  rs_select_cta(planes, scores_copy, P, ransac_n, iters, log1mp, plane8, info);
+  RS_STAMP(6);
   APC_STAMP(0, 2);
 }
 
@@ -414,15 +456,15 @@ k_rs_score(const float4* __restrict__ pts, uint32_t n_max, const uint32_t* n_dev
 // prefix-max over a sortable key, and one thread walks that short list (a handful of entries,
 // one log() each) instead of all num_iterations hypotheses.
 // info = {best iteration | 0xffffffff, n_inliers (filled later), 0, 0}; plane8[4..7] = winner.
-__device__ __noinline__ void rs_select_cta(const double* __restrict__ planes_in, const unsigned long long* scores_in,
-                                           uint32_t n_rows, uint32_t row_stride, uint32_t P, uint32_t ransac_n,
-                                           uint32_t iters, double log1mp, double* __restrict__ plane8,
-                                           uint32_t* __restrict__ info, unsigned long long* __restrict__ scores_copy) {
+// scores = {inliers, error} of every hypothesis, summed over the points by the column CTAs.
+__device__ __noinline__ void rs_select_cta(const double* __restrict__ planes_in, const unsigned long long* scores,
+                                           uint32_t P, uint32_t ransac_n, uint32_t iters, double log1mp,
+                                           double* __restrict__ plane8, uint32_t* __restrict__ info) {
   const double* planes = planes_in;                 // written by k_rs_hypotheses, the previous launch
   __shared__ unsigned long long s_wmax[APC_TILE_THREADS / 32];
   __shared__ unsigned long long s_carry;             // best key of all earlier chunks
-  __shared__ uint32_t s_rec_it[RS_SELECT_CHUNK];     // prefix records of the current chunk, in order
-  __shared__ double s_rec_break[RS_SELECT_CHUNK];    // early-stop bound each record would set
+  __shared__ uint32_t s_rec_it[APC_TILE_THREADS];    // prefix records of the current chunk, in order
+  __shared__ double s_rec_break[APC_TILE_THREADS];   // early-stop bound each record would set
   __shared__ uint32_t s_nrec;
   __shared__ uint32_t sb_it;
   __shared__ double sb_break;
@@ -430,30 +472,16 @@ __device__ __noinline__ void rs_select_cta(const double* __restrict__ planes_in,
   const uint32_t tid = threadIdx.x, lane = tid & 31u, warp = tid >> 5;
   if (tid == 0) { s_carry = 0; sb_it = 0xffffffffu; sb_break = (double)iters; sb_stop = false; }
   __syncthreads();
-  __shared__ ulonglong2 s_half[APC_TILE_THREADS / 2];
-  for (uint32_t c0 = 0; c0 < iters; c0 += APC_TILE_THREADS / 2) {
-    // a chunk of 128 hypotheses: both halves of the CTA add up every other row of the tally table
-    // (two independent load streams per hypothesis), the upper half hands its sums over in smem
-    const uint32_t it = c0 + (tid & 127u);
-    unsigned long long key = 0, inl = 0, err = 0;
+  for (uint32_t c0 = 0; c0 < iters; c0 += APC_TILE_THREADS) {
+    // a chunk of 256 hypotheses, one per thread
+    const uint32_t it = c0 + tid;
+    unsigned long long key = 0, inl = 0;
     if (it < iters) {
-#pragma unroll 13
-      for (uint32_t r = tid >> 7; r < n_rows; r += 2) {   // integer sums: the order is immaterial
-        const ulonglong2 v = __ldcg(reinterpret_cast<const ulonglong2*>(scores_in) + (size_t)r * row_stride + it);
-        inl += v.x;
-        err += v.y;
-      }
-    }
-    if (tid >= 128) s_half[tid - 128] = make_ulonglong2(inl, err);
-    __syncthreads();
-    if (tid >= 128) { inl = 0; err = 0; }
-    if (tid < 128 && it < iters) {
-      inl += s_half[tid].x;
-      err += s_half[tid].y;
+      const ulonglong2 v = __ldcg(reinterpret_cast<const ulonglong2*>(scores) + it);
+      inl = v.x;
+      const unsigned long long err = v.y;
       const double* pl = planes + 4 * (size_t)it;
       const bool valid = !(pl[0] == 0.0 && pl[1] == 0.0 && pl[2] == 0.0 && pl[3] == 0.0);
-      scores_copy[2 * (size_t)it] = inl;
-      scores_copy[2 * (size_t)it + 1] = err;
       // more inliers first, then the smaller error: inl < 2^23, err < 2^40 (4M points x 2^16)
       if (valid && inl > 0) key = (inl << 40) | (0xffffffffffull - (err < 0xffffffffffull ? err : 0xffffffffffull));
     }
@@ -691,13 +719,13 @@ int apc_segment_plane_nobegin(apc_ctx* ctx, const float* xyzi, uint32_t n_max, c
   {
     APC_PROF(ctx, "k_rs_hypotheses", s);
     apc_klaunch(ctx, k_rs_hypotheses, apc_div_up(iters, RS_HYP_THREADS), RS_HYP_THREADS, 0, s, pts, n_max, n_dev, ransac_n, iters, seed, table,
-                                                                              ctx->rs_planes);
+                                                                              ctx->rs_planes, ctx->rs_col_tickets);
   }
   {
     APC_PROF(ctx, "k_rs_score", s);
 #define RS_LAUNCH(CHV)                                                                                              \
   apc_klaunch(ctx, k_rs_score<CHV>, grid, APC_TILE_THREADS, 0, s, pts, n_max, n_dev, ransac_n, iters, ctx->rs_planes, thr, ctx->rs_scores, \
-                                                    log1mp, out_plane, out_info, ctx->rs_scores_copy, ctx->ctrl)
+                                                    log1mp, out_plane, out_info, ctx->rs_scores_copy, ctx->rs_col_tickets, ctx->ctrl)
     if (ch == 20) RS_LAUNCH(20);
     else if (ch == 16) RS_LAUNCH(16);
     else if (ch == 10) RS_LAUNCH(10);

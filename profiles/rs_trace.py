@@ -26,8 +26,10 @@ for k, name in [(1,"prologue"),(2,"scoring"),(3,"flush"),(4,"atom+ticket")]:
     x = a[:,k]-a[:,k-1]
     print(name, "min/med/max ns", x.min(), np.median(x), x.max())
 print("end (stamp4) min/med/max", d[:,4].min(), np.median(d[:,4]), d[:,4].max())
-last = a[a[:,5]>0]
-print("epilogue ns", (last[:,5]-last[:,4]), "end at", last[:,5]-t0)
+col = a[a[:,5]>0]      # the last CTA of each chunk column: its column's tally sum
+print("column sum ns", (col[:,5]-col[:,4]), "end at", col[:,5]-t0)
+last = a[a[:,6]>0]     # the CTA of the last column: the selection
+print("selection ns", (last[:,6]-last[:,5]), "end at", last[:,6]-t0)
 buf2 = None
 sm = a[:, 7]
 order = np.argsort(sm, kind="stable")

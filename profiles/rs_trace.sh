@@ -1,6 +1,6 @@
 #!/bin/bash
-# phase breakdown of k_rs_score (prologue / scoring / flush / ticket / selection) from %globaltimer stamps
-# usage: gpurun --timeout 900 -- 'bash profiles/rs_trace.sh TAG'
+# phase breakdown of k_rs_score (prologue / scoring / flush / ticket / column sums / selection) from %globaltimer stamps
+# usage: bash profiles/rs_trace.sh TAG
 TAG=${1:-r2}
 O=gpurun_out
 mkdir -p $O
