@@ -22,7 +22,7 @@ APC_OK, APC_ERR_CUDA, APC_ERR_BAD_ARG, APC_ERR_KEY_RANGE, APC_ERR_CAPACITY, APC_
 CROP_NUMPY, CROP_TORCH, CROP_OPEN3D = 0, 1, 2
 DEDUP_OFF, DEDUP_OPEN3D, DEDUP_NUMPY, DEDUP_TORCH_COMPAT = 0, 1, 2, 3
 STAGE_NANSKIP, STAGE_DEDUP, STAGE_FINITE, STAGE_CROP = 1, 2, 4, 8
-APC_ICP_POINT_TO_POINT, APC_ICP_POINT_TO_PLANE = 0, 1
+APC_ICP_POINT_TO_POINT, APC_ICP_POINT_TO_PLANE, APC_ICP_GENERALIZED = 0, 1, 2
 APC_ICP_OK, APC_ICP_NO_CORRESPONDENCE, APC_ICP_DEGENERATE = 0, 1, 2
 (CNT_INPUT, CNT_FILTERED, CNT_VOXELS, CNT_AFTER_STAT, CNT_AFTER_RADIUS, CNT_GROUND_INLIERS, CNT_OUTPUT,
  CNT_STATUS) = range(8)
@@ -108,6 +108,8 @@ def _load():
         "apc_cluster_dbscan": [vp, vp, u32, vp, f64, i32, vp, vp, vp, vp],
         "apc_evaluate_registration": [vp, vp, u32, vp, vp, u32, vp, f64, C.POINTER(f64), vp, vp, vp, vp],
         "apc_icp": [vp, vp, u32, vp, vp, vp, u32, vp, f64, C.POINTER(f64), i32, i32, f64, f64, vp, vp, vp, vp, vp],
+        "apc_icp_generalized": [vp, vp, vp, u32, vp, vp, vp, u32, vp, f64, C.POINTER(f64), f64, i32, f64, f64, vp, vp,
+                                vp, vp, vp, vp, vp],
         "apc_segment_plane": [vp, vp, u32, vp, f64, i32, i32, f64, C.c_uint64, vp, vp, vp, vp, vp],
         "apc_segment_plane_scores": [vp, vp, u32, vp],
         "apc_repack": [vp, vp, u32, vp, C.POINTER(OutField), u32, u32, vp, vp],
@@ -149,7 +151,7 @@ SYMBOLS = ["apc_ctx_create", "apc_ctx_destroy", "apc_ctx_set_low_latency", "apc_
            "apc_non_finite_mask", "apc_duplicate_mask", "apc_unique_rows", "apc_select_by_mask", "apc_gather",
            "apc_voxel_downsample", "apc_voxel_downsample_sorted", "apc_voxel_mean_attr", "apc_radius_outliers",
            "apc_statistical_outliers", "apc_estimate_normals", "apc_estimate_normals_knn",
-           "apc_estimate_normals_radius", "apc_cluster_dbscan", "apc_evaluate_registration", "apc_icp", "apc_segment_plane", "apc_segment_plane_scores", "apc_repack", "apc_pipeline_run", "apc_pipeline_run_maps",
+           "apc_estimate_normals_radius", "apc_cluster_dbscan", "apc_evaluate_registration", "apc_icp", "apc_icp_generalized", "apc_segment_plane", "apc_segment_plane_scores", "apc_repack", "apc_pipeline_run", "apc_pipeline_run_maps",
            "apc_pipeline_run_mirrored", "apc_pipeline_run_ex", "apc_graph_capture_pipeline_ex",
            "apc_graph_capture_pipeline", "apc_graph_capture_pipeline_mirrored",
            "apc_graph_launch", "apc_graph_destroy",

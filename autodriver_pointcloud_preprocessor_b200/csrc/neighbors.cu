@@ -1308,6 +1308,7 @@ struct NeighborScratch {
   uint8_t* dbscan_core = nullptr;      // [max_points] core flags
   double* icp_part = nullptr;          // [ICP_MAX_BLOCKS][32] block partials of k_icp_match's moments
   struct IcpState* icp_state = nullptr;   // apc_icp's T, previous metrics and done flag
+  double* gicp_axes[2] = {nullptr, nullptr};   // [max_points][3] regularisation axes of apc_icp_generalized's source, target
 };
 // one scratch set per context, owned by the context (created on first use, freed by apc_ctx_destroy)
 static NeighborScratch* scratch_of(apc_ctx* ctx) {
@@ -1329,7 +1330,7 @@ void apc_neighbors_release(apc_ctx* ctx) {
   void* dbscan[] = {s->dbscan_parent, s->dbscan_id, s->dbscan_core};
   for (void* p : dbscan)
     if (p) cudaFree(p);
-  void* icp[] = {s->icp_part, s->icp_state};
+  void* icp[] = {s->icp_part, s->icp_state, s->gicp_axes[0], s->gicp_axes[1]};
   for (void* p : icp)
     if (p) cudaFree(p);
   delete s;
@@ -3019,5 +3020,165 @@ extern "C" int apc_icp(apc_ctx* ctx, const float* src_xyzi, uint32_t n_src, cons
                                    sc->icp_state, out_T16_dev, out_stats_dev, out_info_dev);
   }
   APC_LAUNCH_CHECK(ctx, "icp");
+  return icp_finish(ctx, n_tgt, n_tgt_dev, s);
+}
+
+// ---- Generalized ICP (Open3D t::pipelines::registration::TransformationEstimationForGeneralizedICP) ------------
+// Contract (oracle/gicp.py): matching, metrics, the loop and the solve are those of point-to-plane; only
+// the per-correspondence system differs.  Every point's covariance gives one regularisation axis a (the
+// eigenvector of its smallest eigenvalue, normal_from_covariance; NaN when an entry is not finite), and Segal's
+// regularised covariance U diag(1, 1, eps) U^T is I - (1 - eps) a a^T.  For s' matched to t:
+//   m = R a_s (R the upper-left 3x3 of the accumulated T), M = 2I - (1 - eps)(m m^T + a_t a_t^T), W = M^-1,
+//   e = s' - t, J = [-[s']x | I]; H = sum J^T W J, b = sum J^T W e, then H x = -b as in point-to-plane.
+//   k_gicp_prep       one thread per point of both clouds, once per call: covariance -> axis (context scratch)
+//   k_icp_match_gicp  the matching of k_icp_match; lane k accumulates entry k of (n, sum d2, H, b) in
+//                     point-to-plane's layout (c_icp_pairs[APC_ICP_POINT_TO_PLANE]), from s', m, a_t and e
+//   k_icp_solve       unchanged, launched as point-to-plane
+__global__ void __launch_bounds__(256)
+k_gicp_prep(const float* __restrict__ src_cov, uint32_t n_src_max, const uint32_t* n_src_dev,
+            const float* __restrict__ tgt_cov, uint32_t n_tgt_max, const uint32_t* n_tgt_dev, double* __restrict__ src_axes,
+            double* __restrict__ tgt_axes, double* __restrict__ out_src_axes, double* __restrict__ out_tgt_axes) {
+  const uint32_t ns = apc_count(n_src_dev, n_src_max), nt = apc_count(n_tgt_dev, n_tgt_max);
+  for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < ns + nt; i += gridDim.x * blockDim.x) {
+    const bool is_src = i < ns;
+    const size_t k = is_src ? i : i - ns;
+    const float* cov = (is_src ? src_cov : tgt_cov) + 9 * k;
+    double C[9], a[3];
+    bool finite = true;
+#pragma unroll
+    for (int u = 0; u < 9; ++u) {
+      C[u] = cov[u];
+      finite = finite && isfinite(C[u]);
+    }
+    if (finite) normal_from_covariance(C, a);
+    else a[0] = a[1] = a[2] = __longlong_as_double(0x7ff8000000000000ll);
+    double* axes = is_src ? src_axes : tgt_axes;
+    double* out = is_src ? out_src_axes : out_tgt_axes;
+#pragma unroll
+    for (int u = 0; u < 3; ++u) {
+      axes[3 * k + u] = a[u];
+      if (out) out[3 * k + u] = a[u];
+    }
+  }
+}
+
+__global__ void __launch_bounds__(128)
+k_icp_match_gicp(const float4* __restrict__ src, uint32_t n_max, const uint32_t* n_dev, const float4* __restrict__ tgt,
+                 const double* __restrict__ src_axes, const double* __restrict__ tgt_axes, GridDev g, float r2,
+                 double one_minus_eps, const IcpState* __restrict__ st, int32_t* __restrict__ corr_out,
+                 double* __restrict__ partials) {
+  if (st->done) return;                                     // the loop has stopped: block-uniform
+  __shared__ double sm[4][32];
+  const uint32_t n = apc_count(n_dev, n_max);
+  const float c = grid_cell_size(g, 0);
+  const uint32_t lane = threadIdx.x & 31u, warp = threadIdx.x >> 5;
+  // lane k: J_pa . W V_pb with V_b = J_b (b < 6) or e (b = 6); pa 7: n, pa 8: sum d2, pa 9: unused lanes
+  const uint32_t pair = c_icp_pairs[APC_ICP_POINT_TO_PLANE][lane], pa = pair & 15u, pb = pair >> 4;
+  double T[12];
+#pragma unroll
+  for (int k = 0; k < 12; ++k) T[k] = st->T[k];
+  double acc = 0.0;
+  for (uint32_t i = (blockIdx.x * blockDim.x + threadIdx.x) >> 5; i < n; i += (gridDim.x * blockDim.x) >> 5) {
+    // the matching of k_icp_match
+    const float4 p = src[i];
+    const double x = p.x, y = p.y, z = p.z;
+    const float4 q = make_float4(icp_row(T, 0, x, y, z), icp_row(T, 1, x, y, z), icp_row(T, 2, x, y, z), 0.0f);
+    uint32_t cs, ps;
+    const uint32_t total = flat27_runs_outside(g, c, q, lane, cs, ps);
+    uint64_t best = ~0ull;
+    for (uint32_t base = 0; base < total; base += 32) {
+      const uint32_t ci = base + lane;
+      const uint32_t at = flat27_at(cs, ps, min(ci, total - 1u));
+      if (ci < total) {
+        const float4 t = g.sorted[at];
+        const float d2 = d2_f32(q.x, q.y, q.z, t.x, t.y, t.z);
+        if (d2 <= r2) best = min(best, ((uint64_t)__float_as_uint(d2) << 32) | __float_as_uint(t.w));
+      }
+    }
+    best = warp_min_u64(best);
+    const bool found = best != ~0ull;                       // warp-uniform
+    const uint32_t j = (uint32_t)best;
+    if (found) {
+      const float4 t = tgt[j];
+      const double sx = q.x, sy = q.y, sz = q.z;
+      const double ex = sx - t.x, ey = sy - t.y, ez = sz - t.z;
+      const double as0 = src_axes[3 * (size_t)i], as1 = src_axes[3 * (size_t)i + 1], as2 = src_axes[3 * (size_t)i + 2];
+      const double a0 = tgt_axes[3 * (size_t)j], a1 = tgt_axes[3 * (size_t)j + 1], a2 = tgt_axes[3 * (size_t)j + 2];
+      const double m0 = (T[0] * as0 + T[1] * as1) + T[2] * as2, m1 = (T[4] * as0 + T[5] * as1) + T[6] * as2,
+                   m2 = (T[8] * as0 + T[9] * as1) + T[10] * as2;
+      const double k = one_minus_eps;
+      const double M00 = 2.0 - k * (m0 * m0 + a0 * a0), M11 = 2.0 - k * (m1 * m1 + a1 * a1),
+                   M22 = 2.0 - k * (m2 * m2 + a2 * a2), M01 = -k * (m0 * m1 + a0 * a1), M02 = -k * (m0 * m2 + a0 * a2),
+                   M12 = -k * (m1 * m2 + a1 * a2);
+      // W = adj(M) / det(M)
+      const double A00 = M11 * M22 - M12 * M12, A01 = M02 * M12 - M01 * M22, A02 = M01 * M12 - M02 * M11;
+      const double inv = 1.0 / ((M00 * A00 + M01 * A01) + M02 * A02);
+      const double W00 = A00 * inv, W01 = A01 * inv, W02 = A02 * inv, W11 = (M00 * M22 - M02 * M02) * inv,
+                   W12 = (M01 * M02 - M00 * M12) * inv, W22 = (M00 * M11 - M01 * M01) * inv;
+      // V_pb: J_b = e_b x s' (b < 3), the unit vector e_(b-3) (3 <= b < 6), or e (b = 6)
+      const double vx = pb == 6 ? ex : pb == 3 ? 1.0 : pb == 1 ? sz : pb == 2 ? -sy : 0.0;
+      const double vy = pb == 6 ? ey : pb == 4 ? 1.0 : pb == 0 ? -sz : pb == 2 ? sx : 0.0;
+      const double vz = pb == 6 ? ez : pb == 5 ? 1.0 : pb == 0 ? sy : pb == 1 ? -sx : 0.0;
+      const double wx = (W00 * vx + W01 * vy) + W02 * vz, wy = (W01 * vx + W11 * vy) + W12 * vz,
+                   wz = (W02 * vx + W12 * vy) + W22 * vz;
+      // J_a . w: (e_a x s') . w = (s' x w)_a for a < 3, w_(a-3) otherwise
+      double val = pa == 0 ? sy * wz - sz * wy : pa == 1 ? sz * wx - sx * wz : pa == 2 ? sx * wy - sy * wx
+                 : pa == 3 ? wx : pa == 4 ? wy : wz;
+      val = pa == 7 ? 1.0 : pa == 8 ? (double)__uint_as_float((uint32_t)(best >> 32)) : pa == 9 ? 0.0 : val;
+      acc += val;
+    }
+    if (lane == 0 && corr_out) corr_out[i] = found ? (int32_t)j : -1;
+  }
+  sm[warp][lane] = acc;
+  __syncthreads();
+  if (threadIdx.x < 32) partials[32 * (size_t)blockIdx.x + lane] = ((sm[0][lane] + sm[1][lane]) + sm[2][lane]) + sm[3][lane];
+}
+
+extern "C" int apc_icp_generalized(apc_ctx* ctx, const float* src_xyzi, const float* src_cov, uint32_t n_src,
+                                   const uint32_t* n_src_dev, const float* tgt_xyzi, const float* tgt_cov, uint32_t n_tgt,
+                                   const uint32_t* n_tgt_dev, double max_correspondence_distance,
+                                   const double* init_T16_host, double epsilon, int max_iteration, double relative_fitness,
+                                   double relative_rmse, double* out_T16_dev, double* out_stats_dev, int32_t* out_info_dev,
+                                   int32_t* out_correspondences, double* out_src_axes_dev, double* out_tgt_axes_dev,
+                                   void* stream) {
+  if (!ctx) return APC_ERR_BAD_ARG;
+  APC_REQUIRE(ctx, out_T16_dev && out_info_dev, "NULL pointer");
+  APC_REQUIRE(ctx, max_iteration >= 0, "max_iteration must be >= 0");
+  APC_REQUIRE(ctx, src_cov && tgt_cov, "generalized ICP needs the covariances of both clouds");
+  APC_REQUIRE(ctx, std::isfinite(epsilon) && epsilon > 0.0, "epsilon must be finite and > 0");
+  NeighborScratch* sc = scratch_of(ctx);
+  for (double*& axes : sc->gicp_axes)       // before the first launch: the call can be captured in a graph
+    if (!axes) APC_CUDA(ctx, cudaMalloc((void**)&axes, (size_t)ctx->max_points * 3 * sizeof(double)));
+  cudaStream_t s = (cudaStream_t)stream;
+  bool empty = false;
+  int rc = icp_begin(ctx, src_xyzi, n_src, tgt_xyzi, n_tgt, n_tgt_dev, max_correspondence_distance, init_T16_host,
+                     out_stats_dev, out_correspondences, nullptr, out_T16_dev, out_info_dev,
+                     max_iteration > 0 ? APC_ICP_NO_CORRESPONDENCE : APC_ICP_OK, &empty, s);
+  if (rc) return rc;
+  if (out_src_axes_dev && n_src) APC_CUDA(ctx, cudaMemsetAsync(out_src_axes_dev, 0, (size_t)n_src * 3 * sizeof(double), s));
+  if (out_tgt_axes_dev && n_tgt) APC_CUDA(ctx, cudaMemsetAsync(out_tgt_axes_dev, 0, (size_t)n_tgt * 3 * sizeof(double), s));
+  if (empty) return APC_OK;
+  {
+    APC_PROF(ctx, "k_gicp_prep", s);
+    k_gicp_prep<<<min(apc_div_up(n_src + n_tgt, 256), (uint32_t)APC_SM_COUNT * 8), 256, 0, s>>>(
+        src_cov, n_src, n_src_dev, tgt_cov, n_tgt, n_tgt_dev, sc->gicp_axes[0], sc->gicp_axes[1], out_src_axes_dev,
+        out_tgt_axes_dev);
+  }
+  const float r32 = (float)max_correspondence_distance;
+  const uint32_t bq = icp_blocks(n_src);
+  for (int j = 0; j < max_iteration; ++j) {
+    {
+      APC_PROF(ctx, "k_icp_match_gicp", s);
+      k_icp_match_gicp<<<bq, 128, 0, s>>>(reinterpret_cast<const float4*>(src_xyzi), n_src, n_src_dev,
+                                          reinterpret_cast<const float4*>(tgt_xyzi), sc->gicp_axes[0], sc->gicp_axes[1],
+                                          sc->grid[0].d, r32 * r32, 1.0 - epsilon, sc->icp_state, out_correspondences,
+                                          sc->icp_part);
+    }
+    APC_PROF(ctx, "k_icp_solve", s);
+    k_icp_solve<<<1, ICP_SOLVE_WARPS * 32, 0, s>>>(sc->icp_part, bq, n_src, n_src_dev, APC_ICP_POINT_TO_PLANE, j,
+                                                   relative_fitness, relative_rmse, sc->icp_state, out_T16_dev,
+                                                   out_stats_dev, out_info_dev);
+  }
+  APC_LAUNCH_CHECK(ctx, "icp_generalized");
   return icp_finish(ctx, n_tgt, n_tgt_dev, s);
 }

@@ -375,6 +375,27 @@ class Context:
                              _ptr(info), _ptr(corr), _stream()))
         return T, stats, info, corr[:n_src]
 
+    def icp_generalized(self, src_xyzi, src_cov, tgt_xyzi, tgt_cov, max_correspondence_distance, init=None,
+                        epsilon=1e-3, max_iteration=30, relative_fitness=1e-6, relative_rmse=1e-6, want_axes=False,
+                        n_src_dev=None, n_tgt_dev=None):
+        """``apc_icp_generalized`` with float32 covariances ``[n, 3, 3]`` (contiguous, on the device).  Returns the
+        tuple of :meth:`icp`, plus the regularisation axes ``(float64[n_src, 3], float64[n_tgt, 3])`` when
+        ``want_axes``; no host synchronisation."""
+        n_src, n_tgt = src_xyzi.shape[0], tgt_xyzi.shape[0]
+        T = self._empty((4, 4), torch.float64)
+        stats = self._empty((2,), torch.float64)
+        info = self._empty((4,), torch.int32)
+        corr = self._empty((max(n_src, 1),), torch.int32)
+        axes_s = self._empty((max(n_src, 1), 3), torch.float64) if want_axes else None
+        axes_t = self._empty((max(n_tgt, 1), 3), torch.float64) if want_axes else None
+        self._ok(lib.apc_icp_generalized(self.h, _ptr(src_xyzi), _ptr(src_cov), n_src, _ptr(n_src_dev), _ptr(tgt_xyzi),
+                                         _ptr(tgt_cov), n_tgt, _ptr(n_tgt_dev), float(max_correspondence_distance),
+                                         _t16(init), float(epsilon), int(max_iteration), float(relative_fitness),
+                                         float(relative_rmse), _ptr(T), _ptr(stats), _ptr(info), _ptr(corr),
+                                         _ptr(axes_s), _ptr(axes_t), _stream()))
+        out = (T, stats, info, corr[:n_src])
+        return out + (axes_s[:n_src], axes_t[:n_tgt]) if want_axes else out
+
     # ---- ransac ------------------------------------------------------------------------------------
     def segment_plane(self, xyzi, distance_threshold, ransac_n, num_iterations, probability, seed=0,
                       sample_table=None, n_dev=None):

@@ -274,6 +274,28 @@ class PointCloud:
         self.point["normals"] = self._home(normals.contiguous())
         return self
 
+    def estimate_covariances(self, max_nn=20, radius=None):
+        """Open3D ``estimate_covariances``: sets ``point['covariances']`` (float32 N x 3 x 3) to the covariance of
+        every point's neighbourhood, the float32 rounding of what ``estimate_normals`` computes with the same
+        arguments; ``normals`` are left alone.  The search follows the arguments as in :meth:`estimate_normals`,
+        with the same ranges (both: hybrid; ``max_nn`` only: KNN; ``radius`` only: every point within it;
+        neither: ``ValueError``).  A point with fewer than 3 neighbours gets the identity.
+
+        :meth:`transform` does not rotate covariances: estimate them in the frame the cloud is registered in."""
+        if radius is None and max_nn is None:
+            raise ValueError("estimate_covariances needs max_nn, radius or both")
+        if self._n() == 0:
+            self.point["covariances"] = self._home(torch.zeros((0, 3, 3), dtype=torch.float32, device="cuda"))
+            return self
+        if radius is None:
+            _, _, cov = self._ctx().estimate_normals_knn(self._xyzi(), int(max_nn), want_cov=True)
+        elif max_nn is None:
+            _, _, cov = self._ctx().estimate_normals_radius(self._xyzi(), float(radius), want_cov=True)
+        else:
+            _, _, cov = self._ctx().estimate_normals(self._xyzi(), int(max_nn), float(radius), want_cov=True)
+        self.point["covariances"] = self._home(cov.to(torch.float32).contiguous())
+        return self
+
     def __repr__(self):
         n = 0 if self.is_empty() else len(self.point["positions"])
         return f"PointCloud on {self.device} [{n} points] attributes: {sorted(k for k in self.point if k != 'positions')}"

@@ -1,16 +1,20 @@
-"""``open3d.t.pipelines.registration`` look-alike: single-scale ICP and ``evaluate_registration`` on the GPU.
+"""``open3d.t.pipelines.registration`` look-alike: single-scale ICP (point-to-point, point-to-plane, generalized) and
+``evaluate_registration`` on the GPU.
 
 The whole ICP loop runs on the device (``apc_icp``): the call synchronises once, at the end.  Definitions, and
-where they differ from Open3D, are in ``oracle/registration.py``; in short:
+where they differ from Open3D, are in ``oracle/registration.py`` and ``oracle/gicp.py``; in short:
 
 * every iteration transforms the original source by the float64 transform accumulated so far and rounds to
   float32 (Open3D re-transforms its float32 cloud in place);
 * a source point's correspondence is the nearest target point by the float32 squared distance with ties to the
   lower index, kept when ``d2 <= float32(max_correspondence_distance)^2`` (Open3D: ``d2 < r^2``);
-* point-to-plane stops with ``RuntimeError`` when its 6x6 system is not positive definite (every normal parallel,
-  for example), where Open3D would solve it anyway.
+* point-to-plane and generalized ICP stop with ``RuntimeError`` when their 6x6 system is not positive definite (every
+  normal parallel, for example), where Open3D would solve it anyway;
+* generalized ICP takes only each covariance's axis of least variance, and regularises it as Segal et al. do
+  (``I - (1 - epsilon) a a^T``).  An isotropic covariance has no such axis: the identity that neighbourhoods of
+  fewer than 3 points get is treated as a horizontal plane.
 
-Not modelled: multi-scale ICP, colored / generalized ICP, robust kernels and per-iteration callbacks.
+Not modelled: multi-scale ICP, colored ICP, robust kernels and per-iteration callbacks.
 """
 from __future__ import annotations
 
@@ -40,6 +44,26 @@ class TransformationEstimationPointToPlane:
 
     def __repr__(self):
         return "TransformationEstimationPointToPlane"
+
+
+class TransformationEstimationForGeneralizedICP:
+    """Generalized ICP (Segal et al. 2009, plane-to-plane): one Gauss-Newton step of ``sum e^T W e`` per iteration,
+    ``W = (R C_s R^T + C_t)^-1`` from the regularised covariances of both clouds (``point['covariances']``, or
+    estimated with :meth:`PointCloud.estimate_covariances` defaults when a cloud has none).  ``epsilon`` is the
+    variance kept along each covariance's axis of least variance."""
+    method = _capi.APC_ICP_GENERALIZED
+
+    def __init__(self, epsilon=1e-3, kernel=None):
+        if kernel is not None:
+            raise NotImplementedError("robust kernels are not modelled")
+        epsilon = float(epsilon)
+        if not (math.isfinite(epsilon) and epsilon > 0):
+            raise ValueError("epsilon must be finite and > 0")
+        self.epsilon = epsilon
+        self.kernel = None
+
+    def __repr__(self):
+        return f"TransformationEstimationForGeneralizedICP(epsilon={self.epsilon})"
 
 
 class ICPConvergenceCriteria:
@@ -95,6 +119,19 @@ def _result(source: PointCloud, T, stats, corr, info=None) -> RegistrationResult
                               bool(info[1]) if info is not None else False, int(info[0]) if info is not None else 0)
 
 
+def _covariances(cloud: PointCloud) -> torch.Tensor:
+    """float32 ``[n, 3, 3]`` on the GPU: the cloud's ``covariances``, or ``estimate_covariances()`` of its positions
+    (the cloud itself is not modified)."""
+    if "covariances" not in cloud.point:
+        cov = cloud._like({"positions": cloud.point["positions"]}).estimate_covariances().point["covariances"]
+    else:
+        cov = cloud.point["covariances"]
+    cov = PointCloud._gpu(cov).to(torch.float32).contiguous()
+    if tuple(cov.shape) != (cloud._n(), 3, 3):
+        raise ValueError(f"covariances must be [{cloud._n()}, 3, 3], got {tuple(cov.shape)}")
+    return cov
+
+
 def evaluate_registration(source: PointCloud, target: PointCloud, max_correspondence_distance,
                           transformation=None) -> RegistrationResult:
     """Open3D ``evaluate_registration``: fitness, inlier rmse and correspondences of ``source`` moved by
@@ -115,8 +152,14 @@ def icp(source: PointCloud, target: PointCloud, max_correspondence_distance, ini
         estimation_method=None, criteria=None, voxel_size=-1.0, callback_after_iteration=None) -> RegistrationResult:
     """Open3D ``icp`` (single scale).  ``voxel_size > 0`` downsamples both clouds first, as Open3D does.  Raises
     ``RuntimeError`` when an iteration finds no correspondence, when point-to-plane runs on a target without
-    ``normals`` or its system is degenerate, and ``NotImplementedError`` for ``callback_after_iteration`` (the
-    loop never returns to the host)."""
+    ``normals`` or its system (or generalized ICP's) is degenerate, and ``NotImplementedError`` for
+    ``callback_after_iteration`` (the loop never returns to the host).
+
+    Generalized ICP uses each cloud's ``covariances`` when present and otherwise estimates them with
+    ``estimate_covariances()`` defaults; the caller's clouds are not modified.  With ``voxel_size > 0`` they are
+    always estimated on the downsampled clouds: a voxel mean of covariances keeps at most 20 fractional bits
+    (about 1e-6), the size of a planar neighbourhood's smallest eigenvalue, so averaged covariances lose their
+    planes."""
     if callback_after_iteration is not None:
         raise NotImplementedError("callback_after_iteration: the ICP loop runs on the GPU without visiting the host")
     _check_distance(max_correspondence_distance)
@@ -125,7 +168,10 @@ def icp(source: PointCloud, target: PointCloud, max_correspondence_distance, ini
     if crit.max_iteration < 0:
         raise ValueError("max_iteration must be >= 0")
     T0 = _transform(init_source_to_target)
+    generalized = estimation.method == _capi.APC_ICP_GENERALIZED
     if voxel_size > 0:
+        if generalized:                          # not carried: estimated on the downsampled clouds below
+            source, target = (c._like({k: v for k, v in c.point.items() if k != "covariances"}) for c in (source, target))
         source, target = source.voxel_down_sample(voxel_size), target.voxel_down_sample(voxel_size)
     point_to_plane = estimation.method == _capi.APC_ICP_POINT_TO_PLANE
     if point_to_plane and "normals" not in target.point:
@@ -135,17 +181,23 @@ def icp(source: PointCloud, target: PointCloud, max_correspondence_distance, ini
     if n_src == 0 or n_tgt == 0:
         raise RuntimeError("Source and/or Target pointcloud is empty.")
     ctx = get_context(max(n_src, n_tgt), source.device.index if source.device.kind == "CUDA" else None)
-    normals = None
-    if point_to_plane:
-        normals = PointCloud._gpu(target.point["normals"]).to(torch.float32).contiguous()
-    T, stats, info, corr = ctx.icp(source._xyzi(), target._xyzi(), float(max_correspondence_distance), T0,
-                                   estimation.method, normals, crit.max_iteration, crit.relative_fitness,
-                                   crit.relative_rmse)
+    if generalized:
+        src_cov, tgt_cov = _covariances(source), _covariances(target)
+        T, stats, info, corr = ctx.icp_generalized(source._xyzi(), src_cov, target._xyzi(), tgt_cov,
+                                                   float(max_correspondence_distance), T0, estimation.epsilon,
+                                                   crit.max_iteration, crit.relative_fitness, crit.relative_rmse)
+    else:
+        normals = None
+        if point_to_plane:
+            normals = PointCloud._gpu(target.point["normals"]).to(torch.float32).contiguous()
+        T, stats, info, corr = ctx.icp(source._xyzi(), target._xyzi(), float(max_correspondence_distance), T0,
+                                       estimation.method, normals, crit.max_iteration, crit.relative_fitness,
+                                       crit.relative_rmse)
     ctx.check()                                   # the one synchronisation of the call
     info = info.cpu().numpy()
     if info[2] == _capi.APC_ICP_NO_CORRESPONDENCE:
         raise RuntimeError(_NO_CORRESPONDENCE)
     if info[2] == _capi.APC_ICP_DEGENERATE:
-        raise RuntimeError("point-to-plane ICP: the linear system is not positive definite (degenerate geometry, "
-                           "e.g. all target normals parallel)")
+        raise RuntimeError(f"{'generalized' if generalized else 'point-to-plane'} ICP: the linear system is not "
+                           "positive definite (degenerate geometry, e.g. all target normals parallel)")
     return _result(source, T.cpu().numpy(), stats, corr, info)

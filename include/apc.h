@@ -290,7 +290,7 @@ int apc_cluster_dbscan(apc_ctx* ctx, const float* xyzi, uint32_t n_max, const ui
 
 /* ---- (3b) ICP registration (Open3D t.pipelines.registration) -------------------------- */
 
-enum { APC_ICP_POINT_TO_POINT = 0, APC_ICP_POINT_TO_PLANE = 1 };
+enum { APC_ICP_POINT_TO_POINT = 0, APC_ICP_POINT_TO_PLANE = 1, APC_ICP_GENERALIZED = 2 };
 enum { APC_ICP_OK = 0, APC_ICP_NO_CORRESPONDENCE = 1, APC_ICP_DEGENERATE = 2 };
 
 /* evaluate_registration(source, target, max_correspondence_distance, transformation) (Open3D
@@ -329,6 +329,28 @@ int apc_icp(apc_ctx* ctx, const float* src_xyzi, uint32_t n_src, const uint32_t*
             double max_correspondence_distance, const double* init_T16_host, int method, int max_iteration,
             double relative_fitness, double relative_rmse, double* out_T16_dev, double* out_stats_dev,
             int32_t* out_info_dev, int32_t* out_correspondences, void* stream);
+
+/* icp(source, target, max_correspondence_distance, init, TransformationEstimationForGeneralizedICP(epsilon),
+ * criteria) (Open3D t::pipelines::registration::ICP with TransformationEstimationForGeneralizedICP; the
+ * covariances are those of t::geometry::PointCloud::EstimateCovariances).  Matching, metrics, the loop, its
+ * statuses and outputs are those of apc_icp with APC_ICP_POINT_TO_PLANE; only the per-correspondence system
+ * differs (Segal et al. 2009, plane-to-plane).  Every point's regularisation axis a is the eigenvector of the
+ * smallest eigenvalue of its covariance (the solver of apc_estimate_normals; NaN when an entry is not finite), and
+ * its regularised covariance I - (1 - epsilon) a a^T = U diag(1, 1, epsilon) U^T.  For s' matched to t:
+ * W = (R C_s,reg R^T + C_t,reg)^-1 with R the rotation of the T accumulated so far, e = s' - t,
+ * J = [-[s']x | I]; one Gauss-Newton step of sum e^T W e solves (sum J^T W J) x = -(sum J^T W e) by Cholesky
+ * (APC_ICP_DEGENERATE when it is not positive definite or not finite).  An isotropic covariance has no defined
+ * axis: the identity (neighbourhoods of fewer than 3 points) gives (0, 0, 1), a zero covariance the axis 0 and so
+ * C_reg = I.  src_cov / tgt_cov float32[9 * n] (row-major 3x3 per point).  out_src_axes_dev / out_tgt_axes_dev
+ * double[3 * n] (may be NULL) receive the axes used, 0 beyond the device count or when a cloud is empty.  The
+ * axes are computed once per call (k_gicp_prep).  No host synchronisation; the call can be captured in a CUDA
+ * graph.  APC_ERR_BAD_ARG: everything apc_icp rejects, NULL covariances, epsilon not finite or not > 0. */
+int apc_icp_generalized(apc_ctx* ctx, const float* src_xyzi, const float* src_cov, uint32_t n_src, const uint32_t* n_src_dev,
+                        const float* tgt_xyzi, const float* tgt_cov, uint32_t n_tgt, const uint32_t* n_tgt_dev,
+                        double max_correspondence_distance, const double* init_T16_host, double epsilon, int max_iteration,
+                        double relative_fitness, double relative_rmse, double* out_T16_dev, double* out_stats_dev,
+                        int32_t* out_info_dev, int32_t* out_correspondences,
+                        double* out_src_axes_dev, double* out_tgt_axes_dev, void* stream);
 
 /* ---- (4) RANSAC ground plane --------------------------------------------------------- */
 
