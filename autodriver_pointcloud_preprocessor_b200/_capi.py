@@ -14,7 +14,7 @@ LIB_PATH = os.path.join(PKG, "libapc.so")
 
 APC_MAX_FIELDS = 16
 APC_MAX_CLOUDS = 8
-APC_MAX_NEIGHBORS = 1024   # statistical nb_neighbors and normals max_nn
+APC_MAX_NEIGHBORS = 1024   # statistical nb_neighbors, normals and FPFH max_nn
 APC_MAX_TRANSFORMS = 3
 APC_MAX_MIRRORS = 8
 
@@ -110,6 +110,9 @@ def _load():
         "apc_icp": [vp, vp, u32, vp, vp, vp, u32, vp, f64, C.POINTER(f64), i32, i32, f64, f64, vp, vp, vp, vp, vp],
         "apc_icp_generalized": [vp, vp, vp, u32, vp, vp, vp, u32, vp, f64, C.POINTER(f64), f64, i32, f64, f64, vp, vp,
                                 vp, vp, vp, vp, vp],
+        "apc_compute_fpfh": [vp, vp, vp, u32, vp, i32, f64, vp, vp, vp, vp],
+        "apc_compute_fpfh_knn": [vp, vp, vp, u32, vp, i32, vp, vp, vp, vp],
+        "apc_correspondences_from_features": [vp, vp, u32, vp, vp, u32, vp, i32, i32, f64, vp, vp, vp, vp],
         "apc_segment_plane": [vp, vp, u32, vp, f64, i32, i32, f64, C.c_uint64, vp, vp, vp, vp, vp],
         "apc_segment_plane_scores": [vp, vp, u32, vp],
         "apc_repack": [vp, vp, u32, vp, C.POINTER(OutField), u32, u32, vp, vp],
@@ -151,7 +154,8 @@ SYMBOLS = ["apc_ctx_create", "apc_ctx_destroy", "apc_ctx_set_low_latency", "apc_
            "apc_non_finite_mask", "apc_duplicate_mask", "apc_unique_rows", "apc_select_by_mask", "apc_gather",
            "apc_voxel_downsample", "apc_voxel_downsample_sorted", "apc_voxel_mean_attr", "apc_radius_outliers",
            "apc_statistical_outliers", "apc_estimate_normals", "apc_estimate_normals_knn",
-           "apc_estimate_normals_radius", "apc_cluster_dbscan", "apc_evaluate_registration", "apc_icp", "apc_icp_generalized", "apc_segment_plane", "apc_segment_plane_scores", "apc_repack", "apc_pipeline_run", "apc_pipeline_run_maps",
+           "apc_estimate_normals_radius", "apc_cluster_dbscan", "apc_evaluate_registration", "apc_icp", "apc_icp_generalized", "apc_compute_fpfh",
+           "apc_compute_fpfh_knn", "apc_correspondences_from_features", "apc_segment_plane", "apc_segment_plane_scores", "apc_repack", "apc_pipeline_run", "apc_pipeline_run_maps",
            "apc_pipeline_run_mirrored", "apc_pipeline_run_ex", "apc_graph_capture_pipeline_ex",
            "apc_graph_capture_pipeline", "apc_graph_capture_pipeline_mirrored",
            "apc_graph_launch", "apc_graph_destroy",

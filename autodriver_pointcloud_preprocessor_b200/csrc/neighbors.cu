@@ -1309,6 +1309,10 @@ struct NeighborScratch {
   double* icp_part = nullptr;          // [ICP_MAX_BLOCKS][32] block partials of k_icp_match's moments
   struct IcpState* icp_state = nullptr;   // apc_icp's T, previous metrics and done flag
   double* gicp_axes[2] = {nullptr, nullptr};   // [max_points][3] regularisation axes of apc_icp_generalized's source, target
+  float* spfh = nullptr;               // [max_points][33] SPFH between the two passes of apc_compute_fpfh(_knn)
+  unsigned long long* feat_best[2] = {nullptr, nullptr};   // [max_points] (d2 bits, index) minima of the feature search
+  int32_t* feat_pairs = nullptr;       // [max_points][2] mutually consistent pairs of apc_correspondences_from_features
+  uint32_t* feat_count = nullptr;      // [2] pair counts: all, mutual
 };
 // one scratch set per context, owned by the context (created on first use, freed by apc_ctx_destroy)
 static NeighborScratch* scratch_of(apc_ctx* ctx) {
@@ -1332,6 +1336,9 @@ void apc_neighbors_release(apc_ctx* ctx) {
     if (p) cudaFree(p);
   void* icp[] = {s->icp_part, s->icp_state, s->gicp_axes[0], s->gicp_axes[1]};
   for (void* p : icp)
+    if (p) cudaFree(p);
+  void* feat[] = {s->spfh, s->feat_best[0], s->feat_best[1], s->feat_pairs, s->feat_count};
+  for (void* p : feat)
     if (p) cudaFree(p);
   delete s;
   ctx->neighbors = nullptr;
@@ -3181,4 +3188,438 @@ extern "C" int apc_icp_generalized(apc_ctx* ctx, const float* src_xyzi, const fl
   }
   APC_LAUNCH_CHECK(ctx, "icp_generalized");
   return icp_finish(ctx, n_tgt, n_tgt_dev, s);
+}
+
+// ---- FPFH features (Open3D t::pipelines::registration::ComputeFPFHFeature) -----------------------------------
+// Contract (oracle/features.py).  Neighbourhoods are those of the normals stage: hybrid (the max_nn nearest within
+// float32(r)^2, k_normals_wide's walk) or KNN (the max_nn nearest, k_normals_knn's level climb + stragglers), kept
+// through a WarpKeep of (d2 bits << 32 | index) keys and sorted, so entry 0 is at d2 = 0 (the query or a duplicate).
+//   pass 0  the pair features (float64) of the query with entries 1..m-1 -> 33 bin counts in per-warp shared
+//           counters (integer: order-free) -> SPFH = count * (100 / (m - 1)), float32
+//   pass 1  the same search again (cheaper than storing n * max_nn lists); lane j sums spfh[k][j] / d2_k over the
+//           entries with d2 > 0 in key order (float64), each group of 11 is scaled by 100 / its sum (the group sum
+//           taken sequentially over the 11 bin totals), spfh[i] is added, float32
+// One warp per query.  Points the grid cannot key are never queried: their SPFH, feature and count stay 0.
+#define FPFH_BINS 33
+#define FPFH_PI 3.141592653589793
+#define FPFH_2PI 6.283185307179586
+
+// Bins of Open3D's ComputePairFeatures(p1, n1, p2, n2) (float64); false when a feature is not finite (no bin).
+// The swap test is |a1| < |a2| (Open3D: acos|a1| > acos|a2|, equal except where acos rounds two values together).
+__device__ __forceinline__ bool fpfh_pair_bins(float4 p1, const double (&n1)[3], float4 p2, const double (&n2)[3],
+                                               uint32_t& b0, uint32_t& b1, uint32_t& b2) {
+  const double dx = (double)p2.x - (double)p1.x, dy = (double)p2.y - (double)p1.y, dz = (double)p2.z - (double)p1.z;
+  const double d = sqrt((dx * dx + dy * dy) + dz * dz);
+  double f0 = 0.0, f1 = 0.0, f2 = 0.0;
+  if (d != 0.0) {
+    const double a1 = ((n1[0] * dx + n1[1] * dy) + n1[2] * dz) / d;
+    const double a2 = ((n2[0] * dx + n2[1] * dy) + n2[2] * dz) / d;
+    const bool swap = fabs(a1) < fabs(a2);
+    const double u0 = swap ? n2[0] : n1[0], u1 = swap ? n2[1] : n1[1], u2 = swap ? n2[2] : n1[2];
+    const double t0 = swap ? n1[0] : n2[0], t1 = swap ? n1[1] : n2[1], t2 = swap ? n1[2] : n2[2];
+    const double e0 = swap ? -dx : dx, e1 = swap ? -dy : dy, e2 = swap ? -dz : dz;
+    double v0 = e1 * u2 - e2 * u1, v1 = e2 * u0 - e0 * u2, v2 = e0 * u1 - e1 * u0;
+    const double vn = sqrt((v0 * v0 + v1 * v1) + v2 * v2);
+    if (vn != 0.0) {
+      f2 = swap ? -a2 : a1;
+      v0 = v0 / vn; v1 = v1 / vn; v2 = v2 / vn;
+      const double w0 = u1 * v2 - u2 * v1, w1 = u2 * v0 - u0 * v2, w2 = u0 * v1 - u1 * v0;
+      f1 = (v0 * t0 + v1 * t1) + v2 * t2;
+      f0 = atan2((w0 * t0 + w1 * t1) + w2 * t2, (u0 * t0 + u1 * t1) + u2 * t2);
+    }
+  }
+  if (!(isfinite(f0) && isfinite(f1) && isfinite(f2))) return false;
+  b0 = (uint32_t)fmin(fmax(floor((11.0 * (f0 + FPFH_PI)) / FPFH_2PI), 0.0), 10.0);
+  b1 = (uint32_t)fmin(fmax(floor((11.0 * (f1 + 1.0)) * 0.5), 0.0), 10.0);
+  b2 = (uint32_t)fmin(fmax(floor((11.0 * (f2 + 1.0)) * 0.5), 0.0), 10.0);
+  return true;
+}
+
+// One query's pass over its sorted neighbourhood buf[0, m) (warp-collective).  cnt: this warp's 33 shared counters.
+template <int PASS>
+__device__ __forceinline__ void fpfh_of_keys(const unsigned long long* buf, uint32_t m, const float4* __restrict__ pts,
+                                             const float* __restrict__ normals, float4 q, uint32_t orig, uint32_t lane,
+                                             uint32_t* cnt, float* __restrict__ spfh, float* __restrict__ feat,
+                                             uint32_t* __restrict__ counts) {
+  if (PASS == 0) {
+    cnt[lane] = 0u;
+    if (lane == 0) cnt[32] = 0u;
+    __syncwarp();
+    const double n1[3] = {(double)normals[3 * (size_t)orig], (double)normals[3 * (size_t)orig + 1],
+                          (double)normals[3 * (size_t)orig + 2]};
+    for (uint32_t i = 1 + lane; i < m; i += 32) {
+      const uint32_t k = (uint32_t)buf[i];
+      const double n2[3] = {(double)normals[3 * (size_t)k], (double)normals[3 * (size_t)k + 1],
+                            (double)normals[3 * (size_t)k + 2]};
+      uint32_t b0, b1, b2;
+      if (fpfh_pair_bins(q, n1, pts[k], n2, b0, b1, b2)) {
+        atomicAdd(&cnt[b0], 1u);
+        atomicAdd(&cnt[11u + b1], 1u);
+        atomicAdd(&cnt[22u + b2], 1u);
+      }
+    }
+    __syncwarp();
+    const double incr = m > 1 ? 100.0 / (double)(m - 1) : 0.0;
+    spfh[(size_t)FPFH_BINS * orig + lane] = (float)((double)cnt[lane] * incr);
+    if (lane == 0) {
+      spfh[(size_t)FPFH_BINS * orig + 32] = (float)((double)cnt[32] * incr);
+      if (counts) counts[orig] = m;
+    }
+    __syncwarp();
+  } else {
+    double acc = 0.0, acc32 = 0.0;                               // lane j: bin j; lane 0 also bin 32
+    for (uint32_t i = 1; i < m; ++i) {
+      const unsigned long long key = buf[i];
+      const float d2 = __uint_as_float((uint32_t)(key >> 32));
+      if (d2 > 0.0f) {
+        const float* row = spfh + (size_t)FPFH_BINS * (uint32_t)key;
+        acc = acc + (double)row[lane] / (double)d2;
+        if (lane == 0) acc32 = acc32 + (double)row[32] / (double)d2;
+      }
+    }
+    double scale[3];
+#pragma unroll
+    for (int gidx = 0; gidx < 3; ++gidx) {
+      double sum = __shfl_sync(0xffffffffu, acc, 11 * gidx);
+      for (int t = 1; t < 11; ++t) {
+        const int j = 11 * gidx + t;
+        const double v = j < 32 ? __shfl_sync(0xffffffffu, acc, j) : __shfl_sync(0xffffffffu, acc32, 0);
+        sum = sum + v;
+      }
+      scale[gidx] = sum != 0.0 ? 100.0 / sum : 0.0;
+    }
+    const float* own = spfh + (size_t)FPFH_BINS * orig;
+    const double sl = lane < 11 ? scale[0] : lane < 22 ? scale[1] : scale[2];
+    feat[(size_t)FPFH_BINS * orig + lane] = (float)(acc * sl + (double)own[lane]);
+    if (lane == 0) feat[(size_t)FPFH_BINS * orig + 32] = (float)(acc32 * scale[2] + (double)own[32]);
+  }
+}
+
+// Hybrid search: k_normals_wide's 27-cell walk and WarpKeep, the kept keys sorted.
+template <int PASS>
+__global__ void __launch_bounds__(128)
+k_fpfh_hybrid(uint32_t n_max, const uint32_t* n_dev, GridDev g, const float4* __restrict__ pts,
+              const float* __restrict__ normals, float r2, uint32_t max_nn, uint32_t cap, float* __restrict__ spfh,
+              float* __restrict__ feat, uint32_t* __restrict__ counts, const ApcCtrl* __restrict__ ctrl) {
+  __shared__ uint32_t s_cnt[4][FPFH_BINS];
+  const uint32_t n = grid_sorted_count(g, ctrl, apc_count(n_dev, n_max));
+  const float c = grid_cell_size(g, 0);
+  const uint32_t lane = threadIdx.x & 31u, w = threadIdx.x >> 5;
+  unsigned long long* buf = reinterpret_cast<unsigned long long*>(wide_smem) + (size_t)w * cap;
+  for (uint32_t j = (blockIdx.x * blockDim.x + threadIdx.x) >> 5; j < n; j += (gridDim.x * blockDim.x) >> 5) {
+    const float4 q = g.sorted[j];
+    const uint32_t orig = __float_as_uint(q.w);
+    uint32_t cs, ps;
+    const uint32_t total = flat27_runs(g, c, q, lane, cs, ps);
+    WarpKeep<unsigned long long> wk;
+    wk.init(buf, cap, max_nn);
+    uint32_t in_radius = 0;
+    for (uint32_t base = 0; base < total; base += 32) {
+      const uint32_t ci = base + lane;
+      const uint32_t at = flat27_at(cs, ps, min(ci, total - 1u));
+      unsigned long long key = 0;
+      bool inside = false;
+      if (ci < total) {
+        const float4 p = g.sorted[at];
+        const float d2 = d2_f32(q.x, q.y, q.z, p.x, p.y, p.z);
+        inside = d2 <= r2;
+        key = ((unsigned long long)__float_as_uint(d2) << 32) | __float_as_uint(p.w);
+      }
+      in_radius += __popc(__ballot_sync(0xffffffffu, inside));
+      wk.add(key, inside, lane);
+    }
+    wk.finish(lane);
+    const uint32_t m = min(in_radius, max_nn);
+    warp_sort(buf, m, lane);
+    fpfh_of_keys<PASS>(buf, m, pts, normals, q, orig, lane, s_cnt[w], spfh, feat, counts);
+    __syncwarp();                                                  // buf is reused by the next query
+  }
+}
+
+// KNN search: k_normals_knn's level climb; pass 0 lists the queries no level covers, pass 1 reuses that list.
+template <int PASS>
+__global__ void __launch_bounds__(KNN_WARPS * 32)
+k_fpfh_knn(uint32_t n_max, const uint32_t* n_dev, GridDev g, const float4* __restrict__ pts, const float* __restrict__ normals,
+           uint32_t k, uint32_t cap, float* __restrict__ spfh, float* __restrict__ feat, uint32_t* __restrict__ counts,
+           uint32_t* __restrict__ stragglers, ApcCtrl* ctrl) {
+  __shared__ uint32_t s_cnt[KNN_WARPS][FPFH_BINS];
+  const uint32_t n = apc_count(n_dev, n_max);
+  const uint32_t n_sorted = grid_sorted_count(g, ctrl, n);
+  const uint32_t k_eff = min(k, n);
+  const uint32_t lane = threadIdx.x & 31u, w = threadIdx.x >> 5;
+  unsigned long long* buf = reinterpret_cast<unsigned long long*>(wide_smem) + (size_t)w * cap;
+  for (uint32_t j = blockIdx.x * KNN_WARPS + w; j < n_sorted; j += gridDim.x * KNN_WARPS) {
+    const float4 q = g.sorted[j];
+    const uint32_t orig = __float_as_uint(q.w);
+    if (knn_levels(g, n_max, q, k_eff, buf, cap, 1, lane)) {
+      warp_sort(buf, k_eff, lane);
+      fpfh_of_keys<PASS>(buf, k_eff, pts, normals, q, orig, lane, s_cnt[w], spfh, feat, counts);
+    } else if (PASS == 0 && lane == 0) {
+      stragglers[atomicAdd(&ctrl->counters[CTR_STRAGGLERS], 1u)] = orig;
+    }
+    __syncwarp();
+  }
+}
+
+template <int PASS>
+__global__ void __launch_bounds__(KNN_WARPS * 32)
+k_fpfh_knn_stragglers(const float4* __restrict__ pts, const float* __restrict__ normals, uint32_t n_max, const uint32_t* n_dev,
+                      uint32_t k, uint32_t cap, const uint32_t* __restrict__ stragglers, const ApcCtrl* ctrl,
+                      float* __restrict__ spfh, float* __restrict__ feat, uint32_t* __restrict__ counts) {
+  __shared__ uint32_t s_cnt[KNN_WARPS][FPFH_BINS];
+  const uint32_t n = apc_count(n_dev, n_max);
+  const uint32_t k_eff = min(k, n);
+  const uint32_t n_str = ctrl->counters[CTR_STRAGGLERS];
+  const uint32_t lane = threadIdx.x & 31u, w = threadIdx.x >> 5;
+  unsigned long long* buf = reinterpret_cast<unsigned long long*>(wide_smem) + (size_t)w * cap;
+  for (uint32_t sidx = blockIdx.x * KNN_WARPS + w; sidx < n_str; sidx += gridDim.x * KNN_WARPS) {
+    const uint32_t orig = stragglers[sidx];
+    const float4 q = pts[orig];
+    knn_brute(pts, n, q, k_eff, buf, cap, lane);
+    warp_sort(buf, k_eff, lane);
+    fpfh_of_keys<PASS>(buf, k_eff, pts, normals, q, orig, lane, s_cnt[w], spfh, feat, counts);
+    __syncwarp();
+  }
+}
+
+static int fpfh_run(apc_ctx* ctx, const float* xyzi, const float* normals, uint32_t n_max, const uint32_t* n_dev,
+                    int max_nn, double radius, bool knn, float* out_features, float* out_spfh, uint32_t* out_counts,
+                    cudaStream_t s) {
+  APC_REQUIRE(ctx, max_nn >= 1 && max_nn <= APC_MAX_NEIGHBORS,
+              "max_nn must be in 1..APC_MAX_NEIGHBORS (" APC_STRINGIFY(APC_MAX_NEIGHBORS) ")");
+  const float r32 = (float)radius;
+  if (!knn) APC_REQUIRE(ctx, radius > 0.0 && r32 > 0.0f && std::isfinite(r32 * r32), "radius must be finite and > 0");
+  if (n_max == 0) return APC_OK;
+  APC_REQUIRE(ctx, xyzi && normals && out_features, "NULL pointer");
+  APC_REQUIRE(ctx, n_max <= ctx->max_points, "more points than the context was created for");
+  // everything is allocated before the first launch
+  const int which = knn ? 1 : 0;
+  int rc = apc_neighbors_prepare(ctx, which);
+  if (rc) return rc;
+  NeighborScratch* sc = scratch_of(ctx);
+  if (!out_spfh && !sc->spfh) APC_CUDA(ctx, cudaMalloc((void**)&sc->spfh, (size_t)ctx->max_points * FPFH_BINS * sizeof(float)));
+  float* spfh = out_spfh ? out_spfh : sc->spfh;
+  rc = apc_begin(ctx, s);
+  if (rc) return rc;
+  APC_CUDA(ctx, cudaMemsetAsync(out_features, 0, (size_t)n_max * FPFH_BINS * sizeof(float), s));
+  APC_CUDA(ctx, cudaMemsetAsync(spfh, 0, (size_t)n_max * FPFH_BINS * sizeof(float), s));
+  if (out_counts) APC_CUDA(ctx, cudaMemsetAsync(out_counts, 0, (size_t)n_max * sizeof(uint32_t), s));
+  GridHost& g = sc->grid[which];
+  const float4* pts = reinterpret_cast<const float4*>(xyzi);
+  if (knn) rc = grid_build(ctx, g, pts, n_max, n_dev, 0.0f, true, s);
+  else rc = grid_build(ctx, g, pts, n_max, n_dev, r32 * 1.00390625f, false, s, false, CTR_CURSOR_NORMALS, true);
+  if (rc) return rc;
+  const uint32_t cap = wide_cap((uint32_t)max_nn);
+  const size_t smem = (size_t)4 * cap * sizeof(unsigned long long);
+  const uint32_t bq = min(apc_div_up(n_max, 4), (uint32_t)APC_SM_COUNT * 16);   // one warp per query, grid-stride
+  if (knn) {
+    {
+      APC_PROF(ctx, "k_fpfh_knn_spfh", s);
+      k_fpfh_knn<0><<<bq, KNN_WARPS * 32, smem, s>>>(n_max, n_dev, g.d, pts, normals, (uint32_t)max_nn, cap, spfh,
+                                                     out_features, out_counts, sc->stragglers, ctx->ctrl);
+    }
+    {
+      APC_PROF(ctx, "k_fpfh_knn_stragglers_spfh", s);
+      k_fpfh_knn_stragglers<0><<<APC_SM_COUNT * 2, KNN_WARPS * 32, smem, s>>>(
+          pts, normals, n_max, n_dev, (uint32_t)max_nn, cap, sc->stragglers, ctx->ctrl, spfh, out_features, out_counts);
+    }
+    {
+      APC_PROF(ctx, "k_fpfh_knn", s);
+      k_fpfh_knn<1><<<bq, KNN_WARPS * 32, smem, s>>>(n_max, n_dev, g.d, pts, normals, (uint32_t)max_nn, cap, spfh,
+                                                     out_features, out_counts, sc->stragglers, ctx->ctrl);
+    }
+    {
+      APC_PROF(ctx, "k_fpfh_knn_stragglers", s);
+      k_fpfh_knn_stragglers<1><<<APC_SM_COUNT * 2, KNN_WARPS * 32, smem, s>>>(
+          pts, normals, n_max, n_dev, (uint32_t)max_nn, cap, sc->stragglers, ctx->ctrl, spfh, out_features, out_counts);
+    }
+  } else {
+    {
+      APC_PROF(ctx, "k_fpfh_hybrid_spfh", s);
+      k_fpfh_hybrid<0><<<bq, 128, smem, s>>>(n_max, n_dev, g.d, pts, normals, r32 * r32, (uint32_t)max_nn, cap, spfh,
+                                             out_features, out_counts, ctx->ctrl);
+    }
+    {
+      APC_PROF(ctx, "k_fpfh_hybrid", s);
+      k_fpfh_hybrid<1><<<bq, 128, smem, s>>>(n_max, n_dev, g.d, pts, normals, r32 * r32, (uint32_t)max_nn, cap, spfh,
+                                             out_features, out_counts, ctx->ctrl);
+    }
+  }
+  APC_PROF(ctx, "k_grid_clean", s);
+  k_grid_clean<<<dim3(min(apc_div_up(n_max, 256), (uint32_t)APC_SM_COUNT * 4), g.d.levels), 256, 0, s>>>(n_max, n_dev, g.d);
+  APC_LAUNCH_CHECK(ctx, "compute_fpfh");
+  return APC_OK;
+}
+
+extern "C" int apc_compute_fpfh(apc_ctx* ctx, const float* xyzi, const float* normals, uint32_t n_max, const uint32_t* n_dev,
+                                int max_nn, double radius, float* out_features, float* out_spfh,
+                                uint32_t* out_neighbor_counts, void* stream) {
+  if (!ctx) return APC_ERR_BAD_ARG;
+  return fpfh_run(ctx, xyzi, normals, n_max, n_dev, max_nn, radius, false, out_features, out_spfh, out_neighbor_counts,
+                  (cudaStream_t)stream);
+}
+
+extern "C" int apc_compute_fpfh_knn(apc_ctx* ctx, const float* xyzi, const float* normals, uint32_t n_max,
+                                    const uint32_t* n_dev, int max_nn, float* out_features, float* out_spfh,
+                                    uint32_t* out_neighbor_counts, void* stream) {
+  if (!ctx) return APC_ERR_BAD_ARG;
+  return fpfh_run(ctx, xyzi, normals, n_max, n_dev, max_nn, 0.0, true, out_features, out_spfh, out_neighbor_counts,
+                  (cudaStream_t)stream);
+}
+
+// ---- correspondences_from_features (Open3D t::pipelines::registration::CorrespondencesFromFeatures) ------------
+// Contract (oracle/features.py): d2 = sum_j (a_j - b_j)^2 in float32, increasing j, unfused; a row's match is the
+// other set's row with the smallest (d2, index) among the finite d2, none when no d2 is finite.  Brute force,
+// O(n_a * n_b * dim) like Open3D's CUDA KNN:
+//   k_feat_nn      one thread per query row (held in registers), the other set's rows through shared-memory tiles;
+//                  the rows are split across blockIdx.y and the splits combine by a 64-bit atomicMin on
+//                  (d2 bits << 32 | index), a total order, so the result does not depend on the schedule
+//   k_feat_pairs   tiles of 1024 source rows in index order: the pairs (i, nn_st[i]) of the rows with a match and,
+//                  with the mutual filter, of those with nn_ts[nn_st[i]] == i, compacted in order (apc_scan.cuh)
+//   k_feat_select  the mutual set when it has more than ratio * n_src pairs, else the unfiltered set (fell_back)
+#define FEAT_THREADS 128
+#define FEAT_TILE 64
+
+template <int DMAX>
+__global__ void __launch_bounds__(FEAT_THREADS)
+k_feat_nn(const float* __restrict__ a, uint32_t na_max, const uint32_t* na_dev, const float* __restrict__ b, uint32_t nb_max,
+          const uint32_t* nb_dev, uint32_t dim, uint32_t rows_per_split, unsigned long long* __restrict__ best) {
+  __shared__ float s_b[FEAT_TILE * DMAX];
+  const uint32_t na = apc_count(na_dev, na_max), nb = apc_count(nb_dev, nb_max);
+  const uint32_t i = blockIdx.x * FEAT_THREADS + threadIdx.x;
+  const uint32_t t0 = blockIdx.y * rows_per_split, t1 = min(t0 + rows_per_split, nb);
+  if (blockIdx.x * FEAT_THREADS >= na || t0 >= t1) return;       // block-uniform
+  float q[DMAX];
+#pragma unroll
+  for (uint32_t d = 0; d < DMAX; ++d) q[d] = (i < na && d < dim) ? a[(size_t)i * dim + d] : 0.0f;
+  unsigned long long key = ~0ull;
+  for (uint32_t tb = t0; tb < t1; tb += FEAT_TILE) {
+    const uint32_t rows = min((uint32_t)FEAT_TILE, t1 - tb);
+    __syncthreads();
+    for (uint32_t e = threadIdx.x; e < rows * dim; e += FEAT_THREADS) s_b[e] = b[(size_t)tb * dim + e];
+    __syncthreads();
+    for (uint32_t r = 0; r < rows; ++r) {
+      const float* row = s_b + r * dim;
+      float d2 = 0.0f;
+#pragma unroll
+      for (uint32_t d = 0; d < DMAX; ++d)
+        if (d < dim) {
+          const float x = __fsub_rn(q[d], row[d]);
+          d2 = __fadd_rn(d2, __fmul_rn(x, x));
+        }
+      if (d2 <= 3.402823466e38f) key = min(key, ((unsigned long long)__float_as_uint(d2) << 32) | (tb + r));   // NaN, inf: never
+    }
+  }
+  if (i < na && key != ~0ull) atomicMin(&best[i], key);
+}
+
+__global__ void __launch_bounds__(APC_TILE_THREADS)
+k_feat_pairs(uint32_t n_max, const uint32_t* n_dev, const unsigned long long* __restrict__ best_st,
+             const unsigned long long* __restrict__ best_ts, int32_t* __restrict__ nearest, int32_t* __restrict__ pairs_all,
+             int32_t* __restrict__ pairs_mut, uint32_t* count2, uint64_t* state_all, uint64_t* state_mut,
+             const ApcCtrl* ctrl, uint32_t n_tiles) {
+  __shared__ uint32_t sm_all[34], sm_mut[34];
+  const uint32_t n = apc_count(n_dev, n_max);
+  const uint32_t tile = blockIdx.x;
+  bool keep[APC_TILE_ITEMS], mut[APC_TILE_ITEMS];
+  int32_t nn[APC_TILE_ITEMS];
+#pragma unroll
+  for (int k = 0; k < APC_TILE_ITEMS; ++k) {
+    const uint32_t i = tile * APC_TILE_POINTS + k * APC_TILE_THREADS + threadIdx.x;
+    nn[k] = (i < n && best_st[i] != ~0ull) ? (int32_t)(uint32_t)best_st[i] : -1;
+    keep[k] = nn[k] >= 0;
+    mut[k] = keep[k] && best_ts && best_ts[nn[k]] != ~0ull && (uint32_t)best_ts[nn[k]] == i;
+    if (nearest && i < n_max) nearest[i] = nn[k];
+  }
+  uint32_t rank[APC_TILE_ITEMS];
+  uint32_t base = tile_compact_offsets(keep, rank, sm_all, state_all, tile, ctrl->epoch, &count2[0], n_tiles);
+#pragma unroll
+  for (int k = 0; k < APC_TILE_ITEMS; ++k)
+    if (keep[k]) {
+      pairs_all[2 * (size_t)(base + rank[k])] = (int32_t)(tile * APC_TILE_POINTS + k * APC_TILE_THREADS + threadIdx.x);
+      pairs_all[2 * (size_t)(base + rank[k]) + 1] = nn[k];
+    }
+  if (best_ts) {                                                   // block-uniform
+    base = tile_compact_offsets(mut, rank, sm_mut, state_mut, tile, ctrl->epoch, &count2[1], n_tiles);
+#pragma unroll
+    for (int k = 0; k < APC_TILE_ITEMS; ++k)
+      if (mut[k]) {
+        pairs_mut[2 * (size_t)(base + rank[k])] = (int32_t)(tile * APC_TILE_POINTS + k * APC_TILE_THREADS + threadIdx.x);
+        pairs_mut[2 * (size_t)(base + rank[k]) + 1] = nn[k];
+      }
+  }
+}
+
+// Open3D keeps the mutual set when it has more than ratio * n_src pairs and otherwise warns and falls back.
+__global__ void __launch_bounds__(256)
+k_feat_select(uint32_t n_max, const uint32_t* n_dev, const uint32_t* __restrict__ count2, int mutual, double ratio,
+              const int32_t* __restrict__ pairs_mut, int32_t* __restrict__ pairs, uint32_t* __restrict__ info) {
+  const uint32_t n = apc_count(n_dev, n_max);
+  const bool use_mut = mutual && (double)count2[1] > ratio * (double)n;
+  if (blockIdx.x == 0 && threadIdx.x == 0) {
+    info[0] = use_mut ? count2[1] : count2[0];
+    info[1] = (mutual && !use_mut) ? 1u : 0u;
+  }
+  if (!use_mut) return;
+  const uint32_t e_end = 2u * count2[1];
+  for (uint32_t e = blockIdx.x * blockDim.x + threadIdx.x; e < e_end; e += gridDim.x * blockDim.x) pairs[e] = pairs_mut[e];
+}
+
+static int feat_search(apc_ctx* ctx, const float* a, uint32_t na, const uint32_t* na_dev, const float* b, uint32_t nb,
+                       const uint32_t* nb_dev, uint32_t dim, unsigned long long* best, cudaStream_t s) {
+  APC_CUDA(ctx, cudaMemsetAsync(best, 0xff, (size_t)na * sizeof(unsigned long long), s));
+  if (nb == 0) return APC_OK;
+  const uint32_t blocks_a = apc_div_up(na, FEAT_THREADS), tiles_b = apc_div_up(nb, FEAT_TILE);
+  const uint32_t splits = max(1u, min(apc_div_up(APC_SM_COUNT * 4, blocks_a), tiles_b));   // >= 4 blocks per SM
+  const uint32_t rows_per_split = apc_div_up(tiles_b, splits) * FEAT_TILE;
+  const dim3 grid(blocks_a, apc_div_up(nb, rows_per_split));
+  APC_PROF(ctx, "k_feat_nn", s);
+  if (dim <= 33) k_feat_nn<33><<<grid, FEAT_THREADS, 0, s>>>(a, na, na_dev, b, nb, nb_dev, dim, rows_per_split, best);
+  else k_feat_nn<64><<<grid, FEAT_THREADS, 0, s>>>(a, na, na_dev, b, nb, nb_dev, dim, rows_per_split, best);
+  return APC_OK;
+}
+
+extern "C" int apc_correspondences_from_features(apc_ctx* ctx, const float* src, uint32_t n_src, const uint32_t* n_src_dev,
+                                                 const float* tgt, uint32_t n_tgt, const uint32_t* n_tgt_dev, int dim,
+                                                 int mutual_filter, double ratio, int32_t* out_pairs,
+                                                 int32_t* out_nearest, uint32_t* out_info_dev, void* stream) {
+  if (!ctx) return APC_ERR_BAD_ARG;
+  APC_REQUIRE(ctx, (src || !n_src) && (tgt || !n_tgt) && out_pairs && out_info_dev, "NULL pointer");   // empty: may be NULL
+  APC_REQUIRE(ctx, dim >= 1 && dim <= 64, "dim must be in 1..64");
+  APC_REQUIRE(ctx, std::isfinite(ratio) && ratio >= 0.0, "mutual_consistency_ratio must be finite and >= 0");
+  APC_REQUIRE(ctx, n_src <= ctx->max_points && n_tgt <= ctx->max_points, "more rows than the context was created for");
+  const uint32_t n_tiles = apc_div_up(n_src, APC_TILE_POINTS);
+  APC_REQUIRE(ctx, n_tiles <= ctx->max_tiles, "more rows than the context was created for");
+  // everything is allocated before the first launch
+  NeighborScratch* sc = scratch_of(ctx);
+  const size_t M = ctx->max_points;
+  for (auto& p : sc->feat_best)
+    if (!p) APC_CUDA(ctx, cudaMalloc((void**)&p, M * sizeof(unsigned long long)));
+  if (!sc->feat_pairs) APC_CUDA(ctx, cudaMalloc((void**)&sc->feat_pairs, M * 2 * sizeof(int32_t)));
+  if (!sc->feat_count) APC_CUDA(ctx, cudaMalloc((void**)&sc->feat_count, 2 * sizeof(uint32_t)));
+  cudaStream_t s = (cudaStream_t)stream;
+  int rc = apc_begin(ctx, s);
+  if (rc) return rc;
+  APC_CUDA(ctx, cudaMemsetAsync(out_info_dev, 0, 2 * sizeof(uint32_t), s));
+  if (n_src == 0) return APC_OK;
+  rc = feat_search(ctx, src, n_src, n_src_dev, tgt, n_tgt, n_tgt_dev, (uint32_t)dim, sc->feat_best[0], s);
+  if (rc) return rc;
+  const bool mutual = mutual_filter != 0;
+  if (mutual && n_tgt) {
+    rc = feat_search(ctx, tgt, n_tgt, n_tgt_dev, src, n_src, n_src_dev, (uint32_t)dim, sc->feat_best[1], s);
+    if (rc) return rc;
+  }
+  {
+    APC_PROF(ctx, "k_feat_pairs", s);
+    k_feat_pairs<<<n_tiles, APC_TILE_THREADS, 0, s>>>(n_src, n_src_dev, sc->feat_best[0],
+                                                      (mutual && n_tgt) ? sc->feat_best[1] : nullptr, out_nearest,
+                                                      out_pairs, sc->feat_pairs, sc->feat_count, ctx->scan_state[0],
+                                                      ctx->scan_state[1], ctx->ctrl, n_tiles);
+  }
+  if (mutual && !n_tgt) APC_CUDA(ctx, cudaMemsetAsync(sc->feat_count + 1, 0, sizeof(uint32_t), s));
+  APC_PROF(ctx, "k_feat_select", s);
+  k_feat_select<<<min(apc_div_up(2 * n_src, 256), (uint32_t)APC_SM_COUNT * 4), 256, 0, s>>>(
+      n_src, n_src_dev, sc->feat_count, mutual ? 1 : 0, ratio, sc->feat_pairs, out_pairs, out_info_dev);
+  APC_LAUNCH_CHECK(ctx, "correspondences_from_features");
+  return APC_OK;
 }

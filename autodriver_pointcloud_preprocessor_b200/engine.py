@@ -396,6 +396,40 @@ class Context:
         out = (T, stats, info, corr[:n_src])
         return out + (axes_s[:n_src], axes_t[:n_tgt]) if want_axes else out
 
+    # ---- features --------------------------------------------------------------------------------------
+    def compute_fpfh(self, xyzi, normals, max_nn, radius=None, want_spfh=False, want_counts=False, n_dev=None):
+        """FPFH of every point (``apc_compute_fpfh``: hybrid search, or ``apc_compute_fpfh_knn`` when ``radius`` is
+        None).  ``normals`` float32 ``[n, 3]`` contiguous on the device.  Returns ``(features float32[n, 33],
+        spfh float32[n, 33] | None, counts int32[n] | None)``; no host synchronisation."""
+        n = xyzi.shape[0]
+        feat = self._empty((max(n, 1), 33), torch.float32)
+        spfh = self._empty((max(n, 1), 33), torch.float32) if want_spfh else None
+        counts = self._empty((max(n, 1),), torch.int32) if want_counts else None
+        if radius is None:
+            rc = lib.apc_compute_fpfh_knn(self.h, _ptr(xyzi), _ptr(normals), n, _ptr(n_dev), int(max_nn), _ptr(feat),
+                                          _ptr(spfh), _ptr(counts), _stream())
+        else:
+            rc = lib.apc_compute_fpfh(self.h, _ptr(xyzi), _ptr(normals), n, _ptr(n_dev), int(max_nn), float(radius),
+                                      _ptr(feat), _ptr(spfh), _ptr(counts), _stream())
+        self._ok(rc)
+        return feat[:n], (spfh[:n] if spfh is not None else None), (counts[:n] if counts is not None else None)
+
+    def correspondences_from_features(self, src, tgt, mutual_filter=False, mutual_consistency_ratio=0.1,
+                                      want_nearest=False, n_src_dev=None, n_tgt_dev=None):
+        """``apc_correspondences_from_features`` on float32 ``[n, dim]`` rows (contiguous, on the device).  Returns
+        ``(pairs int32[n_src, 2], info int32[2] {count, fell_back}, nearest int32[n_src] | None)`` on the device;
+        the first ``count`` rows of ``pairs`` are valid.  No host synchronisation."""
+        n_src, n_tgt = src.shape[0], tgt.shape[0]
+        dim = src.shape[1] if src.dim() == 2 else 0
+        pairs = self._empty((max(n_src, 1), 2), torch.int32)
+        info = self._empty((2,), torch.int32)
+        nearest = self._empty((max(n_src, 1),), torch.int32) if want_nearest else None
+        self._ok(lib.apc_correspondences_from_features(self.h, _ptr(src), n_src, _ptr(n_src_dev), _ptr(tgt), n_tgt,
+                                                       _ptr(n_tgt_dev), int(dim), int(bool(mutual_filter)),
+                                                       float(mutual_consistency_ratio), _ptr(pairs), _ptr(nearest),
+                                                       _ptr(info), _stream()))
+        return pairs[:n_src], info, (nearest[:n_src] if nearest is not None else None)
+
     # ---- ransac ------------------------------------------------------------------------------------
     def segment_plane(self, xyzi, distance_threshold, ransac_n, num_iterations, probability, seed=0,
                       sample_table=None, n_dev=None):

@@ -1,5 +1,6 @@
-"""``open3d.t.pipelines.registration`` look-alike: single-scale ICP (point-to-point, point-to-plane, generalized) and
-``evaluate_registration`` on the GPU.
+"""``open3d.t.pipelines.registration`` look-alike: single-scale ICP (point-to-point, point-to-plane, generalized),
+``evaluate_registration``, FPFH features (``compute_fpfh_feature``) and matching in feature space
+(``correspondences_from_features``) on the GPU.
 
 The whole ICP loop runs on the device (``apc_icp``): the call synchronises once, at the end.  Definitions, and
 where they differ from Open3D, are in ``oracle/registration.py`` and ``oracle/gicp.py``; in short:
@@ -14,11 +15,24 @@ where they differ from Open3D, are in ``oracle/registration.py`` and ``oracle/gi
   (``I - (1 - epsilon) a a^T``).  An isotropic covariance has no such axis: the identity that neighbourhoods of
   fewer than 3 points get is treated as a horizontal plane.
 
-Not modelled: multi-scale ICP, colored ICP, robust kernels and per-iteration callbacks.
+FPFH and feature matching (``oracle/features.py``):
+
+* the neighbourhoods are those of ``estimate_normals``: hybrid (``max_nn`` and ``radius``) or KNN (``max_nn``
+  only); radius-only search and ``indices=`` are not modelled.  Open3D's pair features and 3 x 11 bins; a pair
+  whose feature is not finite (a NaN normal) adds to no bin.  The swap test of the pair feature compares ``|a1| <
+  |a2|`` where Open3D compares their ``acos``; the SPFH multiplies each count by ``100 / (m - 1)`` once, and the
+  FPFH sums in a fixed order, so results can differ from Open3D's in the last float32 bits;
+* a feature row's match is the other set's row with the smallest float32 squared distance, ties to the lower
+  index; rows whose distances are all NaN have no match and no pair.  The search is brute force,
+  O(n_source * n_target * 33).
+
+Not modelled: multi-scale ICP, colored ICP, robust kernels, per-iteration callbacks and global registration
+(RANSAC / FGR on feature correspondences).
 """
 from __future__ import annotations
 
 import math
+import warnings
 
 import numpy as np
 import torch
@@ -201,3 +215,55 @@ def icp(source: PointCloud, target: PointCloud, max_correspondence_distance, ini
         raise RuntimeError(f"{'generalized' if generalized else 'point-to-plane'} ICP: the linear system is not "
                            "positive definite (degenerate geometry, e.g. all target normals parallel)")
     return _result(source, T.cpu().numpy(), stats, corr, info)
+
+
+def compute_fpfh_feature(input: PointCloud, max_nn=100, radius=None, indices=None) -> Tensor:
+    """Open3D ``compute_fpfh_feature``: float32 ``Tensor [N, 33]`` on the cloud's device.  ``max_nn`` with ``radius``
+    is the hybrid search (the ``max_nn`` nearest within ``radius``), ``max_nn`` alone the KNN search; the cloud needs
+    ``normals``.  Raises ``RuntimeError`` without normals and ``NotImplementedError`` for a radius-only search or
+    ``indices``."""
+    if indices is not None:
+        raise NotImplementedError("compute_fpfh_feature: indices= is not modelled")
+    if max_nn is None:
+        raise NotImplementedError("compute_fpfh_feature: the radius-only search is not modelled; pass max_nn")
+    if "normals" not in input.point:
+        raise RuntimeError("compute_fpfh_feature requires normals: call estimate_normals() first")
+    n = input._n()
+    if n == 0:
+        return input._home(torch.zeros((0, 33), dtype=torch.float32, device="cuda"))
+    normals = PointCloud._gpu(input.point["normals"]).to(torch.float32).contiguous()
+    if tuple(normals.shape) != (n, 3):
+        raise ValueError(f"normals must be [{n}, 3], got {tuple(normals.shape)}")
+    feat, _, _ = input._ctx().compute_fpfh(input._xyzi(), normals, int(max_nn),
+                                           None if radius is None else float(radius))
+    return input._home(feat.contiguous())
+
+
+def correspondences_from_features(source_features, target_features, mutual_filter=False,
+                                  mutual_consistency_ratio=0.1) -> Tensor:
+    """Open3D ``correspondences_from_features``: int64 ``Tensor [K, 2]`` of ``(source row, target row)`` pairs in
+    ascending source row, each source row with its nearest target row in feature space.  With ``mutual_filter``
+    only the pairs whose target row's nearest source row is the source row itself are kept, unless there are no
+    more than ``mutual_consistency_ratio * n_source`` of them: then the unfiltered pairs are returned with a
+    warning, as Open3D does.  Source rows without a finite distance (NaN features) have no pair."""
+    src = source_features.t if isinstance(source_features, Tensor) else torch.as_tensor(source_features)
+    tgt = target_features.t if isinstance(target_features, Tensor) else torch.as_tensor(target_features)
+    if src.dim() != 2 or tgt.dim() != 2 or src.shape[1] != tgt.shape[1]:
+        raise ValueError(f"features must be [n, dim] with the same dim, got {tuple(src.shape)} and {tuple(tgt.shape)}")
+    ratio = float(mutual_consistency_ratio)
+    if not (math.isfinite(ratio) and ratio >= 0):
+        raise ValueError("mutual_consistency_ratio must be finite and >= 0")
+    on_cuda = src.is_cuda
+    dev = src.device.index if on_cuda else None
+    home = (lambda t: Tensor(t)) if on_cuda else (lambda t: Tensor(t.cpu()))
+    if src.shape[0] == 0 or tgt.shape[0] == 0:
+        return home(torch.zeros((0, 2), dtype=torch.int64, device="cuda"))
+    ctx = get_context(max(src.shape[0], tgt.shape[0]), dev)
+    src = (src if src.is_cuda else src.cuda(ctx.device)).to(torch.float32).contiguous()
+    tgt = (tgt if tgt.is_cuda else tgt.cuda(ctx.device)).to(torch.float32).contiguous()
+    pairs, info, _ = ctx.correspondences_from_features(src, tgt, bool(mutual_filter), ratio)
+    count, fell_back = (int(v) for v in info.cpu().tolist())      # the one synchronisation of the call
+    if fell_back:
+        warnings.warn("Too few correspondences after mutual filter, fall back to original correspondences.",
+                      RuntimeWarning, stacklevel=2)
+    return home(pairs[:count].to(torch.int64))

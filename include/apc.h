@@ -352,6 +352,44 @@ int apc_icp_generalized(apc_ctx* ctx, const float* src_xyzi, const float* src_co
                         int32_t* out_info_dev, int32_t* out_correspondences,
                         double* out_src_axes_dev, double* out_tgt_axes_dev, void* stream);
 
+/* ---- (3c) FPFH features and feature matching (Open3D t.pipelines.registration) --------- */
+
+/* compute_fpfh_feature(input, max_nn, radius) (Open3D t::pipelines::registration::ComputeFPFHFeature, hybrid
+ * search).  Contract (oracle/features.py): the neighbourhood of estimate_normals' hybrid search (the max_nn nearest
+ * of the points with d2 <= float32(radius)^2 by (d2, index), query included), m points; entry 0 is at d2 = 0 and is
+ * skipped as Open3D skips it.  SPFH: the 3 x 11 bins of Open3D's pair features (float64) of the query with entries
+ * 1..m-1, each count times 100 / (m - 1) (all zero for m <= 1); a pair whose feature is not finite adds to no bin.
+ * FPFH: spfh[k] / d2_k summed over the entries with d2 > 0 in key order (float64), each group of 11 scaled by
+ * 100 / its sum, plus spfh[i].  normals float32[3 * n_max]; out_features and out_spfh float32[33 * n_max] (out_spfh
+ * may be NULL); out_neighbor_counts uint32[n_max] (m, may be NULL).  Points the grid cannot key get zeros and are
+ * in no neighbourhood.  max_nn in 1..APC_MAX_NEIGHBORS and radius finite and > 0 (APC_ERR_BAD_ARG otherwise).
+ * Two passes of the search; no host synchronisation, the call can be captured in a CUDA graph. */
+int apc_compute_fpfh(apc_ctx* ctx, const float* xyzi, const float* normals, uint32_t n_max, const uint32_t* n_dev,
+                     int max_nn, double radius, float* out_features, float* out_spfh,
+                     uint32_t* out_neighbor_counts, void* stream);
+
+/* compute_fpfh_feature(input, max_nn) (KNN search): the same, with the neighbourhood of apc_estimate_normals_knn
+ * (the min(max_nn, n) points first in the order (d2, index), no distance bound). */
+int apc_compute_fpfh_knn(apc_ctx* ctx, const float* xyzi, const float* normals, uint32_t n_max, const uint32_t* n_dev,
+                         int max_nn, float* out_features, float* out_spfh, uint32_t* out_neighbor_counts,
+                         void* stream);
+
+/* correspondences_from_features(source_features, target_features, mutual_filter, mutual_consistency_ratio) (Open3D
+ * t::pipelines::registration::CorrespondencesFromFeatures).  Rows of dim (1..64) float32 values, row-major.  The
+ * match of source row i is the target row with the smallest (d2, index), d2 = sum_j (a_j - b_j)^2 in float32 in
+ * increasing j, unfused; NaN and infinite d2 never win, and a row without a finite d2 has no match.
+ * out_pairs int32[2 * n_src]: the first count rows hold (i, match) in ascending i, for every source row with a match
+ * or, with mutual_filter, only those whose match's own match is i - unless that set has no more than
+ * ratio * n_src pairs, when the unfiltered set is returned and fell_back is 1 (Open3D warns).  out_nearest
+ * int32[n_src] (may be NULL): every row's match, -1 for none.  out_info_dev uint32[2] (device) = {count,
+ * fell_back}.  Brute force, O(n_src * n_tgt * dim) per direction (the target-to-source search runs only with
+ * mutual_filter).  APC_ERR_BAD_ARG: NULL pointers, dim outside 1..64, ratio not finite or < 0, more rows than
+ * max_points.  No host synchronisation; the call can be captured in a CUDA graph. */
+int apc_correspondences_from_features(apc_ctx* ctx, const float* src, uint32_t n_src, const uint32_t* n_src_dev,
+                                      const float* tgt, uint32_t n_tgt, const uint32_t* n_tgt_dev, int dim,
+                                      int mutual_filter, double ratio, int32_t* out_pairs, int32_t* out_nearest,
+                                      uint32_t* out_info_dev, void* stream);
+
 /* ---- (4) RANSAC ground plane --------------------------------------------------------- */
 
 /* segment_plane(distance_threshold, ransac_n, num_iterations, probability) (pp.py:533-543).
