@@ -24,6 +24,7 @@ DEDUP_OFF, DEDUP_OPEN3D, DEDUP_NUMPY, DEDUP_TORCH_COMPAT = 0, 1, 2, 3
 STAGE_NANSKIP, STAGE_DEDUP, STAGE_FINITE, STAGE_CROP = 1, 2, 4, 8
 APC_ICP_POINT_TO_POINT, APC_ICP_POINT_TO_PLANE, APC_ICP_GENERALIZED = 0, 1, 2
 APC_ICP_OK, APC_ICP_NO_CORRESPONDENCE, APC_ICP_DEGENERATE = 0, 1, 2
+APC_FGR_OK, APC_FGR_TOO_FEW, APC_FGR_DEGENERATE = 0, 1, 2
 (CNT_INPUT, CNT_FILTERED, CNT_VOXELS, CNT_AFTER_STAT, CNT_AFTER_RADIUS, CNT_GROUND_INLIERS, CNT_OUTPUT,
  CNT_STATUS) = range(8)
 
@@ -113,6 +114,9 @@ def _load():
         "apc_compute_fpfh": [vp, vp, vp, u32, vp, i32, f64, vp, vp, vp, vp],
         "apc_compute_fpfh_knn": [vp, vp, vp, u32, vp, i32, vp, vp, vp, vp],
         "apc_correspondences_from_features": [vp, vp, u32, vp, vp, u32, vp, i32, i32, f64, vp, vp, vp, vp],
+        "apc_fgr_from_features": [vp, vp, u32, vp, vp, u32, vp, vp, vp, i32, f64, i32, i32, f64, i32, f64, i32, i32,
+                                  C.c_uint64, vp, vp, vp, vp],
+        "apc_fgr": [vp, vp, u32, vp, vp, u32, vp, vp, u32, vp, f64, i32, i32, f64, i32, vp, vp, vp, vp],
         "apc_segment_plane": [vp, vp, u32, vp, f64, i32, i32, f64, C.c_uint64, vp, vp, vp, vp, vp],
         "apc_segment_plane_scores": [vp, vp, u32, vp],
         "apc_repack": [vp, vp, u32, vp, C.POINTER(OutField), u32, u32, vp, vp],
@@ -155,7 +159,7 @@ SYMBOLS = ["apc_ctx_create", "apc_ctx_destroy", "apc_ctx_set_low_latency", "apc_
            "apc_voxel_downsample", "apc_voxel_downsample_sorted", "apc_voxel_mean_attr", "apc_radius_outliers",
            "apc_statistical_outliers", "apc_estimate_normals", "apc_estimate_normals_knn",
            "apc_estimate_normals_radius", "apc_cluster_dbscan", "apc_evaluate_registration", "apc_icp", "apc_icp_generalized", "apc_compute_fpfh",
-           "apc_compute_fpfh_knn", "apc_correspondences_from_features", "apc_segment_plane", "apc_segment_plane_scores", "apc_repack", "apc_pipeline_run", "apc_pipeline_run_maps",
+           "apc_compute_fpfh_knn", "apc_correspondences_from_features", "apc_fgr_from_features", "apc_fgr", "apc_segment_plane", "apc_segment_plane_scores", "apc_repack", "apc_pipeline_run", "apc_pipeline_run_maps",
            "apc_pipeline_run_mirrored", "apc_pipeline_run_ex", "apc_graph_capture_pipeline_ex",
            "apc_graph_capture_pipeline", "apc_graph_capture_pipeline_mirrored",
            "apc_graph_launch", "apc_graph_destroy",

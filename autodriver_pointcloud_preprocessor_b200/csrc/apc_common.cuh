@@ -236,6 +236,14 @@ __device__ __forceinline__ uint32_t apc_count(const uint32_t* n_dev, uint32_t n_
 
 __device__ __forceinline__ uint32_t lane_id() { return threadIdx.x & 31u; }
 
+// Counter-based random stream of RANSAC's hypotheses and FGR's tuples (oracle/ransac.py: splitmix64)
+__device__ __forceinline__ uint64_t splitmix64_dev(uint64_t x) {
+  uint64_t z = x + 0x9E3779B97F4A7C15ull;
+  z = (z ^ (z >> 30)) * 0xBF58476D1CE4E5B9ull;
+  z = (z ^ (z >> 27)) * 0x94D049BB133111EBull;
+  return z ^ (z >> 31);
+}
+
 __device__ __forceinline__ uint32_t warp_sum_u32(uint32_t v) {
   return __reduce_add_sync(0xffffffffu, v);
 }

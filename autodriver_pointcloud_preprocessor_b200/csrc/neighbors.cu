@@ -1313,6 +1313,8 @@ struct NeighborScratch {
   unsigned long long* feat_best[2] = {nullptr, nullptr};   // [max_points] (d2 bits, index) minima of the feature search
   int32_t* feat_pairs = nullptr;       // [max_points][2] mutually consistent pairs of apc_correspondences_from_features
   uint32_t* feat_count = nullptr;      // [2] pair counts: all, mutual
+  int32_t* fgr_pairs = nullptr;        // [3 * max_points][2] FGR's tuple pairs, or the unused pairs of its feature search
+  struct FgrState* fgr_state = nullptr;   // apc_fgr(_from_features)' normalisation, tuple counts and loop outputs
 };
 // one scratch set per context, owned by the context (created on first use, freed by apc_ctx_destroy)
 static NeighborScratch* scratch_of(apc_ctx* ctx) {
@@ -1337,7 +1339,7 @@ void apc_neighbors_release(apc_ctx* ctx) {
   void* icp[] = {s->icp_part, s->icp_state, s->gicp_axes[0], s->gicp_axes[1]};
   for (void* p : icp)
     if (p) cudaFree(p);
-  void* feat[] = {s->spfh, s->feat_best[0], s->feat_best[1], s->feat_pairs, s->feat_count};
+  void* feat[] = {s->spfh, s->feat_best[0], s->feat_best[1], s->feat_pairs, s->feat_count, s->fgr_pairs, s->fgr_state};
   for (void* p : feat)
     if (p) cudaFree(p);
   delete s;
@@ -3602,6 +3604,8 @@ extern "C" int apc_correspondences_from_features(apc_ctx* ctx, const float* src,
   if (rc) return rc;
   APC_CUDA(ctx, cudaMemsetAsync(out_info_dev, 0, 2 * sizeof(uint32_t), s));
   if (n_src == 0) return APC_OK;
+  // rows no pair reaches (source rows without a match) read as -1 rather than as whatever the buffer held
+  APC_CUDA(ctx, cudaMemsetAsync(out_pairs, 0xff, (size_t)n_src * 2 * sizeof(int32_t), s));
   rc = feat_search(ctx, src, n_src, n_src_dev, tgt, n_tgt, n_tgt_dev, (uint32_t)dim, sc->feat_best[0], s);
   if (rc) return rc;
   const bool mutual = mutual_filter != 0;
@@ -3622,4 +3626,439 @@ extern "C" int apc_correspondences_from_features(apc_ctx* ctx, const float* src,
       n_src, n_src_dev, sc->feat_count, mutual ? 1 : 0, ratio, sc->feat_pairs, out_pairs, out_info_dev);
   APC_LAUNCH_CHECK(ctx, "correspondences_from_features");
   return APC_OK;
+}
+
+// ---- Fast Global Registration (Open3D pipelines::registration::FastGlobalRegistration) ---------------------------
+// Contract (oracle/fgr.py): the pairs (the mutual set of the feature search, or the caller's in-range pairs), the
+// tuple test on a counter-based stream, normalisation by the means of both clouds and the largest centred norm D,
+// then iteration_number Gauss-Newton steps of sum s |p - T q|^2 with s = (par / (|r|^2 + par))^2 and the
+// graduated par, and finally the inverse of T in metres.
+//   k_fgr_pairs    (apc_fgr) tiles of 1024 input pairs in order: the pairs with both indices inside their clouds,
+//                  compacted in order (apc_scan.cuh); the others are dropped
+//   k_fgr_tuples   tiles of `steps` x 1024 trials in trial order: each trial draws its three pairs (splitmix64_dev)
+//                  and tests the edge ratios in float64; the tile's accept ballots stay in shared memory while one
+//                  cross-tile scan places the tile, then the first maximum_tuple_count accepted tuples are written
+//   k_fgr_norm     one block: means and D of both clouds in a fixed order, par, T = I, TOO_FEW
+//   k_fgr_accum    one warp per pair, grid-stride: q' = T q, r, s; lane k accumulates moment k of the three axes'
+//                  rows in point-to-plane's layout (c_icp_pairs[APC_ICP_POINT_TO_PLANE]); block rows of 32 partials
+//   k_icp_solve    unchanged, launched as point-to-plane without a convergence test: T = update T, or DEGENERATE
+//   k_fgr_final    the inverse in metres and the info
+// iteration_number (accum, solve) pairs are launched up front and return at once after a DEGENERATE step, so the call
+// makes no host synchronisation.  Launch configurations depend on host sizes only and every sum has a fixed order.
+#define FGR_TRIALS_PER_PAIR 100u
+#define FGR_MIN_PAIRS 10u
+#define FGR_TUPLE_MAX_STEPS 128u   // a tile of tuple trials holds at most 128 x 1024 (16 KB of ballots)
+
+struct FgrState {
+  double mu_s[3], mu_t[3];
+  double g, par0;
+  uint32_t used, accepted, trials;
+  double icp_T[16], icp_stats[2];   // outputs of k_icp_solve
+  int32_t icp_info[4];
+};
+
+__global__ void __launch_bounds__(APC_TILE_THREADS)
+k_fgr_pairs(const int32_t* __restrict__ in, uint32_t n_max, const uint32_t* n_dev, uint32_t n_src_max,
+            const uint32_t* n_src_dev, uint32_t n_tgt_max, const uint32_t* n_tgt_dev, int32_t* __restrict__ out,
+            uint32_t* count, uint64_t* state, const ApcCtrl* ctrl, uint32_t n_tiles) {
+  __shared__ uint32_t sm[34];
+  const uint32_t n = apc_count(n_dev, n_max), ns = apc_count(n_src_dev, n_src_max), nt = apc_count(n_tgt_dev, n_tgt_max);
+  bool keep[APC_TILE_ITEMS];
+  int32_t a[APC_TILE_ITEMS], b[APC_TILE_ITEMS];
+#pragma unroll
+  for (int k = 0; k < APC_TILE_ITEMS; ++k) {
+    const uint32_t e = blockIdx.x * APC_TILE_POINTS + k * APC_TILE_THREADS + threadIdx.x;
+    a[k] = b[k] = -1;
+    if (e < n) {
+      a[k] = in[2 * (size_t)e];
+      b[k] = in[2 * (size_t)e + 1];
+    }
+    keep[k] = a[k] >= 0 && (uint32_t)a[k] < ns && b[k] >= 0 && (uint32_t)b[k] < nt;
+  }
+  uint32_t rank[APC_TILE_ITEMS];
+  const uint32_t base = tile_compact_offsets(keep, rank, sm, state, blockIdx.x, ctrl->epoch, count, n_tiles);
+#pragma unroll
+  for (int k = 0; k < APC_TILE_ITEMS; ++k)
+    if (keep[k]) {
+      out[2 * (size_t)(base + rank[k])] = a[k];
+      out[2 * (size_t)(base + rank[k]) + 1] = b[k];
+    }
+}
+
+__device__ __forceinline__ uint32_t fgr_draw(uint64_t seed, uint32_t t, uint32_t k, uint32_t K) {
+  const uint64_t z = splitmix64_dev(seed + ((uint64_t)t << 32) + k);
+  return (uint32_t)(((z >> 32) * (uint64_t)K) >> 32);
+}
+// sqrt((dx*dx + dy*dy) + dz*dz) in float64, unfused
+__device__ __forceinline__ double fgr_len(float4 a, float4 b) {
+  const double dx = __dsub_rn(a.x, b.x), dy = __dsub_rn(a.y, b.y), dz = __dsub_rn(a.z, b.z);
+  return __dsqrt_rn(__dadd_rn(__dadd_rn(__dmul_rn(dx, dx), __dmul_rn(dy, dy)), __dmul_rn(dz, dz)));
+}
+__device__ __forceinline__ bool fgr_accept(const float4* __restrict__ src, const float4* __restrict__ tgt,
+                                           const int32_t* __restrict__ pairs, uint64_t seed, uint32_t t, uint32_t K,
+                                           double scale) {
+  float4 p[3], q[3];
+#pragma unroll
+  for (uint32_t k = 0; k < 3; ++k) {
+    const uint32_t c = fgr_draw(seed, t, k, K);
+    p[k] = src[pairs[2 * (size_t)c]];
+    q[k] = tgt[pairs[2 * (size_t)c + 1]];
+  }
+  bool ok = true;
+#pragma unroll
+  for (int e = 0; e < 3; ++e) {
+    const double li = fgr_len(p[e], p[(e + 1) % 3]), lj = fgr_len(q[e], q[(e + 1) % 3]);
+    ok = ok && __dmul_rn(li, scale) < lj && lj < __ddiv_rn(li, scale);
+  }
+  return ok;
+}
+
+// Trial t of tile b is item j (0..3) of thread x at step u: t = (b * steps + u) * 1024 + j * 256 + x, so ballot word
+// w = u * 32 + j * 8 + warp holds the trials w * 32 + lane of the tile, and word order is trial order.
+__global__ void __launch_bounds__(256)
+k_fgr_tuples(const float4* __restrict__ src, const float4* __restrict__ tgt, const int32_t* __restrict__ pairs,
+             const uint32_t* K_dev, uint32_t K_max, uint32_t steps, uint64_t seed, double scale, uint32_t max_count,
+             int32_t* __restrict__ out, FgrState* __restrict__ fst, uint64_t* state, const ApcCtrl* ctrl, uint32_t n_tiles) {
+  __shared__ uint32_t bits[FGR_TUPLE_MAX_STEPS * 32], before[FGR_TUPLE_MAX_STEPS * 32];
+  __shared__ uint32_t sm_total, sm_scan;
+  const uint32_t K = apc_count(K_dev, K_max), n_trials = FGR_TRIALS_PER_PAIR * K;
+  const uint32_t lane = threadIdx.x & 31u, warp = threadIdx.x >> 5, words = steps * 32u;
+  const uint32_t t0 = blockIdx.x * steps * 1024u;
+  for (uint32_t u = 0; u < steps; ++u)
+#pragma unroll
+    for (uint32_t j = 0; j < 4; ++j) {
+      const uint32_t t = t0 + u * 1024u + j * 256u + threadIdx.x;
+      const uint32_t b = __ballot_sync(0xffffffffu, t < n_trials && fgr_accept(src, tgt, pairs, seed, t, K, scale));
+      if (lane == 0) bits[u * 32u + j * 8u + warp] = b;
+    }
+  __syncthreads();
+  if (warp == 0) {                                  // exclusive prefix of the words' counts, in word order
+    uint32_t carry = 0;
+    for (uint32_t w0 = 0; w0 < words; w0 += 32) {
+      const uint32_t c = __popc(bits[w0 + lane]);
+      uint32_t incl = c;
+#pragma unroll
+      for (int o = 1; o < 32; o <<= 1) {
+        const uint32_t v = __shfl_up_sync(0xffffffffu, incl, o);
+        if (lane >= (uint32_t)o) incl += v;
+      }
+      before[w0 + lane] = carry + incl - c;
+      carry += __shfl_sync(0xffffffffu, incl, 31);
+    }
+    if (lane == 0) sm_total = carry;
+  }
+  __syncthreads();
+  const uint32_t total = sm_total;
+  const uint32_t excl = scan_two_level(state, blockIdx.x, n_tiles, ctrl->epoch, total, &sm_scan);
+  if (blockIdx.x == n_tiles - 1 && threadIdx.x == 0) fst->accepted = excl + total;
+  if (excl >= max_count) return;                    // block-uniform
+  for (uint32_t u = 0; u < steps; ++u)
+    for (uint32_t j = 0; j < 4; ++j) {
+      const uint32_t w = u * 32u + j * 8u + warp, word = bits[w];
+      if (!((word >> lane) & 1u)) continue;
+      const uint32_t rank = excl + before[w] + __popc(word & ((1u << lane) - 1u));
+      if (rank >= max_count) continue;
+      const uint32_t t = t0 + u * 1024u + j * 256u + threadIdx.x;
+      for (uint32_t k = 0; k < 3; ++k) {
+        const uint32_t c = fgr_draw(seed, t, k, K);
+        out[2 * (3 * (size_t)rank + k)] = pairs[2 * (size_t)c];
+        out[2 * (3 * (size_t)rank + k) + 1] = pairs[2 * (size_t)c + 1];
+      }
+      if (rank == max_count - 1) fst->trials = t + 1;
+    }
+}
+
+// block-wide reductions of k_fgr_norm (1024 threads) in a fixed order; the max propagates NaN
+__device__ __forceinline__ double fgr_max_nan(double a, double b) { return (b > a || b != b) ? b : a; }
+template <bool MAX>
+__device__ __forceinline__ double fgr_block_reduce(double v, double* sm) {
+  const uint32_t lane = threadIdx.x & 31u, warp = threadIdx.x >> 5;
+#pragma unroll
+  for (int o = 16; o; o >>= 1) {
+    const double x = __shfl_down_sync(0xffffffffu, v, o);
+    v = MAX ? fgr_max_nan(v, x) : v + x;
+  }
+  __syncthreads();                                  // sm is reused by the next reduction
+  if (lane == 0) sm[warp] = v;
+  __syncthreads();
+  if (warp == 0) {
+    v = sm[lane];
+#pragma unroll
+    for (int o = 16; o; o >>= 1) {
+      const double x = __shfl_down_sync(0xffffffffu, v, o);
+      v = MAX ? fgr_max_nan(v, x) : v + x;
+    }
+    if (lane == 0) sm[32] = v;
+  }
+  __syncthreads();
+  return sm[32];
+}
+
+__global__ void __launch_bounds__(1024)
+k_fgr_norm(const float4* __restrict__ src, uint32_t n_src_max, const uint32_t* n_src_dev, const float4* __restrict__ tgt,
+           uint32_t n_tgt_max, const uint32_t* n_tgt_dev, const uint32_t* K_dev, uint32_t K_max, int tuple_test,
+           uint32_t max_count, int absolute, FgrState* __restrict__ fst, IcpState* __restrict__ ist) {
+  __shared__ double sm[33];
+  const float4* pts[2] = {src, tgt};
+  const uint32_t n[2] = {apc_count(n_src_dev, n_src_max), apc_count(n_tgt_dev, n_tgt_max)};
+  double mu[2][3], dmax = 0.0;
+  for (int c = 0; c < 2; ++c) {
+    double sx = 0.0, sy = 0.0, sz = 0.0;
+    for (uint32_t i = threadIdx.x; i < n[c]; i += blockDim.x) {
+      const float4 p = pts[c][i];
+      sx += p.x; sy += p.y; sz += p.z;
+    }
+    mu[c][0] = fgr_block_reduce<false>(sx, sm) / (double)n[c];
+    mu[c][1] = fgr_block_reduce<false>(sy, sm) / (double)n[c];
+    mu[c][2] = fgr_block_reduce<false>(sz, sm) / (double)n[c];
+    for (uint32_t i = threadIdx.x; i < n[c]; i += blockDim.x) {
+      const float4 p = pts[c][i];
+      const double dx = p.x - mu[c][0], dy = p.y - mu[c][1], dz = p.z - mu[c][2];
+      dmax = fgr_max_nan(dmax, sqrt((dx * dx + dy * dy) + dz * dz));
+    }
+  }
+  const double D = fgr_block_reduce<true>(dmax, sm);
+  if (threadIdx.x) return;
+  const uint32_t K = apc_count(K_dev, K_max);
+  const uint32_t used = tuple_test ? 3u * min(fst->accepted, max_count) : K;
+  for (int k = 0; k < 3; ++k) {
+    fst->mu_s[k] = mu[0][k];
+    fst->mu_t[k] = mu[1][k];
+  }
+  fst->g = absolute ? 1.0 : D;
+  fst->par0 = absolute ? D : 1.0;
+  fst->used = used;
+  for (int k = 0; k < 16; ++k) ist->T[k] = (k % 5 == 0) ? 1.0 : 0.0;
+  ist->prev_f = ist->prev_r = 0.0;
+  ist->done = used < FGR_MIN_PAIRS;
+  ist->iterations = 0;
+}
+
+__global__ void __launch_bounds__(128)
+k_fgr_accum(const float4* __restrict__ src, const float4* __restrict__ tgt, const int32_t* __restrict__ pairs,
+            const FgrState* __restrict__ fst, const IcpState* __restrict__ ist, int iteration, int decrease_mu,
+            double max_corr, double division_factor, double* __restrict__ partials) {
+  if (ist->done) return;                                    // block-uniform
+  __shared__ double sm[4][32];
+  const uint32_t lane = threadIdx.x & 31u, warp = threadIdx.x >> 5;
+  const uint32_t pair = c_icp_pairs[APC_ICP_POINT_TO_PLANE][lane], pa = pair & 15u, pb = pair >> 4;
+  double par = fst->par0;                                   // the schedule's steps at 0, 4, 8, ... <= iteration
+  if (decrease_mu)
+    for (int j = 0; j <= iteration && par > max_corr; j += 4) par /= division_factor;
+  const double g = fst->g;
+  const double ms[3] = {fst->mu_s[0], fst->mu_s[1], fst->mu_s[2]}, mt[3] = {fst->mu_t[0], fst->mu_t[1], fst->mu_t[2]};
+  double T[12];
+#pragma unroll
+  for (int k = 0; k < 12; ++k) T[k] = ist->T[k];
+  const uint32_t n = fst->used;
+  double acc = 0.0;
+  for (uint32_t i = (blockIdx.x * blockDim.x + threadIdx.x) >> 5; i < n; i += (gridDim.x * blockDim.x) >> 5) {
+    const float4 ps = src[pairs[2 * (size_t)i]], pt = tgt[pairs[2 * (size_t)i + 1]];
+    const double p[3] = {(ps.x - ms[0]) / g, (ps.y - ms[1]) / g, (ps.z - ms[2]) / g};
+    const double q[3] = {(pt.x - mt[0]) / g, (pt.y - mt[1]) / g, (pt.z - mt[2]) / g};
+    double qt[3], r[3];
+#pragma unroll
+    for (int a = 0; a < 3; ++a) {
+      qt[a] = ((T[4 * a] * q[0] + T[4 * a + 1] * q[1]) + T[4 * a + 2] * q[2]) + T[4 * a + 3];
+      r[a] = p[a] - qt[a];
+    }
+    double s = par / (((r[0] * r[0] + r[1] * r[1]) + r[2] * r[2]) + par);
+    s = s * s;
+    const double w = lane == 0 ? 1.0 : s;                   // lane 0 counts the pairs
+#pragma unroll
+    for (int a = 0; a < 3; ++a) {
+      double v[10] = {0.0, 0.0, 0.0, 0.0, 0.0, 0.0, r[a], 1.0, 0.0, 0.0};
+      if (a == 0) { v[1] = -qt[2]; v[2] = qt[1]; v[3] = -1.0; }
+      if (a == 1) { v[0] = qt[2]; v[2] = -qt[0]; v[4] = -1.0; }
+      if (a == 2) { v[0] = -qt[1]; v[1] = qt[0]; v[5] = -1.0; }
+      acc += w * (icp_pick(v, pa) * icp_pick(v, pb));
+    }
+  }
+  sm[warp][lane] = acc;
+  __syncthreads();
+  if (threadIdx.x < 32) partials[32 * (size_t)blockIdx.x + lane] = ((sm[0][lane] + sm[1][lane]) + sm[2][lane]) + sm[3][lane];
+}
+
+// rotation R^T, translation mu_t - R^T mu_s - g R^T t of the normalised T = [R | t]
+__global__ void k_fgr_final(const FgrState* __restrict__ fst, const IcpState* __restrict__ ist, const uint32_t* in_dev,
+                            uint32_t in_max, const uint32_t* K_dev, uint32_t K_max, int tuple_test, uint32_t max_count,
+                            double* __restrict__ out_T, int32_t* __restrict__ out_info) {
+  const uint32_t K = apc_count(K_dev, K_max), in = apc_count(in_dev, in_max);
+  const bool too_few = fst->used < FGR_MIN_PAIRS;
+  const double* T = ist->T;
+  double R[3][3], t[3];
+  for (int a = 0; a < 3; ++a) {
+    for (int b = 0; b < 3; ++b) R[a][b] = too_few ? (a == b ? 1.0 : 0.0) : T[4 * b + a];     // R^T
+    t[a] = T[4 * a + 3];
+  }
+  for (int a = 0; a < 3; ++a) {
+    const double rs = (R[a][0] * fst->mu_s[0] + R[a][1] * fst->mu_s[1]) + R[a][2] * fst->mu_s[2];
+    const double rt = (R[a][0] * t[0] + R[a][1] * t[1]) + R[a][2] * t[2];
+    for (int b = 0; b < 3; ++b) out_T[4 * a + b] = R[a][b];
+    out_T[4 * a + 3] = too_few ? 0.0 : (fst->mu_t[a] - rs) - fst->g * rt;
+    out_T[12 + a] = 0.0;
+  }
+  out_T[15] = 1.0;
+  out_info[0] = too_few ? 0 : (int32_t)ist->iterations;
+  out_info[1] = (int32_t)in;
+  out_info[2] = (int32_t)fst->used;
+  out_info[3] = too_few ? APC_FGR_TOO_FEW : (fst->icp_info[2] == APC_ICP_DEGENERATE ? APC_FGR_DEGENERATE : APC_FGR_OK);
+  out_info[4] = !tuple_test ? 0 : (int32_t)(fst->accepted >= max_count ? fst->trials : FGR_TRIALS_PER_PAIR * K);
+  out_info[5] = (int32_t)(in - K);
+}
+
+static int fgr_check(apc_ctx* ctx, const float* src_xyzi, uint32_t n_src, const float* tgt_xyzi, uint32_t n_tgt,
+                     double division_factor, double max_corr, int iteration_number, double* out_T16_dev,
+                     int32_t* out_info_dev) {
+  APC_REQUIRE(ctx, (src_xyzi || !n_src) && (tgt_xyzi || !n_tgt) && out_T16_dev && out_info_dev, "NULL pointer");
+  APC_REQUIRE(ctx, n_src <= ctx->max_points && n_tgt <= ctx->max_points, "more points than the context was created for");
+  APC_REQUIRE(ctx, std::isfinite(division_factor) && division_factor > 1.0, "division_factor must be finite and > 1");
+  APC_REQUIRE(ctx, std::isfinite(max_corr) && max_corr > 0.0, "maximum_correspondence_distance must be finite and > 0");
+  APC_REQUIRE(ctx, iteration_number >= 0, "iteration_number must be >= 0");
+  return APC_OK;
+}
+
+// Scratch (allocated before the first launch): the pairs of the feature search, the used pairs, the loop's state.
+static int fgr_scratch(apc_ctx* ctx) {
+  NeighborScratch* sc = scratch_of(ctx);
+  const size_t M = ctx->max_points;
+  if (!sc->feat_pairs) APC_CUDA(ctx, cudaMalloc((void**)&sc->feat_pairs, M * 2 * sizeof(int32_t)));
+  if (!sc->feat_count) APC_CUDA(ctx, cudaMalloc((void**)&sc->feat_count, 2 * sizeof(uint32_t)));
+  if (!sc->fgr_pairs) APC_CUDA(ctx, cudaMalloc((void**)&sc->fgr_pairs, 3 * M * 2 * sizeof(int32_t)));
+  if (!sc->fgr_state) APC_CUDA(ctx, cudaMalloc((void**)&sc->fgr_state, sizeof(FgrState)));
+  if (!sc->icp_part) APC_CUDA(ctx, cudaMalloc((void**)&sc->icp_part, (size_t)ICP_MAX_BLOCKS * 32 * sizeof(double)));
+  if (!sc->icp_state) APC_CUDA(ctx, cudaMalloc((void**)&sc->icp_state, sizeof(IcpState)));
+  return APC_OK;
+}
+
+// Everything after the pairs: sc->feat_pairs holds K = feat_count[1] (<= K_max) pairs, in = the pairs before
+// dropping.  The tuple test runs when max_count > 0.
+static int fgr_run(apc_ctx* ctx, const float* src_xyzi, uint32_t n_src, const uint32_t* n_src_dev, const float* tgt_xyzi,
+                   uint32_t n_tgt, const uint32_t* n_tgt_dev, uint32_t K_max, const uint32_t* in_dev, uint32_t in_max,
+                   double division_factor, int absolute, int decrease_mu, double max_corr, int iteration_number,
+                   double tuple_scale, uint32_t max_count, uint64_t seed, double* out_T16_dev, int32_t* out_info_dev,
+                   int32_t* out_pairs_used, cudaStream_t s) {
+  NeighborScratch* sc = scratch_of(ctx);
+  FgrState* fst = sc->fgr_state;
+  const float4* src = reinterpret_cast<const float4*>(src_xyzi);
+  const float4* tgt = reinterpret_cast<const float4*>(tgt_xyzi);
+  const uint32_t* K_dev = sc->feat_count + 1;
+  const bool tuple_test = max_count > 0;
+  const int32_t* used = sc->feat_pairs;
+  uint32_t used_max = K_max;
+  if (tuple_test) {
+    int32_t* out = out_pairs_used ? out_pairs_used : sc->fgr_pairs;
+    const uint64_t trials = (uint64_t)FGR_TRIALS_PER_PAIR * K_max;
+    uint32_t steps = 1;
+    while ((trials + steps * 1024ull - 1) / (steps * 1024ull) > ctx->max_tiles) steps *= 2;
+    APC_REQUIRE(ctx, steps <= FGR_TUPLE_MAX_STEPS, "more pairs than the context can test");
+    const uint32_t n_tiles = (uint32_t)((trials + steps * 1024ull - 1) / (steps * 1024ull));
+    if (n_tiles) {
+      APC_PROF(ctx, "k_fgr_tuples", s);
+      k_fgr_tuples<<<n_tiles, 256, 0, s>>>(src, tgt, sc->feat_pairs, K_dev, K_max, steps, seed, tuple_scale, max_count,
+                                           out, fst, ctx->scan_state[2], ctx->ctrl, n_tiles);
+    }
+    used = out;
+    used_max = 3 * max_count;
+  } else if (out_pairs_used && K_max) {
+    APC_CUDA(ctx, cudaMemcpyAsync(out_pairs_used, sc->feat_pairs, (size_t)K_max * 2 * sizeof(int32_t),
+                                  cudaMemcpyDeviceToDevice, s));
+  }
+  {
+    APC_PROF(ctx, "k_fgr_norm", s);
+    k_fgr_norm<<<1, 1024, 0, s>>>(src, n_src, n_src_dev, tgt, n_tgt, n_tgt_dev, K_dev, K_max, tuple_test ? 1 : 0,
+                                  max_count, absolute, fst, sc->icp_state);
+  }
+  const uint32_t bq = min(apc_div_up(used_max, 4), (uint32_t)ICP_MAX_BLOCKS);
+  for (int j = 0; bq && j < iteration_number; ++j) {
+    {
+      APC_PROF(ctx, "k_fgr_accum", s);
+      k_fgr_accum<<<bq, 128, 0, s>>>(src, tgt, used, fst, sc->icp_state, j, decrease_mu, max_corr, division_factor,
+                                     sc->icp_part);
+    }
+    APC_PROF(ctx, "k_icp_solve", s);
+    k_icp_solve<<<1, ICP_SOLVE_WARPS * 32, 0, s>>>(sc->icp_part, bq, 1, nullptr, APC_ICP_POINT_TO_PLANE, j, -1.0, -1.0,
+                                                   sc->icp_state, fst->icp_T, fst->icp_stats, fst->icp_info);
+  }
+  APC_PROF(ctx, "k_fgr_final", s);
+  k_fgr_final<<<1, 1, 0, s>>>(fst, sc->icp_state, in_dev, in_max, K_dev, K_max, tuple_test ? 1 : 0, max_count,
+                              out_T16_dev, out_info_dev);
+  APC_LAUNCH_CHECK(ctx, "fgr");
+  return APC_OK;
+}
+
+extern "C" int apc_fgr_from_features(apc_ctx* ctx, const float* src_xyzi, uint32_t n_src, const uint32_t* n_src_dev,
+                                     const float* tgt_xyzi, uint32_t n_tgt, const uint32_t* n_tgt_dev,
+                                     const float* src_feat, const float* tgt_feat, int dim, double division_factor,
+                                     int use_absolute_scale, int decrease_mu, double maximum_correspondence_distance,
+                                     int iteration_number, double tuple_scale, int maximum_tuple_count, int tuple_test,
+                                     uint64_t seed, double* out_T16_dev, int32_t* out_info_dev,
+                                     int32_t* out_pairs_used, void* stream) {
+  if (!ctx) return APC_ERR_BAD_ARG;
+  int rc = fgr_check(ctx, src_xyzi, n_src, tgt_xyzi, n_tgt, division_factor, maximum_correspondence_distance,
+                     iteration_number, out_T16_dev, out_info_dev);
+  if (rc) return rc;
+  APC_REQUIRE(ctx, (src_feat || !n_src) && (tgt_feat || !n_tgt), "NULL pointer");
+  APC_REQUIRE(ctx, dim >= 1 && dim <= 64, "dim must be in 1..64");
+  APC_REQUIRE(ctx, tuple_scale > 0.0 && tuple_scale <= 1.0, "tuple_scale must be in (0, 1]");
+  APC_REQUIRE(ctx, maximum_tuple_count >= 1 && (uint32_t)maximum_tuple_count <= ctx->max_points,
+              "maximum_tuple_count must be in 1..max_points");
+  const uint32_t n_tiles = apc_div_up(n_src, APC_TILE_POINTS);
+  APC_REQUIRE(ctx, n_tiles <= ctx->max_tiles, "more rows than the context was created for");
+  NeighborScratch* sc = scratch_of(ctx);
+  for (auto& p : sc->feat_best)
+    if (!p) APC_CUDA(ctx, cudaMalloc((void**)&p, (size_t)ctx->max_points * sizeof(unsigned long long)));
+  rc = fgr_scratch(ctx);
+  if (rc) return rc;
+  cudaStream_t s = (cudaStream_t)stream;
+  rc = apc_begin(ctx, s);
+  if (rc) return rc;
+  APC_CUDA(ctx, cudaMemsetAsync(sc->fgr_state, 0, sizeof(FgrState), s));
+  APC_CUDA(ctx, cudaMemsetAsync(sc->feat_count, 0, 2 * sizeof(uint32_t), s));
+  if (n_src && n_tgt) {
+    rc = feat_search(ctx, src_feat, n_src, n_src_dev, tgt_feat, n_tgt, n_tgt_dev, (uint32_t)dim, sc->feat_best[0], s);
+    if (!rc) rc = feat_search(ctx, tgt_feat, n_tgt, n_tgt_dev, src_feat, n_src, n_src_dev, (uint32_t)dim, sc->feat_best[1], s);
+    if (rc) return rc;
+    APC_PROF(ctx, "k_feat_pairs", s);
+    k_feat_pairs<<<n_tiles, APC_TILE_THREADS, 0, s>>>(n_src, n_src_dev, sc->feat_best[0], sc->feat_best[1], nullptr,
+                                                      sc->fgr_pairs, sc->feat_pairs, sc->feat_count, ctx->scan_state[0],
+                                                      ctx->scan_state[1], ctx->ctrl, n_tiles);
+  }
+  const uint32_t K_max = n_tgt ? n_src : 0;
+  return fgr_run(ctx, src_xyzi, n_src, n_src_dev, tgt_xyzi, n_tgt, n_tgt_dev, K_max, sc->feat_count + 1, K_max,
+                 division_factor, use_absolute_scale ? 1 : 0, decrease_mu ? 1 : 0, maximum_correspondence_distance,
+                 iteration_number, tuple_scale, tuple_test ? (uint32_t)maximum_tuple_count : 0u, seed, out_T16_dev,
+                 out_info_dev, out_pairs_used, s);
+}
+
+extern "C" int apc_fgr(apc_ctx* ctx, const float* src_xyzi, uint32_t n_src, const uint32_t* n_src_dev,
+                       const float* tgt_xyzi, uint32_t n_tgt, const uint32_t* n_tgt_dev, const int32_t* pairs,
+                       uint32_t n_pairs, const uint32_t* n_pairs_dev, double division_factor, int use_absolute_scale,
+                       int decrease_mu, double maximum_correspondence_distance, int iteration_number,
+                       double* out_T16_dev, int32_t* out_info_dev, int32_t* out_pairs_used, void* stream) {
+  if (!ctx) return APC_ERR_BAD_ARG;
+  int rc = fgr_check(ctx, src_xyzi, n_src, tgt_xyzi, n_tgt, division_factor, maximum_correspondence_distance,
+                     iteration_number, out_T16_dev, out_info_dev);
+  if (rc) return rc;
+  APC_REQUIRE(ctx, pairs || !n_pairs, "NULL pointer");
+  APC_REQUIRE(ctx, n_pairs <= ctx->max_points, "more pairs than the context was created for");
+  const uint32_t n_tiles = apc_div_up(n_pairs, APC_TILE_POINTS);
+  APC_REQUIRE(ctx, n_tiles <= ctx->max_tiles, "more pairs than the context was created for");
+  rc = fgr_scratch(ctx);
+  if (rc) return rc;
+  NeighborScratch* sc = scratch_of(ctx);
+  cudaStream_t s = (cudaStream_t)stream;
+  rc = apc_begin(ctx, s);
+  if (rc) return rc;
+  APC_CUDA(ctx, cudaMemsetAsync(sc->fgr_state, 0, sizeof(FgrState), s));
+  APC_CUDA(ctx, cudaMemsetAsync(sc->feat_count, 0, 2 * sizeof(uint32_t), s));
+  if (n_tiles) {
+    APC_PROF(ctx, "k_fgr_pairs", s);
+    k_fgr_pairs<<<n_tiles, APC_TILE_THREADS, 0, s>>>(pairs, n_pairs, n_pairs_dev, n_src, n_src_dev, n_tgt, n_tgt_dev,
+                                                     sc->feat_pairs, sc->feat_count + 1, ctx->scan_state[0], ctx->ctrl,
+                                                     n_tiles);
+  }
+  return fgr_run(ctx, src_xyzi, n_src, n_src_dev, tgt_xyzi, n_tgt, n_tgt_dev, n_pairs, n_pairs_dev, n_pairs,
+                 division_factor, use_absolute_scale ? 1 : 0, decrease_mu ? 1 : 0, maximum_correspondence_distance,
+                 iteration_number, 1.0, 0u, 0, out_T16_dev, out_info_dev, out_pairs_used, s);
 }

@@ -22,13 +22,6 @@ APC_TRACE_EXPORT(ransac)
 #define RS_CHUNK 16
 #define RS_MAX_N 16
 
-__device__ __forceinline__ uint64_t splitmix64_dev(uint64_t x) {
-  uint64_t z = x + 0x9E3779B97F4A7C15ull;
-  z = (z ^ (z >> 30)) * 0xBF58476D1CE4E5B9ull;
-  z = (z ^ (z >> 27)) * 0x94D049BB133111EBull;
-  return z ^ (z >> 31);
-}
-
 __device__ __forceinline__ void plane_from_moments(double cx, double cy, double cz, double xx, double xy, double xz,
                                                    double yy, double yz, double zz, double* out) {
   const double det_x = __dsub_rn(__dmul_rn(yy, zz), __dmul_rn(yz, yz));

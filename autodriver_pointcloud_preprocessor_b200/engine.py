@@ -430,6 +430,45 @@ class Context:
                                                        _ptr(info), _stream()))
         return pairs[:n_src], info, (nearest[:n_src] if nearest is not None else None)
 
+    def fgr_from_features(self, src_xyzi, tgt_xyzi, src_feat, tgt_feat, division_factor=1.4, use_absolute_scale=False,
+                          decrease_mu=True, maximum_correspondence_distance=0.025, iteration_number=64,
+                          tuple_scale=0.95, maximum_tuple_count=1000, tuple_test=True, seed=0, n_src_dev=None,
+                          n_tgt_dev=None):
+        """``apc_fgr_from_features`` on xyzi clouds and float32 ``[n, dim]`` feature rows (contiguous, on the device).
+        Returns ``(T float64[4,4], info int32[6] {iterations, pairs in, pairs used, APC_FGR_* status, trials, pairs
+        dropped}, pairs_used int32[cap, 2])`` on the device, with no host synchronisation; the first ``pairs used``
+        rows of ``pairs_used`` are valid."""
+        n_src, n_tgt = src_xyzi.shape[0], tgt_xyzi.shape[0]
+        dim = src_feat.shape[1] if src_feat.dim() == 2 else 0
+        T = self._empty((4, 4), torch.float64)
+        info = self._empty((6,), torch.int32)
+        cap = 3 * min(max(int(maximum_tuple_count), 1), self.max_points) if tuple_test else n_src   # larger: rejected
+        used = self._empty((max(cap, 1), 2), torch.int32)
+        self._ok(lib.apc_fgr_from_features(self.h, _ptr(src_xyzi), n_src, _ptr(n_src_dev), _ptr(tgt_xyzi), n_tgt,
+                                           _ptr(n_tgt_dev), _ptr(src_feat), _ptr(tgt_feat), int(dim),
+                                           float(division_factor), int(bool(use_absolute_scale)),
+                                           int(bool(decrease_mu)), float(maximum_correspondence_distance),
+                                           int(iteration_number), float(tuple_scale), int(maximum_tuple_count),
+                                           int(bool(tuple_test)), int(seed) & 0xFFFFFFFFFFFFFFFF, _ptr(T), _ptr(info),
+                                           _ptr(used), _stream()))
+        return T, info, used
+
+    def fgr(self, src_xyzi, tgt_xyzi, pairs, division_factor=1.4, use_absolute_scale=False, decrease_mu=True,
+            maximum_correspondence_distance=0.025, iteration_number=64, n_src_dev=None, n_tgt_dev=None,
+            n_pairs_dev=None):
+        """``apc_fgr`` on int32 ``[K, 2]`` pairs (contiguous, on the device).  Returns the tuple of
+        :meth:`fgr_from_features` (``pairs_used`` int32[K, 2]); no host synchronisation."""
+        n_src, n_tgt, n_pairs = src_xyzi.shape[0], tgt_xyzi.shape[0], pairs.shape[0]
+        T = self._empty((4, 4), torch.float64)
+        info = self._empty((6,), torch.int32)
+        used = self._empty((max(n_pairs, 1), 2), torch.int32)
+        self._ok(lib.apc_fgr(self.h, _ptr(src_xyzi), n_src, _ptr(n_src_dev), _ptr(tgt_xyzi), n_tgt, _ptr(n_tgt_dev),
+                             _ptr(pairs), n_pairs, _ptr(n_pairs_dev), float(division_factor),
+                             int(bool(use_absolute_scale)), int(bool(decrease_mu)),
+                             float(maximum_correspondence_distance), int(iteration_number), _ptr(T), _ptr(info),
+                             _ptr(used), _stream()))
+        return T, info, used
+
     # ---- ransac ------------------------------------------------------------------------------------
     def segment_plane(self, xyzi, distance_threshold, ransac_n, num_iterations, probability, seed=0,
                       sample_table=None, n_dev=None):

@@ -1,6 +1,7 @@
 """``open3d.t.pipelines.registration`` look-alike: single-scale ICP (point-to-point, point-to-plane, generalized),
-``evaluate_registration``, FPFH features (``compute_fpfh_feature``) and matching in feature space
-(``correspondences_from_features``) on the GPU.
+``evaluate_registration``, FPFH features (``compute_fpfh_feature``), matching in feature space
+(``correspondences_from_features``) and Fast Global Registration (``registration_fgr_based_on_feature_matching``,
+``registration_fgr_based_on_correspondence``) on the GPU.
 
 The whole ICP loop runs on the device (``apc_icp``): the call synchronises once, at the end.  Definitions, and
 where they differ from Open3D, are in ``oracle/registration.py`` and ``oracle/gicp.py``; in short:
@@ -26,8 +27,15 @@ FPFH and feature matching (``oracle/features.py``):
   index; rows whose distances are all NaN have no match and no pair.  The search is brute force,
   O(n_source * n_target * 33).
 
-Not modelled: multi-scale ICP, colored ICP, robust kernels, per-iteration callbacks and global registration
-(RANSAC / FGR on feature correspondences).
+Fast Global Registration (``oracle/fgr.py``, Zhou, Park and Koltun 2016):
+
+* the feature entry starts from the mutual set of the feature matching, with no ratio fallback;
+* the tuple test draws its triples from a counter-based stream seeded with ``option.seed`` (0 when None), where
+  Open3D uses its own random generator: results are reproducible but not Open3D's draws;
+* the transform accumulates and the original target is transformed every iteration (Open3D moves its copy of the
+  target in place); fewer than 10 pairs after the tuple test warn and return the identity.
+
+Not modelled: multi-scale ICP, colored ICP, robust kernels, per-iteration callbacks and RANSAC global registration.
 """
 from __future__ import annotations
 
@@ -267,3 +275,103 @@ def correspondences_from_features(source_features, target_features, mutual_filte
         warnings.warn("Too few correspondences after mutual filter, fall back to original correspondences.",
                       RuntimeWarning, stacklevel=2)
     return home(pairs[:count].to(torch.int64))
+
+
+class FastGlobalRegistrationOption:
+    """Open3D's ``FastGlobalRegistrationOption``.  ``seed`` (None means 0) seeds the tuple test's draws."""
+
+    def __init__(self, division_factor=1.4, use_absolute_scale=False, decrease_mu=True,
+                 maximum_correspondence_distance=0.025, iteration_number=64, tuple_scale=0.95,
+                 maximum_tuple_count=1000, tuple_test=True, seed=None):
+        self.division_factor = float(division_factor)
+        self.use_absolute_scale = bool(use_absolute_scale)
+        self.decrease_mu = bool(decrease_mu)
+        self.maximum_correspondence_distance = float(maximum_correspondence_distance)
+        self.iteration_number = int(iteration_number)
+        self.tuple_scale = float(tuple_scale)
+        self.maximum_tuple_count = int(maximum_tuple_count)
+        self.tuple_test = bool(tuple_test)
+        self.seed = None if seed is None else int(seed)
+        if not (math.isfinite(self.division_factor) and self.division_factor > 1):
+            raise ValueError("division_factor must be finite and > 1")
+        if not (math.isfinite(self.maximum_correspondence_distance) and self.maximum_correspondence_distance > 0):
+            raise ValueError("maximum_correspondence_distance must be finite and > 0")
+        if self.iteration_number < 0:
+            raise ValueError("iteration_number must be >= 0")
+        if not (0 < self.tuple_scale <= 1):
+            raise ValueError("tuple_scale must be in (0, 1]")
+        if self.maximum_tuple_count < 1:
+            raise ValueError("maximum_tuple_count must be >= 1")
+
+    def __repr__(self):
+        return (f"FastGlobalRegistrationOption(division_factor={self.division_factor}, "
+                f"use_absolute_scale={self.use_absolute_scale}, decrease_mu={self.decrease_mu}, "
+                f"maximum_correspondence_distance={self.maximum_correspondence_distance}, "
+                f"iteration_number={self.iteration_number}, tuple_scale={self.tuple_scale}, "
+                f"maximum_tuple_count={self.maximum_tuple_count}, tuple_test={self.tuple_test}, seed={self.seed})")
+
+
+def _fgr_result(source: PointCloud, T, info) -> RegistrationResult:
+    """The one synchronisation of an FGR call: status, warning or error, and the result."""
+    info = info.cpu().numpy()
+    if info[3] == _capi.APC_FGR_TOO_FEW:
+        warnings.warn(f"Fast Global Registration: only {int(info[2])} correspondences (fewer than 10), returning the "
+                      "identity.", RuntimeWarning, stacklevel=3)
+    if info[3] == _capi.APC_FGR_DEGENERATE:
+        raise RuntimeError("Fast Global Registration: the linear system is not positive definite (degenerate or "
+                           "non-finite correspondences)")
+    corr = torch.full((source._n(),), -1, dtype=torch.int64, device="cuda")
+    return RegistrationResult(Tensor(T.cpu()), source._home(corr), 0.0, 0.0, False, int(info[0]))
+
+
+def _fgr_clouds(source: PointCloud, target: PointCloud):
+    n_src, n_tgt = source._n(), target._n()
+    ctx = get_context(max(n_src, n_tgt, 1), source.device.index if source.device.kind == "CUDA" else None)
+    return ctx, source._xyzi(), target._xyzi()
+
+
+def registration_fgr_based_on_feature_matching(source: PointCloud, target: PointCloud, source_feature, target_feature,
+                                               option=None) -> RegistrationResult:
+    """Open3D ``registration_fgr_based_on_feature_matching``: Fast Global Registration (Zhou, Park and Koltun 2016)
+    of ``source`` onto ``target`` from their features (``[n, dim]``, as :func:`compute_fpfh_feature` returns them).
+    The pairs are the mutual nearest neighbours in feature space, filtered by the tuple test.  The result carries
+    only the transformation (float64, CPU) and ``num_iterations``: ``fitness = inlier_rmse = 0`` and every
+    correspondence is -1, as in Open3D.  Warns and returns the identity with fewer than 10 pairs; raises
+    ``RuntimeError`` when the linear system is degenerate."""
+    opt = option if option is not None else FastGlobalRegistrationOption()
+    fs = source_feature.t if isinstance(source_feature, Tensor) else torch.as_tensor(source_feature)
+    ft = target_feature.t if isinstance(target_feature, Tensor) else torch.as_tensor(target_feature)
+    if fs.dim() != 2 or ft.dim() != 2 or fs.shape[1] != ft.shape[1]:
+        raise ValueError(f"features must be [n, dim] with the same dim, got {tuple(fs.shape)} and {tuple(ft.shape)}")
+    if fs.shape[0] != source._n() or ft.shape[0] != target._n():
+        raise ValueError(f"features have {fs.shape[0]} and {ft.shape[0]} rows for clouds of {source._n()} and "
+                         f"{target._n()} points")
+    ctx, src, tgt = _fgr_clouds(source, target)
+    fs = (fs if fs.is_cuda else fs.cuda(ctx.device)).to(torch.float32).contiguous()
+    ft = (ft if ft.is_cuda else ft.cuda(ctx.device)).to(torch.float32).contiguous()
+    T, info, _ = ctx.fgr_from_features(src, tgt, fs, ft, opt.division_factor, opt.use_absolute_scale, opt.decrease_mu,
+                                       opt.maximum_correspondence_distance, opt.iteration_number, opt.tuple_scale,
+                                       opt.maximum_tuple_count, opt.tuple_test, 0 if opt.seed is None else opt.seed)
+    ctx.check()
+    return _fgr_result(source, T, info)
+
+
+def registration_fgr_based_on_correspondence(source: PointCloud, target: PointCloud, corres,
+                                             option=None) -> RegistrationResult:
+    """Open3D ``registration_fgr_based_on_correspondence``: Fast Global Registration on the given ``(source index,
+    target index)`` pairs (int64 ``[K, 2]``, as :func:`correspondences_from_features` returns them), without the
+    tuple test.  Raises ``ValueError`` for an index outside its cloud; otherwise as
+    :func:`registration_fgr_based_on_feature_matching`."""
+    opt = option if option is not None else FastGlobalRegistrationOption()
+    c = corres.t if isinstance(corres, Tensor) else torch.as_tensor(corres)
+    if c.dim() != 2 or c.shape[1] != 2:
+        raise ValueError(f"corres must be [K, 2], got {tuple(c.shape)}")
+    c = c.to(torch.int64)
+    if c.shape[0] and (bool((c < 0).any()) or int(c[:, 0].max()) >= source._n() or int(c[:, 1].max()) >= target._n()):
+        raise ValueError("corres holds an index outside its point cloud")
+    ctx, src, tgt = _fgr_clouds(source, target)
+    pairs = c.to(device=ctx.device, dtype=torch.int32).contiguous()
+    T, info, _ = ctx.fgr(src, tgt, pairs, opt.division_factor, opt.use_absolute_scale, opt.decrease_mu,
+                         opt.maximum_correspondence_distance, opt.iteration_number)
+    ctx.check()
+    return _fgr_result(source, T, info)

@@ -380,7 +380,8 @@ int apc_compute_fpfh_knn(apc_ctx* ctx, const float* xyzi, const float* normals, 
  * increasing j, unfused; NaN and infinite d2 never win, and a row without a finite d2 has no match.
  * out_pairs int32[2 * n_src]: the first count rows hold (i, match) in ascending i, for every source row with a match
  * or, with mutual_filter, only those whose match's own match is i - unless that set has no more than
- * ratio * n_src pairs, when the unfiltered set is returned and fell_back is 1 (Open3D warns).  out_nearest
+ * ratio * n_src pairs, when the unfiltered set is returned and fell_back is 1 (Open3D warns); the rows past the
+ * unfiltered set's count are (-1, -1).  out_nearest
  * int32[n_src] (may be NULL): every row's match, -1 for none.  out_info_dev uint32[2] (device) = {count,
  * fell_back}.  Brute force, O(n_src * n_tgt * dim) per direction (the target-to-source search runs only with
  * mutual_filter).  APC_ERR_BAD_ARG: NULL pointers, dim outside 1..64, ratio not finite or < 0, more rows than
@@ -389,6 +390,54 @@ int apc_correspondences_from_features(apc_ctx* ctx, const float* src, uint32_t n
                                       const float* tgt, uint32_t n_tgt, const uint32_t* n_tgt_dev, int dim,
                                       int mutual_filter, double ratio, int32_t* out_pairs, int32_t* out_nearest,
                                       uint32_t* out_info_dev, void* stream);
+
+enum { APC_FGR_OK = 0, APC_FGR_TOO_FEW = 1, APC_FGR_DEGENERATE = 2 };
+
+/* registration_fgr_based_on_feature_matching(source, target, source_feature, target_feature, option) (Open3D
+ * pipelines::registration::FastGlobalRegistrationBasedOnFeatureMatching; Zhou, Park, Koltun 2016).  Contract
+ * (oracle/fgr.py):
+ *   pairs: the mutual set of apc_correspondences_from_features (every source row whose match's own match is itself,
+ *     in ascending row), never the fallback;
+ *   tuple test (tuple_test != 0): K pairs, trials t = 0 .. 100 K - 1; draw k of trial t is ((z >> 32) * K) >> 32
+ *     with z = splitmix64(seed + (t << 32) + k); the tuple is accepted iff on each edge (0,1), (1,2), (2,0)
+ *     li * tuple_scale < lj and lj < li / tuple_scale (l = sqrt((dx*dx + dy*dy) + dz*dz), float64, the source
+ *     points' li, the target points' lj), and its three pairs are kept in draw order, in trial order, up to
+ *     maximum_tuple_count tuples;
+ *   normalisation: the means of all points of each cloud, D the largest centred norm; relative scale divides by D
+ *     and starts with par = 1, use_absolute_scale keeps metres and starts with par = D;
+ *   iteration_number Gauss-Newton steps of sum s |p - T q|^2, s = (par / (|r|^2 + par))^2, from T = I, with
+ *     par /= division_factor before iterations 0, 4, 8, ... while par > maximum_correspondence_distance
+ *     (decrease_mu); the 6x6 system is solved as point-to-plane ICP's (APC_FGR_DEGENERATE when it is not positive
+ *     definite or not finite: the loop stops) and T = Rz Ry Rx update T;
+ *   out_T16_dev double[16] (device, row-major): the source-to-target transform in metres, [R^T | mu_t - R^T mu_s -
+ *     g R^T t] (g = D relative, 1 absolute); fewer than 10 pairs reaching the loop is APC_FGR_TOO_FEW and gives the
+ *     identity, 0 iterations.
+ * out_info_dev int32[6] (device) = {iterations, pairs in, pairs used, APC_FGR_* status, trials (the index of the
+ * last trial examined + 1, 0 without the tuple test), pairs dropped}.  out_pairs_used int32[2 * cap] (may be NULL):
+ * the pairs used, in order; cap = 3 * maximum_tuple_count with the tuple test, n_src without.  Features are rows of
+ * dim float32 values as apc_correspondences_from_features takes them.  No host synchronisation; launch
+ * configurations depend on the host sizes only, and the call can be captured in a CUDA graph.  APC_ERR_BAD_ARG:
+ * NULL pointers, sizes above the context's max_points, dim outside 1..64, division_factor not finite or not > 1,
+ * maximum_correspondence_distance not finite or not > 0, iteration_number < 0, tuple_scale outside (0, 1],
+ * maximum_tuple_count outside 1..max_points. */
+int apc_fgr_from_features(apc_ctx* ctx, const float* src_xyzi, uint32_t n_src, const uint32_t* n_src_dev,
+                          const float* tgt_xyzi, uint32_t n_tgt, const uint32_t* n_tgt_dev, const float* src_feat,
+                          const float* tgt_feat, int dim, double division_factor, int use_absolute_scale,
+                          int decrease_mu, double maximum_correspondence_distance, int iteration_number,
+                          double tuple_scale, int maximum_tuple_count, int tuple_test, uint64_t seed,
+                          double* out_T16_dev, int32_t* out_info_dev, int32_t* out_pairs_used, void* stream);
+
+/* registration_fgr_based_on_correspondence(source, target, corres, option) (Open3D
+ * FastGlobalRegistrationBasedOnCorrespondence): the normalisation, loop and outputs of apc_fgr_from_features on the
+ * caller's pairs int32[2 * n_pairs] (source index, target index; the device count n_pairs_dev, may be NULL), with
+ * no tuple test (trials = 0).  A pair with an index outside its cloud's count is never read: it is dropped and
+ * counted.  out_pairs_used int32[2 * n_pairs] (may be NULL): the pairs kept, in order.  APC_ERR_BAD_ARG as
+ * apc_fgr_from_features, and NULL pairs with n_pairs > 0. */
+int apc_fgr(apc_ctx* ctx, const float* src_xyzi, uint32_t n_src, const uint32_t* n_src_dev, const float* tgt_xyzi,
+            uint32_t n_tgt, const uint32_t* n_tgt_dev, const int32_t* pairs, uint32_t n_pairs,
+            const uint32_t* n_pairs_dev, double division_factor, int use_absolute_scale, int decrease_mu,
+            double maximum_correspondence_distance, int iteration_number, double* out_T16_dev, int32_t* out_info_dev,
+            int32_t* out_pairs_used, void* stream);
 
 /* ---- (4) RANSAC ground plane --------------------------------------------------------- */
 
