@@ -70,7 +70,6 @@ struct apc_ctx {
   float* knn_avg = nullptr;         // [max_points]
   double* red_a = nullptr;          // reduction ping-pong
   double* red_b = nullptr;
-  uint32_t* nb_count = nullptr;     // [max_points]
   // ransac
   double* rs_planes = nullptr;      // [max_iters*4]
   unsigned long long* rs_scores = nullptr;  // per-CTA tally rows of k_rs_score {inliers, err}, column by column
@@ -99,7 +98,6 @@ struct apc_ctx {
   // the difference between two runs.  -1 = off.
   int launch_budget = -1;
   mutable int launch_seq = 0;       // launches issued since apc_begin
-  bool fold_begin = false;          // run_pipeline -> apc_frontend_nobegin: k_dedup_insert does k_begin's work (see apc_begin_folded)
 };
 
 // RAII timer around one kernel launch; a no-op unless profiling is enabled on the context.
@@ -133,9 +131,6 @@ struct ProfScope {
 int apc_set_error(apc_ctx* ctx, int code, const char* what, cudaError_t ce = cudaSuccess);
 // bumps the epoch; every public entry point calls it first
 int apc_begin(apc_ctx* ctx, cudaStream_t s);
-// The same without the k_begin launch: the first kernel of the call bumps the epoch and zeroes the counters
-// itself (begin_in_kernel below) - it must neither read them nor run concurrently with a kernel that does.
-int apc_begin_folded(apc_ctx* ctx);
 
 #define APC_CUDA(ctx, call)                                                \
   do {                                                                     \
@@ -193,17 +188,10 @@ __device__ __forceinline__ void pdl_enter() {
 // ---- device helpers ----------------------------------------------------------------------
 #ifdef __CUDACC__
 
-// k_begin's work, done by the first 32 threads of one CTA of the call's first kernel
-__device__ __forceinline__ void begin_in_kernel(ApcCtrl* ctrl) {
-  if (threadIdx.x == 0) ctrl->epoch = ctrl->epoch + 1u;
-  if (threadIdx.x < 30) ctrl->counters[threadIdx.x] = 0u;
-}
-
 // The pipeline's eight output counters (APC_CNT_*), assembled from the stages' device counters by the
-// kernel that runs last: the ticket-last CTA of k_rs_final when the pipeline ends with ground removal
-// (one launch less on every scan of the C1 / C2 configurations), else the one-thread k_pipeline_counts.
+// one-thread k_pipeline_counts, the last kernel of every pipeline run.
 struct CountsEpilogue {
-  const uint32_t* dc;          // the context's dev_counts (NULL: no epilogue)
+  const uint32_t* dc;          // the context's dev_counts
   uint32_t* out;               // uint32[8]
   uint32_t n_input, last;
   int has_vox, has_stat, has_rad, has_ground;

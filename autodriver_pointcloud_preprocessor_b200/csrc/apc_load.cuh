@@ -114,12 +114,10 @@ struct TilePoint {
 // GENERIC = false compiles the FAST16 path only (the host launches that instantiation when every
 // segment qualifies): the byte-record decoder is a lot of code, and keeping it out of the common
 // kernel keeps the hot loop inside the instruction cache.
-// `last_use`: the caller is the last reader of these bytes (k_frontend, after k_dedup_insert): streaming loads
-// (ld.global.cs, evict-first) so that the dead input does not push the lanes' hash tables out of the L2.
 template <bool GENERIC>
 __device__ __forceinline__ void load_tile(const SegDev& s, uint32_t tile_local, bool test_nan,
                                           uint8_t* stage, uint64_t* bar,
-                                          TilePoint (&pt)[APC_TILE_ITEMS], bool last_use = false) {
+                                          TilePoint (&pt)[APC_TILE_ITEMS]) {
   const uint32_t first = tile_local * APC_TILE_POINTS;
   const uint32_t in_tile = min(APC_TILE_POINTS, s.n - first);
   if (!GENERIC || s.fast16) {
@@ -129,7 +127,7 @@ __device__ __forceinline__ void load_tile(const SegDev& s, uint32_t tile_local, 
       const uint32_t e = j * APC_TILE_THREADS + threadIdx.x;
       pt[j].valid = e < in_tile;
       float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
-      if (pt[j].valid) v = last_use ? __ldcs(src + e) : ld_stream_f4(src + e);
+      if (pt[j].valid) v = ld_stream_f4(src + e);
       bool nn = true;
       if (test_nan) {
         if ((s.nan_words & 1u) && is_nan_f(v.x)) nn = false;

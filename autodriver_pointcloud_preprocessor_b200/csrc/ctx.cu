@@ -79,21 +79,13 @@ extern "C" int apc_ctx_destroy(apc_ctx* ctx) {
   for (cudaEvent_t e : ctx->prof.ev) cudaEventDestroy(e);
   void* ptrs[] = {ctx->ctrl, ctx->vox_slots, ctx->vox_acc, ctx->vox_rank, ctx->p2slot,
                   ctx->dedup_slots, ctx->sorted_pts, ctx->knn_avg, ctx->red_a,
-                  ctx->red_b, ctx->nb_count, ctx->rs_planes, ctx->rs_scores, ctx->rs_scores_copy, ctx->rs_col_tickets, ctx->rs_partials, ctx->buf_a, ctx->buf_b,
+                  ctx->red_b, ctx->rs_planes, ctx->rs_scores, ctx->rs_scores_copy, ctx->rs_col_tickets, ctx->rs_partials, ctx->buf_a, ctx->buf_b,
                   ctx->mask_a, ctx->idx_a, ctx->idx_b, ctx->dev_counts, ctx->nrm_scratch};
   for (void* p : ptrs)
     if (p) cudaFree(p);
   for (auto* p : ctx->scan_state)
     if (p) cudaFree(p);
   delete ctx;
-  return APC_OK;
-}
-
-int apc_begin_folded(apc_ctx* ctx) {
-  int cur = -1;
-  if (cudaGetDevice(&cur) == cudaSuccess && cur != ctx->device)
-    return apc_set_error(ctx, APC_ERR_BAD_ARG, "the context lives on another device than the calling thread's current one");
-  ctx->launch_seq = 0;
   return APC_OK;
 }
 
@@ -134,7 +126,6 @@ extern "C" int apc_ctx_create(int device, uint32_t max_points, apc_ctx** out) {
   A(dalloc(&ctx->knn_avg, M));
   A(dalloc(&ctx->red_a, red));
   A(dalloc(&ctx->red_b, red));
-  A(dalloc(&ctx->nb_count, M));
   A(dalloc(&ctx->rs_planes, (size_t)ctx->rs_max_iters * 4));
   // per-CTA tally rows of k_rs_score: <= 2 CTAs per SM, 20 hypotheses each, plus one padded row per launch
   A(dalloc(&ctx->rs_scores, (size_t)(APC_SM_COUNT * 2 * 20 + ctx->rs_max_iters + 64) * 2));

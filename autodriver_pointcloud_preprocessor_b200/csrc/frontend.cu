@@ -8,7 +8,6 @@
 // pp.py:469 (remove_non_finite_points), pp.py:482,487,490 (transform), utils.py:240-301
 // (crop_pointcloud), utils.py:271,297 + pp.py:542 (select_by_mask / select_by_index),
 // pointcloud_concatenator.py:1-5 (merge N sensors into one cloud in a target frame).
-#include <cstdlib>
 
 #include "apc_load.cuh"
 APC_TRACE_EXPORT(frontend)
@@ -34,8 +33,6 @@ struct FrontendParams {
   uint32_t* out_count;
   uint64_t* scan_state;
   ApcCtrl* ctrl;
-  uint32_t do_begin;      // k_dedup_insert is the first kernel of the call: CTA 0 does k_begin's work
-  uint32_t stream_in;     // k_frontend reads the input with evict-first loads (APC_STREAM_IN, A/B knob)
 };
 
 // ---- duplicate removal: 64-bit open-addressing slots {fingerprint:32 | lowest point index:32} -----
@@ -134,7 +131,6 @@ __global__ void __launch_bounds__(APC_TILE_THREADS) k_dedup_insert(const __grid_
   __shared__ __align__(8) uint64_t bar;
   pdl_enter();
   const uint32_t tile = blockIdx.x;
-  if (prm.do_begin && tile == 0) begin_in_kernel(prm.ctrl);   // nothing in this kernel reads the epoch or the counters
   const uint32_t si = find_segment(prm, tile);
   const SegDev& s = prm.seg[si];
   TilePoint pt[APC_TILE_ITEMS];
@@ -191,7 +187,7 @@ __global__ void __launch_bounds__(APC_TILE_THREADS) k_frontend(const __grid_cons
   const uint32_t epoch = prm.ctrl->epoch;
   TilePoint pt[APC_TILE_ITEMS];
   APC_STAMP(1, 0);
-  load_tile<GENERIC>(s, tile - s.tile_begin, prm.skip_nans != 0, stage, &bar, pt, prm.stream_in != 0);
+  load_tile<GENERIC>(s, tile - s.tile_begin, prm.skip_nans != 0, stage, &bar, pt);
 
   bool keep[APC_TILE_ITEMS];
   uint32_t gidx[APC_TILE_ITEMS];
@@ -396,10 +392,9 @@ static int build_params(apc_ctx* ctx, const apc_cloud_desc* clouds, uint32_t n_c
     }
   }
   prm.slots = ctx->dedup_slots;
-  // the duplicate table is all touched once per scan (4 slots per 32-byte sector, one point in four
-  // slots): APC_DEDUP_SHRINK = 1 uses half of it (load 0.5, half the sectors), 0 all of it
-  static const uint32_t shrink = []() { const char* e = getenv("APC_DEDUP_SHRINK"); return e ? (uint32_t)atoi(e) & 3u : 0u; }();
-  prm.slot_mask = (ctx->hash_cap >> shrink) - 1;
+  // the whole duplicate table (one point in four slots): using half of it (load 0.5, half the 32-byte
+  // sectors touched per scan) was slower, 69.7 vs 68.1 us/scan
+  prm.slot_mask = ctx->hash_cap - 1;
   prm.p2slot = ctx->p2slot;
   prm.ctrl = ctx->ctrl;
   *total_points = points;
@@ -499,10 +494,6 @@ int apc_frontend_nobegin(apc_ctx* ctx, const apc_cloud_desc* clouds, uint32_t n_
   rc = set_smem(ctx, smem);
   if (rc) return rc;
   const bool generic = smem != 0;   // some segment needs the byte-record decoder
-  APC_REQUIRE(ctx, !ctx->fold_begin || prm.dedup, "folded begin needs the duplicate-insert kernel");
-  prm.do_begin = ctx->fold_begin ? 1u : 0u;
-  static const uint32_t stream_in = []() { const char* e = getenv("APC_STREAM_IN"); return e ? (uint32_t)atoi(e) : 0u; }();
-  prm.stream_in = stream_in;
   if (prm.dedup) {
     APC_PROF(ctx, "k_dedup_insert", s);
     if (generic) apc_klaunch(ctx, k_dedup_insert<true>, prm.n_tiles, APC_TILE_THREADS, smem, s, prm);

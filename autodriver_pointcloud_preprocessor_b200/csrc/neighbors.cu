@@ -11,12 +11,11 @@
 // size c0 * 2^l; the key packs (level:4 | ix:19 | iy:19 | iz:19).  Points are counting-
 // sorted per level into cell-contiguous arrays, so a query reads its 27 neighbour cells as
 // 27 short contiguous runs.  Queries run in level-0 sorted order so the lanes of a warp
-// share cells.  Radius search uses one level with c0 = r * (1 + 2^-10); KNN climbs levels
+// share cells.  Radius search uses one level with c0 = 2r * (1 + 2^-10); KNN climbs levels
 // until the k-th distance is covered by the 27-cell block, and the rare points that never
 // are (fewer than k points in range of the coarsest level) fall to an exact brute-force
 // kernel.  The table is cleaned by the points that own rank 0 of their cell, not by memset.
 #include <cmath>
-#include <cstdlib>
 #include <cstring>
 #include "apc_scan.cuh"
 #include "apc_grid.cuh"
@@ -232,75 +231,8 @@ __device__ __forceinline__ uint32_t grid_sorted_count(const GridDev& g, const Ap
 }
 
 // ---- radius query -----------------------------------------------------------------------------
-// Neighbours of q within r2 among the first `n_cells` cells of the centre-first order (1 = own cell
-// only, 27 = the whole block), stopping at nb_points unless the exact count is wanted.
-__device__ __forceinline__ uint32_t radius_count(const GridDev& g, float c, float4 q, float r2, uint32_t nb_points,
-                                                 int need_counts, int n_cells) {
-  int32_t ix, iy, iz;
-  grid_coord_g(g, c, q.x, q.y, q.z, ix, iy, iz);  // succeeded at insert time
-  uint32_t cnt = 0;
-  // own cell first, then faces, edges, corners: when only the keep/drop decision is wanted
-  // most points reach nb_points inside their own cell and stop there.  The first probe of the
-  // NEXT cell is in flight while the current cell's points are scanned.
-  uint64_t key = grid_key(0, ix, iy, iz);
-  uint32_t home = grid_home(g, key);
-  uint4 first = grid_load(g, home);
-  for (int c27 = 0; c27 < n_cells && (need_counts || cnt < nb_points); ++c27) {
-    const uint64_t key_now = key;
-    const uint32_t home_now = home;
-    const uint4 first_now = first;
-    if (c27 + 1 < n_cells) {
-      const int code = c_cell_order[c27 + 1];
-      key = grid_key(0, ix + code % 3 - 1, iy + (code / 3) % 3 - 1, iz + code / 9 - 1);
-      home = grid_home(g, key);
-      first = grid_load(g, home);
-    }
-    uint32_t b, f;
-    if (!grid_resolve(g, key_now, home_now, first_now, b, f)) continue;
-    const uint32_t e = b + f;
-    // four points per round: their loads are independent, the exit test runs once per round
-    for (uint32_t t = b; t < e && (need_counts || cnt < nb_points); t += 4) {
-      float4 p[4];
-#pragma unroll
-      for (int u = 0; u < 4; ++u) p[u] = g.sorted[min(t + u, e - 1)];
-#pragma unroll
-      for (int u = 0; u < 4; ++u)
-        cnt += (t + u < e && d2_f32(q.x, q.y, q.z, p[u].x, p[u].y, p[u].z) <= r2) ? 1u : 0u;
-    }
-  }
-  return cnt;
-}
-
-__global__ void __launch_bounds__(128)
-k_radius_query(uint32_t n_max, const uint32_t* n_dev, GridDev g, float r2, uint32_t nb_points, int need_counts,
-               uint8_t* __restrict__ mask, uint32_t* __restrict__ counts, const ApcCtrl* __restrict__ ctrl) {
-  pdl_enter();
-  const uint32_t n = grid_sorted_count(g, ctrl, apc_count(n_dev, n_max));
-  const float c = grid_cell_size(g, 0);
-  APC_STAMP(0, 0);
-  for (uint32_t j = blockIdx.x * blockDim.x + threadIdx.x; j < n; j += gridDim.x * blockDim.x) {
-    const float4 q = g.sorted[j];
-    const uint32_t orig = __float_as_uint(q.w);
-    const uint32_t cnt = radius_count(g, c, q, r2, nb_points, need_counts, 27);
-    mask[orig] = cnt >= nb_points ? 1 : 0;
-    if (counts) counts[orig] = cnt;
-  }
-  APC_STAMP(0, 1);
-}
-
-// ---- radius query over cells of 2r: own cell, then only the neighbours the r-ball can reach ------
-// With a cell edge of 2r (+ slack) the ball around q reaches, along every axis, at most ONE of the two
-// neighbouring cells (the one behind the nearer face), so 1 + 7 cells cover it instead of 27, and a
-// neighbour (a face, edge or corner cell) is visited only if the ball reaches its box: sum over the
-// offset axes of gap^2 <= r^2, gap = distance from q to that face.  On a voxelised 128-beam scan the
-// own cell alone settles 95 % of the keep / drop decisions (cells of r: 75 %), and the others probe
-// 3 to 7 cells, not 26 (profiles/r2p_radius_ab.json).  The set of points tested against d2 <= r2 is a
-// superset of the ball either way, so counts and decisions are bit-identical to the 27-cell walk.
-// Slack: the cell index is floor(fl(x * fl(1/c))) (grid_coord_g), two roundings of 2^-24 each, so a point
-// of the cell below has x < ix*c*(1 + 2^-23) and one of the cell above x >= (ix+1)*c*(1 - 2^-23); the
-// products, differences and d2 below each carry a relative rounding error of 2^-24.  gap is therefore shortened by 1e-6 * (|q| + c) + 1e-5 * r (8x the worst
-// case); if that ever leaves BOTH faces of an axis within reach (coordinates of tens of kilometres) the
-// query falls back to the 27-cell walk.
+// cnt + the neighbours of q within r2 in the run [b, b + f) of the cell-sorted array, stopping at nb_points
+// unless the exact count is wanted.
 __device__ __forceinline__ uint32_t radius_scan_run(const GridDev& g, uint32_t b, uint32_t f, float4 q, float r2,
                                                     uint32_t nb_points, int need_counts, uint32_t cnt) {
   const uint32_t e = b + f;
@@ -316,6 +248,49 @@ __device__ __forceinline__ uint32_t radius_scan_run(const GridDev& g, uint32_t b
   return cnt;
 }
 
+// Neighbours of q within r2 in the whole 27-cell block, stopping at nb_points unless the exact count is wanted.
+__device__ __forceinline__ uint32_t radius_count(const GridDev& g, float c, float4 q, float r2, uint32_t nb_points,
+                                                 int need_counts) {
+  int32_t ix, iy, iz;
+  grid_coord_g(g, c, q.x, q.y, q.z, ix, iy, iz);  // succeeded at insert time
+  uint32_t cnt = 0;
+  // own cell first, then faces, edges, corners: when only the keep/drop decision is wanted
+  // most points reach nb_points inside their own cell and stop there.  The first probe of the
+  // NEXT cell is in flight while the current cell's points are scanned.
+  uint64_t key = grid_key(0, ix, iy, iz);
+  uint32_t home = grid_home(g, key);
+  uint4 first = grid_load(g, home);
+  for (int c27 = 0; c27 < 27 && (need_counts || cnt < nb_points); ++c27) {
+    const uint64_t key_now = key;
+    const uint32_t home_now = home;
+    const uint4 first_now = first;
+    if (c27 + 1 < 27) {
+      const int code = c_cell_order[c27 + 1];
+      key = grid_key(0, ix + code % 3 - 1, iy + (code / 3) % 3 - 1, iz + code / 9 - 1);
+      home = grid_home(g, key);
+      first = grid_load(g, home);
+    }
+    uint32_t b, f;
+    if (!grid_resolve(g, key_now, home_now, first_now, b, f)) continue;
+    cnt = radius_scan_run(g, b, f, q, r2, nb_points, need_counts, cnt);
+  }
+  return cnt;
+}
+
+// ---- radius query over cells of 2r: own cell, then only the neighbours the r-ball can reach ------
+// With a cell edge of 2r (+ slack) the ball around q reaches, along every axis, at most ONE of the two
+// neighbouring cells (the one behind the nearer face), so 1 + 7 cells cover it instead of 27, and a
+// neighbour (a face, edge or corner cell) is visited only if the ball reaches its box: sum over the
+// offset axes of gap^2 <= r^2, gap = distance from q to that face.  On a voxelised 128-beam scan the
+// own cell alone settles 95 % of the keep / drop decisions (cells of r: 75 %), and the others probe
+// 3 to 7 cells, not 26 (profiles/r2p_radius_ab.json).  The set of points tested against d2 <= r2 is a
+// superset of the ball either way, so counts and decisions are bit-identical to the 27-cell walk.
+// Slack: the cell index is floor(fl(x * fl(1/c))) (grid_coord_g), two roundings of 2^-24 each, so a point
+// of the cell below has x < ix*c*(1 + 2^-23) and one of the cell above x >= (ix+1)*c*(1 - 2^-23); the
+// products, differences and d2 below each carry a relative rounding error of 2^-24.  gap is therefore shortened by 1e-6 * (|q| + c) + 1e-5 * r (8x the worst
+// case); if that ever leaves BOTH faces of an axis within reach (coordinates of tens of kilometres) the
+// query falls back to the 27-cell walk.
+//
 // `self` = position of q itself in the cell-sorted array (q = g.sorted[self]).  The own cell is scanned
 // OUTWARDS from that position, two records on either side per round: arrival order inside a cell follows
 // the order of the input (LiDAR firing order), so the records next to q are its neighbours along the scan
@@ -367,7 +342,7 @@ __device__ __forceinline__ uint32_t radius_count_oct(const GridDev& g, float c, 
     gap2[a] = __fmul_rn(gmin, gmin);
     both |= fmaxf(gl, gh) <= reach;
   }
-  if (both) return radius_count(g, c, q, r2, nb_points, need_counts, 27);
+  if (both) return radius_count(g, c, q, r2, nb_points, need_counts);
   const float reach2 = __fmul_rn(reach, reach);
   // faces, edges, corner: the nearer a box, the likelier it holds the missing neighbours.  One cell at a
   // time: probing the cells of a round together (7 table round trips -> 2) was slower, alone and with all
@@ -401,248 +376,26 @@ k_radius_query_oct(uint32_t n_max, const uint32_t* n_dev, GridDev g, float r, fl
   APC_STAMP(0, 1);
 }
 
-// Decision-only variant (keep iff >= nb_points within r) - an A/B knob that lost, see radius_decide.  The per-thread walk above
-// costs what its SLOWEST lane costs: two thirds of its warp instructions were the own-cell loop running on for
-// the one or two lanes of a warp that do not find nb_points near themselves (profiles/r2v_ncu_full.csv,
-// hot_lines).  Here every lane scans outwards for at most `own_rounds` rounds (8 records); the lanes still
-// short of nb_points are then served by the WHOLE WARP, one after the other: the rest of the lane's own cell
-// 32 records at a time (ballot + popc), then lanes 1..7 resolve the <= 7 box-pruned neighbour cells in one
-// round trip and the warp walks their runs as one flat list.  A warp with more than `coop_max` such lanes
-// (a sparse region: everybody is short) lets them walk alone as before - there the per-thread walk keeps all
-// lanes busy.  Counts may overshoot nb_points (whole batches are counted); the decision is the same.
-__global__ void __launch_bounds__(128)
-k_radius_decide_oct(uint32_t n_max, const uint32_t* n_dev, GridDev g, float r, float r2, uint32_t nb_points,
-                    uint8_t* __restrict__ mask, const ApcCtrl* __restrict__ ctrl, uint32_t own_rounds, uint32_t coop_max) {
-  pdl_enter();
-  const uint32_t n = grid_sorted_count(g, ctrl, apc_count(n_dev, n_max));
-  const float c = grid_cell_size(g, 0);
-  const uint32_t lane = lane_id();
-  const float reach = r * 1.00001f, reach2 = __fmul_rn(reach, reach);
-  APC_STAMP(0, 0);
-  for (uint32_t base = blockIdx.x * blockDim.x; base < n; base += gridDim.x * blockDim.x) {
-    const uint32_t j = base + threadIdx.x;
-    const bool live = j < n;
-    float4 q = make_float4(0.f, 0.f, 0.f, 0.f);
-    int32_t ix = 0, iy = 0, iz = 0;
-    uint32_t cnt = 0, b = 0, e = 0, up = 0, down = 0;
-    bool pending = false;
-    if (live) {
-      q = g.sorted[j];
-      grid_coord_g(g, c, q.x, q.y, q.z, ix, iy, iz);  // succeeded at insert time
-      uint32_t f;
-      if (grid_lookup(g, grid_key(0, ix, iy, iz), b, f) && j >= b && j < b + f) {
-        e = b + f;
-        cnt = 1u;                                   // q itself
-        up = j + 1;
-        down = j;
-        for (uint32_t round = 0; round < own_rounds && cnt < nb_points && (up < e || down > b); ++round) {
-          float4 p[4];
-          bool ok[4];
-#pragma unroll
-          for (int u = 0; u < 2; ++u) {
-            ok[u] = up + u < e;
-            p[u] = g.sorted[ok[u] ? up + u : j];
-            ok[2 + u] = down >= b + 1 + u;
-            p[2 + u] = g.sorted[ok[2 + u] ? down - 1 - u : j];
-          }
-#pragma unroll
-          for (int u = 0; u < 4; ++u) cnt += (ok[u] && d2_f32(q.x, q.y, q.z, p[u].x, p[u].y, p[u].z) <= r2) ? 1u : 0u;
-          up = min(up + 2, e);
-          down = down >= b + 2 ? down - 2 : b;
-        }
-        pending = cnt < nb_points;
-      } else {
-        cnt = radius_count_oct(g, c, q, j, r, r2, nb_points, 0);   // (a record outside its own cell's run: not reachable)
-      }
-    }
-    uint32_t bal = __ballot_sync(0xffffffffu, pending);
-    if (bal && (uint32_t)__popc(bal) <= coop_max) {
-      while (bal) {
-        const uint32_t L = __ffs(bal) - 1u;
-        bal &= bal - 1u;
-        const float qx = __shfl_sync(0xffffffffu, q.x, L), qy = __shfl_sync(0xffffffffu, q.y, L), qz = __shfl_sync(0xffffffffu, q.z, L);
-        uint32_t cL = __shfl_sync(0xffffffffu, cnt, L);
-        const uint32_t bL = __shfl_sync(0xffffffffu, b, L), eL = __shfl_sync(0xffffffffu, e, L);
-        const uint32_t upL = __shfl_sync(0xffffffffu, up, L), downL = __shfl_sync(0xffffffffu, down, L);
-        const int32_t ixL = __shfl_sync(0xffffffffu, ix, L), iyL = __shfl_sync(0xffffffffu, iy, L), izL = __shfl_sync(0xffffffffu, iz, L);
-        // 1. what is left of the own cell: [bL, downL) and [upL, eL)
-        const uint32_t lo_n = downL - bL, tot = lo_n + (eL - upL);
-        for (uint32_t t0 = 0; t0 < tot && cL < nb_points; t0 += 32) {
-          const uint32_t t = t0 + lane;
-          bool hit = false;
-          if (t < tot) {
-            const float4 p = g.sorted[t < lo_n ? bL + t : upL + (t - lo_n)];
-            hit = d2_f32(qx, qy, qz, p.x, p.y, p.z) <= r2;
-          }
-          cL += __popc(__ballot_sync(0xffffffffu, hit));
-        }
-        if (cL < nb_points) {
-          // 2. the neighbour cells the ball reaches (same pruning as radius_count_oct)
-          const float qa[3] = {qx, qy, qz};
-          const int32_t ia[3] = {ixL, iyL, izL};
-          int32_t dir[3];
-          float gap2[3];
-          bool both = false;
-#pragma unroll
-          for (int a = 0; a < 3; ++a) {
-            const float lo = __fmul_rn((float)ia[a], c), hi = __fmul_rn((float)(ia[a] + 1), c);
-            const float slack = 1e-6f * (fabsf(qa[a]) + c) + 1e-5f * r;
-            const float gl = fmaxf(0.0f, __fsub_rn(__fsub_rn(qa[a], lo), slack)), gh = fmaxf(0.0f, __fsub_rn(__fsub_rn(hi, qa[a]), slack));
-            dir[a] = gl <= gh ? -1 : 1;
-            const float gmin = fminf(gl, gh);
-            gap2[a] = __fmul_rn(gmin, gmin);
-            both |= fmaxf(gl, gh) <= reach;
-          }
-          if (both) {                                 // slack not small against r: the lane walks all 27 cells itself
-            uint32_t full = 0;
-            if (lane == L) full = radius_count(g, c, q, r2, nb_points, 0, 27);
-            cL = __shfl_sync(0xffffffffu, full, L);
-          } else {
-            uint32_t ns = 0, nf = 0;
-            if (lane >= 1u && lane < 8u) {
-              const float s2 = ((lane & 1u) ? gap2[0] : 0.0f) + ((lane & 2u) ? gap2[1] : 0.0f) + ((lane & 4u) ? gap2[2] : 0.0f);
-              if (s2 <= reach2) {
-                const uint64_t key = grid_key(0, ixL + ((lane & 1u) ? dir[0] : 0), iyL + ((lane & 2u) ? dir[1] : 0),
-                                              izL + ((lane & 4u) ? dir[2] : 0));
-                uint32_t bb, ff;
-                if (grid_lookup(g, key, bb, ff)) { ns = bb; nf = ff; }
-              }
-            }
-            uint32_t incl = nf;
-#pragma unroll
-            for (int o = 1; o < 8; o <<= 1) {
-              const uint32_t v = __shfl_up_sync(0xffffffffu, incl, o);
-              if (lane >= (uint32_t)o) incl += v;
-            }
-            const uint32_t ps = incl - nf;                       // first flat index of lane's run
-            const uint32_t total = __shfl_sync(0xffffffffu, incl, 7);
-            for (uint32_t t0 = 0; t0 < total && cL < nb_points; t0 += 32) {
-              const uint32_t t = t0 + lane;
-              const uint32_t flat = min(t, total - 1u);
-              uint32_t run = 0;                                  // largest m in 1..7 with ps[m] <= flat
-#pragma unroll
-              for (int step = 4; step > 0; step >>= 1) {
-                const uint32_t mid = run + step;
-                const uint32_t v = __shfl_sync(0xffffffffu, ps, mid & 31u);
-                if (mid < 8u && v <= flat) run = mid;
-              }
-              const uint32_t rs = __shfl_sync(0xffffffffu, ns, run), rp = __shfl_sync(0xffffffffu, ps, run);
-              bool hit = false;
-              if (t < total) {
-                const float4 p = g.sorted[rs + (flat - rp)];
-                hit = d2_f32(qx, qy, qz, p.x, p.y, p.z) <= r2;
-              }
-              cL += __popc(__ballot_sync(0xffffffffu, hit));
-            }
-          }
-        }
-        if (lane == L) cnt = cL;
-      }
-    } else if (pending) {
-      cnt = radius_count_oct(g, c, q, j, r, r2, nb_points, 0);
-    }
-    if (live) mask[__float_as_uint(q.w)] = cnt >= nb_points ? 1 : 0;
-  }
-  APC_STAMP(0, 1);
-}
+// Cell edge of the radius grid: 2r, + 2^-10 slack so that d2 <= r2 never reaches past the neighbouring cell.
+// Against cells of r and the 27-cell walk, cells of 2r and the pruned walk above give +6 % saturated
+// throughput (profiles/r2p_radius_ab.json).
+static float radius_cell(float r32) { return r32 * 2.0f * 1.0009765625f; }
 
-// Cell edge of the radius grid in units of r (+ 2^-10 slack so that d2 <= r2 never reaches past the
-// neighbouring cell): >= 2 = the pruned 8-cell walk above (default 2), 1 = the 27-cell walk (APC_RADIUS_CELL).
-static float radius_cell_mult() {
-  static const float m = []() {
-    const char* e = getenv("APC_RADIUS_CELL");
-    const float v = e ? (float)atof(e) : 2.0f;
-    return v >= 2.0f ? v : 1.0f;
-  }();
-  return m;
-}
-static float radius_cell(float r32) { return r32 * radius_cell_mult() * 1.0009765625f; }
-
-// The keep / drop decision in two launches (the exact counts are not wanted):
-//   fast  every point against its OWN cell only - one probe, one or two rounds of loads, every thread
-//         done within the same few microseconds; the few that did not reach nb_points there are
-//         appended (warp-aggregated) to a pending list;
-//   slow  the pending points against the whole 27-cell block.
-// Idea: one launch doing both keeps ALL threads' registers resident until the slowest walker of each CTA
-// is through its 27 dependent probes.  Measured (APC_RADIUS_SPLIT=1, profiles/r2g_knobs.json): the own-cell
-// pass takes 10.6 us, but the pending pass still takes 23 us (its walkers are the whole cost) and saturated
-// throughput does not move (70.5 vs 70.8 us/scan), for one more launch of latency: OFF by default.
-#define CTR_RADIUS_PENDING 23
-__global__ void __launch_bounds__(128)
-k_radius_fast(uint32_t n_max, const uint32_t* n_dev, GridDev g, float r2, uint32_t nb_points, uint8_t* __restrict__ mask,
-              uint32_t* __restrict__ pending, ApcCtrl* ctrl) {
-  const uint32_t n = grid_sorted_count(g, ctrl, apc_count(n_dev, n_max));
-  const float c = grid_cell_size(g, 0);
-  const uint32_t lane = lane_id();
-  for (uint32_t base = blockIdx.x * blockDim.x; base < n; base += gridDim.x * blockDim.x) {
-    const uint32_t j = base + threadIdx.x;
-    bool open = false;
-    if (j < n) {
-      const float4 q = g.sorted[j];
-      const uint32_t cnt = radius_count(g, c, q, r2, nb_points, 0, 1);
-      open = cnt < nb_points;
-      if (!open) mask[__float_as_uint(q.w)] = 1;
-    }
-    const uint32_t bal = __ballot_sync(0xffffffffu, open);
-    if (bal) {
-      uint32_t at = 0;
-      if (lane == 0) at = atomicAdd(&ctrl->counters[CTR_RADIUS_PENDING], (uint32_t)__popc(bal));
-      at = __shfl_sync(0xffffffffu, at, 0);
-      if (open) pending[at + __popc(bal & ((1u << lane) - 1u))] = j;
-    }
-  }
-}
-__global__ void __launch_bounds__(128)
-k_radius_slow(GridDev g, float r2, uint32_t nb_points, uint8_t* __restrict__ mask, const uint32_t* __restrict__ pending,
-              const ApcCtrl* __restrict__ ctrl) {
-  const uint32_t n = ctrl->counters[CTR_RADIUS_PENDING];
-  const float c = grid_cell_size(g, 0);
-  for (uint32_t k = blockIdx.x * blockDim.x + threadIdx.x; k < n; k += gridDim.x * blockDim.x) {
-    const float4 q = g.sorted[pending[k]];
-    const uint32_t cnt = radius_count(g, c, q, r2, nb_points, 0, 27);
-    mask[__float_as_uint(q.w)] = cnt >= nb_points ? 1 : 0;
-  }
-}
-
-// decision-only radius query: the single launch (default) or the split (APC_RADIUS_SPLIT=1)
-static int radius_decide(apc_ctx* ctx, const GridDev& g, uint32_t n_max, const uint32_t* n_dev, float r, float r2,
-                         uint32_t nb_points, uint8_t* mask, cudaStream_t s) {
-  static const bool split = []() { const char* e = getenv("APC_RADIUS_SPLIT"); return e && atoi(e) != 0; }();
+// The radius query over the built grid: keep / drop decisions into `mask`, and the exact counts into `counts`
+// when it is not NULL.  For the decision alone one launch of the per-thread walk measured best:
+//  - an own-cell pass that lists the points still short of nb_points, then a pass over that list: the first
+//    takes 10.6 us, the second still 23 us, saturated throughput does not move (70.5 vs 70.8 us/scan) and the
+//    split costs one more launch of latency (profiles/r2g_knobs.json);
+//  - the whole warp serving, one after the other, the lanes its own-cell rounds left short: 24.3 vs 21.9 us
+//    alone, 67.7 vs 64.8 us/scan with all lanes busy (profiles/r2p_radius_ab.json);
+//  - blocks of 64 or 256 threads instead of 128: no difference (profiles/r2ab_fold_lanes.json).
+static int radius_query(apc_ctx* ctx, const GridDev& g, uint32_t n_max, const uint32_t* n_dev, float r,
+                        uint32_t nb_points, uint8_t* mask, uint32_t* counts, cudaStream_t s) {
   const uint32_t bq = min(apc_div_up(n_max, 128), (uint32_t)APC_SM_COUNT * 16);
-  if (radius_cell_mult() >= 2.0f) {
-    // APC_RADIUS_COOP = "own_rounds,coop_max": warp-cooperative service of the lanes left short (k_radius_decide_oct).
-    // Default coop_max = 0 = the per-thread walk k_radius_query_oct: the cooperative variant LOST the A/B (24.3 vs
-    // 21.9 us alone, 67.7 vs 64.8 us/scan with all lanes busy at 2,8; 33.4 us at 2,32; profiles/r2p_radius_ab.json)
-    static const uint32_t own_rounds = []() { const char* e = getenv("APC_RADIUS_COOP"); return e ? (uint32_t)atoi(e) : 2u; }();
-    static const uint32_t coop_max = []() {
-      const char* e = getenv("APC_RADIUS_COOP");
-      const char* comma = e ? strchr(e, ',') : nullptr;
-      return comma ? (uint32_t)atoi(comma + 1) : 0u;
-    }();
-    APC_PROF(ctx, "k_radius_query", s);
-    if (coop_max)
-      apc_klaunch(ctx, k_radius_decide_oct, bq, 128, 0, s, n_max, n_dev, g, r, r2, nb_points, mask, ctx->ctrl, own_rounds, coop_max);
-    else {
-      static const uint32_t blk = []() { const char* e = getenv("APC_RADIUS_BLOCK"); const int v = e ? atoi(e) : 128; return (uint32_t)((v == 64 || v == 256) ? v : 128); }();
-      const uint32_t bqb = min(apc_div_up(n_max, blk), (uint32_t)APC_SM_COUNT * (2048u / blk));
-      apc_klaunch(ctx, k_radius_query_oct, bqb, blk, 0, s, n_max, n_dev, g, r, r2, nb_points, 0, mask, nullptr, ctx->ctrl);
-    }
-    APC_LAUNCH_CHECK(ctx, "k_radius_query_oct");
-    return APC_OK;
-  }
-  if (!split) {
-    APC_PROF(ctx, "k_radius_query", s);
-    apc_klaunch(ctx, k_radius_query, bq, 128, 0, s, n_max, n_dev, g, r2, nb_points, 0, mask, nullptr, ctx->ctrl);
-    APC_LAUNCH_CHECK(ctx, "k_radius_query");
-    return APC_OK;
-  }
-  {
-    APC_PROF(ctx, "k_radius_fast", s);
-    k_radius_fast<<<bq, 128, 0, s>>>(n_max, n_dev, g, r2, nb_points, mask, ctx->nb_count, ctx->ctrl);
-  }
-  APC_PROF(ctx, "k_radius_slow", s);
-  k_radius_slow<<<min(bq, (uint32_t)APC_SM_COUNT * 4), 128, 0, s>>>(g, r2, nb_points, mask, ctx->nb_count, ctx->ctrl);
-  APC_LAUNCH_CHECK(ctx, "k_radius_fast/slow");
+  APC_PROF(ctx, "k_radius_query", s);
+  apc_klaunch(ctx, k_radius_query_oct, bq, 128, 0, s, n_max, n_dev, g, r, r * r, nb_points, counts ? 1 : 0, mask, counts,
+              ctx->ctrl);
+  APC_LAUNCH_CHECK(ctx, "k_radius_query_oct");
   return APC_OK;
 }
 
@@ -684,9 +437,12 @@ struct TopK {
 //      sequential float32 sum as oracle/outliers.py.
 #define KNN_CAP 1024
 #define KNN_WARPS 4
+// newcomers in a batch of 32 above which the batch is sorted and merged instead of inserted one by one
+// (2 / 4 / 6 / 10: within 2 %, 32: twice the time; profiles/r2x_knn_ab.json)
+#define KNN_MERGE_MIN 6u
 __global__ void __launch_bounds__(KNN_WARPS * 32)
 k_knn_query(uint32_t n_max, const uint32_t* n_dev, GridDev g, uint32_t k, float* __restrict__ avg,
-            uint32_t* __restrict__ stragglers, ApcCtrl* ctrl, uint32_t start_fill, int exact_margin, uint32_t merge_min) {
+            uint32_t* __restrict__ stragglers, ApcCtrl* ctrl) {
   __shared__ uint32_t s_buf[KNN_WARPS][KNN_CAP];
   const uint32_t n = apc_count(n_dev, n_max);
   const uint32_t n_sorted = grid_sorted_count(g, ctrl, n);
@@ -699,20 +455,10 @@ k_knn_query(uint32_t n_max, const uint32_t* n_dev, GridDev g, uint32_t k, float*
     const float4 q = g.sorted[j];
     const uint32_t orig = __float_as_uint(q.w);
     bool done = false;
-    // Optional starting level (start_fill > 0, an A/B knob that lost): the finest level whose OWN cell already
-    // holds start_fill points (lane l reads the population of the query's cell at level l through the slot
-    // recorded at insert time: two dependent loads for all levels at once).
-    uint32_t level0 = 0;
-    if (start_fill) {
-      uint32_t fill = 0;
-      if (lane < g.levels) {
-        const uint32_t sl = g.slot[(size_t)lane * n_max + orig];
-        if (sl != GRID_NOSLOT) fill = g.slots[sl].fill;
-      }
-      const uint32_t okm = __ballot_sync(0xffffffffu, fill >= start_fill);
-      level0 = okm ? (uint32_t)__ffs(okm) - 1u : g.levels - 1u;
-    }
-    for (uint32_t level = level0; level < g.levels && !done; ++level) {
+    // Always from level 0: starting at the finest level whose own cell already holds 5 / 10 / 16 points
+    // examines more candidates than the failed levels cost (2.49 / 2.94 / 3.34 ms against 1.86 ms on the C4
+    // scan, profiles/r2x_knn_ab.json).
+    for (uint32_t level = 0; level < g.levels && !done; ++level) {
       const float c = g.cell[level];
       int32_t ix, iy, iz;
       if (!grid_coord_g(g, c, q.x, q.y, q.z, ix, iy, iz)) continue;
@@ -733,16 +479,13 @@ k_knn_query(uint32_t n_max, const uint32_t* n_dev, GridDev g, uint32_t k, float*
       const uint32_t total = __shfl_sync(0xffffffffu, incl, 31);
       if (total < k_eff) continue;
       const float4* sp = g.sorted + (size_t)level * n_max;
-      // every point closer than `safe` lies inside the 27-cell block: the cell edge plus (exact_margin) the
-      // query's distance to the nearest face of its own cell, less 0.1 % for the rounding of the cell index
-      float safe = c;
-      if (exact_margin) {
-        const float mx = fminf(__fsub_rn(q.x, __fmul_rn((float)ix, c)), __fsub_rn(__fmul_rn((float)(ix + 1), c), q.x));
-        const float my = fminf(__fsub_rn(q.y, __fmul_rn((float)iy, c)), __fsub_rn(__fmul_rn((float)(iy + 1), c), q.y));
-        const float mz = fminf(__fsub_rn(q.z, __fmul_rn((float)iz, c)), __fsub_rn(__fmul_rn((float)(iz + 1), c), q.z));
-        safe = __fadd_rn(c, fmaxf(0.0f, fminf(mx, fminf(my, mz))));
-      }
-      safe = __fmul_rn(safe, 0.999f);
+      // every point closer than `safe` lies inside the 27-cell block: the cell edge plus the query's distance
+      // to the nearest face of its own cell (1859 against 1961 us for the cell edge alone on the C4 scan,
+      // profiles/r2x_knn_ab.json), less 0.1 % for the rounding of the cell index
+      const float fx = fminf(__fsub_rn(q.x, __fmul_rn((float)ix, c)), __fsub_rn(__fmul_rn((float)(ix + 1), c), q.x));
+      const float fy = fminf(__fsub_rn(q.y, __fmul_rn((float)iy, c)), __fsub_rn(__fmul_rn((float)(iy + 1), c), q.y));
+      const float fz = fminf(__fsub_rn(q.z, __fmul_rn((float)iz, c)), __fsub_rn(__fmul_rn((float)(iz + 1), c), q.z));
+      const float safe = __fmul_rn(__fadd_rn(c, fmaxf(0.0f, fminf(fx, fminf(fy, fz)))), 0.999f);
       if (k_eff <= 32u) {
         // 2'. k <= 32 (the reference's default is 20): the k best live in REGISTERS, lane i holding the
         // i-th smallest distance so far.  A batch of 32 candidates is screened with one ballot against
@@ -767,7 +510,7 @@ k_knn_query(uint32_t n_max, const uint32_t* n_dev, GridDev g, uint32_t k, float*
             d2 = d2_f32(q.x, q.y, q.z, p.x, p.y, p.z);
           }
           uint32_t cand = __ballot_sync(0xffffffffu, d2 < kth);
-          if ((uint32_t)__popc(cand) > merge_min) {
+          if ((uint32_t)__popc(cand) > KNN_MERGE_MIN) {
             // many of the batch beat the current k-th value (always the first batch of a pass, often the second):
             // sort the batch across the lanes (bitonic network, 15 shuffle stages) and merge it with the sorted
             // `val` - reversed batch, element-wise minimum = the 32 smallest of the union as a bitonic sequence,
@@ -1070,12 +813,12 @@ template <> __device__ __forceinline__ unsigned long long knn_key<unsigned long 
 
 // The KNN grid's level climb for query q (warp-collective), shared by k_knn_query_wide and k_normals_knn:
 // per level, lanes 0..26 resolve the 27 cells, the flat candidate list streams through a WarpKeep of `cap`
-// keys at buf, and the level stands if the k_eff-th distance is covered by the block (`safe`, exact_margin).
+// keys at buf, and the level stands if the k_eff-th distance is covered by the block (`safe`).
 // Returns true with the k_eff smallest keys in buf[0, k_eff) (unordered); false when no level covers q
 // (a straggler).
 template <typename K>
 __device__ __forceinline__ bool knn_levels(const GridDev& g, uint32_t n_max, float4 q, uint32_t k_eff, K* buf, uint32_t cap,
-                                           int exact_margin, uint32_t lane) {
+                                           uint32_t lane) {
   for (uint32_t level = 0; level < g.levels; ++level) {
     const float c = g.cell[level];
     int32_t ix, iy, iz;
@@ -1096,14 +839,10 @@ __device__ __forceinline__ bool knn_levels(const GridDev& g, uint32_t n_max, flo
     const uint32_t total = __shfl_sync(0xffffffffu, incl, 31);
     if (total < k_eff) continue;
     const float4* sp = g.sorted + (size_t)level * n_max;
-    float safe = c;
-    if (exact_margin) {
-      const float mx = fminf(__fsub_rn(q.x, __fmul_rn((float)ix, c)), __fsub_rn(__fmul_rn((float)(ix + 1), c), q.x));
-      const float my = fminf(__fsub_rn(q.y, __fmul_rn((float)iy, c)), __fsub_rn(__fmul_rn((float)(iy + 1), c), q.y));
-      const float mz = fminf(__fsub_rn(q.z, __fmul_rn((float)iz, c)), __fsub_rn(__fmul_rn((float)(iz + 1), c), q.z));
-      safe = __fadd_rn(c, fmaxf(0.0f, fminf(mx, fminf(my, mz))));
-    }
-    safe = __fmul_rn(safe, 0.999f);
+    const float fx = fminf(__fsub_rn(q.x, __fmul_rn((float)ix, c)), __fsub_rn(__fmul_rn((float)(ix + 1), c), q.x));
+    const float fy = fminf(__fsub_rn(q.y, __fmul_rn((float)iy, c)), __fsub_rn(__fmul_rn((float)(iy + 1), c), q.y));
+    const float fz = fminf(__fsub_rn(q.z, __fmul_rn((float)iz, c)), __fsub_rn(__fmul_rn((float)(iz + 1), c), q.z));
+    const float safe = __fmul_rn(__fadd_rn(c, fmaxf(0.0f, fminf(fx, fminf(fy, fz)))), 0.999f);
     WarpKeep<K> wk;
     wk.init(buf, cap, k_eff);
     for (uint32_t base = 0; base < total; base += 32) {
@@ -1153,11 +892,11 @@ __device__ __forceinline__ void knn_brute(const float4* __restrict__ pts, uint32
 }
 
 // k_knn_query for 64 < k <= APC_MAX_NEIGHBORS: the same level climb, 27-cell flat candidate list and
-// coverage test (`safe`, exact_margin), the candidates through a WarpKeep of wide_cap(k) entries per
+// coverage test (`safe`), the candidates through a WarpKeep of wide_cap(k) entries per
 // warp (dynamic shared memory), the accepted level's k distances sorted and summed by wide_average.
 __global__ void __launch_bounds__(KNN_WARPS * 32)
 k_knn_query_wide(uint32_t n_max, const uint32_t* n_dev, GridDev g, uint32_t k, uint32_t cap, float* __restrict__ avg,
-                 uint32_t* __restrict__ stragglers, ApcCtrl* ctrl, int exact_margin) {
+                 uint32_t* __restrict__ stragglers, ApcCtrl* ctrl) {
   const uint32_t n = apc_count(n_dev, n_max);
   const uint32_t n_sorted = grid_sorted_count(g, ctrl, n);
   const uint32_t k_eff = min(k, n);
@@ -1166,7 +905,7 @@ k_knn_query_wide(uint32_t n_max, const uint32_t* n_dev, GridDev g, uint32_t k, u
   for (uint32_t j = blockIdx.x * KNN_WARPS + w; j < n_sorted; j += gridDim.x * KNN_WARPS) {
     const float4 q = g.sorted[j];
     const uint32_t orig = __float_as_uint(q.w);
-    if (knn_levels(g, n_max, q, k_eff, buf, cap, exact_margin, lane)) {
+    if (knn_levels(g, n_max, q, k_eff, buf, cap, lane)) {
       const float a = wide_average(buf, k_eff, lane);
       if (lane == 0) avg[orig] = a;
     } else if (lane == 0) {
@@ -1395,8 +1134,7 @@ static int grid_build(apc_ctx* ctx, GridHost& g, const float4* pts, uint32_t n_m
   }
   g.d.cell0 = (g.d.levels == 1 && cell_hint > 0.0f) ? cell_hint : 0.0f;
   g.d.inv0 = (reciprocal && g.d.cell0 > 0.0f) ? 1.0f / g.d.cell0 : 0.0f;
-  static const bool cell_list = getenv("APC_NO_CELL_LIST") == nullptr;   // A/B knob
-  g.d.cells = (inserted && cell_list) ? g.cells_buf : nullptr;
+  g.d.cells = inserted ? g.cells_buf : nullptr;
   if (!(g.d.cell0 > 0.0f)) k_grid_cells<<<1, 1, 0, s>>>(ctx->ctrl, cell_hint, g.d.levels, g.d.cell);
   const dim3 grid(bx, g.d.levels);
   if (!inserted) {   // (the pipeline's voxel stage inserts its centroids as it writes them)
@@ -1426,25 +1164,11 @@ int apc_radius_nobegin(apc_ctx* ctx, const float* xyzi, uint32_t n_max, const ui
   if (rc) return rc;
   GridHost& g = scratch_of(ctx)->grid[0];
   const float r32 = (float)radius;
-  const float r2 = r32 * r32;                       // float32(r)^2, rounded once
-  // cells of r (+ slack, so that d2 <= r2 never reaches 2 cells away); measured alternatives at
-  // 200k points: cells of 2r 37 us, one warp per cell group with shuffled broadcasts 85 us,
-  // neighbour-cell lookups issued in rounds of 6-13 32-50 us, this per-thread walk 29-32 us
-  const float cell = radius_cell(r32);
   const float4* pts = reinterpret_cast<const float4*>(xyzi);
-  rc = grid_build(ctx, g, pts, n_max, n_dev, cell, false, s, false, 0, radius_cell_mult() >= 2.0f);
+  rc = grid_build(ctx, g, pts, n_max, n_dev, radius_cell(r32), false, s, false, 0, true);
   if (rc) return rc;
-  if (out_counts) {
-    const uint32_t bq = min(apc_div_up(n_max, 128), (uint32_t)APC_SM_COUNT * 16);
-    APC_PROF(ctx, "k_radius_query", s);
-    if (radius_cell_mult() >= 2.0f)
-      apc_klaunch(ctx, k_radius_query_oct, bq, 128, 0, s, n_max, n_dev, g.d, r32, r2, (uint32_t)nb_points, 1, out_mask, out_counts, ctx->ctrl);
-    else
-      apc_klaunch(ctx, k_radius_query, bq, 128, 0, s, n_max, n_dev, g.d, r2, (uint32_t)nb_points, 1, out_mask, out_counts, ctx->ctrl);
-  } else {
-    rc = radius_decide(ctx, g.d, n_max, n_dev, r32, r2, (uint32_t)nb_points, out_mask, s);
-    if (rc) return rc;
-  }
+  rc = radius_query(ctx, g.d, n_max, n_dev, r32, (uint32_t)nb_points, out_mask, out_counts, s);
+  if (rc) return rc;
   const dim3 grid(min(apc_div_up(n_max, 256), (uint32_t)APC_SM_COUNT * 4), 1);
   APC_PROF(ctx, "k_grid_clean", s);
   k_grid_clean<<<grid, 256, 0, s>>>(n_max, n_dev, g.d);
@@ -1504,8 +1228,8 @@ int apc_radius_grid_view(apc_ctx* ctx, double radius, GridDev* out) {
   if (rc) return rc;
   GridHost& g = scratch_of(ctx)->grid[0];
   g.d.cell0 = radius_cell((float)radius);
-  g.d.inv0 = radius_cell_mult() >= 2.0f ? 1.0f / g.d.cell0 : 0.0f;
-  g.d.cells = getenv("APC_NO_CELL_LIST") ? nullptr : g.cells_buf;   // the caller inserts: it also lists the occupied cells
+  g.d.inv0 = 1.0f / g.d.cell0;
+  g.d.cells = g.cells_buf;   // the caller inserts: it also lists the occupied cells
   *out = g.d;
   return APC_OK;
 }
@@ -1527,9 +1251,9 @@ int apc_radius_select_nobegin(apc_ctx* ctx, const float* xyzi, uint32_t n_max, c
   GridHost& g = scratch_of(ctx)->grid[0];
   const float r32 = (float)radius;
   const float4* pts = reinterpret_cast<const float4*>(xyzi);
-  rc = grid_build(ctx, g, pts, n_max, n_dev, radius_cell(r32), false, s, points_inserted != 0, 0, radius_cell_mult() >= 2.0f);
+  rc = grid_build(ctx, g, pts, n_max, n_dev, radius_cell(r32), false, s, points_inserted != 0, 0, true);
   if (rc) return rc;
-  rc = radius_decide(ctx, g.d, n_max, n_dev, r32, r32 * r32, (uint32_t)nb_points, mask_scratch, s);
+  rc = radius_query(ctx, g.d, n_max, n_dev, r32, (uint32_t)nb_points, mask_scratch, nullptr, s);
   if (rc) return rc;
   const uint32_t n_tiles = apc_div_up(n_max, APC_TILE_POINTS);
   APC_REQUIRE(ctx, n_tiles <= ctx->max_tiles, "more points than the context was created for");
@@ -1573,14 +1297,13 @@ int apc_statistical_nobegin(apc_ctx* ctx, const float* xyzi, uint32_t n_max, con
   rc = grid_build(ctx, g, pts, n_max, n_dev, cell_hint, !(cell_hint > 0.0f), s);
   if (rc) return rc;
   const uint32_t bq = min(apc_div_up(n_max, KNN_WARPS), (uint32_t)APC_SM_COUNT * 16);   // one warp per query, grid-stride
-  static const int margin_env = []() { const char* e = getenv("APC_KNN_MARGIN"); return e ? atoi(e) : 1; }();
   if (nb_neighbors > KNN_KMAX) {
     const uint32_t cap = wide_cap((uint32_t)nb_neighbors);
     const size_t smem = (size_t)KNN_WARPS * cap * sizeof(uint32_t);
     {
       APC_PROF(ctx, "k_knn_query_wide", s);
       k_knn_query_wide<<<bq, KNN_WARPS * 32, smem, s>>>(n_max, n_dev, g.d, (uint32_t)nb_neighbors, cap, avg, sc->stragglers,
-                                                        ctx->ctrl, margin_env);
+                                                        ctx->ctrl);
     }
     {
       APC_PROF(ctx, "k_knn_stragglers_wide", s);
@@ -1590,16 +1313,7 @@ int apc_statistical_nobegin(apc_ctx* ctx, const float* xyzi, uint32_t n_max, con
   } else {
     {
       APC_PROF(ctx, "k_knn_query", s);
-      // APC_KNN_START_FILL: own-cell population that selects the starting level (default 0 = always level 0: skipping
-      // fine levels by this estimate examines more candidates than the failed passes cost - 2.49 / 2.94 / 3.34 ms
-      // against 1.86 ms for a population of 5 / 10 / 16 on the C4 scan);
-      // APC_KNN_MARGIN=0: guaranteed radius = the cell edge only (profiles/r2x_knn_ab.json)
-      static const int fill_env = []() { const char* e = getenv("APC_KNN_START_FILL"); return e ? atoi(e) : -1; }();
-      const uint32_t start_fill = fill_env > 0 ? (uint32_t)fill_env : 0u;
-      // newcomers in a batch of 32 above which the batch is sorted and merged instead of inserted one by one
-      static const uint32_t merge_min = []() { const char* e = getenv("APC_KNN_MERGE_MIN"); return e ? (uint32_t)atoi(e) : 6u; }();
-      k_knn_query<<<bq, KNN_WARPS * 32, 0, s>>>(n_max, n_dev, g.d, (uint32_t)nb_neighbors, avg, sc->stragglers, ctx->ctrl,
-                                                start_fill, margin_env, merge_min);
+      k_knn_query<<<bq, KNN_WARPS * 32, 0, s>>>(n_max, n_dev, g.d, (uint32_t)nb_neighbors, avg, sc->stragglers, ctx->ctrl);
     }
     {
       APC_PROF(ctx, "k_knn_stragglers", s);
@@ -2071,7 +1785,7 @@ k_normals_knn(uint32_t n_max, const uint32_t* n_dev, GridDev g, const float4* __
   for (uint32_t j = blockIdx.x * KNN_WARPS + w; j < n_sorted; j += gridDim.x * KNN_WARPS) {
     const float4 q = g.sorted[j];
     const uint32_t orig = __float_as_uint(q.w);
-    if (knn_levels(g, n_max, q, k_eff, buf, cap, 1, lane)) normals_cov_of_keys(buf, k_eff, pts, q, orig, lane, counts, cov9);
+    if (knn_levels(g, n_max, q, k_eff, buf, cap, lane)) normals_cov_of_keys(buf, k_eff, pts, q, orig, lane, counts, cov9);
     else if (lane == 0) stragglers[atomicAdd(&ctrl->counters[CTR_STRAGGLERS], 1u)] = orig;
     __syncwarp();
   }
@@ -3353,7 +3067,7 @@ k_fpfh_knn(uint32_t n_max, const uint32_t* n_dev, GridDev g, const float4* __res
   for (uint32_t j = blockIdx.x * KNN_WARPS + w; j < n_sorted; j += gridDim.x * KNN_WARPS) {
     const float4 q = g.sorted[j];
     const uint32_t orig = __float_as_uint(q.w);
-    if (knn_levels(g, n_max, q, k_eff, buf, cap, 1, lane)) {
+    if (knn_levels(g, n_max, q, k_eff, buf, cap, lane)) {
       warp_sort(buf, k_eff, lane);
       fpfh_of_keys<PASS>(buf, k_eff, pts, normals, q, orig, lane, s_cnt[w], spfh, feat, counts);
     } else if (PASS == 0 && lane == 0) {

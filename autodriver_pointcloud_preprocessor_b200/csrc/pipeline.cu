@@ -3,8 +3,6 @@
 // counters so that no stage waits for the host, plus CUDA-graph capture / replay of the
 // whole chain (one launch per scan).
 #include <cmath>
-#include <cstdio>
-#include <cstdlib>
 
 #include "apc_grid.cuh"
 APC_TRACE_EXPORT(pipeline)
@@ -23,7 +21,7 @@ int apc_statistical_nobegin(apc_ctx*, const float*, uint32_t, const uint32_t*, i
                             double*, cudaStream_t);
 int apc_segment_plane_nobegin(apc_ctx*, const float*, uint32_t, const uint32_t*, double, int, int, double, uint64_t,
                               const int32_t*, double*, uint8_t*, uint32_t*, float*, uint32_t*, int, cudaStream_t,
-                              const uint32_t*, uint32_t*, const MirrorDev*, const float*, float*, const CountsEpilogue*);
+                              const uint32_t*, uint32_t*, const MirrorDev*, const float*, float*);
 int apc_normals_nobegin(apc_ctx*, const float*, uint32_t, const uint32_t*, int, double, float*, uint32_t*, double*, cudaStream_t);
 int apc_neighbors_prepare(apc_ctx*, int);
 int apc_normals_prepare(apc_ctx*, int);
@@ -36,12 +34,6 @@ __global__ void k_pipeline_counts(const __grid_constant__ CountsEpilogue fin, co
   pdl_enter();
   pipeline_counts_write(fin, ctrl);
   APC_STAMP(0, 0);
-}
-
-// A/B probe (APC_DUMMY_KERNELS=k): k empty launches per scan, to separate "saturated throughput is set
-// by the number of launches" from "... by the work inside them" (profiles/, DESIGN.md section 4).
-__global__ void k_nop(const ApcCtrl* ctrl) {
-  if (threadIdx.x == 99 && ctrl->epoch == 0xffffffffu) printf("never");
 }
 
 __global__ void k_iota(uint32_t* out, uint32_t n_max, const uint32_t* n_dev) {
@@ -78,17 +70,13 @@ static int run_pipeline(apc_ctx* ctx, const apc_cloud_desc* clouds, uint32_t n_c
   const int n_stages = 1 + has_vox + has_stat + has_rad + has_ground;
   const bool has_normals = cfg->normals_enable != 0;
   APC_REQUIRE(ctx, !has_normals || (maps && maps->normals_dev), "normals_enable needs maps.normals_dev");
-  // first kernel = k_dedup_insert (it uses neither the epoch nor the counters): it does k_begin's work
-  // APC_FOLD=1: fold k_begin into k_dedup_insert and the counters into k_rs_final (11 launches per C2 scan instead
-  // of 13).  OFF by default: interleaved A/B, 8 lanes, two runs each - 64.84 / 64.69 us per scan folded against
-  // 63.37 / 63.77 with the two one-CTA launches, and the same single-scan latency (0.133 ms): inside a captured
-  // graph the tiny launches cost less than what they take off the two big kernels' critical paths
-  // (profiles/r2ab_fold_lanes.json).
-  static const bool fold_env = []() { const char* e = getenv("APC_FOLD"); return e && atoi(e) != 0; }();
-  const bool fold_begin = fold_env && cfg->filter.dedup_mode == APC_DEDUP_OPEN3D && n_total > 0;
-  int rc = fold_begin ? apc_begin_folded(ctx) : apc_begin(ctx, s);
+  // k_begin and k_pipeline_counts stay launches of their own.  Folding them into k_dedup_insert and k_rs_final
+  // (11 launches per C2 scan instead of 13) was slower: interleaved A/B, 8 lanes, two runs each - 64.84 / 64.69
+  // us per scan folded against 63.37 / 63.77 with the two one-CTA launches, and the same single-scan latency
+  // (0.133 ms): inside a captured graph the tiny launches cost less than what they take off the two big
+  // kernels' critical paths (profiles/r2ab_fold_lanes.json).
+  int rc = apc_begin(ctx, s);
   if (rc) return rc;
-  ctx->fold_begin = fold_begin;
   uint32_t* dc = ctx->dev_counts;
   float* ping = reinterpret_cast<float*>(ctx->buf_a);
   float* pong = reinterpret_cast<float*>(ctx->buf_b);
@@ -109,9 +97,7 @@ static int run_pipeline(apc_ctx* ctx, const apc_cloud_desc* clouds, uint32_t n_c
   fin.dc = dc;
   fin.out = out_counts_dev;
   fin.n_input = n_total;
-  fin.last = DC_OUT;                     // when the ground stage writes the counters it is the last stage
   fin.has_vox = has_vox; fin.has_stat = has_stat; fin.has_rad = has_rad; fin.has_ground = has_ground;
-  bool counts_done = false;
   uint32_t* const want_row = maps ? maps->out_row_dev : nullptr;
   int sel_left = want_row ? has_stat + has_rad + has_ground : 0;
   const uint32_t* row_in = nullptr;
@@ -125,14 +111,10 @@ static int run_pipeline(apc_ctx* ctx, const apc_cloud_desc* clouds, uint32_t n_c
   uint32_t cur_cnt = DC_FILTERED;
   rc = apc_frontend_nobegin(ctx, clouds, n_clouds, &cfg->filter, cur, maps ? maps->src_idx_dev : nullptr, nullptr,
                             dc + DC_FILTERED, 0, s);
-  ctx->fold_begin = false;
   if (rc) return rc;
-  static const int n_dummy = []() { const char* e = getenv("APC_DUMMY_KERNELS"); return e ? atoi(e) : 0; }();
-  for (int k = 0; k < n_dummy; ++k) k_nop<<<1, 32, 0, s>>>(ctx->ctrl);
   // voxel -> radius with nothing in between: the voxel stage inserts its centroids into the radius
   // grid as it writes them (one launch and one pass over the centroids less)
-  static const bool fuse_grid = getenv("APC_NO_GRID_FUSION") == nullptr;   // A/B knob for profiles/
-  const bool grid_in_voxel = fuse_grid && has_vox && has_rad && !has_stat && n_total > 0;
+  const bool grid_in_voxel = has_vox && has_rad && !has_stat && n_total > 0;
   if (has_vox) {
     float* out = dst();
     GridDev grid{};
@@ -150,9 +132,9 @@ static int run_pipeline(apc_ctx* ctx, const apc_cloud_desc* clouds, uint32_t n_c
     float* out = dst();
     // level-0 cell such that the k nearest of a point on a voxelised surface (one point per
     // voxel_size^2: r_k = voxel_size * sqrt(k / pi)) usually lie inside the first 27-cell block; the
-    // result does not depend on it (the query climbs levels until the k-th distance is covered)
-    static const float hint_scale = []() { const char* e = getenv("APC_KNN_HINT"); return e ? (float)atof(e) : 1.25f; }();   // A/B knob (profiles/r2x_knn_ab.json)
-    const float hint = has_vox ? hint_scale * cfg->voxel_size * fmaxf(2.0f, 1.3f * sqrtf((float)cfg->stat_nb_neighbors / 3.14159265f)) : 0.0f;
+    // result does not depend on it (the query climbs levels until the k-th distance is covered).  The factor
+    // 1.25 was kept against 1.5 and 2.0 (profiles/r2x_knn_ab.json).
+    const float hint = has_vox ? 1.25f * cfg->voxel_size * fmaxf(2.0f, 1.3f * sqrtf((float)cfg->stat_nb_neighbors / 3.14159265f)) : 0.0f;
     rc = apc_statistical_nobegin(ctx, cur, n_total, dc + cur_cnt, cfg->stat_nb_neighbors, cfg->stat_std_ratio, hint,
                                  ctx->mask_a, nullptr, nullptr, s);
     if (rc) return rc;
@@ -193,8 +175,7 @@ static int run_pipeline(apc_ctx* ctx, const apc_cloud_desc* clouds, uint32_t n_c
     rc = apc_segment_plane_nobegin(ctx, cur, n_total, dc + cur_cnt, cfg->ground_distance_threshold, cfg->ground_ransac_n,
                                    cfg->ground_num_iterations, cfg->ground_probability, cfg->ground_seed, nullptr, plane,
                                    nullptr, dc + DC_INFO, out, dc + DC_OUT, 4, s, row_in, rows, last_mir(), nrm_in,
-                                   nrm_in ? maps->normals_dev : nullptr, fold_env && n_total ? &fin : nullptr);
-    counts_done = fold_env && n_total;
+                                   nrm_in ? maps->normals_dev : nullptr);
     if (rc) return rc;
     row_in = rows;
     cur = out;
@@ -204,11 +185,9 @@ static int run_pipeline(apc_ctx* ctx, const apc_cloud_desc* clouds, uint32_t n_c
     k_iota<<<min(apc_div_up(n_total, 256), (uint32_t)APC_SM_COUNT * 4), 256, 0, s>>>(want_row, n_total, dc + cur_cnt);
     APC_LAUNCH_CHECK(ctx, "k_iota");
   }
-  if (!counts_done) {
-    fin.last = cur_cnt;
-    apc_klaunch(ctx, k_pipeline_counts, 1, 1, 0, s, fin, ctx->ctrl);
-    APC_LAUNCH_CHECK(ctx, "k_pipeline_counts");
-  }
+  fin.last = cur_cnt;
+  apc_klaunch(ctx, k_pipeline_counts, 1, 1, 0, s, fin, ctx->ctrl);
+  APC_LAUNCH_CHECK(ctx, "k_pipeline_counts");
   return APC_OK;
 }
 

@@ -15,7 +15,6 @@
 //   - final pass: inlier mask against the winning hypothesis + moment sums for the
 //     least-squares refit, reduced in a fixed order.
 #include <cmath>
-#include <cstdlib>
 #include "apc_scan.cuh"
 APC_TRACE_EXPORT(ransac)
 
@@ -225,7 +224,7 @@ k_rs_hypotheses(const float4* __restrict__ pts, uint32_t n_max, const uint32_t* 
 }
 
 template <int CH>
-__global__ void __launch_bounds__(APC_TILE_THREADS, CH <= 10 ? 3 : 1)
+__global__ void __launch_bounds__(APC_TILE_THREADS, 1)
 k_rs_score(const float4* __restrict__ pts, uint32_t n_max, const uint32_t* n_dev, uint32_t ransac_n, uint32_t iters,
            const double* __restrict__ planes, double thr,
            unsigned long long* scores, double log1mp, double* __restrict__ plane8, uint32_t* __restrict__ info,
@@ -555,8 +554,7 @@ k_rs_final(const float4* __restrict__ pts, uint32_t n_max, const uint32_t* n_dev
            uint32_t* __restrict__ info, double thr, uint8_t* __restrict__ mask, double* __restrict__ partials,
            float4* __restrict__ keep_out, uint32_t* keep_count, uint64_t* scan_state, uint32_t n_tiles, ApcCtrl* ctrl,
            const uint32_t* __restrict__ keep_idx_in, uint32_t* __restrict__ keep_idx_out,
-           const __grid_constant__ MirrorDev mir, const float* __restrict__ nrm_in, float* __restrict__ nrm_out,
-           const __grid_constant__ CountsEpilogue fin) {
+           const __grid_constant__ MirrorDev mir, const float* __restrict__ nrm_in, float* __restrict__ nrm_out) {
   __shared__ double s_red[8][10];
   __shared__ bool s_last;
   __shared__ uint32_t sm_scan[34];
@@ -652,8 +650,6 @@ k_rs_final(const float4* __restrict__ pts, uint32_t n_max, const uint32_t* n_dev
   if (threadIdx.x == 0) {
     const double n = s_tot[0];
     info[1] = (uint32_t)n;
-    // every other CTA has retired its results before its ticket: the stage counters are final
-    if (fin.dc) pipeline_counts_write(fin, ctrl);
     if (n < 1.0) { plane8[0] = plane8[1] = plane8[2] = plane8[3] = 0.0; return; }
     const double cx = s_tot[1] / n, cy = s_tot[2] / n, cz = s_tot[3] / n;
     const double xx = s_tot[4] - n * cx * cx, xy = s_tot[5] - n * cx * cy, xz = s_tot[6] - n * cx * cz;
@@ -667,8 +663,7 @@ int apc_segment_plane_nobegin(apc_ctx* ctx, const float* xyzi, uint32_t n_max, c
                               int ransac_n, int iters, double prob, uint64_t seed, const int32_t* table,
                               double* out_plane, uint8_t* out_mask, uint32_t* out_info, float* out_keep_xyzi,
                               uint32_t* out_keep_count, int scan_slot, cudaStream_t s, const uint32_t* keep_idx_in,
-                              uint32_t* keep_idx_out, const MirrorDev* mir, const float* nrm_in, float* nrm_out,
-                              const CountsEpilogue* fin) {
+                              uint32_t* keep_idx_out, const MirrorDev* mir, const float* nrm_in, float* nrm_out) {
   APC_REQUIRE(ctx, out_plane && out_info && (out_mask || out_keep_xyzi), "NULL output pointer");
   APC_REQUIRE(ctx, !out_keep_xyzi || out_keep_count, "out_keep_count is NULL");
   APC_REQUIRE(ctx, prob > 0.0 && prob <= 1.0, "probability must be in (0, 1]");
@@ -688,24 +683,15 @@ int apc_segment_plane_nobegin(apc_ctx* ctx, const float* xyzi, uint32_t n_max, c
   const float4* pts = reinterpret_cast<const float4*>(xyzi);
   const uint32_t n_tiles = apc_div_up(n_max, APC_TILE_POINTS);
   APC_REQUIRE(ctx, n_tiles <= ctx->max_tiles, "more points than the context was created for");
-  // hypotheses per CTA (CH) and CTAs per SM.  CH = 20 / 16 with ONE CTA per SM (142 / 128 registers, the
-  // default), or CH = 10 / 8 with TWO (80 registers): the same arithmetic per SM.  Measured (APC_RS_CH=10,
-  // profiles/r2g_rs_trace_ch10.txt): the two co-resident CTAs share the issue slots, so a CTA's scoring
-  // phase does not shrink (8.6 vs 8.2 us), the kernel ends later (19.1 vs 16.1 us) and saturated throughput
-  // is the same (70.5 vs 71.2 us/scan): the larger chunk stays.
-  static const uint32_t ch_env = []() { const char* e = getenv("APC_RS_CH"); return e ? (uint32_t)atoi(e) : 20u; }();
-  uint32_t ch;
-  if (ch_env == 20 || ch_env == 16) {
-    const uint32_t pad16 = apc_div_up(iters, 16) * 16, pad20 = apc_div_up(iters, 20) * 20;
-    ch = pad20 < pad16 ? 20u : 16u;               // whichever pads num_iterations less (100 = 5 x 20)
-  } else {
-    const uint32_t pad8 = apc_div_up(iters, 8) * 8, pad10 = apc_div_up(iters, 10) * 10;
-    ch = pad10 <= pad8 ? 10u : 8u;
-  }
+  // hypotheses per CTA (CH) = 20 or 16, with ONE CTA per SM.  Half the chunk (10 / 8) with TWO CTAs per SM does
+  // the same arithmetic per SM, but the two co-resident CTAs share the issue slots, so a CTA's scoring phase
+  // does not shrink (8.6 vs 8.2 us), the kernel ends later (19.1 vs 16.1 us) and saturated throughput is the
+  // same (70.5 vs 71.2 us/scan, profiles/r2g_rs_trace_ch10.txt): the larger chunk stays.
+  const uint32_t pad16 = apc_div_up(iters, 16) * 16, pad20 = apc_div_up(iters, 20) * 20;
+  const uint32_t ch = pad20 < pad16 ? 20u : 16u;   // whichever pads num_iterations less (100 = 5 x 20)
   const uint32_t n_chunks = apc_div_up(iters, ch);
-  const uint32_t ctas_per_sm = ch <= 10 ? 2u : 1u;
-  // every CTA strides over the same number of point tiles; the per-CTA tally rows are sized for <= 2 CTAs per SM
-  const uint32_t gx0 = min(n_tiles, max(1u, (uint32_t)(APC_SM_COUNT * ctas_per_sm) / n_chunks));
+  // every CTA strides over the same number of point tiles
+  const uint32_t gx0 = min(n_tiles, max(1u, (uint32_t)APC_SM_COUNT / n_chunks));
   const uint32_t gx = apc_div_up(n_tiles, apc_div_up(n_tiles, gx0));
   const dim3 grid(gx, n_chunks);
   const double log1mp = prob < 1.0 ? log(1.0 - prob) : -INFINITY;
@@ -720,9 +706,7 @@ int apc_segment_plane_nobegin(apc_ctx* ctx, const float* xyzi, uint32_t n_max, c
   apc_klaunch(ctx, k_rs_score<CHV>, grid, APC_TILE_THREADS, 0, s, pts, n_max, n_dev, ransac_n, iters, ctx->rs_planes, thr, ctx->rs_scores, \
                                                     log1mp, out_plane, out_info, ctx->rs_scores_copy, ctx->rs_col_tickets, ctx->ctrl)
     if (ch == 20) RS_LAUNCH(20);
-    else if (ch == 16) RS_LAUNCH(16);
-    else if (ch == 10) RS_LAUNCH(10);
-    else RS_LAUNCH(8);
+    else RS_LAUNCH(16);
 #undef RS_LAUNCH
   }
   APC_PROF(ctx, "k_rs_final", s);
@@ -730,7 +714,7 @@ int apc_segment_plane_nobegin(apc_ctx* ctx, const float* xyzi, uint32_t n_max, c
                                                   reinterpret_cast<float4*>(out_keep_xyzi), out_keep_count,
                                                   ctx->scan_state[scan_slot], n_tiles, ctx->ctrl, keep_idx_in, keep_idx_out,
                                                   mir && out_keep_xyzi ? *mir : MirrorDev{}, nrm_in,
-                                                  out_keep_xyzi ? nrm_out : nullptr, fin ? *fin : CountsEpilogue{});
+                                                  out_keep_xyzi ? nrm_out : nullptr);
   APC_LAUNCH_CHECK(ctx, "segment_plane");
   return APC_OK;
 }
@@ -746,7 +730,7 @@ extern "C" int apc_segment_plane(apc_ctx* ctx, const float* xyzi, uint32_t n_max
   if (rc) return rc;
   return apc_segment_plane_nobegin(ctx, xyzi, n_max, n_dev, distance_threshold, ransac_n, num_iterations, probability,
                                    seed, sample_table_dev, out_plane_dev, out_inlier_mask, out_info_dev, nullptr, nullptr,
-                                   4, s, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr);
+                                   4, s, nullptr, nullptr, nullptr, nullptr, nullptr);
 }
 
 // Per-hypothesis tallies {inlier count, integer error sum} of the most recent segment_plane call.

@@ -12,7 +12,6 @@
 //               slot; an order-preserving scan over the first-flags numbers the voxels
 // The table is self-cleaning: the thread that finalises a voxel resets its slot, so no
 // per-frame memset of the (capacity x 64 B) table sits on the critical path.
-#include <cstdlib>
 #include "apc_scan.cuh"
 #include "apc_grid.cuh"
 APC_TRACE_EXPORT(voxel)
@@ -42,79 +41,51 @@ __device__ __forceinline__ unsigned long long fixed_intensity(float w, ApcCtrl* 
   return 0ull;
 }
 
-// ITEMS points per thread, their atomics issued in lockstep (all key CAS first, then the probes of the
-// unlucky ones, then the joiners' accumulations).  ITEMS = 1 (default) gives the shortest kernel both
-// alone (15.7 vs 23.5 us: more resident warps hide the dependent atomic chain) and with eight lanes
-// sharing the GPU (68.9 vs 70.5 us/scan, profiles/r2g_knobs.json) although ITEMS = 4 holds half the
-// registers: the atomic round trips, not the register file, set this kernel's cost.  APC_VOX_ITEMS=4.
-template <int ITEMS>
+// One point per thread: the key CAS, the probes when the slot holds another voxel, then a joiner's
+// accumulations.  Four points per thread with their atomics issued in lockstep was slower both alone
+// (23.5 vs 15.7 us: more resident warps hide the dependent atomic chain) and with eight lanes sharing the GPU
+// (70.5 vs 68.9 us/scan, profiles/r2g_knobs.json) although it held half the registers: the atomic round
+// trips, not the register file, set this kernel's cost.
 __global__ void __launch_bounds__(256)
 k_voxel_insert(const float4* __restrict__ pts, uint32_t n_max, const uint32_t* n_dev, float vs,
                VoxSlot* __restrict__ slots, VoxAcc* __restrict__ accs, uint32_t cap_mask, uint32_t* __restrict__ p2slot,
                ApcCtrl* ctrl) {
   pdl_enter();
   const uint32_t n = apc_count(n_dev, n_max);
-  const uint32_t stride = gridDim.x * blockDim.x * ITEMS;
   APC_STAMP(0, 0);
-  for (uint32_t base = blockIdx.x * blockDim.x * ITEMS + threadIdx.x; base < n; base += stride) {
-    float4 p[ITEMS];
-    uint64_t key[ITEMS];
-    uint32_t slot[ITEMS];
-    unsigned long long old[ITEMS];
-    bool live[ITEMS];
-#pragma unroll
-    for (int j = 0; j < ITEMS; ++j) {
-      const uint32_t i = base + j * blockDim.x;
-      live[j] = i < n;
-      p[j] = live[j] ? pts[i] : make_float4(0.f, 0.f, 0.f, 0.f);
+  for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
+    const float4 p = pts[i];
+    uint64_t key = 0;
+    if (!voxel_key(p, vs, key)) {
+      atomicOr(&ctrl->err, APC_DEVERR_KEY_RANGE);
+      p2slot[i] = VOX_NOSLOT;
+      continue;
     }
-#pragma unroll
-    for (int j = 0; j < ITEMS; ++j) {
-      const uint32_t i = base + j * blockDim.x;
-      key[j] = 0;
-      slot[j] = 0;
-      if (live[j] && !voxel_key(p[j], vs, key[j])) {
-        atomicOr(&ctrl->err, APC_DEVERR_KEY_RANGE);
-        p2slot[i] = VOX_NOSLOT;
-        live[j] = false;
-      }
-      // block = the voxel's 2x2 neighbourhood in x, y (bit 0 of either index cleared); sub = its place in it
-      const uint64_t block = key[j] & ~((1ull << 42) | (1ull << 21));
-      const uint32_t sub = (uint32_t)((key[j] >> 42) & 1ull) | ((uint32_t)((key[j] >> 21) & 1ull) << 1);
-      slot[j] = ((((uint32_t)mix64(block)) << 2) & cap_mask) | sub;
+    // block = the voxel's 2x2 neighbourhood in x, y (bit 0 of either index cleared); sub = its place in it
+    const uint64_t block = key & ~((1ull << 42) | (1ull << 21));
+    const uint32_t sub = (uint32_t)((key >> 42) & 1ull) | ((uint32_t)((key >> 21) & 1ull) << 1);
+    uint32_t slot = ((((uint32_t)mix64(block)) << 2) & cap_mask) | sub;
+    unsigned long long old = atomicCAS(&slots[slot].key, VOX_EMPTY, (unsigned long long)key);
+    for (uint32_t probe = 1; old != VOX_EMPTY && old != key && probe <= (cap_mask >> 2); ++probe) {  // next block, same place
+      slot = (slot + 4) & cap_mask;
+      old = atomicCAS(&slots[slot].key, VOX_EMPTY, (unsigned long long)key);
     }
-#pragma unroll
-    for (int j = 0; j < ITEMS; ++j)      // every CAS in flight before any result is looked at
-      old[j] = live[j] ? atomicCAS(&slots[slot[j]].key, VOX_EMPTY, (unsigned long long)key[j]) : VOX_EMPTY;
-#pragma unroll
-    for (int j = 0; j < ITEMS; ++j) {
-      if (!live[j]) continue;
-      for (uint32_t probe = 1; old[j] != VOX_EMPTY && old[j] != key[j] && probe <= (cap_mask >> 2); ++probe) {  // next block, same place
-        slot[j] = (slot[j] + 4) & cap_mask;
-        old[j] = atomicCAS(&slots[slot[j]].key, VOX_EMPTY, (unsigned long long)key[j]);
-      }
-    }
-#pragma unroll
-    for (int j = 0; j < ITEMS; ++j) {
-      if (!live[j]) continue;
-      const uint32_t i = base + j * blockDim.x;
-      VoxSlot* s = &slots[slot[j]];
-      if (old[j] == VOX_EMPTY) {          // owner: nothing to accumulate yet
-        s->owner = i;
-        p2slot[i] = slot[j];
-      } else if (old[j] == key[j]) {      // joins an existing voxel
-        p2slot[i] = slot[j];
-        atomicMin(&s->first, i);
-        VoxAcc* a = &accs[slot[j]];
-        atomicAdd(&a->cnt, 1u);
-        atomicAdd(&a->acc[0], fixed_xyz(p[j].x));
-        atomicAdd(&a->acc[1], fixed_xyz(p[j].y));
-        atomicAdd(&a->acc[2], fixed_xyz(p[j].z));
-        atomicAdd(&a->acc[3], fixed_intensity(p[j].w, ctrl));
-      } else {
-        atomicOr(&ctrl->err, APC_DEVERR_CAPACITY);
-        p2slot[i] = VOX_NOSLOT;
-      }
+    VoxSlot* s = &slots[slot];
+    if (old == VOX_EMPTY) {          // owner: nothing to accumulate yet
+      s->owner = i;
+      p2slot[i] = slot;
+    } else if (old == key) {         // joins an existing voxel
+      p2slot[i] = slot;
+      atomicMin(&s->first, i);
+      VoxAcc* a = &accs[slot];
+      atomicAdd(&a->cnt, 1u);
+      atomicAdd(&a->acc[0], fixed_xyz(p.x));
+      atomicAdd(&a->acc[1], fixed_xyz(p.y));
+      atomicAdd(&a->acc[2], fixed_xyz(p.z));
+      atomicAdd(&a->acc[3], fixed_intensity(p.w, ctrl));
+    } else {
+      atomicOr(&ctrl->err, APC_DEVERR_CAPACITY);
+      p2slot[i] = VOX_NOSLOT;
     }
   }
   APC_STAMP(0, 1);
@@ -259,16 +230,8 @@ int apc_voxel_nobegin(apc_ctx* ctx, const float* xyzi, uint32_t n_max, const uin
   const uint32_t blocks = min(apc_div_up(n_max, 256), (uint32_t)APC_SM_COUNT * 8);
   {
     APC_PROF(ctx, "k_voxel_insert", s);
-    static const int items = []() { const char* e = getenv("APC_VOX_ITEMS"); return e ? atoi(e) : 1; }();
-    if (items >= 4) {
-      const uint32_t ib = min(apc_div_up(n_max, 1024), (uint32_t)APC_SM_COUNT * 8);
-      apc_klaunch(ctx, k_voxel_insert<4>, ib, 256, 0, s, reinterpret_cast<const float4*>(xyzi), n_max, n_dev, voxel_size, ctx->vox_slots,
-                                           ctx->vox_acc, ctx->hash_cap - 1, ctx->p2slot, ctx->ctrl);
-    } else {
-      const uint32_t ib = min(apc_div_up(n_max, 256), (uint32_t)APC_SM_COUNT * 8);
-      apc_klaunch(ctx, k_voxel_insert<1>, ib, 256, 0, s, reinterpret_cast<const float4*>(xyzi), n_max, n_dev, voxel_size, ctx->vox_slots,
-                                           ctx->vox_acc, ctx->hash_cap - 1, ctx->p2slot, ctx->ctrl);
-    }
+    apc_klaunch(ctx, k_voxel_insert, blocks, 256, 0, s, reinterpret_cast<const float4*>(xyzi), n_max, n_dev, voxel_size, ctx->vox_slots,
+                ctx->vox_acc, ctx->hash_cap - 1, ctx->p2slot, ctx->ctrl);
   }
   APC_LAUNCH_CHECK(ctx, "k_voxel_insert");
   const uint32_t n_tiles = apc_div_up(n_max, APC_TILE_POINTS);

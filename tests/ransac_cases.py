@@ -14,7 +14,6 @@ kernel clamps an out-of-range index to ``P - 1``; the oracle does not).
 from __future__ import annotations
 
 import math
-import os
 
 import numpy as np
 
@@ -26,21 +25,17 @@ SM_COUNT = 148
 QCAP = 128
 
 
-def chunk_size(iters: int, knob: int | None = None) -> int:
-    """Hypotheses per scoring CTA: 20 or 16, whichever pads ``iters`` less (the default), or 10 / 8
-    under ``APC_RS_CH=10``."""
-    knob = int(os.environ.get("APC_RS_CH", "20")) if knob is None else knob
+def chunk_size(iters: int) -> int:
+    """Hypotheses per scoring CTA: 20 or 16, whichever pads ``iters`` less."""
     up = lambda a, b: -(-a // b) * b
-    if knob in (20, 16):
-        return 20 if up(iters, 20) < up(iters, 16) else 16
-    return 10 if up(iters, 10) <= up(iters, 8) else 8
+    return 20 if up(iters, 20) < up(iters, 16) else 16
 
 
 def score_grid(n_max: int, iters: int, ch: int) -> tuple[int, int]:
     """``(CTAs striding over the point tiles, chunks)`` of the scoring launch."""
     n_tiles = -(-n_max // TILE_POINTS)
     n_chunks = -(-iters // ch)
-    gx0 = min(n_tiles, max(1, SM_COUNT * (2 if ch <= 10 else 1) // n_chunks))
+    gx0 = min(n_tiles, max(1, SM_COUNT // n_chunks))
     return -(-n_tiles // -(-n_tiles // gx0)), n_chunks
 
 

@@ -4,10 +4,6 @@ full), the packed per-thread count + error accumulator, the prefix-record select
 stop, the final pass, and the argument checks.  Every case asserts, through the band model of
 ``ransac_cases``, that it reaches the path it targets, and prints the counts."""
 import contextlib
-import os
-import re
-import subprocess
-import sys
 
 import numpy as np
 import pytest
@@ -17,7 +13,6 @@ import ransac_cases as rc
 pytestmark = pytest.mark.gpu
 
 torch = pytest.importorskip("torch")
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 NONE = 0xFFFFFFFF
 
 
@@ -328,15 +323,3 @@ def test_bad_arguments_and_recovery(env):
     assert e.value.code == capi.APC_ERR_TOO_FEW
     compare(ctx, pts, 0.2, 5, 50, seed=99)
 
-
-# ---- 10. the APC_RS_CH=10 variant -----------------------------------------------------------------------
-def test_small_chunk_variant():
-    """Cases 1, 2 and 5 with ``APC_RS_CH=10`` (chunks of 8 or 10, two CTAs per SM); the knob is read once
-    per process, so they run in a child interpreter."""
-    env = dict(os.environ, APC_RS_CH="10")
-    r = subprocess.run([sys.executable, "-m", "pytest", "-q", "-s", "-p", "no:cacheprovider", os.path.abspath(__file__),
-                        "-k", "rounding_band or queue_overflow or many_chunks"],
-                       env=env, cwd=ROOT, capture_output=True, text=True, timeout=900)
-    print(r.stdout[-3000:])
-    assert r.returncode == 0, r.stdout[-3000:] + r.stderr[-2000:]
-    assert re.search(r"\b9 passed", r.stdout)

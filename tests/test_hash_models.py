@@ -287,9 +287,9 @@ def test_sources_match_the_models():
     assert set(int(b) for b in re.findall(r"\(int64_t\)q[xyz] \+ (\d+)\)", vk)) == {VOX_BIAS}
     sh = re.search(r"key = \(ux << (\d+)\) \| \(uy << (\d+)\) \| uz;", vk)
     assert (int(sh.group(1)), int(sh.group(2))) == VOX_SHIFTS
-    assert "key[j] & ~((1ull << 42) | (1ull << 21))" in vx
-    assert "slot[j] = ((((uint32_t)mix64(block)) << 2) & cap_mask) | sub;" in vx
-    assert "slot[j] = (slot[j] + 4) & cap_mask;" in vx                   # probing moves block by block
+    assert "key & ~((1ull << 42) | (1ull << 21))" in vx
+    assert "slot = ((((uint32_t)mix64(block)) << 2) & cap_mask) | sub;" in vx
+    assert "slot = (slot + 4) & cap_mask;" in vx                         # probing moves block by block
 
     gk = _body(_src("apc_grid.cuh"), "uint64_t grid_key(uint32_t level, int32_t ix, int32_t iy, int32_t iz)")
     lv = int(re.search(r"\(uint64_t\)level << (\d+)", gk).group(1))
@@ -308,6 +308,6 @@ def test_sources_match_the_models():
     assert "uint64_t want = (uint64_t)levels * M * 4 / 3 + 1024;" in nb
     assert "if (which == 0 && cap < ctx->hash_cap) cap = ctx->hash_cap;" in nb
     assert f"#define KNN_LEVELS {KNN_LEVELS}" in nb
-    assert re.search(r"return r32 \* radius_cell_mult\(\) \* ([0-9.]+)f;", nb).group(1) == repr(RADIUS_CELL_SLACK)
-    assert "const float v = e ? (float)atof(e) : 2.0f;" in nb
+    m = re.search(r"static float radius_cell\(float r32\) \{ return r32 \* ([0-9.]+)f \* ([0-9.]+)f; \}", nb)
+    assert float(m.group(1)) == RADIUS_CELL_MULT and m.group(2) == repr(RADIUS_CELL_SLACK)
     assert nb.count(f"r32 * {NB_CELL_SLACK!r}f") >= 3                   # normals radius, DBSCAN, ICP
