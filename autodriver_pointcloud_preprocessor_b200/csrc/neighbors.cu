@@ -230,6 +230,58 @@ __device__ __forceinline__ uint32_t grid_sorted_count(const GridDev& g, const Ap
   return min(n, ctrl->counters[g.cursor_base]);
 }
 
+// ---- the warp's 27-cell walk ----------------------------------------------------------------------
+// The 27 cells around cell (ix, iy, iz) of `level` as one flat candidate list, for a warp that walks it 32 records
+// at a time: lane l < 27 resolves cell l and keeps its run's start in the level's cell-sorted array (cs) and the
+// flat index of the run's first record (ps); returns the list's length (all lanes).
+__device__ __forceinline__ uint32_t flat27_runs(const GridDev& g, uint32_t level, int32_t ix, int32_t iy, int32_t iz,
+                                                uint32_t lane, uint32_t& cs, uint32_t& ps) {
+  uint32_t s0 = 0, cf = 0;
+  if (lane < 27) {
+    const int dx = (int)(lane % 3u) - 1, dy = (int)((lane / 3u) % 3u) - 1, dz = (int)(lane / 9u) - 1;
+    uint32_t b, f;
+    if (grid_lookup(g, grid_key(level, ix + dx, iy + dy, iz + dz), b, f)) { s0 = b; cf = f; }
+  }
+  uint32_t incl = cf;
+#pragma unroll
+  for (int o = 1; o < 32; o <<= 1) {
+    const uint32_t v = __shfl_up_sync(0xffffffffu, incl, o);
+    if (lane >= (uint32_t)o) incl += v;
+  }
+  cs = s0;
+  ps = incl - cf;
+  return __shfl_sync(0xffffffffu, incl, 31);
+}
+// The same around the level-0 cell of a query taken from the grid (its cell was keyed at insert time).
+__device__ __forceinline__ uint32_t flat27_runs(const GridDev& g, float c, float4 q, uint32_t lane, uint32_t& cs, uint32_t& ps) {
+  int32_t ix, iy, iz;
+  grid_coord_g(g, c, q.x, q.y, q.z, ix, iy, iz);  // succeeded at insert time
+  return flat27_runs(g, 0, ix, iy, iz, lane, cs, ps);
+}
+// Position in the level's cell-sorted array of record `flat` of that list (called by all lanes of the warp).
+__device__ __forceinline__ uint32_t flat27_at(uint32_t cs, uint32_t ps, uint32_t flat) {
+  uint32_t run = 0;                                  // largest cell with ps <= flat
+#pragma unroll
+  for (int step = 16; step > 0; step >>= 1) {
+    const uint32_t mid = run + step;
+    const uint32_t v = __shfl_sync(0xffffffffu, ps, mid & 31u);
+    if (mid < 27u && v <= flat) run = mid;
+  }
+  const uint32_t rs = __shfl_sync(0xffffffffu, cs, run), rp = __shfl_sync(0xffffffffu, ps, run);
+  return rs + (flat - rp);
+}
+// KNN coverage bound, squared: every point closer to q than `safe` lies inside the 27-cell block around q's cell
+// (ix, iy, iz) of edge c.  `safe` is the cell edge plus q's distance to the nearest face of its own cell (1859 against
+// 1961 us for the cell edge alone on the C4 scan, profiles/r2x_knn_ab.json), less 0.1 % for the rounding of the
+// cell index.
+__device__ __forceinline__ float knn_safe2(float4 q, float c, int32_t ix, int32_t iy, int32_t iz) {
+  const float fx = fminf(__fsub_rn(q.x, __fmul_rn((float)ix, c)), __fsub_rn(__fmul_rn((float)(ix + 1), c), q.x));
+  const float fy = fminf(__fsub_rn(q.y, __fmul_rn((float)iy, c)), __fsub_rn(__fmul_rn((float)(iy + 1), c), q.y));
+  const float fz = fminf(__fsub_rn(q.z, __fmul_rn((float)iz, c)), __fsub_rn(__fmul_rn((float)(iz + 1), c), q.z));
+  const float safe = __fmul_rn(__fadd_rn(c, fmaxf(0.0f, fminf(fx, fminf(fy, fz)))), 0.999f);
+  return __fmul_rn(safe, safe);
+}
+
 // ---- radius query -----------------------------------------------------------------------------
 // cnt + the neighbours of q within r2 in the run [b, b + f) of the cell-sorted array, stopping at nb_points
 // unless the exact count is wanted.
@@ -423,18 +475,19 @@ struct TopK {
 
 // One WARP per query (the per-thread version - a sorted list in local memory - ran at 7 active lanes
 // per instruction and 1750 warp instructions per query: profiles, prof_c4).  Per level:
-//   1. lanes 0..26 resolve the 27 neighbour cells in parallel; a warp scan of the run lengths gives
-//      the flat candidate list and tells whether the block holds k points at all;
-//   2. the lanes stride over the flat list (run found by a 5-step shuffle search), compute the
-//      float32 distances and drop their bit patterns (non-negative floats order like integers)
-//      into the warp's shared buffer; longer lists go through the buffer in chunks, each chunk
-//      merged with the k best so far;
+//   1. the warp's 27-cell walk (flat27_runs) gives the flat candidate list and tells whether the block
+//      holds k points at all;
+//   2. the lanes stride over the flat list, compute the float32 distances and drop their bit patterns
+//      (non-negative floats order like integers) into the warp's shared buffer; longer lists go through
+//      the buffer in chunks, each chunk merged with the k best so far;
 //   3. the k-th smallest value is found by a 31-step binary search on the bit pattern (each step a
 //      strided count + REDUX), the k smallest are compacted in place (ties at the k-th value are
 //      interchangeable);
-//   4. the level's answer stands if the k-th distance is covered by the block (same test as before);
-//      then the k values are rank-sorted and summed in ascending order by shuffles - the same
-//      sequential float32 sum as oracle/outliers.py.
+//   4. the level's answer stands if the k-th distance is covered by the block (knn_safe2); then the k
+//      values are rank-sorted and summed in ascending order by shuffles - the same sequential float32
+//      sum as oracle/outliers.py.
+// WarpKeep does steps 2 and 3 for k_knn_query_wide, but in this kernel's place at 32 < k <= 64 it was 20 - 30 %
+// slower on the C4 scan (3476 -> 4572 us at k = 33, 4708 -> 5679 us at k = 64; B200 at 1000 W).
 #define KNN_CAP 1024
 #define KNN_WARPS 4
 // newcomers in a batch of 32 above which the batch is sorted and merged instead of inserted one by one
@@ -462,30 +515,11 @@ k_knn_query(uint32_t n_max, const uint32_t* n_dev, GridDev g, uint32_t k, float*
       const float c = g.cell[level];
       int32_t ix, iy, iz;
       if (!grid_coord_g(g, c, q.x, q.y, q.z, ix, iy, iz)) continue;
-      // 1. the 27 cells, one per lane
-      uint32_t cs = 0, cf = 0;
-      if (lane < 27) {
-        const int dx = (int)(lane % 3u) - 1, dy = (int)((lane / 3u) % 3u) - 1, dz = (int)(lane / 9u) - 1;
-        uint32_t b, f;
-        if (grid_lookup(g, grid_key(level, ix + dx, iy + dy, iz + dz), b, f)) { cs = b; cf = f; }
-      }
-      uint32_t incl = cf;
-#pragma unroll
-      for (int o = 1; o < 32; o <<= 1) {
-        const uint32_t v = __shfl_up_sync(0xffffffffu, incl, o);
-        if (lane >= (uint32_t)o) incl += v;
-      }
-      const uint32_t ps = incl - cf;                               // first flat index of this lane's run
-      const uint32_t total = __shfl_sync(0xffffffffu, incl, 31);
+      uint32_t cs, ps;
+      const uint32_t total = flat27_runs(g, level, ix, iy, iz, lane, cs, ps);
       if (total < k_eff) continue;
       const float4* sp = g.sorted + (size_t)level * n_max;
-      // every point closer than `safe` lies inside the 27-cell block: the cell edge plus the query's distance
-      // to the nearest face of its own cell (1859 against 1961 us for the cell edge alone on the C4 scan,
-      // profiles/r2x_knn_ab.json), less 0.1 % for the rounding of the cell index
-      const float fx = fminf(__fsub_rn(q.x, __fmul_rn((float)ix, c)), __fsub_rn(__fmul_rn((float)(ix + 1), c), q.x));
-      const float fy = fminf(__fsub_rn(q.y, __fmul_rn((float)iy, c)), __fsub_rn(__fmul_rn((float)(iy + 1), c), q.y));
-      const float fz = fminf(__fsub_rn(q.z, __fmul_rn((float)iz, c)), __fsub_rn(__fmul_rn((float)(iz + 1), c), q.z));
-      const float safe = __fmul_rn(__fadd_rn(c, fmaxf(0.0f, fminf(fx, fminf(fy, fz)))), 0.999f);
+      const float bound2 = knn_safe2(q, c, ix, iy, iz);
       if (k_eff <= 32u) {
         // 2'. k <= 32 (the reference's default is 20): the k best live in REGISTERS, lane i holding the
         // i-th smallest distance so far.  A batch of 32 candidates is screened with one ballot against
@@ -495,18 +529,10 @@ k_knn_query(uint32_t n_max, const uint32_t* n_dev, GridDev g, uint32_t k, float*
         float val = inf, kth = inf;
         for (uint32_t base = 0; base < total; base += 32) {
           const uint32_t ci = base + lane;
-          const uint32_t flat = min(ci, total - 1u);
-          uint32_t run = 0;                                        // largest t with ps[t] <= flat
-#pragma unroll
-          for (int step = 16; step > 0; step >>= 1) {
-            const uint32_t mid = run + step;
-            const uint32_t v = __shfl_sync(0xffffffffu, ps, mid & 31u);
-            if (mid < 27u && v <= flat) run = mid;
-          }
-          const uint32_t rs = __shfl_sync(0xffffffffu, cs, run), rp = __shfl_sync(0xffffffffu, ps, run);
+          const uint32_t at = flat27_at(cs, ps, min(ci, total - 1u));
           float d2 = inf;
           if (ci < total) {
-            const float4 p = sp[rs + (flat - rp)];
+            const float4 p = sp[at];
             d2 = d2_f32(q.x, q.y, q.z, p.x, p.y, p.z);
           }
           uint32_t cand = __ballot_sync(0xffffffffu, d2 < kth);
@@ -548,7 +574,7 @@ k_knn_query(uint32_t n_max, const uint32_t* n_dev, GridDev g, uint32_t k, float*
             }
           }
         }
-        if (kth <= __fmul_rn(safe, safe)) {
+        if (kth <= bound2) {
           done = true;
           const float r = sqrtf(val);
           float sum = 0.0f;
@@ -566,17 +592,9 @@ k_knn_query(uint32_t n_max, const uint32_t* n_dev, GridDev g, uint32_t k, float*
         const uint32_t take = min((uint32_t)KNN_CAP - m, total - c0);
         for (uint32_t base = 0; base < take; base += 32) {
           const uint32_t ci = base + lane;
-          const uint32_t flat = c0 + min(ci, take - 1u);
-          uint32_t run = 0;                                        // largest t with ps[t] <= flat
-#pragma unroll
-          for (int step = 16; step > 0; step >>= 1) {
-            const uint32_t mid = run + step;
-            const uint32_t v = __shfl_sync(0xffffffffu, ps, mid & 31u);
-            if (mid < 27u && v <= flat) run = mid;
-          }
-          const uint32_t rs = __shfl_sync(0xffffffffu, cs, run), rp = __shfl_sync(0xffffffffu, ps, run);
+          const uint32_t at = flat27_at(cs, ps, c0 + min(ci, take - 1u));
           if (ci < take) {
-            const float4 p = sp[rs + (flat - rp)];
+            const float4 p = sp[at];
             buf[m + ci] = __float_as_uint(d2_f32(q.x, q.y, q.z, p.x, p.y, p.z));
           }
         }
@@ -617,7 +635,7 @@ k_knn_query(uint32_t n_max, const uint32_t* n_dev, GridDev g, uint32_t k, float*
       uint32_t mx = 0;
       for (uint32_t i = lane; i < k_eff; i += 32) mx = max(mx, buf[i]);
       const float kth = __uint_as_float(__reduce_max_sync(0xffffffffu, mx));
-      if (kth <= __fmul_rn(safe, safe)) done = true;
+      if (kth <= bound2) done = true;
     }
     if (done && k_eff > 32u) {
       for (uint32_t e = lane; e < k_eff; e += 32) {                 // rank sort (k <= 64)
@@ -695,7 +713,7 @@ k_knn_stragglers(const float4* __restrict__ pts, uint32_t n_max, const uint32_t*
   }
 }
 
-// ---- k > 64 (up to APC_MAX_NEIGHBORS): per-warp shared candidate buffers ---------------------------
+// ---- k > 64 (up to APC_MAX_NEIGHBORS; normals: max_nn > 32): per-warp shared candidate buffers -------
 // Keys are compared as unsigned integers and have their top bit clear: float32 d2 bit patterns
 // (non-negative floats order like integers), or (d2 bits << 32 | index) for the normals.
 //
@@ -754,7 +772,7 @@ struct WarpKeep {
   }
 };
 
-// Buffer entries per warp for k > 64: more than k + 32 (a selection always makes room for a batch)
+// Buffer entries per warp of a WarpKeep: more than k + 32 (a selection always makes room for a batch)
 // and at least the power of two warp_sort pads k to.  k = 1024: 1280 entries, 5 KB (KNN) /
 // 10 KB (normals) per warp, 20 / 40 KB per block of 4 warps - under the 48 KB of a default launch.
 static inline uint32_t wide_cap(uint32_t k) {
@@ -812,8 +830,8 @@ template <> __device__ __forceinline__ unsigned long long knn_key<unsigned long 
 }
 
 // The KNN grid's level climb for query q (warp-collective), shared by k_knn_query_wide and k_normals_knn:
-// per level, lanes 0..26 resolve the 27 cells, the flat candidate list streams through a WarpKeep of `cap`
-// keys at buf, and the level stands if the k_eff-th distance is covered by the block (`safe`).
+// per level, the 27-cell flat candidate list (flat27_runs) streams through a WarpKeep of `cap` keys at buf,
+// and the level stands if the k_eff-th distance is covered by the block (knn_safe2).
 // Returns true with the k_eff smallest keys in buf[0, k_eff) (unordered); false when no level covers q
 // (a straggler).
 template <typename K>
@@ -823,42 +841,19 @@ __device__ __forceinline__ bool knn_levels(const GridDev& g, uint32_t n_max, flo
     const float c = g.cell[level];
     int32_t ix, iy, iz;
     if (!grid_coord_g(g, c, q.x, q.y, q.z, ix, iy, iz)) continue;
-    uint32_t cs = 0, cf = 0;
-    if (lane < 27) {
-      const int dx = (int)(lane % 3u) - 1, dy = (int)((lane / 3u) % 3u) - 1, dz = (int)(lane / 9u) - 1;
-      uint32_t b, f;
-      if (grid_lookup(g, grid_key(level, ix + dx, iy + dy, iz + dz), b, f)) { cs = b; cf = f; }
-    }
-    uint32_t incl = cf;
-#pragma unroll
-    for (int o = 1; o < 32; o <<= 1) {
-      const uint32_t v = __shfl_up_sync(0xffffffffu, incl, o);
-      if (lane >= (uint32_t)o) incl += v;
-    }
-    const uint32_t ps = incl - cf;
-    const uint32_t total = __shfl_sync(0xffffffffu, incl, 31);
+    uint32_t cs, ps;
+    const uint32_t total = flat27_runs(g, level, ix, iy, iz, lane, cs, ps);
     if (total < k_eff) continue;
     const float4* sp = g.sorted + (size_t)level * n_max;
-    const float fx = fminf(__fsub_rn(q.x, __fmul_rn((float)ix, c)), __fsub_rn(__fmul_rn((float)(ix + 1), c), q.x));
-    const float fy = fminf(__fsub_rn(q.y, __fmul_rn((float)iy, c)), __fsub_rn(__fmul_rn((float)(iy + 1), c), q.y));
-    const float fz = fminf(__fsub_rn(q.z, __fmul_rn((float)iz, c)), __fsub_rn(__fmul_rn((float)(iz + 1), c), q.z));
-    const float safe = __fmul_rn(__fadd_rn(c, fmaxf(0.0f, fminf(fx, fminf(fy, fz)))), 0.999f);
+    const float bound2 = knn_safe2(q, c, ix, iy, iz);
     WarpKeep<K> wk;
     wk.init(buf, cap, k_eff);
     for (uint32_t base = 0; base < total; base += 32) {
       const uint32_t ci = base + lane;
-      const uint32_t flat = min(ci, total - 1u);
-      uint32_t run = 0;                                          // largest t with ps[t] <= flat
-#pragma unroll
-      for (int step = 16; step > 0; step >>= 1) {
-        const uint32_t mid = run + step;
-        const uint32_t v = __shfl_sync(0xffffffffu, ps, mid & 31u);
-        if (mid < 27u && v <= flat) run = mid;
-      }
-      const uint32_t rs = __shfl_sync(0xffffffffu, cs, run), rp = __shfl_sync(0xffffffffu, ps, run);
+      const uint32_t at = flat27_at(cs, ps, min(ci, total - 1u));
       K key = 0;
       if (ci < total) {
-        const float4 p = sp[rs + (flat - rp)];
+        const float4 p = sp[at];
         key = knn_key<K>(d2_f32(q.x, q.y, q.z, p.x, p.y, p.z), __float_as_uint(p.w));
       }
       wk.add(key, ci < total, lane);
@@ -866,7 +861,7 @@ __device__ __forceinline__ bool knn_levels(const GridDev& g, uint32_t n_max, flo
     wk.finish(lane);
     uint32_t mx = 0;                                             // covered by the block? (the d2 bits of the keys)
     for (uint32_t i = lane; i < k_eff; i += 32) mx = max(mx, (uint32_t)(buf[i] >> (8 * sizeof(K) - 32)));
-    if (__uint_as_float(__reduce_max_sync(0xffffffffu, mx)) <= __fmul_rn(safe, safe)) return true;
+    if (__uint_as_float(__reduce_max_sync(0xffffffffu, mx)) <= bound2) return true;
   }
   return false;
 }
@@ -892,8 +887,8 @@ __device__ __forceinline__ void knn_brute(const float4* __restrict__ pts, uint32
 }
 
 // k_knn_query for 64 < k <= APC_MAX_NEIGHBORS: the same level climb, 27-cell flat candidate list and
-// coverage test (`safe`), the candidates through a WarpKeep of wide_cap(k) entries per
-// warp (dynamic shared memory), the accepted level's k distances sorted and summed by wide_average.
+// coverage test (knn_safe2), the candidates through a WarpKeep of wide_cap(k) entries per warp (dynamic
+// shared memory), the accepted level's k distances sorted and summed by wide_average.
 __global__ void __launch_bounds__(KNN_WARPS * 32)
 k_knn_query_wide(uint32_t n_max, const uint32_t* n_dev, GridDev g, uint32_t k, uint32_t cap, float* __restrict__ avg,
                  uint32_t* __restrict__ stragglers, ApcCtrl* ctrl) {
@@ -1297,28 +1292,23 @@ int apc_statistical_nobegin(apc_ctx* ctx, const float* xyzi, uint32_t n_max, con
   rc = grid_build(ctx, g, pts, n_max, n_dev, cell_hint, !(cell_hint > 0.0f), s);
   if (rc) return rc;
   const uint32_t bq = min(apc_div_up(n_max, KNN_WARPS), (uint32_t)APC_SM_COUNT * 16);   // one warp per query, grid-stride
-  if (nb_neighbors > KNN_KMAX) {
-    const uint32_t cap = wide_cap((uint32_t)nb_neighbors);
+  const uint32_t k = (uint32_t)nb_neighbors;
+  if (k <= KNN_KMAX) {
+    {
+      APC_PROF(ctx, "k_knn_query", s);
+      k_knn_query<<<bq, KNN_WARPS * 32, 0, s>>>(n_max, n_dev, g.d, k, avg, sc->stragglers, ctx->ctrl);
+    }
+    APC_PROF(ctx, "k_knn_stragglers", s);
+    k_knn_stragglers<<<APC_SM_COUNT * 2, 256, 0, s>>>(pts, n_max, n_dev, k, sc->stragglers, ctx->ctrl, avg);
+  } else {
+    const uint32_t cap = wide_cap(k);
     const size_t smem = (size_t)KNN_WARPS * cap * sizeof(uint32_t);
     {
       APC_PROF(ctx, "k_knn_query_wide", s);
-      k_knn_query_wide<<<bq, KNN_WARPS * 32, smem, s>>>(n_max, n_dev, g.d, (uint32_t)nb_neighbors, cap, avg, sc->stragglers,
-                                                        ctx->ctrl);
+      k_knn_query_wide<<<bq, KNN_WARPS * 32, smem, s>>>(n_max, n_dev, g.d, k, cap, avg, sc->stragglers, ctx->ctrl);
     }
-    {
-      APC_PROF(ctx, "k_knn_stragglers_wide", s);
-      k_knn_stragglers_wide<<<APC_SM_COUNT * 2, KNN_WARPS * 32, smem, s>>>(pts, n_max, n_dev, (uint32_t)nb_neighbors, cap,
-                                                                           sc->stragglers, ctx->ctrl, avg);
-    }
-  } else {
-    {
-      APC_PROF(ctx, "k_knn_query", s);
-      k_knn_query<<<bq, KNN_WARPS * 32, 0, s>>>(n_max, n_dev, g.d, (uint32_t)nb_neighbors, avg, sc->stragglers, ctx->ctrl);
-    }
-    {
-      APC_PROF(ctx, "k_knn_stragglers", s);
-      k_knn_stragglers<<<APC_SM_COUNT * 2, 256, 0, s>>>(pts, n_max, n_dev, (uint32_t)nb_neighbors, sc->stragglers, ctx->ctrl, avg);
-    }
+    APC_PROF(ctx, "k_knn_stragglers_wide", s);
+    k_knn_stragglers_wide<<<APC_SM_COUNT * 2, KNN_WARPS * 32, smem, s>>>(pts, n_max, n_dev, k, cap, sc->stragglers, ctx->ctrl, avg);
   }
   const dim3 gridc(min(apc_div_up(n_max, 256), (uint32_t)APC_SM_COUNT * 4), g.d.levels);
   {
@@ -1367,30 +1357,6 @@ extern "C" int apc_statistical_outliers(apc_ctx* ctx, const float* xyzi, uint32_
 // (0, 0, 1).  The neighbourhood is chosen with the float32 distance of the outlier stages and the
 // total order (d2, original index); moments are taken about the query point in float64 (no
 // cancellation whatever the coordinates' magnitude).  oracle/normals.py restates the same steps.
-#define NRM_KMAX 64
-
-struct NearList {
-  unsigned long long key[NRM_KMAX];   // d2 bits << 32 | original index: d2 >= 0, so integer order = (d2, index) order
-  uint32_t pos[NRM_KMAX];             // position of the neighbour in the cell-sorted array
-  uint32_t cnt, worst;
-  __device__ __forceinline__ void find_worst(uint32_t k) {
-    worst = 0;
-    for (uint32_t j = 1; j < k; ++j)
-      if (key[j] > key[worst]) worst = j;
-  }
-  __device__ __forceinline__ void push(unsigned long long kk, uint32_t p, uint32_t k) {
-    if (cnt < k) {
-      key[cnt] = kk;
-      pos[cnt] = p;
-      if (++cnt == k) find_worst(k);
-    } else if (kk < key[worst]) {
-      key[worst] = kk;
-      pos[worst] = p;
-      find_worst(k);
-    }
-  }
-};
-
 __device__ __forceinline__ void cross3(const double* a, const double* b, double* c) {
   c[0] = a[1] * b[2] - a[2] * b[1];
   c[1] = a[2] * b[0] - a[0] * b[2];
@@ -1490,66 +1456,38 @@ __device__ void normal_from_covariance(const double* C, double* nrm) {
   }
 }
 
-__global__ void __launch_bounds__(128)
-k_normals_query(uint32_t n_max, const uint32_t* n_dev, GridDev g, float r2, uint32_t max_nn, float* __restrict__ normals,
-                uint32_t* __restrict__ counts, double* __restrict__ covariances, const ApcCtrl* __restrict__ ctrl) {
-  const uint32_t n = grid_sorted_count(g, ctrl, apc_count(n_dev, n_max));
-  const float c = grid_cell_size(g, 0);
-  for (uint32_t j = blockIdx.x * blockDim.x + threadIdx.x; j < n; j += gridDim.x * blockDim.x) {
-    const float4 q = g.sorted[j];
-    const uint32_t orig = __float_as_uint(q.w);
-    int32_t ix, iy, iz;
-    grid_coord_g(g, c, q.x, q.y, q.z, ix, iy, iz);  // succeeded at insert time
-    NearList nl;
-    nl.cnt = 0;
-    nl.worst = 0;
-    for (int c27 = 0; c27 < 27; ++c27) {
-      const int dx = c27 % 3 - 1, dy = (c27 / 3) % 3 - 1, dz = c27 / 9 - 1;
-      uint32_t b, f;
-      if (!grid_lookup(g, grid_key(0, ix + dx, iy + dy, iz + dz), b, f)) continue;
-      const uint32_t e = b + f;
-      for (uint32_t t = b; t < e; ++t) {
-        const float4 p = g.sorted[t];
-        const float d2 = d2_f32(q.x, q.y, q.z, p.x, p.y, p.z);
-        if (d2 <= r2)
-          nl.push(((unsigned long long)__float_as_uint(d2) << 32) | __float_as_uint(p.w), t, max_nn);
-      }
-    }
-    double C[9] = {1.0, 0.0, 0.0, 0.0, 1.0, 0.0, 0.0, 0.0, 1.0};   // fewer than 3 neighbours: identity
-    if (nl.cnt >= 3) {
-      double s0 = 0.0, s1 = 0.0, s2 = 0.0, m00 = 0.0, m01 = 0.0, m02 = 0.0, m11 = 0.0, m12 = 0.0, m22 = 0.0;
-      for (uint32_t k = 0; k < nl.cnt; ++k) {
-        const float4 p = g.sorted[nl.pos[k]];
-        const double x = (double)p.x - (double)q.x, y = (double)p.y - (double)q.y, z = (double)p.z - (double)q.z;
-        s0 += x; s1 += y; s2 += z;
-        m00 += x * x; m01 += x * y; m02 += x * z; m11 += y * y; m12 += y * z; m22 += z * z;
-      }
-      const double inv = 1.0 / (double)nl.cnt;
-      s0 *= inv; s1 *= inv; s2 *= inv;
-      C[0] = m00 * inv - s0 * s0;
-      C[1] = C[3] = m01 * inv - s0 * s1;
-      C[2] = C[6] = m02 * inv - s0 * s2;
-      C[4] = m11 * inv - s1 * s1;
-      C[5] = C[7] = m12 * inv - s1 * s2;
-      C[8] = m22 * inv - s2 * s2;
-    }
-    double nrm[3];
-    normal_from_covariance(C, nrm);
-    normals[3 * (size_t)orig + 0] = (float)nrm[0];
-    normals[3 * (size_t)orig + 1] = (float)nrm[1];
-    normals[3 * (size_t)orig + 2] = (float)nrm[2];
-    if (counts) counts[orig] = nl.cnt;
-    if (covariances)
-      for (int k = 0; k < 9; ++k) covariances[9 * (size_t)orig + k] = C[k];
+// Covariance of a neighbourhood of n_sel points from float64 moments about the query point that the lanes hold in
+// parts (v: sums of x, y, z, xx, xy, xz, yy, yz, zz): the warp adds them up (warp-collective), lanes 0..8 store cov9
+// of point orig, lane 0 the count.  Fewer than 3 neighbours: identity.
+__device__ __forceinline__ void normals_cov_store(double (&v)[9], uint32_t n_sel, uint32_t orig, uint32_t lane,
+                                                  uint32_t* __restrict__ counts, double* __restrict__ cov9) {
+  double C[9] = {1.0, 0.0, 0.0, 0.0, 1.0, 0.0, 0.0, 0.0, 1.0};
+  if (n_sel >= 3) {
+#pragma unroll
+    for (int k = 0; k < 9; ++k)
+#pragma unroll
+      for (int o = 16; o > 0; o >>= 1) v[k] += __shfl_xor_sync(0xffffffffu, v[k], o);
+    const double inv = 1.0 / (double)n_sel;
+    const double s0 = v[0] * inv, s1 = v[1] * inv, s2 = v[2] * inv;
+    C[0] = v[3] * inv - s0 * s0;
+    C[1] = C[3] = v[4] * inv - s0 * s1;
+    C[2] = C[6] = v[5] * inv - s0 * s2;
+    C[4] = v[6] * inv - s1 * s1;
+    C[5] = C[7] = v[7] * inv - s1 * s2;
+    C[8] = v[8] * inv - s2 * s2;
   }
+  double mine = C[0];                                            // C[lane] without a local-memory array
+#pragma unroll
+  for (int k = 1; k < 9; ++k) mine = lane == (uint32_t)k ? C[k] : mine;
+  if (lane < 9) cov9[9 * (size_t)orig + lane] = mine;
+  if (lane == 0 && counts) counts[orig] = n_sel;
 }
 
-// max_nn <= 32 (the reference's default is 30): one WARP per query, as in k_knn_query.  Lanes 0..26
-// resolve the 27 cells; the lanes stride over the flat candidate list; the max_nn nearest in-radius
-// neighbours by (d2, original index) live in registers, lane i holding the i-th smallest key and the
-// neighbour's position; every lane then contributes its neighbour's moments about the query point
-// and a shuffle tree adds them up in float64.  The eigenvector is computed by k_normals_eigen, one
-// THREAD per point (a serial float64 solve would idle 31 lanes of the warp here).
+// max_nn <= 32 (the reference's default is 30): one WARP per query, as in k_knn_query.  The lanes stride over
+// the 27-cell flat candidate list; the max_nn nearest in-radius neighbours by (d2, original index) live in
+// registers, lane i holding the i-th smallest key and the neighbour's position; every lane then contributes its
+// neighbour's moments about the query point and normals_cov_store adds them up in float64.  The eigenvector is
+// computed by k_normals_eigen, one THREAD per point (a serial float64 solve would idle 31 lanes of the warp here).
 __global__ void __launch_bounds__(128)
 k_normals_cov(uint32_t n_max, const uint32_t* n_dev, GridDev g, float r2, uint32_t max_nn, uint32_t* __restrict__ counts,
               double* __restrict__ cov9, const ApcCtrl* __restrict__ ctrl) {
@@ -1559,36 +1497,13 @@ k_normals_cov(uint32_t n_max, const uint32_t* n_dev, GridDev g, float r2, uint32
   for (uint32_t j = (blockIdx.x * blockDim.x + threadIdx.x) >> 5; j < n; j += (gridDim.x * blockDim.x) >> 5) {
     const float4 q = g.sorted[j];
     const uint32_t orig = __float_as_uint(q.w);
-    int32_t ix, iy, iz;
-    grid_coord_g(g, c, q.x, q.y, q.z, ix, iy, iz);  // succeeded at insert time
-    uint32_t cs = 0, cf = 0;
-    if (lane < 27) {
-      const int dx = (int)(lane % 3u) - 1, dy = (int)((lane / 3u) % 3u) - 1, dz = (int)(lane / 9u) - 1;
-      uint32_t b, f;
-      if (grid_lookup(g, grid_key(0, ix + dx, iy + dy, iz + dz), b, f)) { cs = b; cf = f; }
-    }
-    uint32_t incl = cf;
-#pragma unroll
-    for (int o = 1; o < 32; o <<= 1) {
-      const uint32_t v = __shfl_up_sync(0xffffffffu, incl, o);
-      if (lane >= (uint32_t)o) incl += v;
-    }
-    const uint32_t ps = incl - cf;
-    const uint32_t total = __shfl_sync(0xffffffffu, incl, 31);   // >= 1: the query's own cell holds the query
+    uint32_t cs, ps;
+    const uint32_t total = flat27_runs(g, c, q, lane, cs, ps);   // >= 1: the query's own cell holds the query
     unsigned long long kv = ~0ull, kth = ~0ull;                   // lane i: i-th smallest key so far / the max_nn-th
     uint32_t pv = 0, in_radius = 0;
     for (uint32_t base = 0; base < total; base += 32) {
       const uint32_t ci = base + lane;
-      const uint32_t flat = min(ci, total - 1u);
-      uint32_t run = 0;
-#pragma unroll
-      for (int step = 16; step > 0; step >>= 1) {
-        const uint32_t mid = run + step;
-        const uint32_t v = __shfl_sync(0xffffffffu, ps, mid & 31u);
-        if (mid < 27u && v <= flat) run = mid;
-      }
-      const uint32_t rs = __shfl_sync(0xffffffffu, cs, run), rp = __shfl_sync(0xffffffffu, ps, run);
-      const uint32_t pos = rs + (flat - rp);
+      const uint32_t pos = flat27_at(cs, ps, min(ci, total - 1u));
       // key = (d2 bits : 32 | original index : 26 | tag : 6), ordered by (d2, index) like the oracle; the tag (the
       // lane that holds the entry's sorted position) only rides along through the sorting network below
       unsigned long long key = ~0ull;
@@ -1645,75 +1560,68 @@ k_normals_cov(uint32_t n_max, const uint32_t* n_dev, GridDev g, float r2, uint32
       }
     }
     const uint32_t n_sel = min(in_radius, max_nn);
-    double C[9] = {1.0, 0.0, 0.0, 0.0, 1.0, 0.0, 0.0, 0.0, 1.0};   // fewer than 3 neighbours: identity
-    if (n_sel >= 3) {
-      double v[9] = {0.0, 0.0, 0.0, 0.0, 0.0, 0.0, 0.0, 0.0, 0.0};
-      if (lane < n_sel) {
-        const float4 p = g.sorted[pv];
-        const double x = (double)p.x - (double)q.x, y = (double)p.y - (double)q.y, z = (double)p.z - (double)q.z;
-        v[0] = x; v[1] = y; v[2] = z;
-        v[3] = x * x; v[4] = x * y; v[5] = x * z; v[6] = y * y; v[7] = y * z; v[8] = z * z;
-      }
-#pragma unroll
-      for (int k = 0; k < 9; ++k)
-#pragma unroll
-        for (int o = 16; o > 0; o >>= 1) v[k] += __shfl_xor_sync(0xffffffffu, v[k], o);
-      const double inv = 1.0 / (double)n_sel;
-      const double s0 = v[0] * inv, s1 = v[1] * inv, s2 = v[2] * inv;
-      C[0] = v[3] * inv - s0 * s0;
-      C[1] = C[3] = v[4] * inv - s0 * s1;
-      C[2] = C[6] = v[5] * inv - s0 * s2;
-      C[4] = v[6] * inv - s1 * s1;
-      C[5] = C[7] = v[7] * inv - s1 * s2;
-      C[8] = v[8] * inv - s2 * s2;
+    double v[9] = {0.0, 0.0, 0.0, 0.0, 0.0, 0.0, 0.0, 0.0, 0.0};
+    if (n_sel >= 3 && lane < n_sel) {
+      const float4 p = g.sorted[pv];
+      const double x = (double)p.x - (double)q.x, y = (double)p.y - (double)q.y, z = (double)p.z - (double)q.z;
+      v[0] = x; v[1] = y; v[2] = z;
+      v[3] = x * x; v[4] = x * y; v[5] = x * z; v[6] = y * y; v[7] = y * z; v[8] = z * z;
     }
-    if (lane < 9) cov9[9 * (size_t)orig + lane] = C[lane];
-    if (lane == 0 && counts) counts[orig] = n_sel;
+    normals_cov_store(v, n_sel, orig, lane, counts, cov9);
   }
 }
 
 // Covariance of a kept neighbourhood (warp-collective): buf[0, n_sel) holds the neighbours' 64-bit keys (d2 bits
 // << 32 | original index), unordered.  The float64 moments about q are summed in key order, the same on every run
-// (the keys arrive in the grid's in-cell order, which the build's atomics decide); lanes 0..8 write cov9 of point
-// orig, lane 0 the count.  Fewer than 3 neighbours: identity.
+// (the keys arrive in the grid's in-cell order, which the build's atomics decide), by normals_cov_store.
 __device__ __forceinline__ void normals_cov_of_keys(unsigned long long* buf, uint32_t n_sel, const float4* __restrict__ pts,
                                                     float4 q, uint32_t orig, uint32_t lane, uint32_t* __restrict__ counts,
                                                     double* __restrict__ cov9) {
-  double C[9] = {1.0, 0.0, 0.0, 0.0, 1.0, 0.0, 0.0, 0.0, 1.0};
+  double v[9] = {0.0, 0.0, 0.0, 0.0, 0.0, 0.0, 0.0, 0.0, 0.0};
   if (n_sel >= 3) {
     warp_sort(buf, n_sel, lane);
-    double v[9] = {0.0, 0.0, 0.0, 0.0, 0.0, 0.0, 0.0, 0.0, 0.0};
     for (uint32_t i = lane; i < n_sel; i += 32) {
       const float4 p = pts[(uint32_t)buf[i]];
       const double x = (double)p.x - (double)q.x, y = (double)p.y - (double)q.y, z = (double)p.z - (double)q.z;
       v[0] += x; v[1] += y; v[2] += z;
       v[3] += x * x; v[4] += x * y; v[5] += x * z; v[6] += y * y; v[7] += y * z; v[8] += z * z;
     }
-#pragma unroll
-    for (int k = 0; k < 9; ++k)
-#pragma unroll
-      for (int o = 16; o > 0; o >>= 1) v[k] += __shfl_xor_sync(0xffffffffu, v[k], o);
-    const double inv = 1.0 / (double)n_sel;
-    const double s0 = v[0] * inv, s1 = v[1] * inv, s2 = v[2] * inv;
-    C[0] = v[3] * inv - s0 * s0;
-    C[1] = C[3] = v[4] * inv - s0 * s1;
-    C[2] = C[6] = v[5] * inv - s0 * s2;
-    C[4] = v[6] * inv - s1 * s1;
-    C[5] = C[7] = v[7] * inv - s1 * s2;
-    C[8] = v[8] * inv - s2 * s2;
   }
-  double mine = C[0];                                            // C[lane] without a local-memory array
-#pragma unroll
-  for (int k = 1; k < 9; ++k) mine = lane == (uint32_t)k ? C[k] : mine;
-  if (lane < 9) cov9[9 * (size_t)orig + lane] = mine;
-  if (lane == 0 && counts) counts[orig] = n_sel;
+  normals_cov_store(v, n_sel, orig, lane, counts, cov9);
 }
 
-// 64 < max_nn <= APC_MAX_NEIGHBORS: one warp per query over the same 27-cell flat candidate list as
-// k_normals_cov; the in-radius candidates stream through a WarpKeep of 64-bit keys (d2 bits << 32 |
-// original index: the oracle's total order, so the neighbourhood is exact) of wide_cap(max_nn) entries per
-// warp; the kept keys are sorted, and the lanes read the neighbours by original index from the input and add up
-// their float64 moments about the query point.  k_normals_eigen turns cov9 into normals.
+// Hybrid search around a query taken from the grid (warp-collective): the 27-cell walk, every in-radius candidate's
+// 64-bit key (d2 bits << 32 | original index: the oracle's total order, so the neighbourhood is exact) through a
+// WarpKeep of `cap` entries at buf.  Returns min(in-radius count, max_nn), the number of keys left in buf (unordered).
+__device__ __forceinline__ uint32_t hybrid_keep(const GridDev& g, float c, float4 q, float r2, uint32_t max_nn,
+                                                unsigned long long* buf, uint32_t cap, uint32_t lane) {
+  uint32_t cs, ps;
+  const uint32_t total = flat27_runs(g, c, q, lane, cs, ps);
+  WarpKeep<unsigned long long> wk;
+  wk.init(buf, cap, max_nn);
+  uint32_t in_radius = 0;
+  for (uint32_t base = 0; base < total; base += 32) {
+    const uint32_t ci = base + lane;
+    const uint32_t at = flat27_at(cs, ps, min(ci, total - 1u));
+    unsigned long long key = 0;
+    bool inside = false;
+    if (ci < total) {
+      const float4 p = g.sorted[at];
+      const float d2 = d2_f32(q.x, q.y, q.z, p.x, p.y, p.z);
+      inside = d2 <= r2;
+      key = knn_key<unsigned long long>(d2, __float_as_uint(p.w));
+    }
+    in_radius += __popc(__ballot_sync(0xffffffffu, inside));
+    wk.add(key, inside, lane);
+  }
+  wk.finish(lane);
+  return min(in_radius, max_nn);                                 // == wk.m
+}
+
+// 32 < max_nn <= APC_MAX_NEIGHBORS: one warp per query; hybrid_keep keeps the neighbourhood in a WarpKeep of
+// wide_cap(max_nn) entries per warp, and normals_cov_of_keys sorts the kept keys, reads the neighbours by original
+// index from the input and adds up their float64 moments about the query point.  k_normals_eigen turns cov9 into
+// normals.
 __global__ void __launch_bounds__(128)
 k_normals_wide(uint32_t n_max, const uint32_t* n_dev, GridDev g, const float4* __restrict__ pts, float r2, uint32_t max_nn,
                uint32_t cap, uint32_t* __restrict__ counts, double* __restrict__ cov9, const ApcCtrl* __restrict__ ctrl) {
@@ -1724,49 +1632,7 @@ k_normals_wide(uint32_t n_max, const uint32_t* n_dev, GridDev g, const float4* _
   for (uint32_t j = (blockIdx.x * blockDim.x + threadIdx.x) >> 5; j < n; j += (gridDim.x * blockDim.x) >> 5) {
     const float4 q = g.sorted[j];
     const uint32_t orig = __float_as_uint(q.w);
-    int32_t ix, iy, iz;
-    grid_coord_g(g, c, q.x, q.y, q.z, ix, iy, iz);  // succeeded at insert time
-    uint32_t cs = 0, cf = 0;
-    if (lane < 27) {
-      const int dx = (int)(lane % 3u) - 1, dy = (int)((lane / 3u) % 3u) - 1, dz = (int)(lane / 9u) - 1;
-      uint32_t b, f;
-      if (grid_lookup(g, grid_key(0, ix + dx, iy + dy, iz + dz), b, f)) { cs = b; cf = f; }
-    }
-    uint32_t incl = cf;
-#pragma unroll
-    for (int o = 1; o < 32; o <<= 1) {
-      const uint32_t v = __shfl_up_sync(0xffffffffu, incl, o);
-      if (lane >= (uint32_t)o) incl += v;
-    }
-    const uint32_t ps = incl - cf;
-    const uint32_t total = __shfl_sync(0xffffffffu, incl, 31);
-    WarpKeep<unsigned long long> wk;
-    wk.init(buf, cap, max_nn);
-    uint32_t in_radius = 0;
-    for (uint32_t base = 0; base < total; base += 32) {
-      const uint32_t ci = base + lane;
-      const uint32_t flat = min(ci, total - 1u);
-      uint32_t run = 0;
-#pragma unroll
-      for (int step = 16; step > 0; step >>= 1) {
-        const uint32_t mid = run + step;
-        const uint32_t v = __shfl_sync(0xffffffffu, ps, mid & 31u);
-        if (mid < 27u && v <= flat) run = mid;
-      }
-      const uint32_t rs = __shfl_sync(0xffffffffu, cs, run), rp = __shfl_sync(0xffffffffu, ps, run);
-      unsigned long long key = 0;
-      bool inside = false;
-      if (ci < total) {
-        const float4 p = g.sorted[rs + (flat - rp)];
-        const float d2 = d2_f32(q.x, q.y, q.z, p.x, p.y, p.z);
-        inside = d2 <= r2;
-        key = ((unsigned long long)__float_as_uint(d2) << 32) | __float_as_uint(p.w);
-      }
-      in_radius += __popc(__ballot_sync(0xffffffffu, inside));
-      wk.add(key, inside, lane);
-    }
-    wk.finish(lane);
-    normals_cov_of_keys(buf, min(in_radius, max_nn), pts, q, orig, lane, counts, cov9);   // n_sel == wk.m
+    normals_cov_of_keys(buf, hybrid_keep(g, c, q, r2, max_nn, buf, cap, lane), pts, q, orig, lane, counts, cov9);
     __syncwarp();                                                  // buf is reused by the next query
   }
 }
@@ -1810,7 +1676,7 @@ k_normals_knn_stragglers(const float4* __restrict__ pts, uint32_t n_max, const u
 }
 
 // Radius search (Open3D estimate_normals with radius only): every point with d2 <= float32(r)^2, no cap on the
-// count.  One warp per query over the 27-cell flat candidate list of k_normals_wide, nothing kept: each
+// count.  One warp per query over the 27-cell flat candidate list (flat27_runs), nothing kept: each
 // in-radius neighbour adds its moments about the query in fixed point, rint(d * 2^40 / r) for the 3 first and
 // rint(d d' * 2^40 / r^2) for the 6 second moments, in int64.  Integer sums do not depend on the order the
 // grid's atomics leave inside a cell, so the covariance is bit-identical across runs and input permutations.
@@ -1826,38 +1692,16 @@ k_normals_radius(uint32_t n_max, const uint32_t* n_dev, GridDev g, float r, floa
   for (uint32_t j = (blockIdx.x * blockDim.x + threadIdx.x) >> 5; j < n; j += (gridDim.x * blockDim.x) >> 5) {
     const float4 q = g.sorted[j];
     const uint32_t orig = __float_as_uint(q.w);
-    int32_t ix, iy, iz;
-    grid_coord_g(g, c, q.x, q.y, q.z, ix, iy, iz);  // succeeded at insert time
-    uint32_t cs = 0, cf = 0;
-    if (lane < 27) {
-      const int dx = (int)(lane % 3u) - 1, dy = (int)((lane / 3u) % 3u) - 1, dz = (int)(lane / 9u) - 1;
-      uint32_t b, f;
-      if (grid_lookup(g, grid_key(0, ix + dx, iy + dy, iz + dz), b, f)) { cs = b; cf = f; }
-    }
-    uint32_t incl = cf;
-#pragma unroll
-    for (int o = 1; o < 32; o <<= 1) {
-      const uint32_t v = __shfl_up_sync(0xffffffffu, incl, o);
-      if (lane >= (uint32_t)o) incl += v;
-    }
-    const uint32_t ps = incl - cf;
-    const uint32_t total = __shfl_sync(0xffffffffu, incl, 31);
+    uint32_t cs, ps;
+    const uint32_t total = flat27_runs(g, c, q, lane, cs, ps);
     long long m[9] = {0, 0, 0, 0, 0, 0, 0, 0, 0};
     uint32_t cnt = 0;
     for (uint32_t base = 0; base < total; base += 32) {
       const uint32_t ci = base + lane;
-      const uint32_t flat = min(ci, total - 1u);
-      uint32_t run = 0;
-#pragma unroll
-      for (int step = 16; step > 0; step >>= 1) {
-        const uint32_t mid = run + step;
-        const uint32_t v = __shfl_sync(0xffffffffu, ps, mid & 31u);
-        if (mid < 27u && v <= flat) run = mid;
-      }
-      const uint32_t rs = __shfl_sync(0xffffffffu, cs, run), rp = __shfl_sync(0xffffffffu, ps, run);
+      const uint32_t at = flat27_at(cs, ps, min(ci, total - 1u));
       bool inside = false;
       if (ci < total) {
-        const float4 p = g.sorted[rs + (flat - rp)];
+        const float4 p = g.sorted[at];
         inside = d2_f32(q.x, q.y, q.z, p.x, p.y, p.z) <= r2;
         if (inside) {
           const double x = (double)p.x - (double)q.x, y = (double)p.y - (double)q.y, z = (double)p.z - (double)q.z;
@@ -1907,13 +1751,11 @@ k_normals_eigen(uint32_t n_max, const uint32_t* n_dev, const double* __restrict_
 }
 
 // Allocations of the normals stage (grid + covariance scratch): must run outside stream capture.
-int apc_normals_prepare(apc_ctx* ctx, int max_nn) {
+int apc_normals_prepare(apc_ctx* ctx) {
   int rc = apc_neighbors_prepare(ctx, 0);
   if (rc) return rc;
   NeighborScratch* sc = scratch_of(ctx);
-  // k_normals_cov (max_nn <= 32) and k_normals_wide (max_nn > 64) hand their covariances to k_normals_eigen
-  const bool via_cov = max_nn <= 32 || max_nn > NRM_KMAX;
-  if (via_cov && !sc->cov) APC_CUDA(ctx, cudaMalloc((void**)&sc->cov, (size_t)ctx->max_points * 9 * sizeof(double)));
+  if (!sc->cov) APC_CUDA(ctx, cudaMalloc((void**)&sc->cov, (size_t)ctx->max_points * 9 * sizeof(double)));
   return APC_OK;
 }
 
@@ -1926,7 +1768,8 @@ int apc_normals_nobegin(apc_ctx* ctx, const float* xyzi, uint32_t n_max, const u
               "max_nn must be in 1..APC_MAX_NEIGHBORS (" APC_STRINGIFY(APC_MAX_NEIGHBORS) ") and radius > 0");
   int rc = apc_neighbors_prepare(ctx, 0);
   if (rc) return rc;
-  GridHost& g = scratch_of(ctx)->grid[0];
+  NeighborScratch* sc = scratch_of(ctx);
+  GridHost& g = sc->grid[0];
   const float r32 = (float)radius;
   const float4* pts = reinterpret_cast<const float4*>(xyzi);
   // cells of r * (1 + 2^-8) indexed by one multiply with the host-rounded reciprocal (grid_coord_g): the three IEEE
@@ -1935,30 +1778,25 @@ int apc_normals_nobegin(apc_ctx* ctx, const float* xyzi, uint32_t n_max, const u
   // the range the division with its 2^-10 margin guaranteed.
   rc = grid_build(ctx, g, pts, n_max, n_dev, r32 * 1.00390625f, false, s, false, CTR_CURSOR_NORMALS, true);
   if (rc) return rc;
-  if (max_nn <= 32 || max_nn > NRM_KMAX) {
-    // warp per query -> covariances (caller's buffer or context scratch), then thread per point -> eigenvector
-    NeighborScratch* sc = scratch_of(ctx);
-    double* cov = out_cov;
-    if (!cov) {
-      if (!sc->cov) APC_CUDA(ctx, cudaMalloc((void**)&sc->cov, (size_t)ctx->max_points * 9 * sizeof(double)));
-      cov = sc->cov;
-    }
-    const uint32_t bq = min(apc_div_up(n_max, 4), (uint32_t)APC_SM_COUNT * 16);
-    if (max_nn <= 32) {
-      APC_PROF(ctx, "k_normals_cov", s);
-      k_normals_cov<<<bq, 128, 0, s>>>(n_max, n_dev, g.d, r32 * r32, (uint32_t)max_nn, out_counts, cov, ctx->ctrl);
-    } else {
-      const uint32_t cap = wide_cap((uint32_t)max_nn);
-      APC_PROF(ctx, "k_normals_wide", s);
-      k_normals_wide<<<bq, 128, (size_t)4 * cap * sizeof(unsigned long long), s>>>(n_max, n_dev, g.d, pts, r32 * r32, (uint32_t)max_nn,
-                                                                                   cap, out_counts, cov, ctx->ctrl);
-    }
+  // warp per query -> covariances (caller's buffer or context scratch), then thread per point -> eigenvector
+  double* cov = out_cov;
+  if (!cov) {
+    if (!sc->cov) APC_CUDA(ctx, cudaMalloc((void**)&sc->cov, (size_t)ctx->max_points * 9 * sizeof(double)));
+    cov = sc->cov;
+  }
+  const uint32_t bq = min(apc_div_up(n_max, 4), (uint32_t)APC_SM_COUNT * 16);
+  if (max_nn <= 32) {
+    APC_PROF(ctx, "k_normals_cov", s);
+    k_normals_cov<<<bq, 128, 0, s>>>(n_max, n_dev, g.d, r32 * r32, (uint32_t)max_nn, out_counts, cov, ctx->ctrl);
+  } else {
+    const uint32_t cap = wide_cap((uint32_t)max_nn);
+    APC_PROF(ctx, "k_normals_wide", s);
+    k_normals_wide<<<bq, 128, (size_t)4 * cap * sizeof(unsigned long long), s>>>(n_max, n_dev, g.d, pts, r32 * r32, (uint32_t)max_nn,
+                                                                                 cap, out_counts, cov, ctx->ctrl);
+  }
+  {
     APC_PROF(ctx, "k_normals_eigen", s);
     k_normals_eigen<<<min(apc_div_up(n_max, 256), (uint32_t)APC_SM_COUNT * 8), 256, 0, s>>>(n_max, n_dev, cov, out_normals);
-  } else {
-    const uint32_t bq = min(apc_div_up(n_max, 128), (uint32_t)APC_SM_COUNT * 16);
-    APC_PROF(ctx, "k_normals_query", s);
-    k_normals_query<<<bq, 128, 0, s>>>(n_max, n_dev, g.d, r32 * r32, (uint32_t)max_nn, out_normals, out_counts, out_cov, ctx->ctrl);
   }
   const dim3 grid(min(apc_div_up(n_max, 256), (uint32_t)APC_SM_COUNT * 4), 1);
   APC_PROF(ctx, "k_grid_clean", s);
@@ -2086,42 +1924,6 @@ extern "C" int apc_estimate_normals_radius(apc_ctx* ctx, const float* xyzi, uint
 // relaxed stores: every value stored is an ancestor, so the trees stay the same whichever store lands last.
 // Points the grid cannot key (APC_ERR_KEY_RANGE) are never in the cell-sorted array: they are in no one's N,
 // stay non-core and keep the label -1.
-
-// The 27 cells around q as one flat candidate list, for a warp that walks it 32 records at a time: lane l < 27
-// resolves cell l and keeps its run's start in the cell-sorted array (cs) and the flat index of the run's first
-// record (ps); returns the list's length (all lanes).  This is k_normals_radius's walk; that kernel keeps its inline
-// copy because calling these helpers changes its instruction schedule.
-__device__ __forceinline__ uint32_t flat27_runs(const GridDev& g, float c, float4 q, uint32_t lane, uint32_t& cs, uint32_t& ps) {
-  int32_t ix, iy, iz;
-  grid_coord_g(g, c, q.x, q.y, q.z, ix, iy, iz);  // succeeded at insert time
-  uint32_t s0 = 0, cf = 0;
-  if (lane < 27) {
-    const int dx = (int)(lane % 3u) - 1, dy = (int)((lane / 3u) % 3u) - 1, dz = (int)(lane / 9u) - 1;
-    uint32_t b, f;
-    if (grid_lookup(g, grid_key(0, ix + dx, iy + dy, iz + dz), b, f)) { s0 = b; cf = f; }
-  }
-  uint32_t incl = cf;
-#pragma unroll
-  for (int o = 1; o < 32; o <<= 1) {
-    const uint32_t v = __shfl_up_sync(0xffffffffu, incl, o);
-    if (lane >= (uint32_t)o) incl += v;
-  }
-  cs = s0;
-  ps = incl - cf;
-  return __shfl_sync(0xffffffffu, incl, 31);
-}
-// Position in g.sorted of record `flat` of that list (called by all lanes of the warp).
-__device__ __forceinline__ uint32_t flat27_at(uint32_t cs, uint32_t ps, uint32_t flat) {
-  uint32_t run = 0;                                  // largest cell with ps <= flat
-#pragma unroll
-  for (int step = 16; step > 0; step >>= 1) {
-    const uint32_t mid = run + step;
-    const uint32_t v = __shfl_sync(0xffffffffu, ps, mid & 31u);
-    if (mid < 27u && v <= flat) run = mid;
-  }
-  const uint32_t rs = __shfl_sync(0xffffffffu, cs, run), rp = __shfl_sync(0xffffffffu, ps, run);
-  return rs + (flat - rp);
-}
 
 __device__ __forceinline__ uint32_t ld_relaxed_u32(const uint32_t* p) {
   uint32_t v;
@@ -2381,13 +2183,31 @@ __device__ __forceinline__ uint32_t flat27_runs_outside(const GridDev& g, float 
   int32_t ix, iy, iz;
   cs = ps = 0;
   if (!grid_coord_g(g, c, q.x, q.y, q.z, ix, iy, iz)) return 0;
-  return flat27_runs(g, c, q, lane, cs, ps);
+  return flat27_runs(g, 0, ix, iy, iz, lane, cs, ps);
 }
 // warp minimum of a 64-bit key: high words, then the low words of the lanes that hold the high minimum
 __device__ __forceinline__ uint64_t warp_min_u64(uint64_t k) {
   const uint32_t hi = __reduce_min_sync(0xffffffffu, (uint32_t)(k >> 32));
   const uint32_t lo = __reduce_min_sync(0xffffffffu, (uint32_t)(k >> 32) == hi ? (uint32_t)k : 0xffffffffu);
   return ((uint64_t)hi << 32) | lo;
+}
+// ICP's correspondence search for the transformed source point q (warp-collective): the smallest (d2 bits << 32 |
+// index) key over the target points with d2 <= r2 in the 27 cells around q, the same in every lane; all ones when
+// there is none.
+__device__ __forceinline__ uint64_t icp_best(const GridDev& g, float c, float4 q, float r2, uint32_t lane) {
+  uint32_t cs, ps;
+  const uint32_t total = flat27_runs_outside(g, c, q, lane, cs, ps);
+  uint64_t best = ~0ull;
+  for (uint32_t base = 0; base < total; base += 32) {
+    const uint32_t ci = base + lane;
+    const uint32_t at = flat27_at(cs, ps, min(ci, total - 1u));
+    if (ci < total) {
+      const float4 t = g.sorted[at];
+      const float d2 = d2_f32(q.x, q.y, q.z, t.x, t.y, t.z);
+      if (d2 <= r2) best = min(best, ((uint64_t)__float_as_uint(d2) << 32) | __float_as_uint(t.w));
+    }
+  }
+  return warp_min_u64(best);
 }
 
 __global__ void k_icp_init(IcpT16 init, IcpState* __restrict__ st, double* __restrict__ out_T, double* __restrict__ out_stats,
@@ -2425,19 +2245,7 @@ k_icp_match(const float4* __restrict__ src, uint32_t n_max, const uint32_t* n_de
     const float4 p = src[i];
     const double x = p.x, y = p.y, z = p.z;
     const float4 q = make_float4(icp_row(T, 0, x, y, z), icp_row(T, 1, x, y, z), icp_row(T, 2, x, y, z), 0.0f);
-    uint32_t cs, ps;
-    const uint32_t total = flat27_runs_outside(g, c, q, lane, cs, ps);
-    uint64_t best = ~0ull;
-    for (uint32_t base = 0; base < total; base += 32) {
-      const uint32_t ci = base + lane;
-      const uint32_t at = flat27_at(cs, ps, min(ci, total - 1u));
-      if (ci < total) {
-        const float4 t = g.sorted[at];
-        const float d2 = d2_f32(q.x, q.y, q.z, t.x, t.y, t.z);
-        if (d2 <= r2) best = min(best, ((uint64_t)__float_as_uint(d2) << 32) | __float_as_uint(t.w));
-      }
-    }
-    best = warp_min_u64(best);
+    const uint64_t best = icp_best(g, c, q, r2, lane);
     const bool found = best != ~0ull;                       // warp-uniform
     const uint32_t j = (uint32_t)best;
     const float d2 = __uint_as_float((uint32_t)(best >> 32));
@@ -2802,23 +2610,10 @@ k_icp_match_gicp(const float4* __restrict__ src, uint32_t n_max, const uint32_t*
   for (int k = 0; k < 12; ++k) T[k] = st->T[k];
   double acc = 0.0;
   for (uint32_t i = (blockIdx.x * blockDim.x + threadIdx.x) >> 5; i < n; i += (gridDim.x * blockDim.x) >> 5) {
-    // the matching of k_icp_match
     const float4 p = src[i];
     const double x = p.x, y = p.y, z = p.z;
     const float4 q = make_float4(icp_row(T, 0, x, y, z), icp_row(T, 1, x, y, z), icp_row(T, 2, x, y, z), 0.0f);
-    uint32_t cs, ps;
-    const uint32_t total = flat27_runs_outside(g, c, q, lane, cs, ps);
-    uint64_t best = ~0ull;
-    for (uint32_t base = 0; base < total; base += 32) {
-      const uint32_t ci = base + lane;
-      const uint32_t at = flat27_at(cs, ps, min(ci, total - 1u));
-      if (ci < total) {
-        const float4 t = g.sorted[at];
-        const float d2 = d2_f32(q.x, q.y, q.z, t.x, t.y, t.z);
-        if (d2 <= r2) best = min(best, ((uint64_t)__float_as_uint(d2) << 32) | __float_as_uint(t.w));
-      }
-    }
-    best = warp_min_u64(best);
+    const uint64_t best = icp_best(g, c, q, r2, lane);
     const bool found = best != ~0ull;                       // warp-uniform
     const uint32_t j = (uint32_t)best;
     if (found) {
@@ -3011,7 +2806,7 @@ __device__ __forceinline__ void fpfh_of_keys(const unsigned long long* buf, uint
   }
 }
 
-// Hybrid search: k_normals_wide's 27-cell walk and WarpKeep, the kept keys sorted.
+// Hybrid search: k_normals_wide's hybrid_keep, the kept keys sorted.
 template <int PASS>
 __global__ void __launch_bounds__(128)
 k_fpfh_hybrid(uint32_t n_max, const uint32_t* n_dev, GridDev g, const float4* __restrict__ pts,
@@ -3025,27 +2820,7 @@ k_fpfh_hybrid(uint32_t n_max, const uint32_t* n_dev, GridDev g, const float4* __
   for (uint32_t j = (blockIdx.x * blockDim.x + threadIdx.x) >> 5; j < n; j += (gridDim.x * blockDim.x) >> 5) {
     const float4 q = g.sorted[j];
     const uint32_t orig = __float_as_uint(q.w);
-    uint32_t cs, ps;
-    const uint32_t total = flat27_runs(g, c, q, lane, cs, ps);
-    WarpKeep<unsigned long long> wk;
-    wk.init(buf, cap, max_nn);
-    uint32_t in_radius = 0;
-    for (uint32_t base = 0; base < total; base += 32) {
-      const uint32_t ci = base + lane;
-      const uint32_t at = flat27_at(cs, ps, min(ci, total - 1u));
-      unsigned long long key = 0;
-      bool inside = false;
-      if (ci < total) {
-        const float4 p = g.sorted[at];
-        const float d2 = d2_f32(q.x, q.y, q.z, p.x, p.y, p.z);
-        inside = d2 <= r2;
-        key = ((unsigned long long)__float_as_uint(d2) << 32) | __float_as_uint(p.w);
-      }
-      in_radius += __popc(__ballot_sync(0xffffffffu, inside));
-      wk.add(key, inside, lane);
-    }
-    wk.finish(lane);
-    const uint32_t m = min(in_radius, max_nn);
+    const uint32_t m = hybrid_keep(g, c, q, r2, max_nn, buf, cap, lane);
     warp_sort(buf, m, lane);
     fpfh_of_keys<PASS>(buf, m, pts, normals, q, orig, lane, s_cnt[w], spfh, feat, counts);
     __syncwarp();                                                  // buf is reused by the next query

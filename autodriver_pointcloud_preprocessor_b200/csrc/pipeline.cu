@@ -24,7 +24,7 @@ int apc_segment_plane_nobegin(apc_ctx*, const float*, uint32_t, const uint32_t*,
                               const uint32_t*, uint32_t*, const MirrorDev*, const float*, float*);
 int apc_normals_nobegin(apc_ctx*, const float*, uint32_t, const uint32_t*, int, double, float*, uint32_t*, double*, cudaStream_t);
 int apc_neighbors_prepare(apc_ctx*, int);
-int apc_normals_prepare(apc_ctx*, int);
+int apc_normals_prepare(apc_ctx*);
 int apc_sort_prepare(apc_ctx*);
 
 // dev_counts layout inside the context
@@ -197,7 +197,7 @@ static int prepare(apc_ctx* ctx, const apc_pipeline_cfg* cfg) {
   if (!rc && cfg->stat_enable) rc = apc_neighbors_prepare(ctx, 1);
   if (!rc && cfg->filter.dedup_mode >= APC_DEDUP_NUMPY) rc = apc_sort_prepare(ctx);
   if (!rc && cfg->normals_enable) {
-    rc = apc_normals_prepare(ctx, cfg->normals_max_nn);
+    rc = apc_normals_prepare(ctx);
     if (!rc && cfg->ground_enable && !ctx->nrm_scratch)
       APC_CUDA(ctx, cudaMalloc((void**)&ctx->nrm_scratch, (size_t)ctx->max_points * 3 * sizeof(float)));
   }

@@ -24,7 +24,7 @@ from autodriver_pointcloud_preprocessor_b200 import _capi, engine
 
 RUNS = 10
 KERNELS = ("k_grid_insert", "k_grid_assign", "k_grid_scatter", "k_normals_knn", "k_normals_knn_stragglers",
-           "k_normals_radius", "k_normals_cov", "k_normals_query", "k_normals_wide", "k_normals_eigen", "k_grid_clean")
+           "k_normals_radius", "k_normals_cov", "k_normals_wide", "k_normals_eigen", "k_grid_clean")
 
 
 def voxel_cloud(ctx, desc, fcfg, voxel_size):

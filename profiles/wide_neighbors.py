@@ -1,9 +1,9 @@
-"""Cost of the neighbourhood sizes above 64 (the *_wide kernels) next to the sizes below, on one GPU:
+"""Cost of the large neighbourhood sizes (the *_wide kernels: k > 64, max_nn > 32) next to the sizes below, on one GPU:
 eager pipeline runs with every kernel bracketed by CUDA events (``ctx.profile(True)``).
 
-* statistical outlier removal on the C4 scan (1.5 M points, 0.05 m voxels), k in {20, 64, 65, 100, 256, 1024};
+* statistical outlier removal on the C4 scan (1.5 M points, 0.05 m voxels), k in {20, 33, 48, 64, 65, 100, 256, 1024};
 * normal estimation on the reference's default configuration (262 144-point scan, duplicate removal,
-  non-finite filter, ROI crop, 0.01 m voxels, radius 0.1 m), max_nn in {30, 64, 65, 100, 256}.
+  non-finite filter, ROI crop, 0.01 m voxels, radius 0.1 m), max_nn in {30, 33, 48, 64, 65, 100, 256}.
 
 Per configuration: one warm-up run, then RUNS profiled runs; the JSON holds the mean time per launch of
 every kernel of the stage and the stage total, with the GPU's name and power limit.
@@ -18,7 +18,7 @@ from autodriver_pointcloud_preprocessor_b200 import _capi, engine, synth
 RUNS = 10
 STAT_KERNELS = ("k_grid_insert", "k_grid_assign", "k_grid_scatter", "k_knn_query", "k_knn_stragglers", "k_knn_query_wide",
                 "k_knn_stragglers_wide", "k_grid_clean", "stat_reduce_mask")
-NRM_KERNELS = ("k_normals_cov", "k_normals_query", "k_normals_wide", "k_normals_eigen")
+NRM_KERNELS = ("k_normals_cov", "k_normals_wide", "k_normals_eigen")
 
 
 def gpu_info():
@@ -54,7 +54,7 @@ def main():
     m = synth.pack_cloud(synth.lidar_scan(seed=500, n_beams=128, n_az=2048, n_points=1_500_000), "xyzi16")
     ctx = engine.Context(max_points=m.width)
     desc = engine.make_cloud_desc(m.fields, m.point_step, m.width, torch.frombuffer(bytearray(m.data), dtype=torch.uint8).cuda())
-    for k in (20, 64, 65, 100, 256, 1024):
+    for k in (20, 33, 48, 64, 65, 100, 256, 1024):
         pcfg = engine.make_pipeline_cfg(engine.make_filter_cfg(skip_nans=True, remove_nan=True, remove_inf=True), voxel_size=0.05,
                                         statistical=dict(nb_neighbors=k, std_ratio=2.0))
         r = dict(k=k, **profile_stage(ctx, desc, pcfg, STAT_KERNELS))
@@ -66,7 +66,7 @@ def main():
     ctx = engine.Context(max_points=m.width)
     desc = engine.make_cloud_desc(m.fields, m.point_step, m.width, torch.frombuffer(bytearray(m.data), dtype=torch.uint8).cuda())
     fcfg = engine.make_filter_cfg(skip_nans=True, dedup_mode=_capi.DEDUP_OPEN3D, remove_nan=True, remove_inf=True, crop=bench.CROP)
-    for nn in (30, 64, 65, 100, 256):
+    for nn in (30, 33, 48, 64, 65, 100, 256):
         pcfg = engine.make_pipeline_cfg(fcfg, voxel_size=0.01, normals=dict(radius=0.1, max_nn=nn))
         r = dict(max_nn=nn, **profile_stage(ctx, desc, pcfg, NRM_KERNELS))
         print("normals", json.dumps(r), flush=True)

@@ -1,4 +1,4 @@
-"""GPU parity tests of normal estimation (pp.py:521-530; csrc/neighbors.cu k_normals_query) against
+"""GPU parity tests of normal estimation (pp.py:521-530; csrc/neighbors.cu k_normals_cov / k_normals_wide) against
 oracle/normals.py.  Neighbour counts are integer work (bit-exact); covariances and normals are
 floating point: covariance within 1e-9 relative to its largest entry, normals within 1e-5 per
 component (sign included) wherever the two smallest eigenvalues are separated, and an eigen-residual

@@ -1,6 +1,7 @@
-"""Statistical outlier removal and normal estimation with 64 < k <= APC_MAX_NEIGHBORS (1024): the wide
-kernels (k_knn_query_wide / k_knn_stragglers_wide, k_normals_wide) against the oracle, the dispatch that
-keeps k <= 64 on the existing kernels, the cap, the fused pipeline and its graph, and the node."""
+"""Statistical outlier removal and normal estimation with large neighbourhoods (up to APC_MAX_NEIGHBORS = 1024):
+the wide kernels (k_knn_query_wide / k_knn_stragglers_wide above k = 64, k_normals_wide above max_nn = 32) against
+the oracle, the dispatch between them and the smaller-k kernels, the cap, the fused pipeline and its graph, and the
+node."""
 import numpy as np
 import pytest
 
@@ -46,7 +47,7 @@ def assert_statistical(ctx, xyzi, host, k, ratio, brute=False):
     assert np.array_equal(mask.cpu().numpy().astype(bool), ref_mask)
 
 
-@pytest.mark.parametrize("k", [65, 100, 256, 1024])
+@pytest.mark.parametrize("k", [33, 64, 65, 100, 256, 1024])
 def test_statistical_wide_parity(env, k):
     ctx = env["ctx"]
     host = outlier_cloud(env)
@@ -73,19 +74,20 @@ def launched(ctx, fn):
         ctx.profile(False)
 
 
-def test_dispatch_keeps_k_up_to_64_on_the_existing_kernels(env):
+def test_dispatch_thresholds(env):
+    """Statistical: k <= 64 on k_knn_query / k_knn_stragglers, above it the *_wide kernels.  Normals: max_nn <= 32
+    on k_normals_cov, above it k_normals_wide."""
     ctx = env["ctx"]
     xyzi = to_xyzi(outlier_cloud(env))
-    names = launched(ctx, lambda: ctx.statistical_outliers(xyzi, 64, 2.0))
-    assert "k_knn_query" in names and "k_knn_stragglers" in names
-    assert "k_knn_query_wide" not in names and "k_knn_stragglers_wide" not in names
-    names = launched(ctx, lambda: ctx.statistical_outliers(xyzi, 65, 2.0))
-    assert "k_knn_query_wide" in names and "k_knn_stragglers_wide" in names
-    assert "k_knn_query" not in names and "k_knn_stragglers" not in names
-    kernels = {"k_normals_cov", "k_normals_query", "k_normals_wide"}
-    for max_nn, want in ((32, "k_normals_cov"), (64, "k_normals_query"), (65, "k_normals_wide")):
+    kernels = {"k_knn_query", "k_knn_stragglers", "k_knn_query_wide", "k_knn_stragglers_wide"}
+    for k, want in ((32, {"k_knn_query", "k_knn_stragglers"}), (33, {"k_knn_query", "k_knn_stragglers"}),
+                    (64, {"k_knn_query", "k_knn_stragglers"}), (65, {"k_knn_query_wide", "k_knn_stragglers_wide"})):
+        names = launched(ctx, lambda: ctx.statistical_outliers(xyzi, k, 2.0))
+        assert names & kernels == want, (k, names)
+    kernels = {"k_normals_cov", "k_normals_wide"}
+    for max_nn, want in ((32, "k_normals_cov"), (33, "k_normals_wide"), (64, "k_normals_wide"), (65, "k_normals_wide")):
         names = launched(ctx, lambda: ctx.estimate_normals(xyzi, max_nn, 0.5))
-        assert names & kernels == {want}, (max_nn, names)
+        assert names & kernels == {want} and "k_normals_eigen" in names, (max_nn, names)
 
 
 def test_cap_is_refused_and_the_context_stays_usable(env):
@@ -115,7 +117,7 @@ def dense_surface(seed=5):
     return p
 
 
-@pytest.mark.parametrize("max_nn,radius", [(65, 0.2), (100, 0.25), (512, 0.5)])
+@pytest.mark.parametrize("max_nn,radius", [(33, 0.2), (65, 0.2), (100, 0.25), (512, 0.5)])
 def test_normals_wide_parity(env, max_nn, radius):
     from oracle import normals as onrm
     from test_gpu_normals import check_normals
